@@ -23,6 +23,12 @@ with the EMA teacher update folded in.  Nothing is skipped.
            /root/reference) on the host cores, BASELINE.json configs[0] (2 clips x 8 crops); the oracle port only if no
            reference checkout travelled.  `gpu_torch_baseline`: the same reference step on this GPU under torch eager +
            bf16 autocast (what a user of the reference gets on this box today), outside the timed region.
+
+--dump-outputs DIR: after the timed steps, writes what the last timed step handed its caller as DIR/<name>.npy, so that
+two builds run with the same arguments (hence the same seeded inputs) can be compared output for output.  train / nat:
+loss (float64), and of the model state the step updated -- params (trained parameters), teacher (EMA teacher encoder),
+adam_exp_avg, adam_exp_avg_sq -- each a fixed seeded sample of 2^21 elements in optimizer_state_dict() name order.
+hear: embeddings (the same kind of sample) and timestamps.  float32 unless noted; about 32 MiB in all.
 """
 from __future__ import annotations
 
@@ -50,6 +56,7 @@ SPEC = [(512, 10, 5)] + [(512, 3, 2)] * 4 + [(512, 2, 2)]
 MASKER = dict(target_masks_per_context=4, context_mask_prob=0.65, context_mask_length=10, target_prob=0.25,
               target_length=10, ratio_cutoff=0.1)   # configs/masker/AudioSet.yaml
 HEAR_CLIPS = 256
+DUMP_SAMPLE = 1 << 21         # elements kept of each output larger than this (--dump-outputs)
 HBM_WRITE_PEAK_GBS = 3906.0   # measured: torch memset / fill of 1 GiB on this pool's B200 (scripts/bw_probe.py)
 
 
@@ -67,6 +74,37 @@ def load_traffic():
     (scripts/kernel_traffic.py -> profiles/r02_kernel_traffic.json); None when absent."""
     p = os.path.join(ROOT, "profiles", "r02_kernel_traffic.json")
     return json.load(open(p)) if os.path.exists(p) else None
+
+
+def dump_outputs(out_dir, outputs):
+    """Writes each tensor of `outputs` as out_dir/<name>.npy (float64 stays float64, anything else becomes float32).
+    A tensor of more than DUMP_SAMPLE elements is reduced to the elements at DUMP_SAMPLE fixed positions of its
+    flattened form (seed 0, ascending): the same positions for every run and build with the same output size."""
+    import numpy as np
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in outputs.items():
+        t = t.detach()
+        if t.numel() > DUMP_SAMPLE:
+            idx = np.sort(np.random.default_rng(0).choice(t.numel(), size=DUMP_SAMPLE, replace=False))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        t = t.cpu().double() if t.dtype == torch.float64 else t.cpu().float()
+        np.save(os.path.join(out_dir, name + ".npy"), t.numpy())
+
+
+def _train_outputs(model, loss):
+    """The last training step's loss and the model state it updated, for --dump-outputs."""
+    import torch
+
+    opt = model.optimizer_state_dict()
+    params = dict(model.named_parameters())
+    names = opt["param_names"]
+    return {"loss": loss.double(),
+            "params": torch.cat([params[n].detach().reshape(-1) for n in names]),
+            "teacher": torch.cat([p.detach().reshape(-1) for p in model.teacher_encoder.parameters()]),
+            "adam_exp_avg": torch.cat([opt["state"][n]["exp_avg"].reshape(-1) for n in names]),
+            "adam_exp_avg_sq": torch.cat([opt["state"][n]["exp_avg_sq"].reshape(-1) for n in names])}
 
 
 # ===================================================================================================== FLOP model
@@ -291,6 +329,8 @@ def run_native(args):
     barrier()
     launches = _lib.kernel_launches() - k0
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, _train_outputs(model, loss))
     ms_total = max_over_ranks(e0.elapsed_time(e1))
     ms_step = ms_total / args.steps
     value = world * B * args.steps / (ms_total / 1e3)
@@ -481,6 +521,8 @@ def run_hear(args):
     launches = _lib.kernel_launches() - k0
     clocks = sampler.stop() if sampler else None
     assert tuple(emb.shape) == (n, 996, 768) and tuple(ts.shape) == (n, 996) and bool(torch.isfinite(emb).all())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"embeddings": emb, "timestamps": ts})
     ms_total = max_over_ranks(e0.elapsed_time(e1))
     ms_step = ms_total / args.steps
     value = world * n * args.steps / (ms_total / 1e3)
@@ -697,7 +739,13 @@ def main():
     ap.add_argument("--no-gpu-baseline", action="store_true")
     ap.add_argument("--deterministic", action="store_true",
                     help="time the step with bit-reproducible reductions (ops.set_deterministic); not the default bench line")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step to DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of this implementation's timed step (--impl native)")
     args.warmup = max(args.warmup, 3) if args.impl == "native" else args.warmup
     if args.impl == "reference":
         run_reference(args)

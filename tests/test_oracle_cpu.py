@@ -371,7 +371,7 @@ def test_lightning_base_is_used_when_available():
     assert issubclass(w.JEPA, _lightning.Base) and hasattr(w.JEPA, "log_dict") and hasattr(w.JEPA, "save_hyperparameters")
 
 
-def test_hf_feature_extractor_and_reference_staging():
+def test_hf_feature_extractor_and_reference_staging(tmp_path):
     from wavjepa_b200 import hf
     ext = hf.WavJEPAFeatureExtractor.from_pretrained("labhamlet/wavjepa-base", trust_remote_code=True)
     out = ext([torch.ones(5), torch.ones(8)], return_tensors="pt")
@@ -379,9 +379,23 @@ def test_hf_feature_extractor_and_reference_staging():
     assert tuple(ext(torch.zeros(160000))["input_values"].shape) == (1, 160000)
     with pytest.raises(ValueError):
         ext(torch.zeros(10), sampling_rate=44100)
-    # the staged reference copy (bench.py's reference arms on the GPU box) is byte-identical to the checkout
+    # the staged reference copy (bench.py's reference arms) is a byte-identical copy of a checkout's hot-path packages,
+    # with a sha256 manifest; checked on a small stand-in checkout in the reference's flat layout
+    import hashlib
     from oracle import stage_reference
-    if os.path.isdir("/root/reference/wavjepa"):
-        dest = stage_reference.stage("/root/reference", os.path.join(ROOT, "baseline", "_ref"))
-        man = json.load(open(os.path.join(dest, "MANIFEST.json")))["files"]
-        assert "wavjepa/jepa.py" in man and "hear_api/runtime.py" in man and len(man) > 20
+    src, dest = tmp_path / "reference", tmp_path / "staged"
+    staged = {"wavjepa/jepa.py": b"class JEPA: pass\n", "wavjepa/extractors/__init__.py": b"",
+              "hear_api/runtime.py": b"def load_model(): pass\n", "hear_configs/WavJEPA.py": b"# config\n",
+              "data_modules/__init__.py": b"", "utils.py": b"def util(): pass\n", "LICENSE": b"MIT\n"}
+    left_out = {"train.py": b"main()\n", "wavjepa/__pycache__/jepa.cpython-312.pyc": b"\0", "wavjepa/clip.wav": b"RIFF",
+                "hear_api/model.ckpt": b"\0"}
+    for rel_path, data in {**staged, **left_out}.items():
+        (src / rel_path).parent.mkdir(parents=True, exist_ok=True)
+        (src / rel_path).write_bytes(data)
+    assert stage_reference.stage(str(src), str(dest)) == str(dest)
+    man = json.load(open(dest / "MANIFEST.json"))["files"]
+    assert sorted(man) == sorted(staged)
+    for rel_path, data in staged.items():
+        assert (dest / rel_path).read_bytes() == data and man[rel_path] == hashlib.sha256(data).hexdigest(), rel_path
+    assert stage_reference.stage(str(tmp_path / "absent"), str(tmp_path / "none")) is None
+    assert not (tmp_path / "none").exists()
