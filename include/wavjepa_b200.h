@@ -310,6 +310,35 @@ int wj_add_bf16(float* a, const void* b_bf16, int64_t n, void* stream);
 int wj_colsum(const void* x, int x_is_bf16, int64_t M, int N, int64_t ld, float* out, void* stream);
 int wj_scale_bf16(void* x_bf16, const float* scale_dev, int64_t n, void* stream);
 
+/* ------------------------------------------------------------------------------------------------------------------
+ * Reference-precision (TF32) inference path: the fp32 feature extraction of hear_api/runtime.py:98-145 with every GEMM
+ * operand rounded to nearest tf32 (the tensor core truncates raw fp32, which doubles the error), fp32 accumulation,
+ * exact erf GELU, fp32 residual stream.  Forward only.
+ *
+ * wj_gemm_tf32: out[b*L + t, n] = epilogue( sum_vc A(vc; t, b) * W[n, vc] ) with an fp32 operand A (wj_operand_t over
+ *   4-byte elements: plain activations or the conv window views) and fp32 W [N, K] (leading dim ldw), both K-major,
+ *   tcgen05.mma.kind::tf32.  K % 32 == 0, N % 128 == 0.  Epilogue: v = acc + bias; act 4: v = GELU_erf(v) (act 0: none);
+ *   v += resid[row % resid_mod or row, n]; out = bf16(v), or fp32 v (rounded to nearest tf32 when round_out).
+ *   accumulate / out2 / aux / out_rows / colsum must be unset. */
+int wj_gemm_tf32(const wj_operand_t* A, const float* W, int64_t ldw, int L, int batch, int N, int K,
+                 const wj_epilogue_t* epi, int round_out, void* stream);
+/* Conv block 0 from fp32 input x [B, Cin, L] and unrounded fp32 weights: fp32 FMA on the CUDA cores, closed-form
+ * GroupNorm statistics (moments / stats workspaces as wj_conv0_gn_gelu_fwd), exact erf GELU; out fp32 [B, L_out, C]
+ * rounded to nearest tf32. */
+int wj_conv0_gn_gelu_fwd_f32(const float* x, const float* w, const float* gamma, const float* beta, int B, int Cin,
+                             int L, int C, int k, int stride, float eps, double* moments, float* stats, float* out,
+                             void* stream);
+/* Attention forward of wj_attn_varlen_fwd (bf16 qkv, Q/K/V and P on the tensor cores in bf16) writing O as fp32
+ * [tokens, D] rounded to nearest tf32.  Head dim 64 and sequences of <= 512 tokens only; other shapes are refused. */
+int wj_attn_varlen_fwd_f32out(const void* qkv_bf16, const int* cu_seqlens, int n_seqs, int max_len, int64_t total_tokens,
+                              int D, int H, float* out_f32, void* stream);
+/* LayerNorm(x + add) with x fp32 and add fp32 (or NULL): out_f32 = the unrounded result, out_tf32 = the result rounded to
+ * nearest tf32 (the next GEMM's operand); either may be NULL.  D as wj_layernorm_fwd. */
+int wj_add_layernorm_fwd_f32(const float* x, const float* add_f32, const float* gamma, const float* beta, float eps,
+                             int M, int D, float* out_f32, float* out_tf32, void* stream);
+/* y[i] = x[i] rounded to nearest tf32 (y may be x). */
+int wj_tf32_round(const float* x, float* y, int64_t n, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

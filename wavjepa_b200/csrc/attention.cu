@@ -357,7 +357,22 @@ using namespace wj;
 
 namespace wj {
 int attn_fwd_tc_launch(const void* qkv, const int* cu, int n_seqs, int max_len, long long total_tokens, int D, int H,
-                       void* out, float* lse2, cudaStream_t st);
+                       void* out, float* lse2, cudaStream_t st, float* out_f32 = nullptr);
+}
+
+// Forward of the TF32 inference path: the same tcgen05 kernels (bf16 Q/K/V and P), O written as fp32 rounded to nearest
+// tf32.  Built for head dim 64 and sequences of <= 512 tokens; other shapes are refused (there is no bf16 fallback).
+extern "C" int wj_attn_varlen_fwd_f32out(const void* qkv_bf16, const int* cu_seqlens, int n_seqs, int max_len,
+                                         int64_t total_tokens, int D, int H, float* out_f32, void* stream) {
+  if (n_seqs <= 0 || max_len <= 0) return WJ_OK;
+  if (D % H != 0 || D / H != 64 || D % 64 != 0 || max_len > 512 || total_tokens <= 0) {
+    set_error("wj_attn_varlen_fwd_f32out: built for head dim 64 and <= 512 tokens (D=%d H=%d max_len=%d)", D, H, max_len);
+    return WJ_ERR_ARG;
+  }
+  const int rc = wj::attn_fwd_tc_launch(qkv_bf16, cu_seqlens, n_seqs, max_len, total_tokens, D, H, nullptr, nullptr,
+                                        WJ_STREAM(stream), out_f32);
+  if (rc == 1) { set_error("wj_attn_varlen_fwd_f32out: tensor-map encoding unavailable"); return WJ_ERR_RUNTIME; }
+  return rc;
 }
 
 extern "C" int wj_attn_varlen_fwd(const void* qkv_bf16, const int* cu_seqlens, int n_seqs, int max_len, int64_t total_tokens,

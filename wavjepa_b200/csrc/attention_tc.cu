@@ -26,6 +26,7 @@ struct AttnTcParams {
   float scale_log2;
   bf16* out;
   float* lse2;
+  float* out_f32;   // F32OUT kernels: O as fp32 rounded to nearest tf32 (the operand of the tf32 out_proj GEMM)
 };
 
 // KT = keys per item (128, 256 or 512 = TMEM columns of S); sequences of 129..512 tokens run as 2..4 query tiles.  With
@@ -100,8 +101,9 @@ template <int EC> __device__ __forceinline__ void tmem_ld_cols(uint32_t taddr, u
   }
 }
 
-template <int DH, int KT>
-__global__ void __launch_bounds__(AttnTcCfg<DH, KT>::THREADS, 512 / KT)
+// (F32OUT at 128 keys: 3 CTAs per SM instead of 4 -- its fp32 epilogue does not fit in 96 registers without spilling)
+template <int DH, int KT, bool F32OUT = false>
+__global__ void __launch_bounds__(AttnTcCfg<DH, KT>::THREADS, (F32OUT && KT == 128) ? 3 : 512 / KT)
 attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tmQ, const AttnTcParams p) {
   using Cfg = AttnTcCfg<DH, KT>;
   constexpr int STAGES = Cfg::STAGES, HALVES = Cfg::HALVES, NW = Cfg::NW;
@@ -355,9 +357,17 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tmQ, const AttnTcParams p
       if (lane == 0) mbar_arrive(bar_done);
       if (row < nq) {
         const float inv = fa / lsum;
+        if constexpr (F32OUT) {
+          float* of = p.out_f32 + static_cast<long long>(start + row) * p.D + head * DH + (HALVES >= 2 ? half * EC : 0);
+#pragma unroll
+          for (int j = 0; j < EC; j += 4)
+            *reinterpret_cast<float4*>(of + j) = make_float4(
+                tf32_round(__uint_as_float(o[j]) * inv), tf32_round(__uint_as_float(o[j + 1]) * inv),
+                tf32_round(__uint_as_float(o[j + 2]) * inv), tf32_round(__uint_as_float(o[j + 3]) * inv));
+        }
         bf16* op = p.out + static_cast<long long>(start + row) * p.D + head * DH + (HALVES >= 2 ? half * EC : 0);
 #pragma unroll
-        for (int j = 0; j < EC; j += 8) {
+        for (int j = 0; j < EC && !F32OUT; j += 8) {
           uint4 w;
           w.x = pack_bf16x2(__uint_as_float(o[j]) * inv, __uint_as_float(o[j + 1]) * inv);
           w.y = pack_bf16x2(__uint_as_float(o[j + 2]) * inv, __uint_as_float(o[j + 3]) * inv);
@@ -704,7 +714,7 @@ typedef CUresult (*PFN_encodeTiledA)(CUtensorMap*, CUtensorMapDataType, cuuint32
 
 // Returns WJ_OK and launches when the problem fits this kernel; 1 when the caller should use the mma.sync kernel.
 int attn_fwd_tc_launch(const void* qkv, const int* cu, int n_seqs, int max_len, long long total_tokens, int D, int H,
-                       void* out, float* lse2, cudaStream_t st) {
+                       void* out, float* lse2, cudaStream_t st, float* out_f32) {
   const int dh = D / H;
   if (max_len > 512 || D % 64 != 0 || (dh != 32 && dh != 64) || total_tokens <= 0) return 1;
   static PFN_encodeTiledA enc = nullptr;
@@ -728,7 +738,7 @@ int attn_fwd_tc_launch(const void* qkv, const int* cu, int n_seqs, int max_len, 
   const int qt = max_len > 256 ? 4 : (max_len > 128 ? 2 : 1);
   p.cu = cu; p.n_seqs = n_seqs; p.D = D; p.H = H; p.items = n_seqs * H;   // units = (sequence, head)
   p.scale_log2 = 1.4426950408889634f / sqrtf(static_cast<float>(dh));
-  p.out = reinterpret_cast<bf16*>(out); p.lse2 = lse2;
+  p.out = reinterpret_cast<bf16*>(out); p.lse2 = lse2; p.out_f32 = out_f32;
   auto go = [&](auto kernel, int smem, int ctas, int threads) -> int {
     cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
     if (e != cudaSuccess) { set_error("attn_fwd_tc attr: %s", cudaGetErrorString(e)); return WJ_ERR_RUNTIME; }
@@ -737,6 +747,12 @@ int attn_fwd_tc_launch(const void* qkv, const int* cu, int n_seqs, int max_len, 
     kernel<<<grid, threads, smem, st>>>(tm, p);
     return check_launch("attn_fwd_tc");
   };
+  if (out_f32 != nullptr) {   // fp32 output: head dim 64 (the encoder), 128 / 256 / 512 keys
+    if (dh != 64) { set_error("attn_fwd_tc: the fp32-output kernels are built for head dim 64 (got %d)", dh); return WJ_ERR_ARG; }
+    if (qt == 4) return go(attn_fwd_tc_kernel<64, 512, true>, AttnTcCfg<64, 512>::SMEM, AttnTcCfg<64, 512>::CTAS, AttnTcCfg<64, 512>::THREADS);
+    if (qt == 2) return go(attn_fwd_tc_kernel<64, 256, true>, AttnTcCfg<64, 256>::SMEM, AttnTcCfg<64, 256>::CTAS, AttnTcCfg<64, 256>::THREADS);
+    return go(attn_fwd_tc_kernel<64, 128, true>, AttnTcCfg<64, 128>::SMEM, AttnTcCfg<64, 128>::CTAS, AttnTcCfg<64, 128>::THREADS);
+  }
   if (dh == 64 && qt == 4) return go(attn_fwd_tc_kernel<64, 512>, AttnTcCfg<64, 512>::SMEM, AttnTcCfg<64, 512>::CTAS, AttnTcCfg<64, 512>::THREADS);
   if (qt == 4) return go(attn_fwd_tc_kernel<32, 512>, AttnTcCfg<32, 512>::SMEM, AttnTcCfg<32, 512>::CTAS, AttnTcCfg<32, 512>::THREADS);
   if (dh == 64 && qt == 1) return go(attn_fwd_tc_kernel<64, 128>, AttnTcCfg<64, 128>::SMEM, AttnTcCfg<64, 128>::CTAS, AttnTcCfg<64, 128>::THREADS);

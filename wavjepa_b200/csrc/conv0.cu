@@ -34,13 +34,15 @@ struct Conv0Args {
   const bf16* x;      // [B, Cin, L]
   const float* w;     // [C, Cin, 10] fp32 master weights (rounded to bf16 on load: autocast semantics)
   int B, Cin, L, L_out, C;
+  const float* xf;    // fp32 input instead of x (the TF32 inference path): neither input nor weights are rounded
 };
 
 __host__ __device__ inline int conv0_moment_count(int Cin) { const int na = Cin * kC0K; return na + na * na; }
 
 // ------------------------------------------------------------------------------------------------ moments
 // grid B, block 512: thread o < NA + NA*NA owns one moment; the instance streams through smem in windows.
-template <int CIN>
+// F32: the TF32 inference path (fp32 input a.xf, unrounded weights)
+template <int CIN, bool F32 = false>
 __global__ void __launch_bounds__(512) conv0_moments_kernel(Conv0Args a, double* __restrict__ mom) {
   constexpr int NA = CIN * kC0K;
   constexpr int NOUT = NA + NA * NA;
@@ -61,7 +63,12 @@ __global__ void __launch_bounds__(512) conv0_moments_kernel(Conv0Args a, double*
     __syncthreads();
     for (int ci = 0; ci < CIN; ++ci) {
       const bf16* src = a.x + (static_cast<size_t>(b) * CIN + ci) * a.L + static_cast<size_t>(t0) * kC0S;
-      for (int i = threadIdx.x; i < win; i += blockDim.x) s_x[ci * WIN + i] = __bfloat162float(src[i]);
+      if constexpr (F32) {
+        const float* srcf = a.xf + (static_cast<size_t>(b) * CIN + ci) * a.L + static_cast<size_t>(t0) * kC0S;
+        for (int i = threadIdx.x; i < win; i += blockDim.x) s_x[ci * WIN + i] = srcf[i];
+      } else {
+        for (int i = threadIdx.x; i < win; i += blockDim.x) s_x[ci * WIN + i] = __bfloat162float(src[i]);
+      }
     }
     __syncthreads();
     if (o < NOUT) {
@@ -78,7 +85,7 @@ __global__ void __launch_bounds__(512) conv0_moments_kernel(Conv0Args a, double*
 }
 
 // grid B, block C: closed-form GroupNorm statistics -> stats[b, c] = (mean, rstd)
-template <int CIN>
+template <int CIN, bool F32 = false>
 __global__ void conv0_stats_kernel(Conv0Args a, const double* __restrict__ mom, float eps, float* __restrict__ stats) {
   constexpr int NA = CIN * kC0K;
   constexpr int NOUT = NA + NA * NA;
@@ -90,7 +97,10 @@ __global__ void conv0_stats_kernel(Conv0Args a, const double* __restrict__ mom, 
   if (c >= a.C) return;
   double w[NA];
 #pragma unroll
-  for (int i = 0; i < NA; ++i) w[i] = static_cast<double>(bf16_round(a.w[static_cast<size_t>(c) * NA + i]));
+  for (int i = 0; i < NA; ++i) {
+    const float wi = a.w[static_cast<size_t>(c) * NA + i];
+    w[i] = static_cast<double>(F32 ? wi : bf16_round(wi));
+  }
   double m = 0.0, q = 0.0;
 #pragma unroll
   for (int i = 0; i < NA; ++i) m += w[i] * s_m[i];
@@ -432,6 +442,60 @@ __global__ void __launch_bounds__(256) conv0_bwd_finalize_kernel(Conv0Args a, co
   }
 }
 
+// Forward of the TF32 inference path: fp32 input and weights, fp32 FMA on the CUDA cores (Cin x 10 MAC per output),
+// closed-form statistics of the unrounded conv output, exact erf GELU, fp32 channels-last [B, L_out, C] output rounded to
+// nearest tf32 (it is the operand of the next conv's implicit GEMM).  (256 clips x 10 s: 16.9 GB written in 8.5 ms,
+// ~2 TB/s -- short of the HBM bound; the exact erff per output is the rest, profiles/r03_bench_hear_precision.json.)
+// grid (ceil(L_out / kC0F32T), B), block C / 2: thread i owns channels 2i, 2i + 1 (weights and affine in registers); a
+// warp writes 256 contiguous bytes of each output row.
+constexpr int kC0F32T = 64;                                 // outputs per block
+constexpr int kC0F32Win = (kC0F32T - 1) * kC0S + kC0K;      // 325 samples
+template <int CIN>
+__global__ void __launch_bounds__(256) conv0_fwd_f32_kernel(Conv0Args a, const float* __restrict__ stats,
+                                                            const float* __restrict__ gamma,
+                                                            const float* __restrict__ beta, float* __restrict__ out) {
+  constexpr int NA = CIN * kC0K;
+  __shared__ float s_x[CIN][kC0F32Win];
+  const int b = blockIdx.y;
+  const int t0 = blockIdx.x * kC0F32T;
+  const int c = 2 * threadIdx.x;
+  for (int ci = 0; ci < CIN; ++ci) {
+    const float* src = a.xf + (static_cast<size_t>(b) * CIN + ci) * a.L;
+    for (int i = threadIdx.x; i < kC0F32Win; i += blockDim.x) {
+      const long long pos = static_cast<long long>(t0) * kC0S + i;
+      s_x[ci][i] = pos < a.L ? src[pos] : 0.f;
+    }
+  }
+  float w0[NA], w1[NA];
+#pragma unroll
+  for (int i = 0; i < NA; ++i) {
+    w0[i] = a.w[static_cast<size_t>(c) * NA + i];
+    w1[i] = a.w[static_cast<size_t>(c + 1) * NA + i];
+  }
+  const float4 st = *reinterpret_cast<const float4*>(stats + (static_cast<size_t>(b) * a.C + c) * 2);   // m0 r0 m1 r1
+  const float sc0 = gamma[c] * st.y, sc1 = gamma[c + 1] * st.w;
+  const float sh0 = beta[c] - st.x * sc0, sh1 = beta[c + 1] - st.z * sc1;
+  __syncthreads();
+  const int nt = min(kC0F32T, a.L_out - t0);
+  float* op = out + (static_cast<size_t>(b) * a.L_out + t0) * a.C + c;
+#pragma unroll 4
+  for (int t = 0; t < nt; ++t) {
+    float y0 = 0.f, y1 = 0.f;
+#pragma unroll
+    for (int ci = 0; ci < CIN; ++ci) {
+#pragma unroll
+      for (int k = 0; k < kC0K; ++k) {
+        const float xv = s_x[ci][t * kC0S + k];
+        y0 = fmaf(xv, w0[ci * kC0K + k], y0);
+        y1 = fmaf(xv, w1[ci * kC0K + k], y1);
+      }
+    }
+    const float g0 = tf32_round(gelu_erf(fmaf(y0, sc0, sh0)));
+    const float g1 = tf32_round(gelu_erf(fmaf(y1, sc1, sh1)));
+    *reinterpret_cast<float2*>(op + static_cast<size_t>(t) * a.C) = make_float2(g0, g1);
+  }
+}
+
 static int check_conv0(int Cin, int C, int k, int stride) {
   if (k != kC0K || stride != kC0S) { set_error("conv0: only k=10, stride=5 is built (got k=%d s=%d)", k, stride); return WJ_ERR_ARG; }
   if (Cin < 1 || Cin > kC0MaxCin) { set_error("conv0: Cin must be 1 or 2"); return WJ_ERR_ARG; }
@@ -453,7 +517,7 @@ extern "C" int wj_conv0_gn_gelu_fwd(const void* x_bf16, const float* w, const fl
   if (rc) return rc;
   cudaStream_t st = WJ_STREAM(stream);
   Conv0Args a;
-  a.x = reinterpret_cast<const bf16*>(x_bf16); a.w = w; a.B = B; a.Cin = Cin; a.L = L; a.C = C;
+  a.x = reinterpret_cast<const bf16*>(x_bf16); a.w = w; a.B = B; a.Cin = Cin; a.L = L; a.C = C; a.xf = nullptr;
   a.L_out = (L - k) / stride + 1;
   const int chunks = (a.L_out + kC0TT - 1) / kC0TT;
   const int cpb = 4;
@@ -483,7 +547,7 @@ extern "C" int wj_conv0_gn_gelu_bwd(const void* x_bf16, const float* w, const fl
   (void)eps; (void)dgelu_bf16;   // GELU' is recomputed (see the kernel); the argument is kept for ABI stability
   cudaStream_t st = WJ_STREAM(stream);
   Conv0Args a;
-  a.x = reinterpret_cast<const bf16*>(x_bf16); a.w = w; a.B = B; a.Cin = Cin; a.L = L; a.C = C;
+  a.x = reinterpret_cast<const bf16*>(x_bf16); a.w = w; a.B = B; a.Cin = Cin; a.L = L; a.C = C; a.xf = nullptr;
   a.L_out = (L - k) / stride + 1;
   const int na = Cin * kC0K;
   const int chunks = (a.L_out + kC0TT - 1) / kC0TT;
@@ -507,4 +571,29 @@ extern "C" int wj_conv0_gn_gelu_bwd(const void* x_bf16, const float* w, const fl
     conv0_bwd_finalize_kernel<2><<<fgrid, fblock, 0, st>>>(a, moments, stats, gamma, red, dw, dgamma, dbeta, nslab);
   }
   return check_launch("conv0_gn_gelu_bwd", 2);
+}
+
+// Conv block 0 of the TF32 inference path (see conv0_fwd_f32_kernel): x fp32 [B, Cin, L], out fp32 [B, L_out, C].
+extern "C" int wj_conv0_gn_gelu_fwd_f32(const float* x, const float* w, const float* gamma, const float* beta, int B,
+                                        int Cin, int L, int C, int k, int stride, float eps, double* moments, float* stats,
+                                        float* out, void* stream) {
+  if (B <= 0) return WJ_OK;
+  int rc = check_conv0(Cin, C, k, stride);
+  if (rc) return rc;
+  if (L < k) { set_error("conv0_f32: input shorter than the kernel"); return WJ_ERR_ARG; }
+  cudaStream_t st = WJ_STREAM(stream);
+  Conv0Args a;
+  a.x = nullptr; a.xf = x; a.w = w; a.B = B; a.Cin = Cin; a.L = L; a.C = C;
+  a.L_out = (L - k) / stride + 1;
+  dim3 grid((a.L_out + kC0F32T - 1) / kC0F32T, B);
+  if (Cin == 1) {
+    conv0_moments_kernel<1, true><<<B, 512, 0, st>>>(a, moments);
+    conv0_stats_kernel<1, true><<<B, C, 0, st>>>(a, moments, eps, stats);
+    conv0_fwd_f32_kernel<1><<<grid, C / 2, 0, st>>>(a, stats, gamma, beta, out);
+  } else {
+    conv0_moments_kernel<2, true><<<B, 512, 0, st>>>(a, moments);
+    conv0_stats_kernel<2, true><<<B, C, 0, st>>>(a, moments, eps, stats);
+    conv0_fwd_f32_kernel<2><<<grid, C / 2, 0, st>>>(a, stats, gamma, beta, out);
+  }
+  return check_launch("conv0_gn_gelu_fwd_f32", 3);
 }

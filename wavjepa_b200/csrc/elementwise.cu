@@ -619,6 +619,20 @@ extern "C" int wj_cast_bf16(const float* x, void* y_bf16, int64_t n, void* strea
   return check_launch("cast_bf16");
 }
 
+// y = x rounded to nearest tf32 (fp32 words with the low 13 mantissa bits zero): the working weights and the layer-0
+// operand of the TF32 inference path.  y may alias x.
+__global__ void tf32_round_kernel(const float* x, float* y, int64_t n) {
+  for (int64_t i = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x; i < n;
+       i += static_cast<int64_t>(gridDim.x) * blockDim.x)
+    y[i] = tf32_round(x[i]);
+}
+
+extern "C" int wj_tf32_round(const float* x, float* y, int64_t n, void* stream) {
+  if (n <= 0) return WJ_OK;
+  tf32_round_kernel<<<grid_for(n), 256, 0, WJ_STREAM(stream)>>>(x, y, n);
+  return check_launch("tf32_round");
+}
+
 extern "C" int wj_colsum(const void* x, int x_is_bf16, int64_t M, int N, int64_t ld, float* out, void* stream) {
   if (M <= 0) return WJ_OK;
   if (N % 2) { set_error("wj_colsum: N must be even"); return WJ_ERR_ARG; }

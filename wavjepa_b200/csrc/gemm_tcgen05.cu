@@ -70,6 +70,7 @@ struct GemmParams {
   long long* dbg;       // optional per-CTA cycle counters (wj_gemm_debug): [0] MMA thread waiting for operands, [1] for a free
                         // accumulator, [2] its total, [3] producer waiting for a free stage, [4] epilogue warp 4 waiting for
                         // an accumulator, [5] its total, [6] tiles, [7] unused
+  int round_tf32;       // tf32 kernel: fp32 outputs are rounded to nearest tf32 (they are the next GEMM's operand)
 };
 
 struct OutMaps {
@@ -128,7 +129,8 @@ __device__ __forceinline__ void seg_coords(const SegInfo& s, int vc, int& c0, in
 // 16-byte vectors with 64-128 contiguous bytes per row per instruction.  Work unit = 16 TMEM lanes x 32 columns;
 // the next unit's TMEM load is in flight during the math of the current one.  `arrive()` hands the accumulator back
 // to the MMA warp as soon as this warp's last tcgen05.ld has completed.
-template <int BN, bool WGRAD, typename Arrive>
+// TF32: the reference-precision inference GEMM (act 4 = exact erf GELU in fp32, no bf16 rounding anywhere).
+template <int BN, bool WGRAD, bool TF32 = false, typename Arrive>
 __device__ __forceinline__ void epilogue_tile(const GemmParams& p, uint32_t t_base, int lane, int lane_grp, int col_q,
                                               int n_blk, int b, int row_in_batch0, long long wgrad_row0, bool have_k,
                                               Arrive arrive, long long out_off = 0) {
@@ -229,7 +231,12 @@ __device__ __forceinline__ void epilogue_tile(const GemmParams& p, uint32_t t_ba
 #pragma unroll
         for (int c = 0; c < 8; ++c) x[c] += bias8[c];
       }
-      if (p.act == 3) {
+      if constexpr (TF32) {
+        if (p.act == 4) {
+#pragma unroll
+          for (int c = 0; c < 8; ++c) x[c] = gelu_erf(x[c]);
+        }
+      } else if (p.act == 3) {
         // the Linear output is bf16 under autocast before it meets the fp32 residual / positional table
 #pragma unroll
         for (int c = 0; c < 8; c += 2) bf16_round2(x[c], x[c + 1]);
@@ -278,6 +285,12 @@ __device__ __forceinline__ void epilogue_tile(const GemmParams& p, uint32_t t_ba
 #pragma unroll
         for (int c = 0; c < 8; ++c) atomicAdd(op + c * p.ld_out, x[c]);
       } else if (p.out_f32) {
+        if constexpr (TF32) {
+          if (p.round_tf32) {
+#pragma unroll
+            for (int c = 0; c < 8; ++c) x[c] = tf32_round(x[c]);
+          }
+        }
         float* op = reinterpret_cast<float*>(p.out) + out_off + orow * p.ld_out + n0;
         if (p.accumulate) {
           red_add_v4(op, x[0], x[1], x[2], x[3]);
@@ -535,15 +548,20 @@ __device__ __forceinline__ void epilogue_tile_tma_aux(const GemmParams& p, const
 }
 
 // MODE 0: A K-major, B K-major (fwd)   MODE 1: A, B MN-major (wgrad)   MODE 2: A K-major, B MN-major (dgrad)
-template <int BN, int MODE, bool HEAVY>
+// TF32 (MODE 0 only): fp32 operands, tcgen05.mma.kind::tf32.  A 128-byte swizzle row holds 64 bf16 or 32 fp32, and one
+// UMMA consumes 32 bytes of K either way, so the shared-memory ring, descriptors and barriers are byte-identical; only
+// the element count of a k-block (KB), the instruction kind and the descriptor's operand formats change.
+template <int BN, int MODE, bool HEAVY, bool TF32 = false>
 __global__ void __launch_bounds__(kThreads, 1)
 gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
             const __grid_constant__ CUtensorMap tmB1, const __grid_constant__ OutMaps om, const GemmParams p) {
+  static_assert(!TF32 || (MODE == 0 && !HEAVY), "the tf32 kernel is the plain forward");
   constexpr bool AUXQ = (MODE == 2 && HEAVY);   // GELU-backward dgrad: TMA-fed factor tiles (see epilogue_tile_tma_aux)
   using C = Cfg<BN, AUXQ>;
   constexpr bool WGRAD = (MODE == 1);
   constexpr bool B_MN = (MODE != 0);
   constexpr int STAGES = C::STAGES;
+  constexpr int KB = TF32 ? BK / 2 : BK;   // elements of K per k-block (128 bytes of each operand row)
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   uint64_t* full_bar = reinterpret_cast<uint64_t*>(smem + STAGES * C::STAGE_BYTES);
@@ -585,7 +603,7 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
   // wgrad : tile -> (split, m_blk, n_blk)
   auto num_kb = [&](int tile) -> int {
     if constexpr (!WGRAD) {
-      return p.K / BK;
+      return p.K / KB;
     } else {
       const int split = tile / (p.m_blocks * p.n_blocks);
       const int kb_total = p.batch * p.kb_per_batch;
@@ -611,7 +629,7 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
           const int n_blk = tile - m_blk * p.n_blocks;
           const int b = m_blk / p.mb_per_batch;
           const int row0 = (m_blk - b * p.mb_per_batch) * BM;
-          const int nkb = p.K / BK;
+          const int nkb = p.K / KB;
           for (int kb = 0; kb < nkb; ++kb) {
             const long long tw = p.dbg ? clock64() : 0;
             mbar_wait_relaxed(&empty_bar[stage], phase ^ 1);
@@ -619,11 +637,11 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
             uint8_t* sa = smem + stage * C::STAGE_BYTES;
             uint8_t* sb = sa + C::A_BYTES;
             int c0, q, po;
-            seg_coords(p.seg, kb * BK, c0, q, po);
+            seg_coords(p.seg, kb * KB, c0, q, po);
             mbar_arrive_expect_tx(&full_bar[stage], C::STAGE_BYTES);
             tma_load_4d(sa, &tmA, &full_bar[stage], c0, q, row0 + po, b);
             if constexpr (!B_MN) {
-              tma_load_2d(sb, &tmB, &full_bar[stage], kb * BK, n_blk * BN);
+              tma_load_2d(sb, &tmB, &full_bar[stage], kb * KB, n_blk * BN);
             } else {
               // dgrad: W is [reduction rows, output cols] row-major -> BN/64 MN-major atoms of 64 reduction rows, all
               // fetched by ONE TMA instruction through a 3-D view {64 cols, rows, column atoms} (the TMA unit is
@@ -676,7 +694,7 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
   } else if (warp == 1) {
     // ======================================================================================= MMA issuer
     if (lane == 0) {
-      constexpr uint32_t idesc = umma_idesc_bf16(BM, BN, WGRAD, B_MN);
+      constexpr uint32_t idesc = TF32 ? umma_idesc_tf32(BM, BN) : umma_idesc_bf16(BM, BN, WGRAD, B_MN);
       int stage = 0;
       uint32_t phase = 0;
       int it = 0;
@@ -708,7 +726,8 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
             else da = umma_smem_desc_sw128(sa + k * 2048, BK * 128, 1024);
             if constexpr (!B_MN) db = umma_smem_desc_sw128(sb + k * 32, 0, 1024);
             else db = umma_smem_desc_sw128(sb + k * 2048, BK * 128, 1024);
-            umma_bf16(d_tmem, da, db, idesc, (kb > 0 || k > 0) ? 1u : 0u);
+            if constexpr (TF32) umma_tf32(d_tmem, da, db, idesc, (kb > 0 || k > 0) ? 1u : 0u);
+            else umma_bf16(d_tmem, da, db, idesc, (kb > 0 || k > 0) ? 1u : 0u);
           }
           umma_commit(&empty_bar[stage]);  // frees the smem slot when these MMAs retire
           if (++stage == STAGES) { stage = 0; phase ^= 1; }
@@ -772,7 +791,7 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
       tc_fence_after();
       const uint32_t t_acc = tmem_base + (static_cast<uint32_t>(lane_grp * 32) << 16) + acc * BN;
       const uint32_t t_base = t_acc + col_q * (CHUNKS * 32);   // (TMA-store paths: CHUNKS consecutive chunks per warp)
-      if constexpr (!WGRAD) {
+      if constexpr (!WGRAD && !TF32) {
         if (p.tma_store) {
           if constexpr (AUXQ) {   // (for dgrad the second instantiation is the GELU-backward path)
             epilogue_tile_tma_aux<BN>(p, om, t_base, ap, lane, lane_grp, col_q, tile, n_blk, b, row_in_batch0,
@@ -786,8 +805,9 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
       }
       long long out_off = 0;
       if constexpr (WGRAD) out_off = static_cast<long long>(tile / (p.m_blocks * p.n_blocks)) * p.split_stride;
-      epilogue_tile<BN, WGRAD>(p, t_acc, lane, lane_grp, col_q, n_blk, b, row_in_batch0,
-                               static_cast<long long>(m_blk) * BM, have_k, [&]() { mbar_arrive(&tempty_bar[acc]); }, out_off);
+      epilogue_tile<BN, WGRAD, TF32>(p, t_acc, lane, lane_grp, col_q, n_blk, b, row_in_batch0,
+                                     static_cast<long long>(m_blk) * BM, have_k, [&]() { mbar_arrive(&tempty_bar[acc]); },
+                                     out_off);
     }
     if (p.tma_store && lane == 0) bulk_wait0();   // all TMA stores of this warp are complete before smem goes away
     if (p.dbg && warp == kEpiWarp0 && lane == 0) {
@@ -1077,7 +1097,8 @@ static PFN_encodeTiled get_encode() {
 }
 
 
-static int encode_map(CUtensorMap* tm, const wj_operand_t* op, const uint32_t box[4]) {
+static int encode_map(CUtensorMap* tm, const wj_operand_t* op, const uint32_t box[4],
+                      CUtensorMapDataType dt = CU_TENSOR_MAP_DATA_TYPE_BFLOAT16) {
   PFN_encodeTiled enc = get_encode();
   if (!enc) { set_error("cuTensorMapEncodeTiled entry point unavailable (no CUDA driver?)"); return WJ_ERR_RUNTIME; }
   cuuint64_t dims[4];
@@ -1085,7 +1106,7 @@ static int encode_map(CUtensorMap* tm, const wj_operand_t* op, const uint32_t bo
   cuuint32_t bx[4], es[4] = {1, 1, 1, 1};
   for (int i = 0; i < 4; ++i) { dims[i] = static_cast<cuuint64_t>(op->dim[i]); bx[i] = box[i]; }
   for (int i = 0; i < 3; ++i) strides[i] = static_cast<cuuint64_t>(op->stride_bytes[i]);
-  CUresult r = enc(tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(op->ptr), dims, strides, bx, es,
+  CUresult r = enc(tm, dt, 4, const_cast<void*>(op->ptr), dims, strides, bx, es,
                    CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) {
@@ -1098,13 +1119,14 @@ static int encode_map(CUtensorMap* tm, const wj_operand_t* op, const uint32_t bo
 }
 
 static int encode_map_2d(CUtensorMap* tm, const void* ptr, uint64_t inner, uint64_t outer, uint64_t stride_bytes,
-                         uint32_t box_inner, uint32_t box_outer) {
+                         uint32_t box_inner, uint32_t box_outer,
+                         CUtensorMapDataType dt = CU_TENSOR_MAP_DATA_TYPE_BFLOAT16) {
   PFN_encodeTiled enc = get_encode();
   if (!enc) { set_error("cuTensorMapEncodeTiled entry point unavailable (no CUDA driver?)"); return WJ_ERR_RUNTIME; }
   cuuint64_t dims[2] = {inner, outer};
   cuuint64_t strides[1] = {stride_bytes};
   cuuint32_t bx[2] = {box_inner, box_outer}, es[2] = {1, 1};
-  CUresult r = enc(tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(ptr), dims, strides, bx, es,
+  CUresult r = enc(tm, dt, 2, const_cast<void*>(ptr), dims, strides, bx, es,
                    CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) {
@@ -1206,11 +1228,11 @@ static bool tile192_ok(const wj_epilogue_t* e, int N) {
          (e->act == 0 || e->act == 1) && e->ld_out % 8 == 0 && reinterpret_cast<uintptr_t>(e->out) % 16 == 0;
 }
 
-template <int BN, int MODE, bool HEAVY>
+template <int BN, int MODE, bool HEAVY, bool TF32 = false>
 static int launch_variant(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMap& tmB1, const OutMaps& om,
                           const GemmParams& p, int grid, cudaStream_t st) {
   static bool attr_set = false;
-  auto kern = gemm_kernel<BN, MODE, HEAVY>;
+  auto kern = gemm_kernel<BN, MODE, HEAVY, TF32>;
   constexpr int kSmem = Cfg<BN, (MODE == 2 && HEAVY)>::SMEM_BYTES;
   if (!attr_set) {
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem);
@@ -1546,4 +1568,51 @@ extern "C" int wj_gemm_dgrad_bf16(const wj_operand_t* A, const void* W, int64_t 
   if (block_n == 192) return launch<192, 2>(tmA, tmB, tmB, om, p, grid, st);
   if (block_n == 256) return launch<256, 2>(tmA, tmB, tmB, om, p, grid, st);
   return launch<128, 2>(tmA, tmB, tmB, om, p, grid, st);
+}
+
+// Reference-precision (TF32) inference GEMM: out[b*L + t, n] = epilogue( sum_vc A(vc; t, b) * W[n, vc] ) with A and W fp32
+// (the caller rounds them to nearest tf32: the tensor core would truncate), K-major, tcgen05.mma.kind::tf32, fp32
+// accumulation.  Epilogue: v = acc + bias; act 4: v = exact erf GELU(v); v += resid; out = v as bf16, or fp32 rounded
+// to nearest tf32 when round_out (an output that is the next GEMM's operand).
+extern "C" int wj_gemm_tf32(const wj_operand_t* A, const float* W, int64_t ldw, int L, int batch, int N, int K,
+                            const wj_epilogue_t* epi, int round_out, void* stream) {
+  if (L <= 0 || batch <= 0) return WJ_OK;
+  constexpr int KB = BK / 2;
+  if (epi == nullptr) { set_error("wj_gemm_tf32: no epilogue"); return WJ_ERR_ARG; }
+  if (K % KB != 0 || N % 128 != 0) { set_error("wj_gemm_tf32: K must be a multiple of 32 and N of 128 (K=%d N=%d)", K, N); return WJ_ERR_ARG; }
+  if (A->seg_width > 0 && (A->seg_width % KB != 0 || K > 4 * A->seg_width)) { set_error("wj_gemm_tf32: bad segment width"); return WJ_ERR_ARG; }
+  if (epi->accumulate || epi->out2 != nullptr || epi->aux != nullptr || epi->out_rows != nullptr || epi->colsum != nullptr ||
+      (epi->act != 0 && epi->act != 4)) {
+    set_error("wj_gemm_tf32: the epilogue takes bias, act 0 / 4 (exact GELU), a residual and a plain output");
+    return WJ_ERR_ARG;
+  }
+  if (round_out && !epi->out_f32) { set_error("wj_gemm_tf32: tf32 rounding needs an fp32 output"); return WJ_ERR_ARG; }
+  if (epi->ld_out % 8 != 0 || reinterpret_cast<uintptr_t>(epi->out) % 16 != 0 ||
+      (epi->resid != nullptr && (epi->ld_resid % 8 != 0 || reinterpret_cast<uintptr_t>(epi->resid) % 16 != 0))) {
+    set_error("wj_gemm_tf32: outputs / residual need 16-byte aligned rows");
+    return WJ_ERR_ARG;
+  }
+  const int block_n = N % 256 == 0 ? 256 : 128;
+  CUtensorMap tmA, tmB;
+  const uint32_t boxA[4] = {KB, 1, BM, 1};
+  int rc = encode_map(&tmA, A, boxA, CU_TENSOR_MAP_DATA_TYPE_FLOAT32);
+  if (rc) return rc;
+  rc = encode_map_2d(&tmB, W, (uint64_t)K, (uint64_t)N, (uint64_t)ldw * 4, KB, (uint32_t)block_n, CU_TENSOR_MAP_DATA_TYPE_FLOAT32);
+  if (rc) return rc;
+  GemmParams p;
+  memset(&p, 0, sizeof(p));
+  p.L = L; p.batch = batch; p.N = N; p.K = K;
+  p.mb_per_batch = (L + BM - 1) / BM;
+  p.m_blocks = batch * p.mb_per_batch;
+  p.n_blocks = N / block_n;
+  p.total_tiles = p.m_blocks * p.n_blocks;
+  fill_seg(p.seg, A);
+  fill_epilogue(p, epi);
+  p.round_tf32 = round_out ? 1 : 0;
+  const int grid = p.total_tiles < num_sms() ? p.total_tiles : num_sms();
+  OutMaps om;
+  memset(&om, 0, sizeof(om));   // (generic epilogue: no TMA stores)
+  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  if (block_n == 256) return launch_variant<256, 0, false, true>(tmA, tmB, tmB, om, p, grid, st);
+  return launch_variant<128, 0, false, true>(tmA, tmB, tmB, om, p, grid, st);
 }

@@ -12,12 +12,16 @@
 namespace wj {
 
 // ------------------------------------------------------------------------------------------------ LayerNorm
-template <int D, typename TIn>
+// TF32 (the reference-precision inference path): the addend is fp32 (add_f32) and the operand copy of the output is fp32
+// rounded to nearest tf32 (out_tf32, the next GEMM's operand) instead of bf16.
+template <int D, typename TIn, bool TF32 = false>
 __global__ void __launch_bounds__(256) layernorm_fwd_kernel(const TIn* __restrict__ x, const float* __restrict__ gamma,
                                                             const float* __restrict__ beta, float eps, int M,
                                                             float* __restrict__ out_f32, bf16* __restrict__ out_bf16,
                                                             float* __restrict__ stats, float* __restrict__ rowsum,
-                                                            const bf16* __restrict__ add) {
+                                                            const bf16* __restrict__ add,
+                                                            const float* __restrict__ add_f32 = nullptr,
+                                                            float* __restrict__ out_tf32 = nullptr) {
   // add (optional, bf16 [M, D]): the row normalised is x + add -- the residual sum y = x + bf16(Linear(...)) of the
   // post-norm layer, formed here in registers so that the GEMM writes 2 bytes per element and y never exists in HBM
   constexpr int PER = D / 32;  // elements per lane, contiguous chunks of 4
@@ -39,7 +43,12 @@ __global__ void __launch_bounds__(256) layernorm_fwd_kernel(const TIn* __restric
       const float2 b = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&u.y));
       v[4 * i] = a.x; v[4 * i + 1] = a.y; v[4 * i + 2] = b.x; v[4 * i + 3] = b.y;
     }
-    if (add != nullptr) {
+    if constexpr (TF32) {
+      if (add_f32 != nullptr) {
+        const float4 f = *reinterpret_cast<const float4*>(add_f32 + base + col);
+        v[4 * i] += f.x; v[4 * i + 1] += f.y; v[4 * i + 2] += f.z; v[4 * i + 3] += f.w;
+      }
+    } else if (add != nullptr) {
       const uint2 u = *reinterpret_cast<const uint2*>(add + base + col);
       const float2 a = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&u.x));
       const float2 b = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&u.y));
@@ -70,7 +79,11 @@ __global__ void __launch_bounds__(256) layernorm_fwd_kernel(const TIn* __restric
     osum += o.x + o.y + o.z + o.w;
     osq += o.x * o.x + o.y * o.y + o.z * o.z + o.w * o.w;
     if (out_f32 != nullptr) *reinterpret_cast<float4*>(out_f32 + base + col) = o;
-    if (out_bf16 != nullptr) {
+    if constexpr (TF32) {
+      if (out_tf32 != nullptr)
+        *reinterpret_cast<float4*>(out_tf32 + base + col) =
+            make_float4(tf32_round(o.x), tf32_round(o.y), tf32_round(o.z), tf32_round(o.w));
+    } else if (out_bf16 != nullptr) {
       uint2 u;
       u.x = pack_bf16x2(o.x, o.y);
       u.y = pack_bf16x2(o.z, o.w);
@@ -442,6 +455,22 @@ extern "C" int wj_add_layernorm_fwd(const float* x, const void* add_bf16, const 
   if (M <= 0) return WJ_OK;
   return launch_ln_fwd<float>(x, gamma, beta, eps, M, D, out_f32, reinterpret_cast<bf16*>(out_bf16), stats, rowsum,
                               WJ_STREAM(stream), reinterpret_cast<const bf16*>(add_bf16));
+}
+
+// LayerNorm(x + add) of the TF32 inference path: x fp32, add fp32 or NULL; out_f32 = the unrounded result (residual
+// stream), out_tf32 = the result rounded to nearest tf32 (the next GEMM's operand); either may be NULL.
+extern "C" int wj_add_layernorm_fwd_f32(const float* x, const float* add_f32, const float* gamma, const float* beta,
+                                        float eps, int M, int D, float* out_f32, float* out_tf32, void* stream) {
+  if (M <= 0) return WJ_OK;
+  const int blocks = (M + 7) / 8;
+  cudaStream_t st = WJ_STREAM(stream);
+  switch (D) {
+#define WJ_LNF(DD) case DD: layernorm_fwd_kernel<DD, float, true><<<blocks, 256, 0, st>>>(x, gamma, beta, eps, M, out_f32, nullptr, nullptr, nullptr, nullptr, add_f32, out_tf32); break;
+    WJ_LNF(128) WJ_LNF(256) WJ_LNF(384) WJ_LNF(512) WJ_LNF(768) WJ_LNF(1024)
+#undef WJ_LNF
+    default: set_error("add_layernorm_fwd_f32: unsupported D=%d (128,256,384,512,768,1024)", D); return WJ_ERR_ARG;
+  }
+  return check_launch("add_layernorm_fwd_f32");
 }
 
 extern "C" int wj_add_layernorm_bwd(const float* dy_f32, const void* dy_bf16, const float* x, const void* add_bf16,

@@ -162,6 +162,19 @@ __device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t desc_a, uint
       "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
       : "memory");
 }
+// D[tmem] (+)= A[smem] * B[smem], tf32 inputs (fp32 words whose low 13 mantissa bits the tensor core ignores), fp32
+// accumulate, issued by ONE thread.  One instruction consumes 32 bytes of K (K = 8), like kind::f16 with K = 16.
+__device__ __forceinline__ void umma_tf32(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc,
+                                          uint32_t accumulate) {
+  asm volatile(
+      "{\n"
+      ".reg .pred p;\n"
+      "setp.ne.b32 p, %4, 0;\n"
+      "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n"
+      "}\n" ::"r"(tmem_d),
+      "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
 // Arrives on `bar` once all previously issued tcgen05.mma of this thread have completed.
 __device__ __forceinline__ void umma_commit(uint64_t* bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar))
@@ -226,6 +239,11 @@ __device__ __forceinline__ uint64_t umma_smem_desc_sw128(uint32_t smem_addr, uin
 __host__ __device__ constexpr uint32_t umma_idesc_bf16(int M, int N, bool a_mn_major, bool b_mn_major) {
   return (1u << 4) | (1u << 7) | (1u << 10) | ((a_mn_major ? 1u : 0u) << 15) | ((b_mn_major ? 1u : 0u) << 16) |
          (static_cast<uint32_t>(N >> 3) << 17) | (static_cast<uint32_t>(M >> 4) << 24);
+}
+// Instruction descriptor for kind::tf32 with tf32 A/B (format 2 in both fields), fp32 D, both operands K-major.
+__host__ __device__ constexpr uint32_t umma_idesc_tf32(int M, int N) {
+  return (1u << 4) | (2u << 7) | (2u << 10) | (static_cast<uint32_t>(N >> 3) << 17) |
+         (static_cast<uint32_t>(M >> 4) << 24);
 }
 
 // ----------------------------------------------------------------------------------------------- CTA pair (cta_group::2)
@@ -437,6 +455,13 @@ __device__ __forceinline__ uint32_t pack_bf16x2(float lo, float hi) {
   return *reinterpret_cast<uint32_t*>(&h);
 }
 __device__ __forceinline__ float bf16_round(float x) { return __bfloat162float(__float2bfloat16_rn(x)); }
+// fp32 -> nearest tf32 (ties away from zero), kept as an fp32 word with the low 13 mantissa bits zero.  The tensor core
+// truncates raw fp32 operands, which doubles the error of the TF32 inference path; operands are rounded as written.
+__device__ __forceinline__ float tf32_round(float x) {
+  uint32_t y;
+  asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(y) : "f"(x));
+  return __uint_as_float(y);
+}
 // Two values rounded to bf16 (round-to-nearest-even) and widened again with ONE pack (F2FP) + two integer ops instead
 // of two F2F conversions: F2F shares the quarter-rate XU pipe with MUFU, which the GELU epilogues saturate.
 __device__ __forceinline__ void bf16_round2(float& a, float& b) {

@@ -93,6 +93,42 @@ class TransformerStack:
             x32, x16 = x2_32, x2_16
         return x32, x16, saved
 
+    def forward_tf32(self, layers: List[LayerW], x32: torch.Tensor, xop: torch.Tensor, cu: torch.Tensor, n_seqs: int,
+                     max_len: int) -> torch.Tensor:
+        """Inference forward at reference precision (the reference's fp32 feature extraction): the same packed layout,
+        `layers` hold fp32 weight matrices rounded to nearest tf32.  x32: [M, d] fp32 residual stream, xop: its copy
+        rounded to nearest tf32.  Returns the fp32 output of the last layer.
+
+        Every GEMM runs on the tf32 tensor cores with operands rounded to nearest as they are written (the tensor core
+        would truncate raw fp32); attention keeps bf16 Q/K/V and P but writes O in fp32; the Linear outputs stay fp32
+        into the residual add; GELU is the exact erf form."""
+        d, H, ff = self.d, self.H, self.ff
+        M = x32.shape[0]
+        dev = x32.device
+        bf, f32 = torch.bfloat16, torch.float32
+        for w in layers:
+            qkv = _empty((M, 3 * d), bf, dev)
+            ops.gemm_tf32(ops.plain_operand(xop), w.w_in, M, 1, qkv, bias=w.b_in)
+            att = _empty((M, d), f32, dev)
+            ops.attn_fwd_f32(qkv, cu, n_seqs, max_len, d, H, att)
+            del qkv
+            o1 = _empty((M, d), f32, dev)
+            ops.gemm_tf32(ops.plain_operand(att), w.w_o, M, 1, o1, bias=w.b_o)
+            del att
+            x1_32 = _empty((M, d), f32, dev)
+            x1_op = _empty((M, d), f32, dev)
+            ops.add_layernorm_fwd_f32(x32, o1, w.g1, w.be1, self.eps, x1_32, x1_op)
+            del o1
+            g = _empty((M, ff), f32, dev)
+            ops.gemm_tf32(ops.plain_operand(x1_op), w.w1, M, 1, g, bias=w.b1, act=ops.ACT_GELU_ERF, round_out=True)
+            o2 = _empty((M, d), f32, dev)
+            ops.gemm_tf32(ops.plain_operand(g), w.w2, M, 1, o2, bias=w.b2)
+            del g
+            x32 = _empty((M, d), f32, dev)
+            xop = _empty((M, d), f32, dev)
+            ops.add_layernorm_fwd_f32(x1_32, o2, w.g2, w.be2, self.eps, x32, xop)
+        return x32
+
     # ------------------------------------------------------------------------------------------------ backward
     def backward(self, layers: List[LayerW], grads: List[LayerG], saved: List[LayerSaved], dx: torch.Tensor,
                  cu: torch.Tensor, n_seqs: int, max_len: int, on_layer_done: Optional[Callable] = None):

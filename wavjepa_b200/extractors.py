@@ -85,11 +85,12 @@ def out_length(spec: Sequence[Sequence[int]], time: int) -> int:
 
 
 # =============================================================================================== kernel orchestration
-def kmajor_weight(w: torch.Tensor, out: Optional[torch.Tensor] = None) -> torch.Tensor:
-    """[O, C, k] fp32 master weight -> [O, k*C] bf16 (tap-major) working copy used by the implicit GEMM."""
+def kmajor_weight(w: torch.Tensor, out: Optional[torch.Tensor] = None, dtype: torch.dtype = torch.bfloat16) -> torch.Tensor:
+    """[O, C, k] fp32 master weight -> [O, k*C] (tap-major) working copy used by the implicit GEMM (bf16, or fp32 for the
+    tf32 GEMM)."""
     O, C, k = w.shape
     if out is None:
-        out = torch.empty(O, k * C, device=w.device, dtype=torch.bfloat16)
+        out = torch.empty(O, k * C, device=w.device, dtype=dtype)
     out.view(O, k, C).copy_(w.detach().permute(0, 2, 1))
     return out
 
@@ -136,6 +137,35 @@ def conv_stack_forward(spec, x16: torch.Tensor, w0: torch.Tensor, gn_w: torch.Te
         sv = ConvSaved()
         sv.x16, sv.moments, sv.stats, sv.acts, sv.pre = x16, moments, stats, acts, pre
     return acts[-1], sv
+
+
+def conv_stack_forward_tf32(spec, x32: torch.Tensor, w0: torch.Tensor, gn_w: torch.Tensor, gn_b: torch.Tensor,
+                            wks: List[torch.Tensor], gn_eps: float = 1e-5) -> torch.Tensor:
+    """Inference at reference precision: x32 [B, Cin, L] fp32 -> features [B, T, C] fp32.  Block 0 in fp32 on the CUDA
+    cores, blocks 1..n as tf32 implicit GEMMs (wks: fp32 tap-major weights rounded to nearest tf32) with the exact GELU.
+    Every block output that feeds another conv is rounded to nearest tf32; the last one (LayerNorm input) is not."""
+    assert x32.dtype == torch.float32 and x32.is_contiguous()
+    B, Cin, L = x32.shape
+    C = spec[0][0]
+    dev = x32.device
+    L0 = (L - 10) // 5 + 1
+    if L0 <= 0:
+        raise WavJepaLibError("input shorter than the first conv kernel")
+    x = torch.empty(B, L0, C, device=dev, dtype=torch.float32)
+    moments, stats = ops.conv0_workspaces(B, Cin, C, dev)
+    ops.conv0_fwd_f32(x32, w0, gn_w, gn_b, x, moments, stats, eps=gn_eps)
+    n = len(spec)
+    for i, (_, k, _) in enumerate(spec[1:], start=1):
+        L_in = x.shape[1]
+        L_out = (L_in - k) // 2 + 1
+        g = torch.empty(B, L_out, C, device=dev, dtype=torch.float32)
+        if L_in % 2 == 0:
+            a_op = ops.conv_operand(x, k)
+        else:
+            a_op = ops.make_operand(x, k * C, L_out, B, row_stride=2 * C, batch_stride=L_in * C)
+        ops.gemm_tf32(a_op, wks[i - 1], L_out, B, g.view(-1, C), act=ops.ACT_GELU_ERF, round_out=i < n - 1)
+        x = g
+    return x
 
 
 def conv_stack_backward(spec, sv: ConvSaved, dh_last: torch.Tensor, w0, gn_w, gn_b, wks, g_w0, g_gn_w, g_gn_b,

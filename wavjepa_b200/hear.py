@@ -12,8 +12,13 @@ B200-first differences (results identical at every returned frame):
     per-clip gain is one kernel, the chunking + per-chunk normalisation (mean / unbiased std INCLUDING the zero
     padding, runtime.py:12-16,133-137) is one kernel, and all B * n_chunks chunks go through the encoder as one
     packed batch whose padded tokens are dropped (they are key-masked in the reference and cut off afterwards);
-  * the encoder runs bf16 operands / fp32 accumulate (the reference runs this path in fp32): features agree with the
-    fp32 reference to <= 1e-2 relative L2 (tests/test_gpu_model.py).
+  * two numerics, chosen with `precision=` on the loaders (hear-eval-kit passes model options through
+    load_model(path, **opts)) or `JEPA.inference_precision`:
+      "bf16" (default)  bf16 operands / fp32 accumulate and a packed-fp16 GELU (the reference runs this path in fp32):
+                        features agree with the fp32 reference to <= 1e-2 relative L2 (tests/test_gpu_model.py);
+      "tf32"            the reference's fp32 feature extraction with every GEMM operand rounded to nearest tf32, fp32
+                        accumulation, residual stream and chunk audio, exact erf GELU: <= 2e-3 relative L2
+                        (tests/test_gpu_tf32.py), at a lower throughput (DESIGN.md 2.1).
 """
 from __future__ import annotations
 
@@ -70,8 +75,12 @@ def embed_chunks(model: JEPA, a: torch.Tensor, gain: Optional[torch.Tensor], uni
     pad, n_chunks, cut_off, total_steps = hear_geometry(L, unit, sr, steps)
     dev = a.device
     starts = (torch.arange(n_chunks, device=dev, dtype=torch.int32) * unit).repeat(B)
-    x16 = torch.empty(B * n_chunks, C, unit, device=dev, dtype=torch.bfloat16)
-    ops.crop_norm(a, starts, n_chunks, unit, x16, None, gain=gain)
+    if model.inference_precision == "tf32":   # conv block 0 reads the fp32 chunks
+        x16 = torch.empty(B * n_chunks, C, unit, device=dev, dtype=torch.float32)
+        ops.crop_norm(a, starts, n_chunks, unit, None, x16, gain=gain)
+    else:
+        x16 = torch.empty(B * n_chunks, C, unit, device=dev, dtype=torch.bfloat16)
+        ops.crop_norm(a, starts, n_chunks, unit, x16, None, gain=gain)
     # The padding mask depends on the geometry only (the same for every clip), so it is built on the HOST and handed over as
     # a pattern that repeats every n_chunks sequences: the packed-token index then needs no device read-back, and calls
     # can be issued back to back without a host synchronisation.
@@ -92,7 +101,7 @@ class RuntimeJEPA(nn.Module):
     """reference hear_api/runtime.py:39-155."""
 
     def __init__(self, in_channels: int, weights, is_spectrogram: bool, process_seconds: float, extractor,
-                 model_size: str, sr: int, device: Optional[str] = None, **kwargs) -> None:
+                 model_size: str, sr: int, device: Optional[str] = None, precision: str = "bf16", **kwargs) -> None:
         super().__init__()
         if is_spectrogram:
             raise WavJepaLibError("spectrogram front-ends are not part of WavJEPA")
@@ -105,6 +114,7 @@ class RuntimeJEPA(nn.Module):
                           transformer_decoder_cfg=TransformerEncoderCFG.create(),
                           transformer_decoder_layers_cfg=TransformerLayerCFG.create(d_model=384), resample_sr=sr,
                           size=model_size, process_audio_seconds=process_seconds)
+        self.model.inference_precision = precision   # "bf16" or "tf32" (ValueError otherwise), see the module docstring
         if weights is None:
             raise TypeError("load_model needs a checkpoint: weights['state_dict'] (the reference fails here too, "
                             "hear_api/runtime.py:64)")
@@ -164,10 +174,11 @@ class RuntimeNatJEPA(RuntimeJEPA):
     the two channels' embeddings averaged (:142-147)."""
 
     def __init__(self, in_channels: int, weights, is_spectrogram: bool, process_seconds: float, extractor,
-                 model_size: str, sr: int, device: Optional[str] = None, **kwargs) -> None:
+                 model_size: str, sr: int, device: Optional[str] = None, precision: str = "bf16", **kwargs) -> None:
         if in_channels != 2:
             raise WavJepaLibError("RuntimeNatJEPA is built for the binaural model (in_channels=2)")
-        super().__init__(in_channels, weights, is_spectrogram, process_seconds, extractor, model_size, sr, device, **kwargs)
+        super().__init__(in_channels, weights, is_spectrogram, process_seconds, extractor, model_size, sr, device,
+                         precision, **kwargs)
         self.output_steps = self.model.extract_audio.total_patches(self.unit_frames) // in_channels
 
     def to_feature(self, audio: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
@@ -210,28 +221,29 @@ def _load_weights(args):
     return torch.load(w, weights_only=False, map_location="cpu")
 
 
-def load_model(*args, **kwargs) -> RuntimeJEPA:
-    """hear_configs/WavJEPA.py:11-35.  args[0]: checkpoint path (or an already loaded dict with 'state_dict')."""
+def load_model(*args, precision: str = "bf16", **kwargs) -> RuntimeJEPA:
+    """hear_configs/WavJEPA.py:11-35.  args[0]: checkpoint path (or an already loaded dict with 'state_dict').
+    precision: "bf16" (default) or "tf32" (reference-precision features, see the module docstring)."""
     extractor = ConvFeatureExtractor(conv_layers_spec=BASE_SPEC, in_channels=1)
     return RuntimeJEPA(in_channels=1, process_seconds=2.01, weights=_load_weights(args), sr=SR, model_size="base",
-                       is_spectrogram=False, extractor=extractor, **kwargs)
+                       is_spectrogram=False, extractor=extractor, precision=precision, **kwargs)
 
 
-def load_model_w2v2(*args, **kwargs) -> RuntimeJEPA:
+def load_model_w2v2(*args, precision: str = "bf16", **kwargs) -> RuntimeJEPA:
     """hear_configs/WavJEPA_w2v2.py:11-35: 7-layer wav2vec2 extractor (stride 320), 4.02 s windows -> 200 tokens."""
     extractor = ConvFeatureExtractor(conv_layers_spec=W2V2_SPEC, in_channels=1)
     return RuntimeJEPA(in_channels=1, process_seconds=4.02, weights=_load_weights(args), sr=SR, model_size="base",
-                       is_spectrogram=False, extractor=extractor, **kwargs)
+                       is_spectrogram=False, extractor=extractor, precision=precision, **kwargs)
 
 
-def load_model_nat(*args, share_weights_over_channels: bool = False, **kwargs) -> RuntimeNatJEPA:
+def load_model_nat(*args, share_weights_over_channels: bool = False, precision: str = "bf16", **kwargs) -> RuntimeNatJEPA:
     """WavJEPA-Nat counterpart of load_model (README.md:93-108 `labhamlet/wavjepa-nat-base`): per-channel extractors
     (wavjepa/extractors/audio_channel_feature_extractor.py), 2 x 200 tokens per 2.01 s window."""
     from .extractors import ConvChannelFeatureExtractor
     extractor = ConvChannelFeatureExtractor(conv_layers_spec=BASE_SPEC, in_channels=2,
                                             share_weights_over_channels=share_weights_over_channels)
     return RuntimeNatJEPA(in_channels=2, process_seconds=2.01, weights=_load_weights(args), sr=SR, model_size="base",
-                          is_spectrogram=False, extractor=extractor, **kwargs)
+                          is_spectrogram=False, extractor=extractor, precision=precision, **kwargs)
 
 
 def get_scene_embeddings(audio, model):

@@ -76,15 +76,17 @@ class WavJEPAModel(nn.Module):
         self.embedding_size = runtime.embedding_size
 
     @classmethod
-    def from_pretrained(cls, checkpoint: Union[str, Dict], nat: Optional[bool] = None, **kwargs) -> "WavJEPAModel":
+    def from_pretrained(cls, checkpoint: Union[str, Dict], nat: Optional[bool] = None, precision: str = "bf16",
+                        **kwargs) -> "WavJEPAModel":
         """checkpoint: path to (or dict of) a Lightning checkpoint with 'state_dict' (hub names cannot be resolved here:
-        there is no network).  nat: build the binaural WavJEPA-Nat runtime (default: inferred from the state-dict keys)."""
+        there is no network).  nat: build the binaural WavJEPA-Nat runtime (default: inferred from the state-dict keys).
+        precision: "bf16" (default) or "tf32" (reference-precision features, wavjepa_b200.hear)."""
         for k in ("trust_remote_code", "force_download"):
             kwargs.pop(k, None)
         ck = hear._load_weights((checkpoint,))
         if nat is None:
             nat = any(k.startswith("extract_audio.cnns.") for k in ck["state_dict"])
-        rt = hear.load_model_nat(ck, **kwargs) if nat else hear.load_model(ck, **kwargs)
+        rt = hear.load_model_nat(ck, precision=precision, **kwargs) if nat else hear.load_model(ck, precision=precision, **kwargs)
         return cls(rt)
 
     def forward(self, input_values: torch.Tensor):
@@ -95,9 +97,10 @@ class WavJEPAModel(nn.Module):
 extractor = WavJEPAFeatureExtractor()
 
 
-def load_model(*args, **kwargs) -> WavJEPAModel:
-    """hear_configs/WavJEPA_huggingface.py:19-24 (there: the hub model; here: args[0] = local checkpoint path / dict)."""
-    model = WavJEPAModel.from_pretrained(args[0], **kwargs)
+def load_model(*args, precision: str = "bf16", **kwargs) -> WavJEPAModel:
+    """hear_configs/WavJEPA_huggingface.py:19-24 (there: the hub model; here: args[0] = local checkpoint path / dict).
+    precision: "bf16" (default) or "tf32"."""
+    model = WavJEPAModel.from_pretrained(args[0], precision=precision, **kwargs)
     model.sample_rate = SAMPLING_RATE
     return model
 

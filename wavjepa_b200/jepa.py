@@ -31,7 +31,7 @@ from ._lightning import Base as _ModuleBase
 from ._lightning import attached_trainer
 from .engine import LayerG, LayerW, TransformerStack
 from .extractors import (ConvChannelFeatureExtractor, ConvFeatureExtractor, conv_stack_backward, conv_stack_forward,
-                         kmajor_weight)
+                         conv_stack_forward_tf32, kmajor_weight)
 from .pos_embed import get_1d_sincos_pos_embed_from_grid
 from .types import ForwardReturn, TransformerEncoderCFG, TransformerLayerCFG
 
@@ -204,6 +204,21 @@ class JEPA(_ModuleBase):
         self._ddp = None
         self.collate_fn = collate_fn
         self.return_dense_preds = True
+        self.inference_precision = "bf16"
+
+    @property
+    def inference_precision(self) -> str:
+        """Numerics of `get_audio_representation`: "bf16" (the default) runs the encoder with bf16 operands and the
+        packed-fp16 tanh-form GELU, ~1e-2 relative L2 from the reference's fp32 features; "tf32" runs the reference's fp32
+        feature extraction with every GEMM operand rounded to nearest tf32, fp32 accumulation and the exact erf GELU
+        (DESIGN.md 2.1).  `forward`, `train_step`, the teacher and the denoiser ignore it."""
+        return self.__dict__.get("_inference_precision", "bf16")
+
+    @inference_precision.setter
+    def inference_precision(self, value: str) -> None:
+        if value not in ("bf16", "tf32"):
+            raise ValueError(f"inference_precision must be 'bf16' or 'tf32', got {value!r}")
+        self.__dict__["_inference_precision"] = value
 
     # ------------------------------------------------------------------------------------------- reference helpers
     def _get_pos_embed_params(self, embedding_dim: int) -> nn.Parameter:
@@ -809,6 +824,7 @@ class JEPA(_ModuleBase):
                                1.0 / world, self.grad_clip, ss, self._flat_w16, self._flat_t, self._flat_t16, e0, e1,
                                ema_decay)
         self._refresh_conv_weights()
+        self._tf32_cache = None   # the tf32 working weights are rebuilt from the updated parameters on their next use
         self._step = self.global_step + 1
 
     # ------------------------------------------------------------------------------------------- optimizer state
@@ -882,6 +898,91 @@ class JEPA(_ModuleBase):
             cache[key] = (rows.contiguous(), cu.contiguous(), reps * int(rows_1.size), int(n_per.max()) if n_per.size else 0)
         return cache[key]
 
+    def _tf32_weights(self) -> dict:
+        """fp32 working copy of the extractor, mapper and encoder weight matrices rounded to nearest tf32 (conv weights
+        tap-major), built on first use and rebuilt when a parameter changed (load_state_dict, optimizer steps) or the flat
+        buffers moved.  Bias and LayerNorm vectors are read from the fp32 masters."""
+        sig = (self._signature(), self._flat_p.data_ptr())
+        cache = self.__dict__.get("_tf32_cache")
+        if cache is not None and cache[0] == sig:
+            return cache[1]
+        self._tf32_cache = None
+        flat = ops.tf32_round(self._flat_p[:self._enc_range[1]])   # extractor .. encoder: the leading part of the layout
+        v32 = lambda n: self._view(flat, n)
+        p32 = lambda n: self._view(self._flat_p, n)
+        conv = {}
+        for prefix, spec in self._extractors():
+            for i in range(1, len(spec)):
+                name = f"{prefix}.{i}.0.weight"
+                conv[name] = kmajor_weight(v32(name), dtype=torch.float32)
+        w = dict(layers=self._stack_weights("encoder.", self._enc_stack.n_layers, v32, p32), conv=conv,
+                 mapper=v32("post_extraction_mapper.weight"))
+        self._tf32_cache = (sig, w)
+        return w
+
+    def _local_features_tf32(self, x32: torch.Tensor, w: dict) -> torch.Tensor:
+        """_local_features at reference precision (inference only): fp32 waveform -> conv stack (tf32) -> LayerNorm(512)
+        -> tf32 Linear 512->D (+bias) + positional table, all fp32.  Returns local32 [B*T, D]."""
+        ex = self.extract_audio
+        B = x32.shape[0]
+        T, D = self.total_patches, self.encoder_embedding_dim
+        C = ex.embedding_dim
+        p32 = lambda n: self._view(self._flat_p, n)
+
+        def stack(prefix, x):
+            wks = [w["conv"][f"{prefix}.{i}.0.weight"] for i in range(1, len(ex.conv_layers_spec))]
+            return conv_stack_forward_tf32(ex.conv_layers_spec, x, p32(f"{prefix}.0.0.weight"), p32(f"{prefix}.0.2.weight"),
+                                           p32(f"{prefix}.0.2.bias"), wks)
+
+        if isinstance(ex, ConvChannelFeatureExtractor):
+            Tc = T // ex.in_channels
+            feats = torch.empty(B, T, C, device=x32.device)
+            xs = x32.transpose(0, 1).contiguous()  # [Cin, B, L]: one mono stream per CNN
+            for c in range(ex.in_channels):
+                prefix = f"extract_audio.cnns.{0 if ex.share_weights_over_channels else c}"
+                feats[:, c * Tc:(c + 1) * Tc].copy_(stack(prefix, xs[c].unsqueeze(1)))
+        else:
+            feats = stack("extract_audio.cnn", x32)
+        ln = torch.empty(B * T, C, device=x32.device)
+        ops.add_layernorm_fwd_f32(feats.view(B * T, C), None, p32("feature_norms.weight"), p32("feature_norms.bias"),
+                                  self.feature_norms.eps, None, ln)
+        local32 = torch.empty(B * T, D, device=x32.device)
+        ops.gemm_tf32(ops.plain_operand(ln), w["mapper"], B * T, 1, local32, bias=p32("post_extraction_mapper.bias"),
+                      resid=self._pos_enc, resid_mod=T)
+        return local32
+
+    def _audio_representation_tf32(self, audio: torch.Tensor, padding_mask, host_mask) -> torch.Tensor:
+        """get_audio_representation with inference_precision == "tf32" (same masking semantics)."""
+        dev = self.device
+        w = self._tf32_weights()
+        x32 = audio.to(device=dev, dtype=torch.float32).contiguous()
+        B = x32.shape[0]
+        T, D = self.total_patches, self.encoder_embedding_dim
+        local32 = self._local_features_tf32(x32, w)
+        p32 = lambda n: self._view(self._flat_p, n)
+        if padding_mask is None and host_mask is None:
+            cu = torch.arange(0, (B + 1) * T, T, device=dev, dtype=torch.int32)
+            xs32 = self._enc_stack.forward_tf32(w["layers"], local32, ops.tf32_round(local32), cu, B, T)
+            out = torch.empty(B * T, D, device=dev)
+            ops.layernorm_fwd(xs32, p32("encoder.norm.weight"), p32("encoder.norm.bias"), self.encoder.norm.eps, out,
+                              None, None, None)
+            return out.view(B, T, D)
+        if host_mask is not None:
+            ctx_rows, cu_c, Nc, max_nc = self._periodic_index(host_mask, B, T)
+        else:
+            pm = padding_mask.to(dev).reshape(B, 1, T).contiguous()
+            mi = ops.mask_indices(pm.view(B, T), torch.zeros_like(pm), pm)
+            ctx_rows, cu_c, Nc, max_nc = mi.ctx_rows, mi.cu_c, mi.Nc, mi.max_nc
+        xc32 = torch.empty(Nc, D, device=dev)
+        ops.gather_rows(local32, ctx_rows, Nc, xc32, None)
+        xs32 = self._enc_stack.forward_tf32(w["layers"], xc32, ops.tf32_round(xc32), cu_c, B, max_nc)
+        packed = torch.empty(Nc, D, device=dev)
+        ops.layernorm_fwd(xs32, p32("encoder.norm.weight"), p32("encoder.norm.bias"), self.encoder.norm.eps, packed,
+                          None, None, None)
+        out = torch.zeros(B * T, D, device=dev)
+        ops.scatter_rows(packed, ctx_rows, Nc, out)
+        return out.view(B, T, D)
+
     def get_audio_representation(self, audio: torch.Tensor, padding_mask: Optional[torch.Tensor] = None,
                                  host_mask=None) -> torch.Tensor:
         """reference wavjepa/jepa.py:456-467: student encoder (incl. final norm) features [B, T, D] fp32.  Tokens
@@ -892,6 +993,8 @@ class JEPA(_ModuleBase):
         self.eval()
         self._ensure_ready()
         self._sync_weights()
+        if self.inference_precision == "tf32":
+            return self._audio_representation_tf32(audio, padding_mask, host_mask)
         dev = self.device
         x16 = audio.to(device=dev, dtype=torch.bfloat16).contiguous()
         B = x16.shape[0]

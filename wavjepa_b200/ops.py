@@ -14,6 +14,7 @@ from . import _lib
 from ._lib import Epilogue, Operand, check
 
 ACT_NONE, ACT_GELU, ACT_DGELU, ACT_BF16 = 0, 1, 2, 3
+ACT_GELU_ERF = 4   # tf32 GEMM only: exact erf GELU in fp32
 
 
 def _stream() -> C.c_void_p:
@@ -32,15 +33,17 @@ def make_operand(t: torch.Tensor, cols: int, rows: int, batch: int = 1, *, row_s
                  batch_stride: Optional[int] = None, nq: int = 1, q_stride: Optional[int] = None,
                  seg_width: int = 0, seg_q: Sequence[int] = (), seg_p: Sequence[int] = (),
                  offset: int = 0) -> Operand:
-    """4-D strided bf16 view (see wj_operand_t).  Strides are in ELEMENTS here."""
-    assert t.dtype == torch.bfloat16
+    """4-D strided view (see wj_operand_t) of a bf16 tensor (wj_gemm_bf16) or an fp32 one (wj_gemm_tf32).  Strides are
+    in ELEMENTS here."""
+    assert t.dtype in (torch.bfloat16, torch.float32)
+    esz = t.element_size()
     op = Operand()
-    op.ptr = _ptr(t) + offset * 2
+    op.ptr = _ptr(t) + offset * esz
     row_stride = cols if row_stride is None else row_stride
     q_stride = row_stride if q_stride is None else q_stride
     batch_stride = rows * row_stride if batch_stride is None else batch_stride
     op.dim[0], op.dim[1], op.dim[2], op.dim[3] = cols, nq, rows, batch
-    op.stride_bytes[0], op.stride_bytes[1], op.stride_bytes[2] = q_stride * 2, row_stride * 2, max(batch_stride, 8) * 2
+    op.stride_bytes[0], op.stride_bytes[1], op.stride_bytes[2] = q_stride * esz, row_stride * esz, max(batch_stride, 8) * esz
     op.seg_width = seg_width
     for i, v in enumerate(seg_q):
         op.seg_q[i] = v
@@ -105,6 +108,37 @@ def gemm(a: Operand, w: torch.Tensor, L: int, batch: int, out: torch.Tensor, *, 
                                 (L * batch * N * 2 if aux is not None else 0))
     check(lib.wj_gemm_bf16(C.byref(a), C.c_void_p(_ptr(w)), C.c_int64(w.stride(0)), L, batch, N, K, C.byref(e),
                            block_n, _stream()))
+
+
+def gemm_tf32(a: Operand, w: torch.Tensor, L: int, batch: int, out: torch.Tensor, *, bias: Optional[torch.Tensor] = None,
+              act: int = ACT_NONE, resid: Optional[torch.Tensor] = None, resid_mod: int = 0,
+              round_out: bool = False) -> None:
+    """out[b*L+t, :] = epilogue(A(t,b) @ w.T) on the tf32 tensor cores: A over an fp32 tensor, w fp32 [N, K], both
+    already rounded to nearest tf32.  act: ACT_NONE or ACT_GELU_ERF; out bf16 or fp32 (round_out: rounded to nearest
+    tf32, for an output that is the next GEMM's operand)."""
+    assert w.dtype == torch.float32 and w.dim() == 2 and w.stride(-1) == 1
+    assert out.dtype in (torch.float32, torch.bfloat16) and out.stride(-1) == 1
+    N, K = w.shape
+    e = Epilogue()
+    e.out = _ptr(out)
+    e.ld_out = out.stride(-2)
+    e.out_f32 = 1 if out.dtype == torch.float32 else 0
+    if bias is not None:
+        assert bias.dtype == torch.float32
+        e.bias = _ptr(bias)
+    if resid is not None:
+        assert resid.dtype == torch.float32 and resid.stride(-1) == 1
+        e.resid = _ptr(resid)
+        e.resid_f32 = 1
+        e.ld_resid = resid.stride(-2)
+        e.resid_mod = resid_mod
+    e.act = act
+    lib = _lib.load()
+    if _lib._profile is not None:
+        _lib._profile.meta = (2.0 * L * batch * N * K, L * batch, N, K, e.act, int(e.out_f32))
+        _lib._profile.nbytes = L * batch * K * 4 + N * K * 4 + L * batch * N * out.element_size()
+    check(lib.wj_gemm_tf32(C.byref(a), C.c_void_p(_ptr(w)), C.c_int64(w.stride(0)), L, batch, N, K, C.byref(e),
+                           1 if round_out else 0, _stream()))
 
 
 def gemm_wgrad(dy: Operand, x: Operand, L: int, batch: int, out: torch.Tensor, *, M: Optional[int] = None,
@@ -303,6 +337,24 @@ def conv0_fwd(x: torch.Tensor, w: torch.Tensor, gamma: torch.Tensor, beta: torch
                                    None, _stream()))
 
 
+def conv0_fwd_f32(x: torch.Tensor, w: torch.Tensor, gamma: torch.Tensor, beta: torch.Tensor, out: torch.Tensor,
+                  moments: torch.Tensor, stats: torch.Tensor, k: int = 10, stride: int = 5, eps: float = 1e-5) -> None:
+    """conv0_fwd of the TF32 inference path: x fp32 [B, Cin, L], unrounded fp32 weights, exact GELU -> out fp32
+    [B, L_out, C] rounded to nearest tf32."""
+    B, Cin, L = x.shape
+    assert x.dtype == torch.float32 and x.is_contiguous() and w.dtype == torch.float32
+    assert out.dtype == torch.float32 and out.is_contiguous()
+    assert moments.dtype == torch.float64 and stats.dtype == torch.float32
+    lib = _lib.load()
+    if _lib._profile is not None:
+        L_out = (L - k) // stride + 1
+        _lib._profile.nbytes = B * (Cin * L * 4 + L_out * w.shape[0] * 4)
+    check(lib.wj_conv0_gn_gelu_fwd_f32(C.c_void_p(_ptr(x)), C.c_void_p(_ptr(w)), C.c_void_p(_ptr(gamma)),
+                                       C.c_void_p(_ptr(beta)), B, Cin, L, w.shape[0], k, stride, C.c_float(eps),
+                                       C.c_void_p(_ptr(moments)), C.c_void_p(_ptr(stats)), C.c_void_p(_ptr(out)),
+                                       _stream()))
+
+
 def conv0_bwd(x, w, gamma, beta, moments, stats, dy, red_scratch, dw, dgamma, dbeta, k: int = 10, stride: int = 5,
               eps: float = 1e-5) -> None:
     """Backward of conv0_fwd from dy (bf16 [B, L_out, C]); GELU' is recomputed from x, nothing else is read."""
@@ -357,6 +409,32 @@ def add_layernorm_fwd(x: torch.Tensor, add: Optional[torch.Tensor], gamma, beta,
         _lib._profile.nbytes = M * D * (4 + 2 * (add is not None) + 4 * (out_f32 is not None) + 2 * (out_bf16 is not None))
     check(lib.wj_add_layernorm_fwd(p(x), p(add), p(gamma), p(beta), C.c_float(eps), M, D, p(out_f32), p(out_bf16),
                                    p(stats), p(rowsum), _stream()))
+
+
+def add_layernorm_fwd_f32(x: torch.Tensor, add: Optional[torch.Tensor], gamma, beta, eps: float, out_f32=None,
+                          out_tf32=None):
+    """LayerNorm(x + add) of the TF32 inference path: x and add fp32 (add may be None); out_f32 unrounded, out_tf32 the
+    same values rounded to nearest tf32 (the next GEMM's operand)."""
+    M, D = x.shape
+    assert x.dtype == torch.float32 and x.is_contiguous()
+    assert add is None or (add.dtype == torch.float32 and add.is_contiguous() and add.shape == x.shape)
+    for o in (out_f32, out_tf32):
+        assert o is None or (o.dtype == torch.float32 and o.is_contiguous() and o.shape == x.shape)
+    lib = _lib.load()
+    p = lambda t: C.c_void_p(_ptr(t))
+    if _lib._profile is not None:
+        _lib._profile.nbytes = M * D * (4 + 4 * (add is not None) + 4 * (out_f32 is not None) + 4 * (out_tf32 is not None))
+    check(lib.wj_add_layernorm_fwd_f32(p(x), p(add), p(gamma), p(beta), C.c_float(eps), M, D, p(out_f32), p(out_tf32),
+                                       _stream()))
+
+
+def tf32_round(x: torch.Tensor, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """x (fp32) rounded to nearest tf32 (into `out`, which may be x)."""
+    assert x.dtype == torch.float32 and x.is_contiguous()
+    out = torch.empty_like(x) if out is None else out
+    assert out.dtype == torch.float32 and out.is_contiguous() and out.numel() == x.numel()
+    check(_lib.load().wj_tf32_round(C.c_void_p(_ptr(x)), C.c_void_p(_ptr(out)), C.c_int64(x.numel()), _stream()))
+    return out
 
 
 def add_layernorm_bwd(dy_f32: Optional[torch.Tensor], dy_bf16: Optional[torch.Tensor], x: torch.Tensor,
@@ -447,6 +525,17 @@ def attn_fwd(qkv: torch.Tensor, cu: torch.Tensor, n_seqs: int, max_len: int, D: 
     if _lib._profile is not None:
         _lib._profile.meta = (0.0, n_seqs, max_len, D, H, qkv.shape[0])
     check(lib.wj_attn_varlen_fwd(p(qkv), p(cu), n_seqs, max_len, C.c_int64(qkv.shape[0]), D, H, p(out), p(lse2), _stream()))
+
+
+def attn_fwd_f32(qkv: torch.Tensor, cu: torch.Tensor, n_seqs: int, max_len: int, D: int, H: int, out: torch.Tensor):
+    """attn_fwd with O written as fp32 rounded to nearest tf32 (head dim 64, <= 512 tokens)."""
+    assert out.dtype == torch.float32 and out.is_contiguous()
+    lib = _lib.load()
+    p = lambda t: C.c_void_p(_ptr(t))
+    if _lib._profile is not None:
+        _lib._profile.meta = (0.0, n_seqs, max_len, D, H, qkv.shape[0])
+    check(lib.wj_attn_varlen_fwd_f32out(p(qkv), p(cu), n_seqs, max_len, C.c_int64(qkv.shape[0]), D, H, p(out),
+                                        _stream()))
 
 
 def attn_bwd(qkv, out, dout, lse2, cu, n_seqs: int, max_len: int, D: int, H: int, dqkv, dbias=None):
