@@ -242,6 +242,14 @@ int wj_attn_varlen_bwd_bias(const void* qkv_bf16, const void* out_bf16, const vo
                             const int* cu_seqlens, int n_seqs, int max_len, int64_t total_tokens, int D, int H,
                             void* dqkv_bf16, float* dbias, void* stream);
 
+/* wj_attn_varlen_bwd_bias that also takes head-dim-64 sequences of 385..400 tokens (the dense binaural WavJEPA-Nat
+ * student of 2 x 200 tokens, fine-tuned through get_audio_representation): the per-query lse / delta then live in the
+ * padding columns of the shared-memory Q rows, so the four 400-row tiles stay resident.  Shorter sequences take exactly
+ * wj_attn_varlen_bwd_bias's kernels. */
+int wj_attn_varlen_bwd_bias_long(const void* qkv_bf16, const void* out_bf16, const void* dout_bf16, const float* lse2,
+                                 const int* cu_seqlens, int n_seqs, int max_len, int64_t total_tokens, int D, int H,
+                                 void* dqkv_bf16, float* dbias, void* stream);
+
 /* Row gather: out[i, :] = src[idx[i], :] (idx NULL = identity, i.e. a cast); fp32 and/or bf16 outputs.
  * contextual_features[~ctx_masks] (wavjepa/jepa.py:399). */
 int wj_gather_rows(const void* src, int src_is_bf16, const int* idx, int N, int D, float* out_f32, void* out_bf16,

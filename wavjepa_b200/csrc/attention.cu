@@ -204,7 +204,10 @@ __global__ void __launch_bounds__(256) attn_fwd_kernel(const bf16* __restrict__ 
 // ------------------------------------------------------------------------------------------------ backward
 // One CTA per (sequence, head); Q, K, V, dO of the whole sequence live in smem (NPAD rows each).
 //   phase A: warps own 16-query blocks -> dQ;  phase B: warps own 16-key blocks -> dK, dV.  No atomics.
-template <int DH>
+// ROWSTATS: the per-query lse / delta live in the padding columns of the Q rows (floats at column DH, DH + 2) instead of
+// two arrays after dO -- 3.5 KB less shared memory, which lets sequences of up to 400 tokens at head dim 64 (the dense
+// WavJEPA-Nat student: two channels x 200 tokens) stay resident; rows past the Q block read as zeros.
+template <int DH, bool ROWSTATS = false>
 __global__ void __launch_bounds__(128, (DH == 32 ? 4 : 3)) attn_bwd_kernel(const bf16* __restrict__ qkv, const bf16* __restrict__ out,
                                                        const bf16* __restrict__ dout, const float* __restrict__ lse2,
                                                        const int* __restrict__ cu, int D, int H, int NPAD, float scale,
@@ -219,6 +222,10 @@ __global__ void __launch_bounds__(128, (DH == 32 ? 4 : 3)) attn_bwd_kernel(const
   bf16* sdO = sV + NPAD * PITCH;
   float* sLse = reinterpret_cast<float*>(sdO + NPAD * PITCH);
   float* sDl = sLse + ((NPAD + 63) & ~63);   // lse / delta rows are read in 64-query blocks: padded (zeros) to 64
+  auto stat = [&](const float* arr, int i, int which) -> float {
+    if constexpr (ROWSTATS) return i < NPAD ? reinterpret_cast<const float*>(sQ + i * PITCH + DH)[which] : 0.f;
+    else return arr[i];
+  };
   const int s = blockIdx.y, h = blockIdx.x;
   const int start = cu[s], n = cu[s + 1] - start;
   if (n <= 0) return;
@@ -250,8 +257,16 @@ __global__ void __launch_bounds__(128, (DH == 32 ? 4 : 3)) attn_bwd_kernel(const
       }
       l = lse2[static_cast<long long>(start + i) * H + h];
     }
-    sLse[i] = l;
-    sDl[i] = dsum;
+    if constexpr (ROWSTATS) {
+      if (i < NPAD) {
+        float* rp = reinterpret_cast<float*>(sQ + i * PITCH + DH);
+        rp[0] = l;
+        rp[1] = dsum;
+      }
+    } else {
+      sLse[i] = l;
+      sDl[i] = dsum;
+    }
   }
   cp_async_wait_all();
   __syncthreads();
@@ -261,8 +276,8 @@ __global__ void __launch_bounds__(128, (DH == 32 ? 4 : 3)) attn_bwd_kernel(const
     uint32_t qf[DH / 16][4], dof[DH / 16][4];
     load_a_frags<DH>(qf, sQ, rb * 16, g, tg);
     load_a_frags<DH>(dof, sdO, rb * 16, g, tg);
-    const float la = sLse[rb * 16 + g], lb = sLse[rb * 16 + g + 8];
-    const float da = sDl[rb * 16 + g], db = sDl[rb * 16 + g + 8];
+    const float la = stat(sLse, rb * 16 + g, 0), lb = stat(sLse, rb * 16 + g + 8, 0);
+    const float da = stat(sDl, rb * 16 + g, 1), db = stat(sDl, rb * 16 + g + 8, 1);
     float dq[DH / 8][4];
 #pragma unroll
     for (int i = 0; i < DH / 8; ++i) dq[i][0] = dq[i][1] = dq[i][2] = dq[i][3] = 0.f;
@@ -316,7 +331,7 @@ __global__ void __launch_bounds__(128, (DH == 32 ? 4 : 3)) attn_bwd_kernel(const
 #pragma unroll
       for (int nt = 0; nt < NT; ++nt) {
         const int q = qb * KB + nt * 8 + 2 * tg;
-        const float l0 = sLse[q], l1 = sLse[q + 1], d0 = sDl[q], d1 = sDl[q + 1];
+        const float l0 = stat(sLse, q, 0), l1 = stat(sLse, q + 1, 0), d0 = stat(sDl, q, 1), d1 = stat(sDl, q + 1, 1);
         const bool q0 = q < n, q1 = q + 1 < n;
         const float p0 = (ka && q0) ? ex2_approx(st[nt][0] * scale_log2 - l0) : 0.f;
         const float p1 = (ka && q1) ? ex2_approx(st[nt][1] * scale_log2 - l1) : 0.f;
@@ -418,9 +433,9 @@ extern "C" int wj_attn_varlen_bwd(const void* qkv_bf16, const void* out_bf16, co
                                  dqkv_bf16, nullptr, stream);
 }
 
-extern "C" int wj_attn_varlen_bwd_bias(const void* qkv_bf16, const void* out_bf16, const void* dout_bf16,
-                                       const float* lse2, const int* cu_seqlens, int n_seqs, int max_len,
-                                       int64_t total_tokens, int D, int H, void* dqkv_bf16, float* dbias, void* stream) {
+static int attn_bwd_bias(const void* qkv_bf16, const void* out_bf16, const void* dout_bf16, const float* lse2,
+                         const int* cu_seqlens, int n_seqs, int max_len, int64_t total_tokens, int D, int H,
+                         void* dqkv_bf16, float* dbias, void* stream, bool allow_rowstats) {
   if (n_seqs <= 0 || max_len <= 0) return WJ_OK;
   const int dh = D / H;
   if (D % H != 0 || (dh != 32 && dh != 64)) { set_error("wj_attn_varlen_bwd: head dim must be 32 or 64"); return WJ_ERR_ARG; }
@@ -444,7 +459,9 @@ extern "C" int wj_attn_varlen_bwd_bias(const void* qkv_bf16, const void* out_bf1
     }
   }
   const int npad = (max_len + 15) & ~15;
-  const size_t smem = static_cast<size_t>(4) * npad * (dh + 8) * 2 + static_cast<size_t>(2) * ((npad + 63) & ~63) * 4;
+  size_t smem = static_cast<size_t>(4) * npad * (dh + 8) * 2 + static_cast<size_t>(2) * ((npad + 63) & ~63) * 4;
+  const bool rowstats = allow_rowstats && dh == 64 && smem > 227 * 1024;   // lse / delta in the Q rows' padding
+  if (rowstats) smem = static_cast<size_t>(4) * npad * (dh + 8) * 2;
   if (smem > 227 * 1024) { set_error("wj_attn_varlen_bwd: sequence of %d tokens (head dim %d) exceeds the shared-memory resident design", max_len, dh); return WJ_ERR_ARG; }
   const float scale = 1.0f / sqrtf(static_cast<float>(dh));
   const float scale_log2 = scale * 1.4426950408889634f;
@@ -454,7 +471,11 @@ extern "C" int wj_attn_varlen_bwd_bias(const void* qkv_bf16, const void* out_bf1
   const bf16* d_o = reinterpret_cast<const bf16*>(dout_bf16);
   bf16* dq = reinterpret_cast<bf16*>(dqkv_bf16);
   cudaError_t e;
-  if (dh == 64) {
+  if (rowstats) {
+    e = cudaFuncSetAttribute(attn_bwd_kernel<64, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem));
+    if (e != cudaSuccess) { set_error("attn_bwd attr: %s", cudaGetErrorString(e)); return WJ_ERR_RUNTIME; }
+    attn_bwd_kernel<64, true><<<grid, 128, smem, WJ_STREAM(stream)>>>(q, o, d_o, lse2, cu_seqlens, D, H, npad, scale, scale_log2, dq);
+  } else if (dh == 64) {
     e = cudaFuncSetAttribute(attn_bwd_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem));
     if (e != cudaSuccess) { set_error("attn_bwd attr: %s", cudaGetErrorString(e)); return WJ_ERR_RUNTIME; }
     attn_bwd_kernel<64><<<grid, 128, smem, WJ_STREAM(stream)>>>(q, o, d_o, lse2, cu_seqlens, D, H, npad, scale, scale_log2, dq);
@@ -466,4 +487,21 @@ extern "C" int wj_attn_varlen_bwd_bias(const void* qkv_bf16, const void* out_bf1
   const int rc = check_launch("attn_varlen_bwd");
   if (rc != WJ_OK || dbias == nullptr) return rc;
   return wj_colsum(dqkv_bf16, 1, total_tokens, 3 * D, 3 * D, dbias, stream);
+}
+
+extern "C" int wj_attn_varlen_bwd_bias(const void* qkv_bf16, const void* out_bf16, const void* dout_bf16,
+                                       const float* lse2, const int* cu_seqlens, int n_seqs, int max_len,
+                                       int64_t total_tokens, int D, int H, void* dqkv_bf16, float* dbias, void* stream) {
+  return attn_bwd_bias(qkv_bf16, out_bf16, dout_bf16, lse2, cu_seqlens, n_seqs, max_len, total_tokens, D, H, dqkv_bf16,
+                       dbias, stream, false);
+}
+
+// The same backward for head-dim-64 sequences of up to 400 tokens (the dense two-channel WavJEPA-Nat student): past 384
+// tokens the per-query lse / delta move into the padding columns of the shared-memory Q rows (attn_bwd_kernel<64, true>).
+extern "C" int wj_attn_varlen_bwd_bias_long(const void* qkv_bf16, const void* out_bf16, const void* dout_bf16,
+                                            const float* lse2, const int* cu_seqlens, int n_seqs, int max_len,
+                                            int64_t total_tokens, int D, int H, void* dqkv_bf16, float* dbias,
+                                            void* stream) {
+  return attn_bwd_bias(qkv_bf16, out_bf16, dout_bf16, lse2, cu_seqlens, n_seqs, max_len, total_tokens, D, H, dqkv_bf16,
+                       dbias, stream, true);
 }

@@ -48,10 +48,12 @@ class TransformerStack:
 
     # ------------------------------------------------------------------------------------------------ forward
     def forward(self, layers: List[LayerW], x32: torch.Tensor, x16: torch.Tensor, cu: torch.Tensor, n_seqs: int,
-                max_len: int, save: bool, layer_hook: Optional[Callable] = None, rowsum_from: int = 1 << 30):
+                max_len: int, save: bool, layer_hook: Optional[Callable] = None, rowsum_from: int = 1 << 30,
+                save_from: int = 0):
         """x32/x16: [M, d] fp32 residual stream and its bf16 copy.  Returns (x32, x16, saved list).
         layer_hook(i, x32, rowsum) is called after layer i (teacher target accumulation); rowsum is produced for
-        layers i >= rowsum_from.
+        layers i >= rowsum_from.  With `save`, layers i >= save_from keep what the backward needs and the saved list
+        holds None for the layers below (a frozen prefix that `backward(stop_at=save_from)` never reaches).
 
         Every Linear writes its output as bf16 (what autocast makes it) through the TMA-store epilogue; the fp32
         residual sum y = x + bf16(Linear) is formed inside the LayerNorm kernel and never stored: the backward
@@ -61,7 +63,11 @@ class TransformerStack:
         dev = x32.device
         bf, f32 = torch.bfloat16, torch.float32
         saved = []
+        keep_all = save
         for i, w in enumerate(layers):
+            save = keep_all and i >= save_from
+            if keep_all and not save:
+                saved.append(None)
             qkv = _empty((M, 3 * d), bf, dev)
             ops.gemm(ops.plain_operand(x16), w.w_in, M, 1, qkv, bias=w.b_in)
             att = _empty((M, d), bf, dev)
@@ -131,18 +137,22 @@ class TransformerStack:
 
     # ------------------------------------------------------------------------------------------------ backward
     def backward(self, layers: List[LayerW], grads: List[LayerG], saved: List[LayerSaved], dx: torch.Tensor,
-                 cu: torch.Tensor, n_seqs: int, max_len: int, on_layer_done: Optional[Callable] = None):
+                 cu: torch.Tensor, n_seqs: int, max_len: int, on_layer_done: Optional[Callable] = None,
+                 stop_at: int = 0, need_dx: bool = True):
         """dx: fp32 [M, d] gradient w.r.t. the stack output (before any final norm).  Accumulates parameter
         gradients into `grads` (pre-zeroed) and returns the gradient w.r.t. the stack input (fp32).
 
         Between layers the gradient travels as a pair (fp32 residual branch, bf16 Linear data gradient -- bf16 is
-        what autocast's Linear backward returns); the pair is summed inside the next LayerNorm backward."""
+        what autocast's Linear backward returns); the pair is summed inside the next LayerNorm backward.
+
+        Layers below `stop_at` are not visited.  need_dx=False: nothing below the lowest visited layer wants its input
+        gradient, so its last data-gradient GEMM is skipped and None is returned."""
         d, H, ff = self.d, self.H, self.ff
         M = dx.shape[0]
         dev = dx.device
         bf, f32 = torch.bfloat16, torch.float32
         dx_b = None   # bf16 half of the gradient w.r.t. the current layer's output
-        for i in range(len(layers) - 1, -1, -1):
+        for i in range(len(layers) - 1, stop_at - 1, -1):
             w, gw, s = layers[i], grads[i], saved[i]
             # ---- LN2 and the MLP
             dy2 = _empty((M, d), f32, dev)
@@ -165,14 +175,20 @@ class TransformerStack:
             datt = _empty((M, d), bf, dev)
             ops.gemm_dgrad(ops.plain_operand(dy1_16), w.w_o, M, 1, datt, K=d, N=d)
             dqkv = _empty((M, 3 * d), bf, dev)
-            ops.attn_bwd(s.qkv, s.att, datt, s.lse, cu, n_seqs, max_len, d, H, dqkv, dbias=gw.b_in)
+            ops.attn_bwd(s.qkv, s.att, datt, s.lse, cu, n_seqs, max_len, d, H, dqkv, dbias=gw.b_in, long_seq=True)
             ops.gemm_wgrad(ops.plain_operand(dqkv), ops.plain_operand(s.x16), M, 1, gw.w_in, accumulate=True)
-            dx_b = _empty((M, d), bf, dev)
-            ops.gemm_dgrad(ops.plain_operand(dqkv), w.w_in, M, 1, dx_b, K=3 * d, N=d)
             dx = dy1
             saved[i] = None
+            if i == stop_at and not need_dx:
+                if on_layer_done is not None:
+                    on_layer_done(i)
+                return None
+            dx_b = _empty((M, d), bf, dev)
+            ops.gemm_dgrad(ops.plain_operand(dqkv), w.w_in, M, 1, dx_b, K=3 * d, N=d)
             if on_layer_done is not None:
                 on_layer_done(i)
+        if not need_dx:
+            return None
         if dx_b is not None:
             ops.add_bf16(dx, dx_b)
         return dx

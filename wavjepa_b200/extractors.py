@@ -123,9 +123,7 @@ def conv_stack_forward(spec, x16: torch.Tensor, w0: torch.Tensor, gn_w: torch.Te
         if L_in % 2 == 0:
             a_op = ops.conv_operand(x, k)
         else:
-            if save:
-                raise WavJepaLibError("training needs even conv input lengths (odd lengths are inference-only)")
-            a_op = ops.make_operand(x, k * C, L_out, B, row_stride=2 * C, batch_stride=L_in * C)
+            a_op = ops.conv_operand_odd(x, k)
         ops.gemm(a_op, wks[i - 1], L_out, B, g.view(-1, C), act=ops.ACT_GELU,
                  out2=h.view(-1, C) if save else None)
         if not save:
@@ -162,7 +160,7 @@ def conv_stack_forward_tf32(spec, x32: torch.Tensor, w0: torch.Tensor, gn_w: tor
         if L_in % 2 == 0:
             a_op = ops.conv_operand(x, k)
         else:
-            a_op = ops.make_operand(x, k * C, L_out, B, row_stride=2 * C, batch_stride=L_in * C)
+            a_op = ops.conv_operand_odd(x, k)
         ops.gemm_tf32(a_op, wks[i - 1], L_out, B, g.view(-1, C), act=ops.ACT_GELU_ERF, round_out=i < n - 1)
         x = g
     return x
@@ -171,7 +169,11 @@ def conv_stack_forward_tf32(spec, x32: torch.Tensor, w0: torch.Tensor, gn_w: tor
 def conv_stack_backward(spec, sv: ConvSaved, dh_last: torch.Tensor, w0, gn_w, gn_b, wks, g_w0, g_gn_w, g_gn_b,
                         g_ws: List[torch.Tensor], gn_eps: float = 1e-5, on_layer_done=None) -> None:
     """dh_last: bf16 [B, T, C] gradient w.r.t. the PRE-activation of the last conv block.  Accumulates into the fp32
-    gradient tensors g_* (shapes of the parameters)."""
+    gradient tensors g_* (shapes of the parameters).
+
+    Odd input lengths (the wav2vec2 extractor's 401-row input of its last block): the weight gradient reads the
+    activations through the forward's strided view (k*C columns per output row, batch pitch L_in*C), and conv_dgrad
+    writes dx with that batch pitch; the trailing input row of a k = 2 block feeds no output and gets a zero gradient."""
     n = len(spec)
     B = dh_last.shape[0]
     C = spec[0][0]
@@ -183,7 +185,8 @@ def conv_stack_backward(spec, sv: ConvSaved, dh_last: torch.Tensor, w0, gn_w, gn
         L_in = x.shape[1]
         L_out = dh.shape[1]
         dwk = torch.empty(C, k * C, device=dev, dtype=torch.float32)
-        ops.gemm_wgrad(ops.make_operand(dh, C, L_out, B), ops.conv_operand(x, k), L_out, B, dwk)
+        x_op = ops.conv_operand(x, k) if L_in % 2 == 0 else ops.conv_operand_odd(x, k)
+        ops.gemm_wgrad(ops.make_operand(dh, C, L_out, B), x_op, L_out, B, dwk)
         g_ws[i - 1].add_(dwk.view(C, k, C).permute(0, 2, 1))
         dx = torch.empty(B, L_in, C, device=dev, dtype=torch.bfloat16)
         if i - 1 >= 1:

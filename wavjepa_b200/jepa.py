@@ -128,6 +128,43 @@ class _LossBridge(torch.autograd.Function):
         return (None, None, *grads)
 
 
+# parameters that `get_audio_representation` reads: the leading span of the flat layout (see JEPA._layout_names)
+_FEATURE_PATH = ("extract_audio.", "feature_norms.", "post_extraction_mapper.", "encoder.")
+
+
+class _FeaturePlan:
+    """Which parts of the feature path train in one differentiable `get_audio_representation` call."""
+    __slots__ = ("names", "conv", "norm", "local", "first_layer")
+
+
+class _FeatureBridge(torch.autograd.Function):
+    """Makes the features of `get_audio_representation` differentiable: the forward runs the saving kernels, the
+    backward runs the hand-written chain (final LayerNorm -> encoder layers -> mapper / feature norm / conv stack) into a
+    gradient buffer owned by this call and hands autograd the gradients of the parameters it asks for.  `audio` is not
+    an input: no gradient reaches the waveform."""
+
+    @staticmethod
+    def forward(ctx, model, inputs, plan, *params):
+        x16, index = inputs   # (a tuple: the waveform is not an input autograd tracks)
+        ctx.model = model
+        ctx.fctx = model._features_saving(x16, index, plan)
+        out, ctx.fctx.out = ctx.fctx.out, None
+        return out
+
+    @staticmethod
+    def backward(ctx, grad_out):
+        c = ctx.fctx
+        if c is None:
+            raise RuntimeError("get_audio_representation: this graph was already backpropagated and its saved "
+                               "activations are freed; run the forward again (retain_graph is not supported)")
+        ctx.fctx = None
+        model = ctx.model
+        gflat = model._features_backward(c, grad_out)
+        needs = ctx.needs_input_grad[3:]
+        grads = [model._view(gflat, n) if needs[i] else None for i, n in enumerate(c.plan.names)]
+        return (None, None, None, *grads)
+
+
 # =================================================================================================== model
 class JEPA(_ModuleBase):
     """A `pytorch_lightning.LightningModule` when Lightning is installed (drop-in for `pl.Trainer.fit`, train.py:244),
@@ -211,7 +248,9 @@ class JEPA(_ModuleBase):
         """Numerics of `get_audio_representation`: "bf16" (the default) runs the encoder with bf16 operands and the
         packed-fp16 tanh-form GELU, ~1e-2 relative L2 from the reference's fp32 features; "tf32" runs the reference's fp32
         feature extraction with every GEMM operand rounded to nearest tf32, fp32 accumulation and the exact erf GELU
-        (DESIGN.md 2.1).  `forward`, `train_step`, the teacher and the denoiser ignore it."""
+        (DESIGN.md 2.1).  `forward`, `train_step`, the teacher and the denoiser ignore it.  "tf32" is inference-only:
+        its features never carry a grad_fn; fine-tuning through `get_audio_representation` runs in "bf16" (DESIGN.md
+        2.2)."""
         return self.__dict__.get("_inference_precision", "bf16")
 
     @inference_precision.setter
@@ -419,30 +458,33 @@ class JEPA(_ModuleBase):
         if gflat is self._flat_g and self._gviews_cache is not None:
             return self._gviews_cache
         g = lambda n: self._view(gflat, n)
-
-        def stack(prefix, n_layers):
-            out = []
-            for i in range(n_layers):
-                b = f"{prefix}layers.{i}."
-                w = LayerG()
-                w.w_in, w.b_in = g(b + "self_attn.in_proj_weight"), g(b + "self_attn.in_proj_bias")
-                w.w_o, w.b_o = g(b + "self_attn.out_proj.weight"), g(b + "self_attn.out_proj.bias")
-                w.w1, w.b1 = g(b + "linear1.weight"), g(b + "linear1.bias")
-                w.w2, w.b2 = g(b + "linear2.weight"), g(b + "linear2.bias")
-                w.g1, w.be1 = g(b + "norm1.weight"), g(b + "norm1.bias")
-                w.g2, w.be2 = g(b + "norm2.weight"), g(b + "norm2.bias")
-                out.append(w)
-            return out
-
-        views = (stack("encoder.", self._enc_stack.n_layers), stack("decoder.", self._dec_stack.n_layers), g)
+        views = (self._stack_grads("encoder.", self._enc_stack.n_layers, g),
+                 self._stack_grads("decoder.", self._dec_stack.n_layers, g), g)
         if gflat is self._flat_g:
             self._gviews_cache = views
         return views
 
+    @staticmethod
+    def _stack_grads(prefix: str, n_layers: int, g: Callable) -> List[LayerG]:
+        out = []
+        for i in range(n_layers):
+            b = f"{prefix}layers.{i}."
+            w = LayerG()
+            w.w_in, w.b_in = g(b + "self_attn.in_proj_weight"), g(b + "self_attn.in_proj_bias")
+            w.w_o, w.b_o = g(b + "self_attn.out_proj.weight"), g(b + "self_attn.out_proj.bias")
+            w.w1, w.b1 = g(b + "linear1.weight"), g(b + "linear1.bias")
+            w.w2, w.b2 = g(b + "linear2.weight"), g(b + "linear2.bias")
+            w.g1, w.be1 = g(b + "norm1.weight"), g(b + "norm1.bias")
+            w.g2, w.be2 = g(b + "norm2.weight"), g(b + "norm2.bias")
+            out.append(w)
+        return out
+
     # ------------------------------------------------------------------------------------------- local features
-    def _local_features(self, x16: torch.Tensor, save: bool):
+    def _local_features(self, x16: torch.Tensor, save: bool, save_conv: Optional[bool] = None):
         """Waveform encoder -> LayerNorm(512) -> Linear 512->D (+bias, bf16) -> + positional table (fp32).
-        reference wavjepa/jepa.py:391-396.  Returns (local32 [B*T, D], ctx pieces for the backward)."""
+        reference wavjepa/jepa.py:391-396.  Returns (local32 [B*T, D], ctx pieces for the backward).
+        save_conv=False (with save): a frozen extractor keeps no activations; only the feature norm saves its stats."""
+        save_conv = save if save_conv is None else (save and save_conv)
         ex = self.extract_audio
         B = x16.shape[0]
         T, D = self.total_patches, self.encoder_embedding_dim
@@ -457,14 +499,14 @@ class JEPA(_ModuleBase):
                 prefix = f"extract_audio.cnns.{0 if ex.share_weights_over_channels else c}"
                 wks = [self._conv_wk[f"{prefix}.{i}.0.weight"] for i in range(1, len(ex.conv_layers_spec))]
                 f, sv = conv_stack_forward(ex.conv_layers_spec, xs[c].unsqueeze(1), p32(f"{prefix}.0.0.weight"),
-                                           p32(f"{prefix}.0.2.weight"), p32(f"{prefix}.0.2.bias"), wks, save)
+                                           p32(f"{prefix}.0.2.weight"), p32(f"{prefix}.0.2.bias"), wks, save_conv)
                 feats[:, c * Tc:(c + 1) * Tc].copy_(f)  # channel-major token order (audio_channel_feature_extractor.py:177-178)
                 conv_saved.append(sv)
         else:
             prefix = "extract_audio.cnn"
             wks = [self._conv_wk[f"{prefix}.{i}.0.weight"] for i in range(1, len(ex.conv_layers_spec))]
             feats, sv = conv_stack_forward(ex.conv_layers_spec, x16, p32(f"{prefix}.0.0.weight"),
-                                           p32(f"{prefix}.0.2.weight"), p32(f"{prefix}.0.2.bias"), wks, save)
+                                           p32(f"{prefix}.0.2.weight"), p32(f"{prefix}.0.2.bias"), wks, save_conv)
             conv_saved.append(sv)
         f2 = feats.view(B * T, C)
         ln16 = torch.empty(B * T, C, device=x16.device, dtype=torch.bfloat16)
@@ -624,9 +666,11 @@ class JEPA(_ModuleBase):
         if on_ready is not None:
             on_ready(0)
 
-    def _local_backward(self, local_saved, dlocal16: torch.Tensor, B: int, g, ready) -> None:
+    def _local_backward(self, local_saved, dlocal16: torch.Tensor, B: int, g, ready, norm: bool = True,
+                        conv: bool = True) -> None:
         """Backward of `_local_features` from the (bf16) gradient of the mapper output on the dense token grid:
-        post_extraction_mapper -> feature_norms -> conv stack(s)."""
+        post_extraction_mapper -> feature_norms -> conv stack(s).  norm=False stops after the mapper, conv=False after
+        the feature norm (frozen parts below them: no data gradient flows there)."""
         T, D = self.total_patches, self.encoder_embedding_dim
         dev = dlocal16.device
         p32 = lambda n: self._view(self._flat_p, n)
@@ -637,12 +681,16 @@ class JEPA(_ModuleBase):
         ops.gemm_wgrad(ops.plain_operand(dlocal16), ops.plain_operand(ln16), B * T, 1,
                        g("post_extraction_mapper.weight"), accumulate=True)
         ready("post_extraction_mapper.weight")
+        if not (norm or conv):
+            return
         dln = torch.empty(B * T, C, device=dev)
         ops.gemm_dgrad(ops.plain_operand(dlocal16), p16("post_extraction_mapper.weight"), B * T, 1, dln, K=D, N=C)
         dfeat = torch.empty(B * T, C, device=dev)
         ops.layernorm_bwd(dln, f2, st, p32("feature_norms.weight"), dfeat, None, g("feature_norms.weight"),
                           g("feature_norms.bias"), None)
         ready("feature_norms.weight")
+        if not conv:
+            return
         # ---- conv stack(s)
         ex = self.extract_audio
         exs = self._extractors()
@@ -983,13 +1031,127 @@ class JEPA(_ModuleBase):
         ops.scatter_rows(packed, ctx_rows, Nc, out)
         return out.view(B, T, D)
 
+    # ------------------------------------------------------------------------------------------- fine-tuning
+    def _feature_grad_plan(self) -> Optional[_FeaturePlan]:
+        """None unless grad mode is on and a feature-path parameter requires grad (the rule of `forward`)."""
+        if not torch.is_grad_enabled():
+            return None
+        params = dict(self.named_parameters())
+        names = [n for n in self._train_names if n.startswith(_FEATURE_PATH)]
+        trainable = [n for n in names if params[n].requires_grad]
+        if not trainable:
+            return None
+        plan = _FeaturePlan()
+        plan.names = names
+        plan.conv = any(n.startswith("extract_audio.") for n in trainable)
+        plan.norm = any(n.startswith("feature_norms.") for n in trainable)
+        plan.local = plan.conv or plan.norm or any(n.startswith("post_extraction_mapper.") for n in trainable)
+        n_layers = self._enc_stack.n_layers
+        layers = [int(n.split(".")[2]) for n in trainable if n.startswith("encoder.layers.")]
+        plan.first_layer = 0 if plan.local else min(layers, default=n_layers)
+        return plan
+
+    def _audio_representation_grad(self, x16, padding_mask, host_mask, plan: _FeaturePlan) -> torch.Tensor:
+        """Differentiable get_audio_representation (same masking semantics and checks as the inference path)."""
+        B, T = x16.shape[0], self.total_patches
+        index = None
+        if host_mask is not None:
+            index = self._periodic_index(host_mask, B, T)
+        elif padding_mask is not None:
+            pm = padding_mask.to(self.device).reshape(B, 1, T).contiguous()
+            mi = ops.mask_indices(pm.view(B, T), torch.zeros_like(pm), pm)
+            index = (mi.ctx_rows, mi.cu_c, mi.Nc, mi.max_nc)
+        params = dict(self.named_parameters())
+        return _FeatureBridge.apply(self, (x16, index), plan, *[params[n] for n in plan.names])
+
+    def _features_saving(self, x16: torch.Tensor, index, plan: _FeaturePlan) -> _Ctx:
+        """Forward of `_FeatureBridge`: the inference kernels plus the activations the backward needs, kept from the
+        lowest trainable point upward.  index: None (dense) or (ctx_rows, cu, Nc, max_len) of the visible rows."""
+        dev = x16.device
+        B = x16.shape[0]
+        T, D = self.total_patches, self.encoder_embedding_dim
+        p32 = lambda n: self._view(self._flat_p, n)
+        c = _Ctx()
+        c.B, c.index, c.plan = B, index, plan
+        local32, local_saved = self._local_features(x16, save=plan.local, save_conv=plan.conv)
+        c.local_saved = local_saved if plan.local else None
+        if index is None:
+            M = B * T
+            c.cu, c.max_len = torch.arange(0, (B + 1) * T, T, device=dev, dtype=torch.int32), T
+            x16r = torch.empty(M, D, device=dev, dtype=torch.bfloat16)
+            ops.gather_rows(local32, None, M, None, x16r)
+            xs32, _, c.enc_saved = self._enc_stack.forward(self._W_enc, local32, x16r, c.cu, B, T, True,
+                                                           save_from=plan.first_layer)
+        else:
+            ctx_rows, c.cu, M, c.max_len = index
+            xc32 = torch.empty(M, D, device=dev)
+            xc16 = torch.empty(M, D, device=dev, dtype=torch.bfloat16)
+            ops.gather_rows(local32, ctx_rows, M, xc32, xc16)
+            xs32, _, c.enc_saved = self._enc_stack.forward(self._W_enc, xc32, xc16, c.cu, B, c.max_len, True,
+                                                           save_from=plan.first_layer)
+        del local32
+        c.out = torch.empty(B, T, D, device=dev) if index is None else torch.zeros(B, T, D, device=dev)
+        packed = c.out.view(B * T, D) if index is None else torch.empty(M, D, device=dev)
+        c.norm_st = torch.empty(M, 2, device=dev)
+        ops.layernorm_fwd(xs32, p32("encoder.norm.weight"), p32("encoder.norm.bias"), self.encoder.norm.eps, packed,
+                          None, c.norm_st, None)
+        if index is not None:
+            ops.scatter_rows(packed, index[0], M, c.out.view(B * T, D))
+        c.xs32, c.M = xs32, M
+        return c
+
+    def _features_backward(self, c: _Ctx, grad_out: torch.Tensor) -> torch.Tensor:
+        """Backward of `_FeatureBridge` from the fp32 gradient of the features [B, T, D].  Returns a gradient buffer
+        over the extractor..encoder span of the flat layout (owned by this call: several graphs may be alive)."""
+        dev = c.xs32.device
+        B, M, plan = c.B, c.M, c.plan
+        T, D = self.total_patches, self.encoder_embedding_dim
+        n_layers = self._enc_stack.n_layers
+        p32 = lambda n: self._view(self._flat_p, n)
+        gflat = torch.zeros(self._enc_range[1], device=dev)
+        g = lambda n: self._view(gflat, n)
+        dy = grad_out.to(device=dev, dtype=torch.float32).contiguous().view(B * T, D)
+        if c.index is not None:   # padded rows are constants: only the visible rows' gradient enters
+            dyp = torch.empty(M, D, device=dev)
+            ops.gather_rows(dy, c.index[0], M, dyp, None)
+            dy = dyp
+        dxs = torch.empty(M, D, device=dev)
+        ops.layernorm_bwd(dy, c.xs32, c.norm_st, p32("encoder.norm.weight"), dxs, None, g("encoder.norm.weight"),
+                          g("encoder.norm.bias"), None)
+        c.xs32 = None
+        if plan.first_layer < n_layers:
+            dx = self._enc_stack.backward(self._W_enc, self._stack_grads("encoder.", n_layers, g), c.enc_saved, dxs,
+                                          c.cu, B, c.max_len, stop_at=plan.first_layer, need_dx=plan.local)
+            if plan.local:
+                # the mapper output is bf16 (autocast), so is its gradient on the dense token grid
+                if c.index is None:
+                    dlocal16 = torch.empty(B * T, D, device=dev, dtype=torch.bfloat16)
+                    ops.gather_rows(dx, None, M, None, dlocal16)
+                else:
+                    dlocal16 = torch.zeros(B * T, D, device=dev, dtype=torch.bfloat16)
+                    ops.scatter_dgelu(dx, c.index[0], None, M, dlocal16)
+                del dx
+                self._local_backward(c.local_saved, dlocal16, B, g, lambda name: None, norm=plan.norm or plan.conv,
+                                     conv=plan.conv)
+        c.enc_saved = c.local_saved = None
+        return gflat
+
     def get_audio_representation(self, audio: torch.Tensor, padding_mask: Optional[torch.Tensor] = None,
                                  host_mask=None) -> torch.Tensor:
         """reference wavjepa/jepa.py:456-467: student encoder (incl. final norm) features [B, T, D] fp32.  Tokens
         hidden by padding_mask (True) are excluded as keys exactly like the reference's key-padding mask; their own
         output rows (which the callers cut off, hear_api/runtime.py:141-142) are returned as zeros.
         host_mask (optional, CPU bool [P, T], P | B): the same padding mask given as a pattern known on the host that
-        repeats every P sequences -- the packed index then needs no device read-back (padding_mask is ignored)."""
+        repeats every P sequences -- the packed index then needs no device read-back (padding_mask is ignored).
+
+        Fine-tuning: in grad mode, when a parameter of the feature path (extract_audio, feature_norms,
+        post_extraction_mapper, encoder) requires grad, the features carry a grad_fn and `backward()` fills `.grad` of
+        the trainable path parameters (everything else keeps grad None).  The values are bit-identical to the no-grad
+        call.  Rows hidden by a padding mask stay constant zeros: gradient flows from the visible rows only (the
+        reference computes values at padded query positions, but no caller reads them).  Frozen parts save nothing and
+        are not backpropagated: a frozen extractor, or encoder layers below the lowest trainable one.  No gradient
+        reaches `audio`, and one graph supports one backward.  inference_precision "tf32" stays forward-only: fine-tuning
+        runs in the "bf16" training numerics (DESIGN.md 2.2)."""
         self.eval()
         self._ensure_ready()
         self._sync_weights()
@@ -999,6 +1161,9 @@ class JEPA(_ModuleBase):
         x16 = audio.to(device=dev, dtype=torch.bfloat16).contiguous()
         B = x16.shape[0]
         T, D = self.total_patches, self.encoder_embedding_dim
+        plan = self._feature_grad_plan()
+        if plan is not None:
+            return self._audio_representation_grad(x16, padding_mask, host_mask, plan)
         local32, _ = self._local_features(x16, save=False)
         p32 = lambda n: self._view(self._flat_p, n)
         if padding_mask is None and host_mask is None:

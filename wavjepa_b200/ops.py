@@ -234,21 +234,63 @@ def conv_operand(x: torch.Tensor, k: int) -> Operand:
                         seg_width=C, seg_q=(0, 1, 0)[:k], seg_p=(0, 0, 1)[:k])
 
 
+def conv_operand_odd(x: torch.Tensor, k: int) -> Operand:
+    """Implicit-GEMM view of channels-last activations x [B, L_in, C] with L_in odd, for a stride-2 Conv1d of width k:
+    output row t reads the k*C contiguous values x[b, 2t : 2t + k, :] (row pitch 2C, batch pitch L_in*C).  Every
+    element it addresses lies inside x: for k = 2 the trailing row x[b, L_in - 1] is never read."""
+    B, L_in, C = x.shape
+    if L_in % 2 == 0 or k not in (2, 3):
+        raise _lib.WavJepaLibError(f"conv_operand_odd: needs an odd input length and k in (2,3); got L={L_in} k={k}")
+    L_out = (L_in - k) // 2 + 1
+    return make_operand(x, k * C, L_out, B, row_stride=2 * C, batch_stride=L_in * C)
+
+
+_conv_rows_cache: dict = {}
+
+
+def _conv_rows(B: int, L_in: int, n: int, parity: int, device) -> torch.Tensor:
+    """int32 [B * n]: physical row b*L_in + 2m + parity of logical output row b*n + m (odd-length conv_dgrad)."""
+    key = (B, L_in, n, parity, str(device))
+    t = _conv_rows_cache.get(key)
+    if t is None:
+        m = torch.arange(n, device=device, dtype=torch.int32)
+        b = torch.arange(B, device=device, dtype=torch.int32)[:, None]
+        t = (b * L_in + 2 * m[None, :] + parity).reshape(-1).contiguous()
+        if len(_conv_rows_cache) >= 16:
+            _conv_rows_cache.clear()
+        _conv_rows_cache[key] = t
+    return t
+
+
 def conv_dgrad(dy: torch.Tensor, wk: torch.Tensor, dx: torch.Tensor, k: int, *, act: int = ACT_NONE,
                aux: Optional[torch.Tensor] = None) -> None:
     """Data gradient of the stride-2 Conv1d: dy [B, L_out, O] bf16, wk [O, k*C] bf16 (k-major), dx [B, L_in, C].
     Even input positions 2m receive taps j=0 (t=m) and j=2 (t=m-1); odd positions 2m+1 receive tap j=1 (t=m):
     two GEMMs over (shifted) views of dy, written with row pitch 2C.  act/aux: optional x aux epilogue
-    (aux = GELU' of the layer below saved by its forward epilogue, same layout as dx)."""
+    (aux = GELU' of the layer below saved by its forward epilogue, same layout as dx).
+
+    Odd L_in: the batch pitch L_in*C is not a multiple of the 2C row pitch, so both GEMMs write (and read aux) through
+    an explicit output-row index (the generic epilogue).  For k = 2 the trailing row L_in - 1 feeds no output: it is
+    written with zeros."""
     B, L_out, O = dy.shape
     _, L_in, C = dx.shape
     assert dy.is_contiguous() and dx.is_contiguous() and wk.shape == (O, k * C)
-    if L_in % 2 != 0:
-        raise _lib.WavJepaLibError("conv_dgrad: odd input length is not supported")
-    half = L_in // 2
     taps_even = (0, 2) if k == 3 else (0,)
     a_even = make_operand(dy, O, L_out, B, seg_width=O, seg_q=(0,) * len(taps_even), seg_p=(0, -1)[:len(taps_even)])
     a_odd = make_operand(dy, O, L_out, B, seg_width=O, seg_q=(0,), seg_p=(0,))
+    if L_in % 2 != 0:
+        assert aux is None or (aux.is_contiguous() and aux.shape == dx.shape)
+        n_even = L_out + 1 if k == 3 else L_out     # k = 3: row L_in - 1 = 2 L_out receives tap 2 of t = L_out - 1
+        n_odd = L_out
+        kw = dict(ld_out=C, act=act, aux=aux, ld_aux=C)
+        gemm_dgrad(a_even, wk, n_even, B, dx, K=len(taps_even) * O, N=C, seg_col_off=[j * C for j in taps_even],
+                   out_rows=_conv_rows(B, L_in, n_even, 0, dx.device), **kw)
+        gemm_dgrad(a_odd, wk, n_odd, B, dx, K=O, N=C, seg_col_off=[C], out_rows=_conv_rows(B, L_in, n_odd, 1, dx.device),
+                   **kw)
+        if k == 2:
+            dx[:, L_in - 1].zero_()
+        return
+    half = L_in // 2
     kw = dict(ld_out=2 * C, act=act, aux=aux, ld_aux=2 * C)
     gemm_dgrad(a_even, wk, half, B, dx, K=len(taps_even) * O, N=C, seg_col_off=[j * C for j in taps_even],
                out_offset=0, aux_offset=0, **kw)
@@ -538,15 +580,19 @@ def attn_fwd_f32(qkv: torch.Tensor, cu: torch.Tensor, n_seqs: int, max_len: int,
                                         _stream()))
 
 
-def attn_bwd(qkv, out, dout, lse2, cu, n_seqs: int, max_len: int, D: int, H: int, dqkv, dbias=None):
-    """dbias (optional, fp32 [3 D]) += column sums of dqkv: the in_proj bias gradient, formed in the kernel's epilogue."""
+def attn_bwd(qkv, out, dout, lse2, cu, n_seqs: int, max_len: int, D: int, H: int, dqkv, dbias=None,
+             long_seq: bool = False):
+    """dbias (optional, fp32 [3 D]) += column sums of dqkv: the in_proj bias gradient, formed in the kernel's epilogue.
+    long_seq: also take head-dim-64 sequences of 385..400 tokens (wj_attn_varlen_bwd_bias_long), which the plain entry
+    point refuses."""
     lib = _lib.load()
     p = lambda t: C.c_void_p(_ptr(t))
     if _lib._profile is not None:
         _lib._profile.meta = (0.0, n_seqs, max_len, D, H, qkv.shape[0])
     assert dbias is None or (dbias.dtype == torch.float32 and dbias.numel() == 3 * D)
-    check(lib.wj_attn_varlen_bwd_bias(p(qkv), p(out), p(dout), p(lse2), p(cu), n_seqs, max_len, C.c_int64(qkv.shape[0]),
-                                      D, H, p(dqkv), p(dbias), _stream()))
+    fn = lib.wj_attn_varlen_bwd_bias_long if long_seq else lib.wj_attn_varlen_bwd_bias
+    check(fn(p(qkv), p(out), p(dout), p(lse2), p(cu), n_seqs, max_len, C.c_int64(qkv.shape[0]), D, H, p(dqkv), p(dbias),
+             _stream()))
 
 
 # ----------------------------------------------------------------------------------------------------- misc
