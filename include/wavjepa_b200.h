@@ -164,6 +164,22 @@ int wj_conv0_gn_gelu_bwd(const void* x_bf16, const float* w, const float* gamma,
                          int L, int C, int k, int stride, float eps, const double* moments, const float* stats,
                          const void* dy_bf16, const void* dgelu_bf16, void* red_scratch, float* dw, float* dgamma,
                          float* dbeta, void* stream);
+/* Backward of the block above down to its input: dx fp32 [B, Cin, L] = the gradient with respect to the bf16 waveform
+ * the forward read (overwritten; samples after the last window get 0), from dY (bf16 [B, L_out, C]).  Per (instance,
+ * channel), with hhat = (z - mean) rstd of the bf16-rounded conv output z and dz = dY GELU'(gamma hhat + beta), all
+ * recomputed from the input window:
+ *   dconv = gamma rstd (dz - sum_t dz / L_out - hhat sum_t dz hhat / L_out)
+ *   dx[b, ci, 5t + j] = sum over the (t, j) covering the sample of sum_c w_bf16[c, ci, j] dconv[b, t, c]
+ * Two passes over dY (the second needs the sums of the first); the channel contraction runs on mma.sync tiles.  The sums
+ * live in per-block slabs and the overlap-add of the two windows covering a sample is a separate fixed-order pass: no
+ * atomics anywhere, dx is bit-identical run to run in the default mode too.  dw / dgamma / dbeta are optional (all
+ * three or NULL): when given they are accumulated exactly as wj_conv0_gn_gelu_bwd in deterministic mode does.
+ * workspace: wj_conv0_bwd_dx_workspace(B, Cin, L, C) bytes, contents on entry irrelevant. */
+long long wj_conv0_bwd_dx_workspace(int B, int Cin, int L, int C);
+int wj_conv0_gn_gelu_bwd_dx(const void* x_bf16, const float* w, const float* gamma, const float* beta, int B, int Cin,
+                            int L, int C, int k, int stride, const double* moments, const float* stats,
+                            const void* dy_bf16, void* workspace, float* dx, float* dw, float* dgamma, float* dbeta,
+                            void* stream);
 
 /* LayerNorm over the last dim (D in {128,256,384,512,768,1024}), biased variance, one warp per row.
  * Writes any of: out_f32, out_bf16, stats [M,2] = (mean, rstd), rowsum [M,2] = (sum, sum of squares of the OUTPUT row).

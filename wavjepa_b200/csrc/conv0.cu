@@ -442,6 +442,168 @@ __global__ void __launch_bounds__(256) conv0_bwd_finalize_kernel(Conv0Args a, co
   }
 }
 
+// Data gradient, the second pass over dY (it needs S1 / S2 of every (instance, channel), which exist only after the first
+// pass): per output t and channel c, with hhat, GELU' and dz recomputed exactly as in conv0_bwd_kernel,
+//   dconv[t, c] = gamma rstd (dz - S1/L_out - hhat S2/L_out)          (GroupNorm backward incl. the statistics' terms)
+//   part[b, t, ci*10 + j] = sum_c w_bf16[c, ci, j] dconv[t, c]          (the channel contraction, K = C, N = 10 taps)
+// The accumulators of n-tiles (2p, 2p + 1) of the conv MMA are, as they stand, the A fragment of a k = 16 MMA over those 16
+// channels (dconv rounded to bf16, like autocast's bf16 conv input gradient), so the contraction needs no shuffle: B is
+// the bf16 weight slice [16 channels x 8 taps] (2 tap tiles, taps 10..15 zero), stored in fragment order in shared memory.
+// Layout as conv0_fwd_kernel: grid (ceil(chunks / chunks_per_block), B), 8 warps each taking 16 outputs of the 128-output
+// tile and all channels.  Every part row t < L_out is written by exactly one lane; the overlap-add of the two windows
+// that cover a sample is left to conv0_dx_gather_kernel (no atomics: bit-identical run to run).
+template <int CIN>
+__global__ void __launch_bounds__(256) conv0_bwd_dx_kernel(Conv0Args a, const float* __restrict__ stats,
+                                                           const float* __restrict__ gamma,
+                                                           const float* __restrict__ beta, const bf16* __restrict__ dy,
+                                                           const double* __restrict__ red, int nslab,
+                                                           float* __restrict__ part, int chunks_per_block) {
+  constexpr int NA = CIN * kC0K;
+  extern __shared__ __align__(16) uint8_t smem_c0[];
+  uint2* s_wb = reinterpret_cast<uint2*>(smem_c0);                   // [CIN][cg 8][pair 4][tap tile 2][lane 32] (b0, b1)
+  bf16* s_w = reinterpret_cast<bf16*>(s_wb + CIN * 8 * 4 * 2 * 32);   // conv weights as in conv0_fwd_kernel
+  float4* s_p = reinterpret_cast<float4*>(s_w + CIN * a.C * 16);      // [C/2 (fragment order)][3]
+  bf16* s_x = reinterpret_cast<bf16*>(s_p + 3 * (a.C / 2));           // [CIN][kC0WinB]
+  const int b = blockIdx.y;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, g = lane >> 2, tg = lane & 3;
+  for (int i = threadIdx.x; i < CIN * a.C * 16; i += blockDim.x) {
+    const int k = i & 15, pos = (i >> 4) % a.C, ci = (i >> 4) / a.C;
+    const int c = c0_chan(pos >> 6, (pos >> 3) & 7, pos & 7);
+    s_w[i] = __float2bfloat16_rn(k < kC0K ? a.w[(static_cast<size_t>(c) * CIN + ci) * kC0K + k] : 0.f);
+  }
+  for (int i = threadIdx.x; i < CIN * 8 * 4 * 2 * 32; i += blockDim.x) {
+    const int ln = i & 31, tt = (i >> 5) & 1, p = (i >> 6) & 3, cg = (i >> 8) & 7, ci = i >> 11;
+    const int tap = tt * 8 + (ln >> 2);
+    const int c = c0_chan(cg, 2 * p, 2 * (ln & 3));   // k = 2tg, 2tg+1 -> c, c+1 (n-tile 2p); k + 8 -> c+2, c+3 (2p+1)
+    uint2 v = make_uint2(0u, 0u);
+    if (tap < kC0K) {
+      const float* wc = a.w + static_cast<size_t>(c) * NA + ci * kC0K + tap;
+      v.x = pack_bf16x2(wc[0], wc[NA]);
+      v.y = pack_bf16x2(wc[2 * NA], wc[3 * NA]);
+    }
+    s_wb[i] = v;
+  }
+  const float invL = 1.0f / a.L_out;
+  for (int i = threadIdx.x; i < a.C / 2; i += blockDim.x) {
+    const int c = c0_chan(i >> 5, (i >> 2) & 7, 2 * (i & 3));
+    const float4 mr = *reinterpret_cast<const float4*>(stats + (static_cast<size_t>(b) * a.C + c) * 2);
+    double s[4] = {0.0, 0.0, 0.0, 0.0};   // S1(c), S1(c+1), S2(c), S2(c+1): slabs added in slab order (as the finalize)
+    for (int sl = 0; sl < nslab; ++sl) {
+      const double* rs = red + (static_cast<size_t>(b) * nslab + sl) * (2 + NA) * a.C + c;
+      s[0] += rs[0]; s[1] += rs[1]; s[2] += rs[a.C]; s[3] += rs[a.C + 1];
+    }
+    s_p[3 * i + 0] = mr;                                                           // (mean0, rstd0, mean1, rstd1)
+    s_p[3 * i + 1] = make_float4(gamma[c], beta[c], gamma[c + 1], beta[c + 1]);
+    s_p[3 * i + 2] = make_float4(static_cast<float>(s[0]) * invL, static_cast<float>(s[2]) * invL,   // S1/L, S2/L
+                                 static_cast<float>(s[1]) * invL, static_cast<float>(s[3]) * invL);
+  }
+  const int n_groups = a.C / 64;
+  for (int ch = 0; ch < chunks_per_block; ++ch) {
+    const int t0 = (blockIdx.x * chunks_per_block + ch) * kC0TT;
+    if (t0 >= a.L_out) break;
+    __syncthreads();
+    load_window_bf16<CIN>(a, b, t0, s_x);
+    __syncthreads();
+    const int tl0 = warp * 16;
+    if (t0 + tl0 >= a.L_out) continue;
+    uint32_t af[CIN][4];
+#pragma unroll
+    for (int ci = 0; ci < CIN; ++ci) conv_a_frag(s_x + ci * kC0WinB, tl0, g, tg, af[ci]);
+    const int ta = t0 + tl0 + g, tb = ta + 8;
+    const bool va = ta < a.L_out, vb = tb < a.L_out;
+    float acc[CIN][2][4];
+#pragma unroll
+    for (int ci = 0; ci < CIN; ++ci)
+#pragma unroll
+      for (int tt = 0; tt < 2; ++tt) acc[ci][tt][0] = acc[ci][tt][1] = acc[ci][tt][2] = acc[ci][tt][3] = 0.f;
+    for (int cg = 0; cg < n_groups; ++cg) {
+      const bf16* pa = dy + (static_cast<size_t>(b) * a.L_out + ta) * a.C + cg * 64 + tg * 16;
+      const bf16* pb = pa + static_cast<size_t>(8) * a.C;
+      uint32_t da[8], db[8];   // dY of this lane's 16 consecutive channels, rows ta / tb (0 past the end)
+      {
+        const uint4 z = make_uint4(0u, 0u, 0u, 0u);
+        const uint4 a0 = va ? *reinterpret_cast<const uint4*>(pa) : z, a1 = va ? *reinterpret_cast<const uint4*>(pa + 8) : z;
+        const uint4 b0 = vb ? *reinterpret_cast<const uint4*>(pb) : z, b1 = vb ? *reinterpret_cast<const uint4*>(pb + 8) : z;
+        da[0] = a0.x; da[1] = a0.y; da[2] = a0.z; da[3] = a0.w; da[4] = a1.x; da[5] = a1.y; da[6] = a1.z; da[7] = a1.w;
+        db[0] = b0.x; db[1] = b0.y; db[2] = b0.z; db[3] = b0.w; db[4] = b1.x; db[5] = b1.y; db[6] = b1.z; db[7] = b1.w;
+      }
+#pragma unroll
+      for (int p = 0; p < 4; ++p) {
+        uint32_t dc[4];   // A fragment of dconv over the 16 channels of n-tiles 2p, 2p + 1
+#pragma unroll
+        for (int h = 0; h < 2; ++h) {
+          const int nt = 2 * p + h;
+          float c[4] = {0.f, 0.f, 0.f, 0.f};
+#pragma unroll
+          for (int ci = 0; ci < CIN; ++ci) {
+            const uint32_t* wp = reinterpret_cast<const uint32_t*>(s_w + (static_cast<size_t>(ci) * a.C + (cg * 8 + nt) * 8 + g) * 16) + tg;
+            mma16816(c, af[ci], wp[0], wp[4]);
+          }
+          const float2 ya = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&da[nt]));
+          const float2 yb = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&db[nt]));
+          const int pi = ((cg * 8 + nt) * 4 + tg) * 3;
+          const float4 mr = s_p[pi], gb = s_p[pi + 1], kk = s_p[pi + 2];
+          bf16_round2(c[0], c[1]);
+          bf16_round2(c[2], c[3]);
+          const float h0 = (c[0] - mr.x) * mr.y, h1 = (c[1] - mr.z) * mr.w;
+          const float h2 = (c[2] - mr.x) * mr.y, h3 = (c[3] - mr.z) * mr.w;
+          const float2 ga = dgelu_h2(fmaf(h0, gb.x, gb.y), fmaf(h1, gb.z, gb.w));
+          const float2 gbv = dgelu_h2(fmaf(h2, gb.x, gb.y), fmaf(h3, gb.z, gb.w));
+          const float z0 = ya.x * ga.x, z1 = ya.y * ga.y, z2 = yb.x * gbv.x, z3 = yb.y * gbv.y;   // dz
+          const float sc0 = gb.x * mr.y, sc1 = gb.z * mr.w;
+          // rows past the end carry no gradient (dz is 0 there, the statistics' terms are not)
+          const float e0 = va ? sc0 * (z0 - kk.x - h0 * kk.y) : 0.f, e1 = va ? sc1 * (z1 - kk.z - h1 * kk.w) : 0.f;
+          const float e2 = vb ? sc0 * (z2 - kk.x - h2 * kk.y) : 0.f, e3 = vb ? sc1 * (z3 - kk.z - h3 * kk.w) : 0.f;
+          dc[2 * h] = pack_bf16x2(e0, e1);
+          dc[2 * h + 1] = pack_bf16x2(e2, e3);
+        }
+        const uint32_t afr[4] = {dc[0], dc[1], dc[2], dc[3]};
+#pragma unroll
+        for (int ci = 0; ci < CIN; ++ci)
+#pragma unroll
+          for (int tt = 0; tt < 2; ++tt) {
+            const uint2 bw = s_wb[(((ci * 8 + cg) * 4 + p) * 2 + tt) * 32 + lane];
+            mma16816(acc[ci][tt], afr, bw.x, bw.y);
+          }
+      }
+    }
+    // accumulator (row g / g + 8, taps tt*8 + 2tg, +1): taps >= 10 exist only for tt = 1, tg > 0
+#pragma unroll
+    for (int ci = 0; ci < CIN; ++ci)
+#pragma unroll
+      for (int tt = 0; tt < 2; ++tt) {
+        const int tap = tt * 8 + 2 * tg;
+        if (tap >= kC0K) continue;
+        if (va) *reinterpret_cast<float2*>(part + (static_cast<size_t>(b) * a.L_out + ta) * NA + ci * kC0K + tap) =
+            make_float2(acc[ci][tt][0], acc[ci][tt][1]);
+        if (vb) *reinterpret_cast<float2*>(part + (static_cast<size_t>(b) * a.L_out + tb) * NA + ci * kC0K + tap) =
+            make_float2(acc[ci][tt][2], acc[ci][tt][3]);
+      }
+  }
+}
+
+// dx[b, ci, s] = part[b, t, ci*10 + j] + part[b, t - 1, ci*10 + j + 5] with t = s / 5, j = s % 5 (each term only where
+// that output exists): the overlap-add of the two stride-5 windows covering sample s, in a fixed order.  Samples after
+// the last window get 0.  One thread per sample.
+template <int CIN>
+__global__ void __launch_bounds__(256) conv0_dx_gather_kernel(const float* __restrict__ part, int B, int L, int L_out,
+                                                              float* __restrict__ dx) {
+  constexpr int NA = CIN * kC0K;
+  const long long n = static_cast<long long>(B) * CIN * L;
+  for (long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; i < n;
+       i += static_cast<long long>(gridDim.x) * blockDim.x) {
+    const int s = static_cast<int>(i % L);
+    const long long bc = i / L;
+    const int ci = static_cast<int>(bc % CIN), b = static_cast<int>(bc / CIN);
+    const int t = s / kC0S, j = s - t * kC0S;
+    const float* pb = part + static_cast<size_t>(b) * L_out * NA + ci * kC0K;
+    float v = 0.f;
+    if (t < L_out) v = pb[static_cast<size_t>(t) * NA + j];
+    if (t >= 1 && t - 1 < L_out) v += pb[static_cast<size_t>(t - 1) * NA + j + kC0S];
+    dx[i] = v;
+  }
+}
+
 // Forward of the TF32 inference path: fp32 input and weights, fp32 FMA on the CUDA cores (Cin x 10 MAC per output),
 // closed-form statistics of the unrounded conv output, exact erf GELU, fp32 channels-last [B, L_out, C] output rounded to
 // nearest tf32 (it is the operand of the next conv's implicit GEMM).  (256 clips x 10 s: 16.9 GB written in 8.5 ms,
@@ -571,6 +733,77 @@ extern "C" int wj_conv0_gn_gelu_bwd(const void* x_bf16, const float* w, const fl
     conv0_bwd_finalize_kernel<2><<<fgrid, fblock, 0, st>>>(a, moments, stats, gamma, red, dw, dgamma, dbeta, nslab);
   }
   return check_launch("conv0_gn_gelu_bwd", 2);
+}
+
+// Backward of block 0 down to the waveform.  The first pass is conv0_bwd_kernel, always on per-block slabs (each sum has
+// one contributor, the slabs are added in order), so S1 / S2 -- and with them dx -- are bit-identical run to run in
+// either mode; then conv0_bwd_dx_kernel (second pass: the data gradient of every output's window into `part`) and the
+// fixed-order overlap-add.  dw / dgamma / dbeta (all or none): the weight-gradient finalize of wj_conv0_gn_gelu_bwd.
+static void conv0_dx_geometry(int B, int Cin, int L, int C, int* L_out, int* nslab, size_t* red_bytes, size_t* part_bytes) {
+  *L_out = (L - kC0K) / kC0S + 1;
+  const int chunks = (*L_out + kC0TT - 1) / kC0TT;
+  *nslab = (chunks + 12) / 13;   // the first pass's grid.x (13 chunks per block, as wj_conv0_gn_gelu_bwd)
+  *red_bytes = static_cast<size_t>(B) * *nslab * (2 + Cin * kC0K) * C * sizeof(double);
+  *part_bytes = static_cast<size_t>(B) * *L_out * Cin * kC0K * sizeof(float);
+}
+
+extern "C" long long wj_conv0_bwd_dx_workspace(int B, int Cin, int L, int C) {
+  if (B <= 0 || L < kC0K) return 0;
+  int L_out, nslab;
+  size_t rb, pb;
+  conv0_dx_geometry(B, Cin, L, C, &L_out, &nslab, &rb, &pb);
+  return static_cast<long long>(rb + pb);
+}
+
+extern "C" int wj_conv0_gn_gelu_bwd_dx(const void* x_bf16, const float* w, const float* gamma, const float* beta, int B,
+                                       int Cin, int L, int C, int k, int stride, const double* moments, const float* stats,
+                                       const void* dy_bf16, void* workspace, float* dx, float* dw, float* dgamma,
+                                       float* dbeta, void* stream) {
+  if (B <= 0) return WJ_OK;
+  int rc = check_conv0(Cin, C, k, stride);
+  if (rc) return rc;
+  if (L < kC0K) { set_error("conv0_bwd_dx: input shorter than the kernel"); return WJ_ERR_ARG; }
+  if (dx == nullptr || workspace == nullptr) { set_error("conv0_bwd_dx: dx and the workspace are required"); return WJ_ERR_ARG; }
+  const int nw = (dw != nullptr) + (dgamma != nullptr) + (dbeta != nullptr);
+  if (nw != 0 && nw != 3) { set_error("conv0_bwd_dx: dw, dgamma and dbeta are given together or not at all"); return WJ_ERR_ARG; }
+  cudaStream_t st = WJ_STREAM(stream);
+  Conv0Args a;
+  a.x = reinterpret_cast<const bf16*>(x_bf16); a.w = w; a.B = B; a.Cin = Cin; a.L = L; a.C = C; a.xf = nullptr;
+  int nslab;
+  size_t red_bytes, part_bytes;
+  conv0_dx_geometry(B, Cin, L, C, &a.L_out, &nslab, &red_bytes, &part_bytes);
+  double* red = reinterpret_cast<double*>(workspace);
+  float* part = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(workspace) + red_bytes);
+  cudaMemsetAsync(red, 0, red_bytes, st);
+  const bf16* dy = reinterpret_cast<const bf16*>(dy_bf16);
+  const int chunks = (a.L_out + kC0TT - 1) / kC0TT;
+  dim3 grid1(nslab, B);
+  const int cpb2 = 4;
+  dim3 grid2((chunks + cpb2 - 1) / cpb2, B);
+  const size_t smem2 = static_cast<size_t>(Cin) * 8 * 4 * 2 * 32 * sizeof(uint2) + static_cast<size_t>(Cin) * C * 16 * 2 +
+                       static_cast<size_t>(C / 2) * 3 * 16 + static_cast<size_t>(Cin) * kC0WinB * 2 + 16;
+  const long long n = static_cast<long long>(B) * Cin * L;
+  const int ggrid = static_cast<int>(std::min<long long>((n + 255) / 256, 148LL * 16));
+  dim3 fgrid((C + 31) / 32), fblock(32, 8);
+  static bool attr_set[2] = {false, false};
+  if (!attr_set[Cin - 1]) {
+    const cudaError_t e = Cin == 1 ? cudaFuncSetAttribute(conv0_bwd_dx_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem2))
+                                   : cudaFuncSetAttribute(conv0_bwd_dx_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem2));
+    if (e != cudaSuccess) { set_error("cudaFuncSetAttribute: %s", cudaGetErrorString(e)); return WJ_ERR_RUNTIME; }
+    attr_set[Cin - 1] = true;
+  }
+  if (Cin == 1) {
+    conv0_bwd_kernel<1><<<grid1, C / 2, 0, st>>>(a, stats, gamma, beta, dy, red, 13, nslab);
+    conv0_bwd_dx_kernel<1><<<grid2, 256, smem2, st>>>(a, stats, gamma, beta, dy, red, nslab, part, cpb2);
+    conv0_dx_gather_kernel<1><<<ggrid, 256, 0, st>>>(part, B, L, a.L_out, dx);
+    if (nw) conv0_bwd_finalize_kernel<1><<<fgrid, fblock, 0, st>>>(a, moments, stats, gamma, red, dw, dgamma, dbeta, nslab);
+  } else {
+    conv0_bwd_kernel<2><<<grid1, C / 2, 0, st>>>(a, stats, gamma, beta, dy, red, 13, nslab);
+    conv0_bwd_dx_kernel<2><<<grid2, 256, smem2, st>>>(a, stats, gamma, beta, dy, red, nslab, part, cpb2);
+    conv0_dx_gather_kernel<2><<<ggrid, 256, 0, st>>>(part, B, L, a.L_out, dx);
+    if (nw) conv0_bwd_finalize_kernel<2><<<fgrid, fblock, 0, st>>>(a, moments, stats, gamma, red, dw, dgamma, dbeta, nslab);
+  }
+  return check_launch("conv0_gn_gelu_bwd_dx", nw ? 4 : 3);
 }
 
 // Conv block 0 of the TF32 inference path (see conv0_fwd_f32_kernel): x fp32 [B, Cin, L], out fp32 [B, L_out, C].

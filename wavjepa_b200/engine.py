@@ -13,7 +13,7 @@ attention operands bf16 with fp32 accumulation, residual stream / LayerNorm / so
 """
 from __future__ import annotations
 
-from typing import Callable, List, Optional
+from typing import Callable, List, Optional, Sequence
 
 import torch
 
@@ -138,7 +138,7 @@ class TransformerStack:
     # ------------------------------------------------------------------------------------------------ backward
     def backward(self, layers: List[LayerW], grads: List[LayerG], saved: List[LayerSaved], dx: torch.Tensor,
                  cu: torch.Tensor, n_seqs: int, max_len: int, on_layer_done: Optional[Callable] = None,
-                 stop_at: int = 0, need_dx: bool = True):
+                 stop_at: int = 0, need_dx: bool = True, need_wgrad: Optional[Sequence[bool]] = None):
         """dx: fp32 [M, d] gradient w.r.t. the stack output (before any final norm).  Accumulates parameter
         gradients into `grads` (pre-zeroed) and returns the gradient w.r.t. the stack input (fp32).
 
@@ -146,7 +146,9 @@ class TransformerStack:
         what autocast's Linear backward returns); the pair is summed inside the next LayerNorm backward.
 
         Layers below `stop_at` are not visited.  need_dx=False: nothing below the lowest visited layer wants its input
-        gradient, so its last data-gradient GEMM is skipped and None is returned."""
+        gradient, so its last data-gradient GEMM is skipped and None is returned.  need_wgrad[i] False (a frozen layer):
+        layer i runs its data-gradient chain only -- no weight-gradient GEMM, no LayerNorm, bias or attention-bias
+        gradient; `grads[i]` is not touched and may be None.  The data gradients are the same bits either way."""
         d, H, ff = self.d, self.H, self.ff
         M = dx.shape[0]
         dev = dx.device
@@ -154,29 +156,37 @@ class TransformerStack:
         dx_b = None   # bf16 half of the gradient w.r.t. the current layer's output
         for i in range(len(layers) - 1, stop_at - 1, -1):
             w, gw, s = layers[i], grads[i], saved[i]
+            wg = need_wgrad is None or need_wgrad[i]
             # ---- LN2 and the MLP
             dy2 = _empty((M, d), f32, dev)
             dy2_16 = _empty((M, d), bf, dev)
-            ops.add_layernorm_bwd(dx, dx_b, s.x1_32, s.o2, s.st2, w.g2, dy2, dy2_16, gw.g2, gw.be2, gw.b2)
-            ops.gemm_wgrad(ops.plain_operand(dy2_16), ops.plain_operand(s.g), M, 1, gw.w2, accumulate=True)
+            ops.add_layernorm_bwd(dx, dx_b, s.x1_32, s.o2, s.st2, w.g2, dy2, dy2_16,
+                                  *((gw.g2, gw.be2, gw.b2) if wg else ()))
+            if wg:
+                ops.gemm_wgrad(ops.plain_operand(dy2_16), ops.plain_operand(s.g), M, 1, gw.w2, accumulate=True)
             dh = _empty((M, ff), bf, dev)
             ops.gemm_dgrad(ops.plain_operand(dy2_16), w.w2, M, 1, dh, K=d, N=ff, act=ops.ACT_DGELU, aux=s.h,
-                           colsum=gw.b1)
-            ops.gemm_wgrad(ops.plain_operand(dh), ops.plain_operand(s.x1_16), M, 1, gw.w1, accumulate=True)
+                           colsum=gw.b1 if wg else None)
+            if wg:
+                ops.gemm_wgrad(ops.plain_operand(dh), ops.plain_operand(s.x1_16), M, 1, gw.w1, accumulate=True)
             dx1_b = _empty((M, d), bf, dev)
             ops.gemm_dgrad(ops.plain_operand(dh), w.w1, M, 1, dx1_b, K=ff, N=d)
             del dh, dy2_16
             # ---- LN1 and the attention block
             dy1 = _empty((M, d), f32, dev)
             dy1_16 = _empty((M, d), bf, dev)
-            ops.add_layernorm_bwd(dy2, dx1_b, s.x32, s.o1, s.st1, w.g1, dy1, dy1_16, gw.g1, gw.be1, gw.b_o)
+            ops.add_layernorm_bwd(dy2, dx1_b, s.x32, s.o1, s.st1, w.g1, dy1, dy1_16,
+                                  *((gw.g1, gw.be1, gw.b_o) if wg else ()))
             del dy2, dx1_b
-            ops.gemm_wgrad(ops.plain_operand(dy1_16), ops.plain_operand(s.att), M, 1, gw.w_o, accumulate=True)
+            if wg:
+                ops.gemm_wgrad(ops.plain_operand(dy1_16), ops.plain_operand(s.att), M, 1, gw.w_o, accumulate=True)
             datt = _empty((M, d), bf, dev)
             ops.gemm_dgrad(ops.plain_operand(dy1_16), w.w_o, M, 1, datt, K=d, N=d)
             dqkv = _empty((M, 3 * d), bf, dev)
-            ops.attn_bwd(s.qkv, s.att, datt, s.lse, cu, n_seqs, max_len, d, H, dqkv, dbias=gw.b_in, long_seq=True)
-            ops.gemm_wgrad(ops.plain_operand(dqkv), ops.plain_operand(s.x16), M, 1, gw.w_in, accumulate=True)
+            ops.attn_bwd(s.qkv, s.att, datt, s.lse, cu, n_seqs, max_len, d, H, dqkv, dbias=gw.b_in if wg else None,
+                         long_seq=True)
+            if wg:
+                ops.gemm_wgrad(ops.plain_operand(dqkv), ops.plain_operand(s.x16), M, 1, gw.w_in, accumulate=True)
             dx = dy1
             saved[i] = None
             if i == stop_at and not need_dx:

@@ -167,9 +167,14 @@ def conv_stack_forward_tf32(spec, x32: torch.Tensor, w0: torch.Tensor, gn_w: tor
 
 
 def conv_stack_backward(spec, sv: ConvSaved, dh_last: torch.Tensor, w0, gn_w, gn_b, wks, g_w0, g_gn_w, g_gn_b,
-                        g_ws: List[torch.Tensor], gn_eps: float = 1e-5, on_layer_done=None) -> None:
+                        g_ws: List[torch.Tensor], gn_eps: float = 1e-5, on_layer_done=None,
+                        dx: Optional[torch.Tensor] = None, weights: bool = True) -> None:
     """dh_last: bf16 [B, T, C] gradient w.r.t. the PRE-activation of the last conv block.  Accumulates into the fp32
     gradient tensors g_* (shapes of the parameters).
+
+    dx (optional, fp32 [B, Cin, L], overwritten): the gradient w.r.t. the waveform, through block 0's data gradient
+    (ops.conv0_bwd_dx).  weights=False (frozen extractor, needs dx): only the data gradients run, no conv weight
+    gradient and no GroupNorm gradient; the g_* are not touched and may be None.
 
     Odd input lengths (the wav2vec2 extractor's 401-row input of its last block): the weight gradient reads the
     activations through the forward's strided view (k*C columns per output row, batch pitch L_in*C), and conv_dgrad
@@ -184,22 +189,28 @@ def conv_stack_backward(spec, sv: ConvSaved, dh_last: torch.Tensor, w0, gn_w, gn
         x = sv.acts[i - 1]
         L_in = x.shape[1]
         L_out = dh.shape[1]
-        dwk = torch.empty(C, k * C, device=dev, dtype=torch.float32)
-        x_op = ops.conv_operand(x, k) if L_in % 2 == 0 else ops.conv_operand_odd(x, k)
-        ops.gemm_wgrad(ops.make_operand(dh, C, L_out, B), x_op, L_out, B, dwk)
-        g_ws[i - 1].add_(dwk.view(C, k, C).permute(0, 2, 1))
-        dx = torch.empty(B, L_in, C, device=dev, dtype=torch.bfloat16)
+        if weights:
+            dwk = torch.empty(C, k * C, device=dev, dtype=torch.float32)
+            x_op = ops.conv_operand(x, k) if L_in % 2 == 0 else ops.conv_operand_odd(x, k)
+            ops.gemm_wgrad(ops.make_operand(dh, C, L_out, B), x_op, L_out, B, dwk)
+            g_ws[i - 1].add_(dwk.view(C, k, C).permute(0, 2, 1))
+        dxi = torch.empty(B, L_in, C, device=dev, dtype=torch.bfloat16)
         if i - 1 >= 1:
-            ops.conv_dgrad(dh, wks[i - 1], dx, k, act=ops.ACT_DGELU, aux=sv.pre[i - 1])
+            ops.conv_dgrad(dh, wks[i - 1], dxi, k, act=ops.ACT_DGELU, aux=sv.pre[i - 1])
         else:
-            ops.conv_dgrad(dh, wks[i - 1], dx, k)
+            ops.conv_dgrad(dh, wks[i - 1], dxi, k)
         sv.acts[i] = None
         sv.pre[i] = None
-        dh = dx
+        dh = dxi
         if on_layer_done is not None:
             on_layer_done(i)
-    red = torch.empty(B, 2 + sv.x16.shape[1] * 10, C, device=dev, dtype=torch.float64)
-    ops.conv0_bwd(sv.x16, w0, gn_w, gn_b, sv.moments, sv.stats, dh, red, g_w0, g_gn_w, g_gn_b, eps=gn_eps)
+    if dx is not None:
+        ops.conv0_bwd_dx(sv.x16, w0, gn_w, gn_b, sv.moments, sv.stats, dh, dx,
+                         *((g_w0, g_gn_w, g_gn_b) if weights else ()))
+    else:
+        assert weights, "a frozen extractor's backward is only run for the waveform gradient"
+        red = torch.empty(B, 2 + sv.x16.shape[1] * 10, C, device=dev, dtype=torch.float64)
+        ops.conv0_bwd(sv.x16, w0, gn_w, gn_b, sv.moments, sv.stats, dh, red, g_w0, g_gn_w, g_gn_b, eps=gn_eps)
     if on_layer_done is not None:
         on_layer_done(0)
 

@@ -133,21 +133,24 @@ _FEATURE_PATH = ("extract_audio.", "feature_norms.", "post_extraction_mapper.", 
 
 
 class _FeaturePlan:
-    """Which parts of the feature path train in one differentiable `get_audio_representation` call."""
-    __slots__ = ("names", "conv", "norm", "local", "first_layer")
+    """Which parts of the feature path train in one differentiable `get_audio_representation` call.  conv / norm /
+    mapper / final_norm / layer_w[i]: some tensor of that part requires grad (its weight gradients are computed);
+    dx: the waveform requires grad (the data gradient runs down to it through every part, trainable or not)."""
+    __slots__ = ("names", "conv", "norm", "mapper", "final_norm", "layer_w", "local", "first_layer", "dx")
 
 
 class _FeatureBridge(torch.autograd.Function):
     """Makes the features of `get_audio_representation` differentiable: the forward runs the saving kernels, the
-    backward runs the hand-written chain (final LayerNorm -> encoder layers -> mapper / feature norm / conv stack) into a
-    gradient buffer owned by this call and hands autograd the gradients of the parameters it asks for.  `audio` is not
-    an input: no gradient reaches the waveform."""
+    backward runs the hand-written chain (final LayerNorm -> encoder layers -> mapper / feature norm / conv stack, down
+    to conv block 0's data gradient when the waveform requires grad) into a gradient buffer owned by this call and hands
+    autograd the gradients of the inputs it asks for.  `audio` is the waveform on the model's device in the caller's
+    dtype; its gradient is returned in that dtype."""
 
     @staticmethod
-    def forward(ctx, model, inputs, plan, *params):
-        x16, index = inputs   # (a tuple: the waveform is not an input autograd tracks)
+    def forward(ctx, model, audio, index, plan, *params):
         ctx.model = model
-        ctx.fctx = model._features_saving(x16, index, plan)
+        ctx.audio_dtype = audio.dtype
+        ctx.fctx = model._features_saving(audio.to(torch.bfloat16).contiguous(), index, plan)
         out, ctx.fctx.out = ctx.fctx.out, None
         return out
 
@@ -159,10 +162,11 @@ class _FeatureBridge(torch.autograd.Function):
                                "activations are freed; run the forward again (retain_graph is not supported)")
         ctx.fctx = None
         model = ctx.model
-        gflat = model._features_backward(c, grad_out)
-        needs = ctx.needs_input_grad[3:]
+        gflat, dx = model._features_backward(c, grad_out)
+        needs = ctx.needs_input_grad[4:]
         grads = [model._view(gflat, n) if needs[i] else None for i, n in enumerate(c.plan.names)]
-        return (None, None, None, *grads)
+        daudio = dx.to(ctx.audio_dtype) if dx is not None and ctx.needs_input_grad[1] else None
+        return (None, daudio, None, None, *grads)
 
 
 # =================================================================================================== model
@@ -249,8 +253,8 @@ class JEPA(_ModuleBase):
         packed-fp16 tanh-form GELU, ~1e-2 relative L2 from the reference's fp32 features; "tf32" runs the reference's fp32
         feature extraction with every GEMM operand rounded to nearest tf32, fp32 accumulation and the exact erf GELU
         (DESIGN.md 2.1).  `forward`, `train_step`, the teacher and the denoiser ignore it.  "tf32" is inference-only:
-        its features never carry a grad_fn; fine-tuning through `get_audio_representation` runs in "bf16" (DESIGN.md
-        2.2)."""
+        its features never carry a grad_fn, whether parameters or the waveform require grad; fine-tuning and the waveform
+        gradient through `get_audio_representation` run in "bf16" (DESIGN.md 2.2, 2.3)."""
         return self.__dict__.get("_inference_precision", "bf16")
 
     @inference_precision.setter
@@ -667,27 +671,31 @@ class JEPA(_ModuleBase):
             on_ready(0)
 
     def _local_backward(self, local_saved, dlocal16: torch.Tensor, B: int, g, ready, norm: bool = True,
-                        conv: bool = True) -> None:
+                        conv: bool = True, dx: Optional[torch.Tensor] = None, wg_mapper: bool = True,
+                        wg_norm: bool = True, wg_conv: bool = True) -> None:
         """Backward of `_local_features` from the (bf16) gradient of the mapper output on the dense token grid:
         post_extraction_mapper -> feature_norms -> conv stack(s).  norm=False stops after the mapper, conv=False after
-        the feature norm (frozen parts below them: no data gradient flows there)."""
+        the feature norm (frozen parts below them: no data gradient flows there).  dx (fp32 [B, Cin, L], overwritten):
+        continue through conv block 0 to the waveform.  wg_* False: that part is frozen, its weight gradients (and bias
+        column sums) are not computed; the data gradient still passes through it."""
         T, D = self.total_patches, self.encoder_embedding_dim
         dev = dlocal16.device
         p32 = lambda n: self._view(self._flat_p, n)
         p16 = lambda n: self._view(self._flat_w16, n)
         conv_saved, f2, ln16, st = local_saved
         C = f2.shape[1]
-        ops.colsum(dlocal16, g("post_extraction_mapper.bias"))
-        ops.gemm_wgrad(ops.plain_operand(dlocal16), ops.plain_operand(ln16), B * T, 1,
-                       g("post_extraction_mapper.weight"), accumulate=True)
+        if wg_mapper:
+            ops.colsum(dlocal16, g("post_extraction_mapper.bias"))
+            ops.gemm_wgrad(ops.plain_operand(dlocal16), ops.plain_operand(ln16), B * T, 1,
+                           g("post_extraction_mapper.weight"), accumulate=True)
         ready("post_extraction_mapper.weight")
         if not (norm or conv):
             return
         dln = torch.empty(B * T, C, device=dev)
         ops.gemm_dgrad(ops.plain_operand(dlocal16), p16("post_extraction_mapper.weight"), B * T, 1, dln, K=D, N=C)
         dfeat = torch.empty(B * T, C, device=dev)
-        ops.layernorm_bwd(dln, f2, st, p32("feature_norms.weight"), dfeat, None, g("feature_norms.weight"),
-                          g("feature_norms.bias"), None)
+        ops.layernorm_bwd(dln, f2, st, p32("feature_norms.weight"), dfeat, None,
+                          *((g("feature_norms.weight"), g("feature_norms.bias")) if wg_norm else (None, None)), None)
         ready("feature_norms.weight")
         if not conv:
             return
@@ -704,22 +712,27 @@ class JEPA(_ModuleBase):
                 # with shared weights every channel pass adds into the SAME gradient region: it is final (and may be
                 # all-reduced) only after the last pass
                 last = (not ex.share_weights_over_channels) or ch == 0
-                self._conv_backward(prefix, ex.conv_layers_spec, sv, dfc, B, Tc, C, g, ready if last else (lambda name: None))
+                # each mono stream's waveform gradient lands in its channel
+                dxc = None if dx is None else torch.empty(B, 1, dx.shape[2], device=dev)
+                self._conv_backward(prefix, ex.conv_layers_spec, sv, dfc, B, Tc, C, g, ready if last else (lambda name: None),
+                                    dxc, wg_conv)
+                if dx is not None:
+                    dx[:, ch:ch + 1].copy_(dxc)
         else:
-            self._conv_backward(exs[0][0], ex.conv_layers_spec, conv_saved[0], dfeat, B, T, C, g, ready)
+            self._conv_backward(exs[0][0], ex.conv_layers_spec, conv_saved[0], dfeat, B, T, C, g, ready, dx, wg_conv)
 
-    def _conv_backward(self, prefix, spec, sv, dfeat, B, T, C, g, ready):
+    def _conv_backward(self, prefix, spec, sv, dfeat, B, T, C, g, ready, dx=None, weights: bool = True):
         n = len(spec)
         dev = dfeat.device
         p32 = lambda nm: self._view(self._flat_p, nm)
         dh = torch.empty(B, T, C, device=dev, dtype=torch.bfloat16)
         ops.scatter_dgelu(dfeat, None, sv.pre[n - 1].view(B * T, C), B * T, dh.view(B * T, C))
         wks = [self._conv_wk[f"{prefix}.{i}.0.weight"] for i in range(1, n)]
-        g_ws = [g(f"{prefix}.{i}.0.weight") for i in range(1, n)]
+        gw = g if weights else (lambda nm: None)
         conv_stack_backward(spec, sv, dh, p32(f"{prefix}.0.0.weight"), p32(f"{prefix}.0.2.weight"),
-                            p32(f"{prefix}.0.2.bias"), wks, g(f"{prefix}.0.0.weight"), g(f"{prefix}.0.2.weight"),
-                            g(f"{prefix}.0.2.bias"), g_ws,
-                            on_layer_done=lambda i: ready(f"{prefix}.{i}.0.weight"))
+                            p32(f"{prefix}.0.2.bias"), wks, gw(f"{prefix}.0.0.weight"), gw(f"{prefix}.0.2.weight"),
+                            gw(f"{prefix}.0.2.bias"), [gw(f"{prefix}.{i}.0.weight") for i in range(1, n)],
+                            on_layer_done=lambda i: ready(f"{prefix}.{i}.0.weight"), dx=dx, weights=weights)
 
     # ------------------------------------------------------------------------------------------- public API
     def forward(self, audio: torch.Tensor, ctx_masks: torch.Tensor, target_indices: torch.Tensor,
@@ -1032,28 +1045,35 @@ class JEPA(_ModuleBase):
         return out.view(B, T, D)
 
     # ------------------------------------------------------------------------------------------- fine-tuning
-    def _feature_grad_plan(self) -> Optional[_FeaturePlan]:
-        """None unless grad mode is on and a feature-path parameter requires grad (the rule of `forward`)."""
+    def _feature_grad_plan(self, audio_grad: bool = False) -> Optional[_FeaturePlan]:
+        """None unless grad mode is on and the waveform (audio_grad) or a feature-path parameter requires grad (the
+        rule of `forward`)."""
         if not torch.is_grad_enabled():
             return None
         params = dict(self.named_parameters())
         names = [n for n in self._train_names if n.startswith(_FEATURE_PATH)]
         trainable = [n for n in names if params[n].requires_grad]
-        if not trainable:
+        if not (trainable or audio_grad):
             return None
         plan = _FeaturePlan()
         plan.names = names
+        plan.dx = audio_grad
         plan.conv = any(n.startswith("extract_audio.") for n in trainable)
         plan.norm = any(n.startswith("feature_norms.") for n in trainable)
-        plan.local = plan.conv or plan.norm or any(n.startswith("post_extraction_mapper.") for n in trainable)
+        plan.mapper = any(n.startswith("post_extraction_mapper.") for n in trainable)
+        plan.final_norm = any(n.startswith("encoder.norm.") for n in trainable)
+        plan.local = plan.conv or plan.norm or plan.mapper or plan.dx
         n_layers = self._enc_stack.n_layers
         layers = [int(n.split(".")[2]) for n in trainable if n.startswith("encoder.layers.")]
+        plan.layer_w = [i in layers for i in range(n_layers)]
         plan.first_layer = 0 if plan.local else min(layers, default=n_layers)
         return plan
 
-    def _audio_representation_grad(self, x16, padding_mask, host_mask, plan: _FeaturePlan) -> torch.Tensor:
-        """Differentiable get_audio_representation (same masking semantics and checks as the inference path)."""
-        B, T = x16.shape[0], self.total_patches
+    def _audio_representation_grad(self, audio, padding_mask, host_mask, plan: _FeaturePlan) -> torch.Tensor:
+        """Differentiable get_audio_representation (same masking semantics and checks as the inference path).  audio:
+        the waveform already on the model's device (moved outside the Function, so that autograd's copy backward
+        returns its gradient to the caller's device)."""
+        B, T = audio.shape[0], self.total_patches
         index = None
         if host_mask is not None:
             index = self._periodic_index(host_mask, B, T)
@@ -1062,7 +1082,7 @@ class JEPA(_ModuleBase):
             mi = ops.mask_indices(pm.view(B, T), torch.zeros_like(pm), pm)
             index = (mi.ctx_rows, mi.cu_c, mi.Nc, mi.max_nc)
         params = dict(self.named_parameters())
-        return _FeatureBridge.apply(self, (x16, index), plan, *[params[n] for n in plan.names])
+        return _FeatureBridge.apply(self, audio, index, plan, *[params[n] for n in plan.names])
 
     def _features_saving(self, x16: torch.Tensor, index, plan: _FeaturePlan) -> _Ctx:
         """Forward of `_FeatureBridge`: the inference kernels plus the activations the backward needs, kept from the
@@ -1073,7 +1093,9 @@ class JEPA(_ModuleBase):
         p32 = lambda n: self._view(self._flat_p, n)
         c = _Ctx()
         c.B, c.index, c.plan = B, index, plan
-        local32, local_saved = self._local_features(x16, save=plan.local, save_conv=plan.conv)
+        # (the waveform gradient runs the whole conv stack backward: its GELU' copies are kept even when it is frozen)
+        local32, local_saved = self._local_features(x16, save=plan.local, save_conv=plan.conv or plan.dx)
+        c.x_shape = x16.shape
         c.local_saved = local_saved if plan.local else None
         if index is None:
             M = B * T
@@ -1100,9 +1122,11 @@ class JEPA(_ModuleBase):
         c.xs32, c.M = xs32, M
         return c
 
-    def _features_backward(self, c: _Ctx, grad_out: torch.Tensor) -> torch.Tensor:
-        """Backward of `_FeatureBridge` from the fp32 gradient of the features [B, T, D].  Returns a gradient buffer
-        over the extractor..encoder span of the flat layout (owned by this call: several graphs may be alive)."""
+    def _features_backward(self, c: _Ctx, grad_out: torch.Tensor):
+        """Backward of `_FeatureBridge` from the fp32 gradient of the features [B, T, D].  Returns (a gradient buffer
+        over the extractor..encoder span of the flat layout, owned by this call: several graphs may be alive; the fp32
+        gradient of the bf16 waveform [B, Cin, L] when plan.dx, else None).  Only the parts with a trainable tensor
+        compute weight gradients."""
         dev = c.xs32.device
         B, M, plan = c.B, c.M, c.plan
         T, D = self.total_patches, self.encoder_embedding_dim
@@ -1116,12 +1140,15 @@ class JEPA(_ModuleBase):
             ops.gather_rows(dy, c.index[0], M, dyp, None)
             dy = dyp
         dxs = torch.empty(M, D, device=dev)
-        ops.layernorm_bwd(dy, c.xs32, c.norm_st, p32("encoder.norm.weight"), dxs, None, g("encoder.norm.weight"),
-                          g("encoder.norm.bias"), None)
+        ops.layernorm_bwd(dy, c.xs32, c.norm_st, p32("encoder.norm.weight"), dxs, None,
+                          *((g("encoder.norm.weight"), g("encoder.norm.bias")) if plan.final_norm else (None, None)),
+                          None)
         c.xs32 = None
+        daudio = torch.empty(c.x_shape, device=dev) if plan.dx else None
         if plan.first_layer < n_layers:
             dx = self._enc_stack.backward(self._W_enc, self._stack_grads("encoder.", n_layers, g), c.enc_saved, dxs,
-                                          c.cu, B, c.max_len, stop_at=plan.first_layer, need_dx=plan.local)
+                                          c.cu, B, c.max_len, stop_at=plan.first_layer, need_dx=plan.local,
+                                          need_wgrad=plan.layer_w)
             if plan.local:
                 # the mapper output is bf16 (autocast), so is its gradient on the dense token grid
                 if c.index is None:
@@ -1131,10 +1158,11 @@ class JEPA(_ModuleBase):
                     dlocal16 = torch.zeros(B * T, D, device=dev, dtype=torch.bfloat16)
                     ops.scatter_dgelu(dx, c.index[0], None, M, dlocal16)
                 del dx
-                self._local_backward(c.local_saved, dlocal16, B, g, lambda name: None, norm=plan.norm or plan.conv,
-                                     conv=plan.conv)
+                self._local_backward(c.local_saved, dlocal16, B, g, lambda name: None,
+                                     norm=plan.norm or plan.conv or plan.dx, conv=plan.conv or plan.dx, dx=daudio,
+                                     wg_mapper=plan.mapper, wg_norm=plan.norm, wg_conv=plan.conv)
         c.enc_saved = c.local_saved = None
-        return gflat
+        return gflat, daudio
 
     def get_audio_representation(self, audio: torch.Tensor, padding_mask: Optional[torch.Tensor] = None,
                                  host_mask=None) -> torch.Tensor:
@@ -1149,21 +1177,35 @@ class JEPA(_ModuleBase):
         the trainable path parameters (everything else keeps grad None).  The values are bit-identical to the no-grad
         call.  Rows hidden by a padding mask stay constant zeros: gradient flows from the visible rows only (the
         reference computes values at padded query positions, but no caller reads them).  Frozen parts save nothing and
-        are not backpropagated: a frozen extractor, or encoder layers below the lowest trainable one.  No gradient
-        reaches `audio`, and one graph supports one backward.  inference_precision "tf32" stays forward-only: fine-tuning
-        runs in the "bf16" training numerics (DESIGN.md 2.2)."""
+        are not backpropagated: a frozen extractor, or encoder layers below the lowest trainable one; frozen layers
+        above it pass the gradient on without computing weight gradients.
+
+        Waveform gradient: in grad mode, when `audio` requires grad (a frozen encoder used as a perceptual or
+        feature-matching loss, input saliency, a network in front of a trainable encoder), the features carry a
+        grad_fn and `backward()` also fills `audio.grad` -- on audio's device, in its dtype (fp32 or bf16): the
+        gradient with respect to the bf16 waveform the model reads, through every block down to conv block 0.  Only
+        the parts with a trainable tensor compute weight gradients, so a fully frozen encoder runs data gradients only.
+        Padded samples still receive the gradient the GroupNorm of block 0 couples them to.  No gradient reaches
+        padding_mask / host_mask.
+
+        One graph supports one backward.  inference_precision "tf32" stays forward-only (no grad_fn, whatever
+        requires grad): fine-tuning and the waveform gradient run in the "bf16" training numerics (DESIGN.md 2.2,
+        2.3)."""
         self.eval()
         self._ensure_ready()
         self._sync_weights()
         if self.inference_precision == "tf32":
             return self._audio_representation_tf32(audio, padding_mask, host_mask)
         dev = self.device
+        plan = self._feature_grad_plan(audio.requires_grad)
+        if plan is not None:
+            if plan.dx:   # moved outside the Function: autograd's copy backward takes the gradient back to audio.device
+                return self._audio_representation_grad(audio.to(device=dev), padding_mask, host_mask, plan)
+            return self._audio_representation_grad(audio.to(device=dev, dtype=torch.bfloat16).contiguous(),
+                                                   padding_mask, host_mask, plan)
         x16 = audio.to(device=dev, dtype=torch.bfloat16).contiguous()
         B = x16.shape[0]
         T, D = self.total_patches, self.encoder_embedding_dim
-        plan = self._feature_grad_plan()
-        if plan is not None:
-            return self._audio_representation_grad(x16, padding_mask, host_mask, plan)
         local32, _ = self._local_features(x16, save=False)
         p32 = lambda n: self._view(self._flat_p, n)
         if padding_mask is None and host_mask is None:

@@ -412,6 +412,31 @@ def conv0_bwd(x, w, gamma, beta, moments, stats, dy, red_scratch, dw, dgamma, db
                                    _stream()))
 
 
+def conv0_bwd_dx_workspace(B: int, Cin: int, L: int, channels: int, device) -> torch.Tensor:
+    """Scratch of conv0_bwd_dx (uint8; its contents on entry do not matter)."""
+    fn = _lib.load()._cdll.wj_conv0_bwd_dx_workspace   # (the raw symbol: it returns a byte count, not a status)
+    fn.restype = C.c_longlong
+    return torch.empty(int(fn(B, Cin, L, channels)), device=device, dtype=torch.uint8)
+
+
+def conv0_bwd_dx(x, w, gamma, beta, moments, stats, dy, dx, dw=None, dgamma=None, dbeta=None, workspace=None,
+                 k: int = 10, stride: int = 5) -> None:
+    """Backward of conv0_fwd down to the waveform: dx fp32 [B, Cin, L] (overwritten) from dy (bf16 [B, L_out, C]).
+    dw / dgamma / dbeta: all three (accumulated, as conv0_bwd) or None (no weight-gradient work)."""
+    B, Cin, L = x.shape
+    assert x.dtype == torch.bfloat16 and x.is_contiguous()
+    assert dy.dtype == torch.bfloat16 and dy.is_contiguous()
+    assert dx.dtype == torch.float32 and dx.is_contiguous() and dx.shape == x.shape
+    if workspace is None:
+        workspace = conv0_bwd_dx_workspace(B, Cin, L, w.shape[0], x.device)
+    lib = _lib.load()
+    p = lambda t: C.c_void_p(_ptr(t))
+    if _lib._profile is not None:
+        _lib._profile.nbytes = 2 * (B * Cin * L * 2 + dy.numel() * 2) + B * Cin * L * 4
+    check(lib.wj_conv0_gn_gelu_bwd_dx(p(x), p(w), p(gamma), p(beta), B, Cin, L, w.shape[0], k, stride, p(moments),
+                                      p(stats), p(dy), p(workspace), p(dx), p(dw), p(dgamma), p(dbeta), _stream()))
+
+
 # ----------------------------------------------------------------------------------------------------- norms
 def layernorm_fwd(x: torch.Tensor, gamma, beta, eps: float, out_f32=None, out_bf16=None, stats=None, rowsum=None):
     M, D = x.shape
