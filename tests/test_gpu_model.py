@@ -680,7 +680,7 @@ def test_denoiser_default_clip_is_the_reference_trainers():
 def test_shared_conv_weights_are_announced_once_final():
     """ADVICE r1: with share_weights_over_channels=True both channel passes add into the same conv gradients; a bucket
     must not be announced (and all-reduced) before the last pass.  A recording reducer checks that nothing changes in
-    flat[offset:] after ready(offset)."""
+    flat[offset:] after ready(offset).  The denoiser's backward announces its buckets the same way."""
     cfg = jo.Cfg(in_channels=2, per_channel=True)
     ex = w.ConvChannelFeatureExtractor(conv_layers_spec=cfg.spec, in_channels=2, share_weights_over_channels=True)
     model = w.JEPA(feature_extractor=ex, transformer_encoder_cfg=w.TransformerEncoderCFG.create(),
@@ -711,14 +711,19 @@ def test_shared_conv_weights_are_announced_once_final():
     audio = torch.randn(2, 2, cfg.target_length, generator=g).bfloat16().to(DEV)
     mk = w.TimeInverseBlockMasker(4, 0.65, 10, 0.25, 10, 0.1, channel_based_masking=True, seed=2, row0=0)
     c_m, t_m, v_m = mk(batch_size=2, n_times=400, in_channels=2)
-    flat = model._flat_g if model._flat_p is not None else None
     model.train_step(audio, c_m, t_m, v_m)
-    flat = model._flat_g
-    assert len(rec.log) > 20
-    offs = [o for o, _, _ in rec.log]
-    assert offs == sorted(offs, reverse=True), "ready() offsets must move from the end of the buffer to its start"
-    for off, s1, s2 in rec.log:
-        assert flat[off:].double().sum().item() == s1 and flat[off:].abs().double().sum().item() == s2, off
+    den = _denoiser(0.25, nr=2)
+    den_rec = Recorder()
+    den.attach_data_parallel(den_rec, sync=False)
+    clean = torch.randn(4, 1, 32159, generator=g).bfloat16().to(DEV)
+    gen = (clean.float() + 0.5 * torch.randn(4, 1, 32159, generator=g).to(DEV)).bfloat16()
+    den.forward_backward(gen, clean)
+    for r, flat in ((rec, model._flat_g), (den_rec, den._core._flat_g)):
+        assert len(r.log) > 20
+        offs = [o for o, _, _ in r.log]
+        assert offs == sorted(offs, reverse=True), "ready() offsets must move from the end of the buffer to its start"
+        for off, s1, s2 in r.log:
+            assert flat[off:].double().sum().item() == s1 and flat[off:].abs().double().sum().item() == s2, off
 
 
 def test_hear_nat_runtime_matches_reference_goldens():

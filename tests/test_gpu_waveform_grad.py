@@ -17,7 +17,7 @@ import torch.nn.functional as F
 pytestmark = pytest.mark.gpu
 
 import wavjepa_b200 as w  # noqa: E402
-from wavjepa_b200 import _lib, hear, ops  # noqa: E402
+from wavjepa_b200 import _lib, hear, jepa, ops  # noqa: E402
 from oracle import inputs as oi  # noqa: E402
 from oracle import jepa_oracle as jo  # noqa: E402
 
@@ -260,7 +260,7 @@ def test_waveform_gradient_matches_the_oracle(name):
 
 
 # ------------------------------------------------------------------------------------------------ contract
-def test_contract_device_dtype_and_unchanged_paths(monkeypatch):
+def test_contract_device_dtype_and_inference_path_saves_nothing(monkeypatch):
     cfg = jo.Cfg()
     model = build(cfg, jo.make_state_dict(cfg, seed=9))
     model.requires_grad_(False)
@@ -269,13 +269,20 @@ def test_contract_device_dtype_and_unchanged_paths(monkeypatch):
     proj = torch.randn(2, cfg.total_patches, cfg.d_model, generator=g).to(DEV)
     with torch.no_grad():
         f0 = model.get_audio_representation(base.to(DEV))
-    # audio not requiring grad, frozen model: the inference path, no graph, no saving kernels
-    calls = []
-    real = model._features_saving
-    monkeypatch.setattr(model, "_features_saving", lambda *a_, **k_: calls.append(1) or real(*a_, **k_))
+    # audio not requiring grad, frozen model: the inference path -- not through _FeatureBridge, no graph, and no
+    # saving kernels: no encoder or conv activations kept, no LayerNorm statistics requested
+    calls, saves = [], []
+    real_bridge = jepa._FeatureBridge.apply
+    monkeypatch.setattr(jepa._FeatureBridge, "apply", lambda *a_, **k_: calls.append(1) or real_bridge(*a_, **k_))
+    real_stack, real_conv, real_ln = model._enc_stack.forward, jepa.conv_stack_forward, ops.layernorm_fwd
+    monkeypatch.setattr(model._enc_stack, "forward", lambda *a_, **k_: saves.append(a_[6]) or real_stack(*a_, **k_))
+    monkeypatch.setattr(jepa, "conv_stack_forward", lambda *a_, **k_: saves.append(a_[6]) or real_conv(*a_, **k_))
+    monkeypatch.setattr(ops, "layernorm_fwd", lambda *a_, **k_: saves.append(a_[6] is not None) or real_ln(*a_, **k_))
     f = model.get_audio_representation(base.to(DEV))
     assert f.grad_fn is None and not f.requires_grad and not calls
+    assert len(saves) == 4 and not any(saves)   # conv stack, feature norm, encoder, final norm
     assert torch.equal(f, f0)
+    saves.clear()
     grads = {}
     for dev in ("cpu", DEV):
         for dt in (torch.float32, torch.bfloat16):
@@ -289,7 +296,7 @@ def test_contract_device_dtype_and_unchanged_paths(monkeypatch):
             grads[(dev, dt)] = a.grad.float().cpu()
             with pytest.raises(RuntimeError, match="already backpropagated"):
                 loss.backward()
-    assert calls   # the waveform-gradient calls ran the saving forward
+    assert calls and all(saves[:4])   # the waveform-gradient calls ran the saving forward
     # every input dtype / device reads the same bf16 waveform: one gradient, returned in each caller's dtype
     assert torch.equal(grads[("cpu", torch.float32)], grads[(DEV, torch.float32)])
     assert torch.equal(grads[(DEV, torch.bfloat16)], grads[(DEV, torch.float32)].bfloat16().float())

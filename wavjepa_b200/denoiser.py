@@ -255,25 +255,6 @@ class Denoiser(_ModuleBase):
         return outs[0][idx], outs[1][idx]
 
     # ------------------------------------------------------------------------------------------- forward / backward
-    def _student_forward(self, x16: torch.Tensor, save: bool):
-        """extractor -> LayerNorm -> mapper -> + positions -> 12 layers -> final LayerNorm on 2N full sequences
-        (wavjepa/denoiser.py:338-346).  Returns (features fp32 [2N*T, D], saved pieces for the backward)."""
-        core = self._core
-        dev = x16.device
-        n2 = x16.shape[0]
-        T, D = self.total_patches, self.encoder_embedding_dim
-        p32 = lambda n: core._view(core._flat_p, n)
-        local32, local_saved = core._local_features(x16, save)
-        l16 = torch.empty(n2 * T, D, device=dev, dtype=torch.bfloat16)
-        ops.gather_rows(local32, None, n2 * T, None, l16)
-        cu = torch.arange(0, (n2 + 1) * T, T, device=dev, dtype=torch.int32)
-        xs32, _, enc_saved = core._enc_stack.forward(core._W_enc, local32, l16, cu, n2, T, save)
-        feats = torch.empty(n2 * T, D, device=dev)
-        st = torch.empty(n2 * T, 2, device=dev) if save else None
-        ops.layernorm_fwd(xs32, p32("encoder.norm.weight"), p32("encoder.norm.bias"), self.encoder.norm.eps, feats,
-                          None, st, None)
-        return feats, (local_saved, enc_saved, xs32, st, cu)
-
     def _run(self, generated_scene: torch.Tensor, clean_scene: torch.Tensor, backward: bool):
         if self.teacher is None:
             raise WavJepaLibError("Denoiser needs its frozen teacher: call _set_teacher(checkpoint) first "
@@ -288,7 +269,10 @@ class Denoiser(_ModuleBase):
         N = gen16.shape[0]
         T, D = self.total_patches, self.encoder_embedding_dim
         x16 = torch.cat([clean16, gen16], dim=0).contiguous()          # halves: [clean | generated]
-        feats, saved = self._student_forward(x16, backward)
+        # the student (wavjepa/denoiser.py:338-346) on 2N full sequences; the backward computes every gradient of the
+        # feature path, whatever requires_grad says
+        plan = core._feature_plan(core._train_names) if backward else None
+        feats, saved = core._features_forward(x16, None, plan)
         with torch.no_grad():
             targets = self.teacher.get_audio_representation(clean16, padding_mask=None).reshape(N * T, D)
         M = N * T * D
@@ -307,19 +291,7 @@ class Denoiser(_ModuleBase):
         if ddp is not None:
             ddp.begin(gflat)
         on_ready = ddp.ready if ddp is not None else None
-        G_enc, _, g = core._grad_views(gflat)
-        ready = (lambda name: on_ready(core._offsets[name][0])) if on_ready is not None else (lambda name: None)
-        local_saved, enc_saved, xs32, st, cu = saved
-        p32 = lambda n: core._view(core._flat_p, n)
-        dxs = torch.empty(2 * N * T, D, device=dev)
-        ops.layernorm_bwd(dfe, xs32, st, p32("encoder.norm.weight"), dxs, None, g("encoder.norm.weight"),
-                          g("encoder.norm.bias"), None)
-        ready("encoder.norm.weight")
-        dx = core._enc_stack.backward(core._W_enc, G_enc, enc_saved, dxs, cu, 2 * N, T,
-                                      lambda i: ready(f"encoder.layers.{i}.self_attn.in_proj_weight"))
-        dlocal16 = torch.empty(2 * N * T, D, device=dev, dtype=bf)     # the mapper output is bf16 under autocast
-        ops.gather_rows(dx, None, 2 * N * T, None, dlocal16)
-        core._local_backward(local_saved, dlocal16, 2 * N, g, ready)
+        core._features_backward(saved, dfe, gflat, on_ready)
         if on_ready is not None:
             on_ready(0)
         world = 1

@@ -20,13 +20,9 @@ import torch
 from . import ops
 
 
-class LayerW:
-    """bf16 working weights + fp32 vectors of one layer (views into the model's flat buffers)."""
-    __slots__ = ("w_in", "b_in", "w_o", "b_o", "w1", "b1", "w2", "b2", "g1", "be1", "g2", "be2")
-
-
-class LayerG:
-    """fp32 gradient views of one layer."""
+class LayerViews:
+    """Views of one layer's tensors into the model's flat buffers: the bf16 working weights + fp32 vectors, or the fp32
+    gradients."""
     __slots__ = ("w_in", "b_in", "w_o", "b_o", "w1", "b1", "w2", "b2", "g1", "be1", "g2", "be2")
 
 
@@ -47,7 +43,7 @@ class TransformerStack:
         self.d, self.H, self.ff, self.n_layers, self.eps = d_model, nhead, dim_ff, n_layers, ln_eps
 
     # ------------------------------------------------------------------------------------------------ forward
-    def forward(self, layers: List[LayerW], x32: torch.Tensor, x16: torch.Tensor, cu: torch.Tensor, n_seqs: int,
+    def forward(self, layers: List[LayerViews], x32: torch.Tensor, x16: torch.Tensor, cu: torch.Tensor, n_seqs: int,
                 max_len: int, save: bool, layer_hook: Optional[Callable] = None, rowsum_from: int = 1 << 30,
                 save_from: int = 0):
         """x32/x16: [M, d] fp32 residual stream and its bf16 copy.  Returns (x32, x16, saved list).
@@ -99,7 +95,7 @@ class TransformerStack:
             x32, x16 = x2_32, x2_16
         return x32, x16, saved
 
-    def forward_tf32(self, layers: List[LayerW], x32: torch.Tensor, xop: torch.Tensor, cu: torch.Tensor, n_seqs: int,
+    def forward_tf32(self, layers: List[LayerViews], x32: torch.Tensor, xop: torch.Tensor, cu: torch.Tensor, n_seqs: int,
                      max_len: int) -> torch.Tensor:
         """Inference forward at reference precision (the reference's fp32 feature extraction): the same packed layout,
         `layers` hold fp32 weight matrices rounded to nearest tf32.  x32: [M, d] fp32 residual stream, xop: its copy
@@ -136,7 +132,7 @@ class TransformerStack:
         return x32
 
     # ------------------------------------------------------------------------------------------------ backward
-    def backward(self, layers: List[LayerW], grads: List[LayerG], saved: List[LayerSaved], dx: torch.Tensor,
+    def backward(self, layers: List[LayerViews], grads: List[LayerViews], saved: List[LayerSaved], dx: torch.Tensor,
                  cu: torch.Tensor, n_seqs: int, max_len: int, on_layer_done: Optional[Callable] = None,
                  stop_at: int = 0, need_dx: bool = True, need_wgrad: Optional[Sequence[bool]] = None):
         """dx: fp32 [M, d] gradient w.r.t. the stack output (before any final norm).  Accumulates parameter

@@ -29,7 +29,7 @@ from . import ops
 from ._lib import WavJepaLibError, require_device
 from ._lightning import Base as _ModuleBase
 from ._lightning import attached_trainer
-from .engine import LayerG, LayerW, TransformerStack
+from .engine import LayerViews, TransformerStack
 from .extractors import (ConvChannelFeatureExtractor, ConvFeatureExtractor, conv_stack_backward, conv_stack_forward,
                          conv_stack_forward_tf32, kmajor_weight)
 from .pos_embed import get_1d_sincos_pos_embed_from_grid
@@ -133,9 +133,10 @@ _FEATURE_PATH = ("extract_audio.", "feature_norms.", "post_extraction_mapper.", 
 
 
 class _FeaturePlan:
-    """Which parts of the feature path train in one differentiable `get_audio_representation` call.  conv / norm /
-    mapper / final_norm / layer_w[i]: some tensor of that part requires grad (its weight gradients are computed);
-    dx: the waveform requires grad (the data gradient runs down to it through every part, trainable or not)."""
+    """Which parts of the feature path a backward through `_features_forward` trains: a differentiable
+    `get_audio_representation` call, or the denoiser's student.  conv / norm / mapper / final_norm / layer_w[i]: some
+    tensor of that part trains (its weight gradients are computed); dx: the waveform gradient is wanted (the data
+    gradient runs down to it through every part, trainable or not)."""
     __slots__ = ("names", "conv", "norm", "mapper", "final_norm", "layer_w", "local", "first_layer", "dx")
 
 
@@ -150,8 +151,7 @@ class _FeatureBridge(torch.autograd.Function):
     def forward(ctx, model, audio, index, plan, *params):
         ctx.model = model
         ctx.audio_dtype = audio.dtype
-        ctx.fctx = model._features_saving(audio.to(torch.bfloat16).contiguous(), index, plan)
-        out, ctx.fctx.out = ctx.fctx.out, None
+        out, ctx.fctx = model._features_forward(audio.to(torch.bfloat16).contiguous(), index, plan)
         return out
 
     @staticmethod
@@ -420,68 +420,66 @@ class JEPA(_ModuleBase):
         self._build_weight_views()
         self._w_sig = sig
 
-    def _extractors(self):
+    def _conv_streams(self, wk: Optional[dict] = None) -> list:
+        """(prefix, weights) of the CNN that serves each conv stream, in channel order: the mono extractor runs one
+        stream over every input channel, the per-channel (Nat) extractor one mono stream per input channel, all through
+        `extract_audio.cnns.0` when it shares weights over channels.  weights: the tap-major working copies of blocks
+        1.. taken from `wk` (`_conv_wk`, or the tf32 copy), or their parameter names when wk is None."""
         ex = self.extract_audio
         if isinstance(ex, ConvChannelFeatureExtractor):
-            n = 1 if ex.share_weights_over_channels else ex.in_channels
-            return [(f"extract_audio.cnns.{c}", ex.conv_layers_spec) for c in range(n)]
-        return [("extract_audio.cnn", ex.conv_layers_spec)]
+            prefixes = [f"extract_audio.cnns.{0 if ex.share_weights_over_channels else c}" for c in range(ex.in_channels)]
+        else:
+            prefixes = ["extract_audio.cnn"]
+        names = lambda p: [f"{p}.{i}.0.weight" for i in range(1, len(ex.conv_layers_spec))]
+        return [(p, names(p) if wk is None else [wk[n] for n in names(p)]) for p in prefixes]
+
+    def _tap_major(self, flat: torch.Tensor, dtype: torch.dtype, old: Optional[dict] = None) -> dict:
+        """Tap-major working copies (kmajor_weight) of the conv weights of blocks 1.. in `flat`, by name, written into
+        the buffers of `old` where it has them."""
+        out = {}
+        for _, names in self._conv_streams():
+            for name in names:
+                if name not in out:   # a CNN shared over channels serves several streams
+                    out[name] = kmajor_weight(self._view(flat, name), (old or {}).get(name), dtype=dtype)
+        return out
 
     def _refresh_conv_weights(self) -> None:
-        if not hasattr(self, "_conv_wk"):
-            self._conv_wk = {}
-        for prefix, spec in self._extractors():
-            for i in range(1, len(spec)):
-                name = f"{prefix}.{i}.0.weight"
-                w = self._view(self._flat_p, name)
-                self._conv_wk[name] = kmajor_weight(w, self._conv_wk.get(name))
+        self._conv_wk = self._tap_major(self._flat_p, torch.bfloat16, getattr(self, "_conv_wk", None))
 
-    def _stack_weights(self, prefix: str, n_layers: int, view16: Callable, view32: Callable) -> List[LayerW]:
+    @staticmethod
+    def _stack_views(prefix: str, n_layers: int, mat: Callable, vec: Callable) -> List[LayerViews]:
+        """Per-layer views of a stack: `mat(name)` views a weight matrix, `vec(name)` a bias or LayerNorm vector (for
+        gradients both are the gradient view)."""
         out = []
         for i in range(n_layers):
             b = f"{prefix}layers.{i}."
-            w = LayerW()
-            w.w_in, w.b_in = view16(b + "self_attn.in_proj_weight"), view32(b + "self_attn.in_proj_bias")
-            w.w_o, w.b_o = view16(b + "self_attn.out_proj.weight"), view32(b + "self_attn.out_proj.bias")
-            w.w1, w.b1 = view16(b + "linear1.weight"), view32(b + "linear1.bias")
-            w.w2, w.b2 = view16(b + "linear2.weight"), view32(b + "linear2.bias")
-            w.g1, w.be1 = view32(b + "norm1.weight"), view32(b + "norm1.bias")
-            w.g2, w.be2 = view32(b + "norm2.weight"), view32(b + "norm2.bias")
+            w = LayerViews()
+            w.w_in, w.b_in = mat(b + "self_attn.in_proj_weight"), vec(b + "self_attn.in_proj_bias")
+            w.w_o, w.b_o = mat(b + "self_attn.out_proj.weight"), vec(b + "self_attn.out_proj.bias")
+            w.w1, w.b1 = mat(b + "linear1.weight"), vec(b + "linear1.bias")
+            w.w2, w.b2 = mat(b + "linear2.weight"), vec(b + "linear2.bias")
+            w.g1, w.be1 = vec(b + "norm1.weight"), vec(b + "norm1.bias")
+            w.g2, w.be2 = vec(b + "norm2.weight"), vec(b + "norm2.bias")
             out.append(w)
         return out
 
     def _build_weight_views(self) -> None:
         p16 = lambda n: self._view(self._flat_w16, n)
         p32 = lambda n: self._view(self._flat_p, n)
-        self._W_enc = self._stack_weights("encoder.", self._enc_stack.n_layers, p16, p32)
-        self._W_dec = self._stack_weights("decoder.", self._dec_stack.n_layers, p16, p32)
-        self._W_tea = self._stack_weights("", self._enc_stack.n_layers, lambda n: self._tview(self._flat_t16, n),
-                                          lambda n: self._tview(self._flat_t, n))
+        self._W_enc = self._stack_views("encoder.", self._enc_stack.n_layers, p16, p32)
+        self._W_dec = self._stack_views("decoder.", self._dec_stack.n_layers, p16, p32)
+        self._W_tea = self._stack_views("", self._enc_stack.n_layers, lambda n: self._tview(self._flat_t16, n),
+                                        lambda n: self._tview(self._flat_t, n))
 
     def _grad_views(self, gflat: torch.Tensor):
         if gflat is self._flat_g and self._gviews_cache is not None:
             return self._gviews_cache
         g = lambda n: self._view(gflat, n)
-        views = (self._stack_grads("encoder.", self._enc_stack.n_layers, g),
-                 self._stack_grads("decoder.", self._dec_stack.n_layers, g), g)
+        views = (self._stack_views("encoder.", self._enc_stack.n_layers, g, g),
+                 self._stack_views("decoder.", self._dec_stack.n_layers, g, g), g)
         if gflat is self._flat_g:
             self._gviews_cache = views
         return views
-
-    @staticmethod
-    def _stack_grads(prefix: str, n_layers: int, g: Callable) -> List[LayerG]:
-        out = []
-        for i in range(n_layers):
-            b = f"{prefix}layers.{i}."
-            w = LayerG()
-            w.w_in, w.b_in = g(b + "self_attn.in_proj_weight"), g(b + "self_attn.in_proj_bias")
-            w.w_o, w.b_o = g(b + "self_attn.out_proj.weight"), g(b + "self_attn.out_proj.bias")
-            w.w1, w.b1 = g(b + "linear1.weight"), g(b + "linear1.bias")
-            w.w2, w.b2 = g(b + "linear2.weight"), g(b + "linear2.bias")
-            w.g1, w.be1 = g(b + "norm1.weight"), g(b + "norm1.bias")
-            w.g2, w.be2 = g(b + "norm2.weight"), g(b + "norm2.bias")
-            out.append(w)
-        return out
 
     # ------------------------------------------------------------------------------------------- local features
     def _local_features(self, x16: torch.Tensor, save: bool, save_conv: Optional[bool] = None):
@@ -494,21 +492,19 @@ class JEPA(_ModuleBase):
         T, D = self.total_patches, self.encoder_embedding_dim
         C = ex.embedding_dim
         p32 = lambda n: self._view(self._flat_p, n)
+        streams = self._conv_streams(self._conv_wk)
         conv_saved = []
         if isinstance(ex, ConvChannelFeatureExtractor):
             Tc = T // ex.in_channels
             feats = torch.empty(B, T, C, device=x16.device, dtype=torch.bfloat16)
             xs = x16.transpose(0, 1).contiguous()  # [Cin, B, L]: one mono stream per CNN
-            for c in range(ex.in_channels):
-                prefix = f"extract_audio.cnns.{0 if ex.share_weights_over_channels else c}"
-                wks = [self._conv_wk[f"{prefix}.{i}.0.weight"] for i in range(1, len(ex.conv_layers_spec))]
+            for c, (prefix, wks) in enumerate(streams):
                 f, sv = conv_stack_forward(ex.conv_layers_spec, xs[c].unsqueeze(1), p32(f"{prefix}.0.0.weight"),
                                            p32(f"{prefix}.0.2.weight"), p32(f"{prefix}.0.2.bias"), wks, save_conv)
                 feats[:, c * Tc:(c + 1) * Tc].copy_(f)  # channel-major token order (audio_channel_feature_extractor.py:177-178)
                 conv_saved.append(sv)
         else:
-            prefix = "extract_audio.cnn"
-            wks = [self._conv_wk[f"{prefix}.{i}.0.weight"] for i in range(1, len(ex.conv_layers_spec))]
+            (prefix, wks), = streams
             feats, sv = conv_stack_forward(ex.conv_layers_spec, x16, p32(f"{prefix}.0.0.weight"),
                                            p32(f"{prefix}.0.2.weight"), p32(f"{prefix}.0.2.bias"), wks, save_conv)
             conv_saved.append(sv)
@@ -701,12 +697,12 @@ class JEPA(_ModuleBase):
             return
         # ---- conv stack(s)
         ex = self.extract_audio
-        exs = self._extractors()
+        streams = self._conv_streams(self._conv_wk)
         if isinstance(ex, ConvChannelFeatureExtractor):
             Tc = T // ex.in_channels
             dfeat3 = dfeat.view(B, T, C)
             for ch in range(ex.in_channels - 1, -1, -1):
-                prefix = exs[0 if ex.share_weights_over_channels else ch][0]
+                prefix, wks = streams[ch]
                 sv = conv_saved[ch]
                 dfc = dfeat3[:, ch * Tc:(ch + 1) * Tc].contiguous().view(B * Tc, C)
                 # with shared weights every channel pass adds into the SAME gradient region: it is final (and may be
@@ -714,20 +710,20 @@ class JEPA(_ModuleBase):
                 last = (not ex.share_weights_over_channels) or ch == 0
                 # each mono stream's waveform gradient lands in its channel
                 dxc = None if dx is None else torch.empty(B, 1, dx.shape[2], device=dev)
-                self._conv_backward(prefix, ex.conv_layers_spec, sv, dfc, B, Tc, C, g, ready if last else (lambda name: None),
-                                    dxc, wg_conv)
+                self._conv_backward(prefix, wks, ex.conv_layers_spec, sv, dfc, B, Tc, C, g,
+                                    ready if last else (lambda name: None), dxc, wg_conv)
                 if dx is not None:
                     dx[:, ch:ch + 1].copy_(dxc)
         else:
-            self._conv_backward(exs[0][0], ex.conv_layers_spec, conv_saved[0], dfeat, B, T, C, g, ready, dx, wg_conv)
+            (prefix, wks), = streams
+            self._conv_backward(prefix, wks, ex.conv_layers_spec, conv_saved[0], dfeat, B, T, C, g, ready, dx, wg_conv)
 
-    def _conv_backward(self, prefix, spec, sv, dfeat, B, T, C, g, ready, dx=None, weights: bool = True):
+    def _conv_backward(self, prefix, wks, spec, sv, dfeat, B, T, C, g, ready, dx=None, weights: bool = True):
         n = len(spec)
         dev = dfeat.device
         p32 = lambda nm: self._view(self._flat_p, nm)
         dh = torch.empty(B, T, C, device=dev, dtype=torch.bfloat16)
         ops.scatter_dgelu(dfeat, None, sv.pre[n - 1].view(B * T, C), B * T, dh.view(B * T, C))
-        wks = [self._conv_wk[f"{prefix}.{i}.0.weight"] for i in range(1, n)]
         gw = g if weights else (lambda nm: None)
         conv_stack_backward(spec, sv, dh, p32(f"{prefix}.0.0.weight"), p32(f"{prefix}.0.2.weight"),
                             p32(f"{prefix}.0.2.bias"), wks, gw(f"{prefix}.0.0.weight"), gw(f"{prefix}.0.2.weight"),
@@ -959,6 +955,18 @@ class JEPA(_ModuleBase):
             cache[key] = (rows.contiguous(), cu.contiguous(), reps * int(rows_1.size), int(n_per.max()) if n_per.size else 0)
         return cache[key]
 
+    def _visible_index(self, B: int, padding_mask, host_mask):
+        """None when every token is visible, else the packed index (ctx_rows, cu, Nc, max_len) of the visible rows of a
+        batch of B sequences: from host_mask when given (`_periodic_index`), else from padding_mask."""
+        T = self.total_patches
+        if host_mask is not None:
+            return self._periodic_index(host_mask, B, T)
+        if padding_mask is None:
+            return None
+        pm = padding_mask.to(self.device).reshape(B, 1, T).contiguous()
+        mi = ops.mask_indices(pm.view(B, T), torch.zeros_like(pm), pm)
+        return mi.ctx_rows, mi.cu_c, mi.Nc, mi.max_nc
+
     def _tf32_weights(self) -> dict:
         """fp32 working copy of the extractor, mapper and encoder weight matrices rounded to nearest tf32 (conv weights
         tap-major), built on first use and rebuilt when a parameter changed (load_state_dict, optimizer steps) or the flat
@@ -971,13 +979,8 @@ class JEPA(_ModuleBase):
         flat = ops.tf32_round(self._flat_p[:self._enc_range[1]])   # extractor .. encoder: the leading part of the layout
         v32 = lambda n: self._view(flat, n)
         p32 = lambda n: self._view(self._flat_p, n)
-        conv = {}
-        for prefix, spec in self._extractors():
-            for i in range(1, len(spec)):
-                name = f"{prefix}.{i}.0.weight"
-                conv[name] = kmajor_weight(v32(name), dtype=torch.float32)
-        w = dict(layers=self._stack_weights("encoder.", self._enc_stack.n_layers, v32, p32), conv=conv,
-                 mapper=v32("post_extraction_mapper.weight"))
+        w = dict(layers=self._stack_views("encoder.", self._enc_stack.n_layers, v32, p32),
+                 conv=self._tap_major(flat, torch.float32), mapper=v32("post_extraction_mapper.weight"))
         self._tf32_cache = (sig, w)
         return w
 
@@ -990,20 +993,19 @@ class JEPA(_ModuleBase):
         C = ex.embedding_dim
         p32 = lambda n: self._view(self._flat_p, n)
 
-        def stack(prefix, x):
-            wks = [w["conv"][f"{prefix}.{i}.0.weight"] for i in range(1, len(ex.conv_layers_spec))]
+        def stack(prefix, wks, x):
             return conv_stack_forward_tf32(ex.conv_layers_spec, x, p32(f"{prefix}.0.0.weight"), p32(f"{prefix}.0.2.weight"),
                                            p32(f"{prefix}.0.2.bias"), wks)
 
+        streams = self._conv_streams(w["conv"])
         if isinstance(ex, ConvChannelFeatureExtractor):
             Tc = T // ex.in_channels
             feats = torch.empty(B, T, C, device=x32.device)
             xs = x32.transpose(0, 1).contiguous()  # [Cin, B, L]: one mono stream per CNN
-            for c in range(ex.in_channels):
-                prefix = f"extract_audio.cnns.{0 if ex.share_weights_over_channels else c}"
-                feats[:, c * Tc:(c + 1) * Tc].copy_(stack(prefix, xs[c].unsqueeze(1)))
+            for c, (prefix, wks) in enumerate(streams):
+                feats[:, c * Tc:(c + 1) * Tc].copy_(stack(prefix, wks, xs[c].unsqueeze(1)))
         else:
-            feats = stack("extract_audio.cnn", x32)
+            feats = stack(*streams[0], x32)
         ln = torch.empty(B * T, C, device=x32.device)
         ops.add_layernorm_fwd_f32(feats.view(B * T, C), None, p32("feature_norms.weight"), p32("feature_norms.bias"),
                                   self.feature_norms.eps, None, ln)
@@ -1012,47 +1014,53 @@ class JEPA(_ModuleBase):
                       resid=self._pos_enc, resid_mod=T)
         return local32
 
-    def _audio_representation_tf32(self, audio: torch.Tensor, padding_mask, host_mask) -> torch.Tensor:
-        """get_audio_representation with inference_precision == "tf32" (same masking semantics)."""
-        dev = self.device
-        w = self._tf32_weights()
-        x32 = audio.to(device=dev, dtype=torch.float32).contiguous()
-        B = x32.shape[0]
+    def _visible_rows(self, local32: torch.Tensor, index, bf16: bool):
+        """The encoder's input rows: all of local32 [B*T, D] (index None) or an fp32 copy of its visible rows, and with
+        bf16 their bf16 copy.  Returns (x32, x16 | None, cu, max_len)."""
         T, D = self.total_patches, self.encoder_embedding_dim
-        local32 = self._local_features_tf32(x32, w)
-        p32 = lambda n: self._view(self._flat_p, n)
-        if padding_mask is None and host_mask is None:
-            cu = torch.arange(0, (B + 1) * T, T, device=dev, dtype=torch.int32)
-            xs32 = self._enc_stack.forward_tf32(w["layers"], local32, ops.tf32_round(local32), cu, B, T)
-            out = torch.empty(B * T, D, device=dev)
-            ops.layernorm_fwd(xs32, p32("encoder.norm.weight"), p32("encoder.norm.bias"), self.encoder.norm.eps, out,
-                              None, None, None)
-            return out.view(B, T, D)
-        if host_mask is not None:
-            ctx_rows, cu_c, Nc, max_nc = self._periodic_index(host_mask, B, T)
+        dev = local32.device
+        if index is None:
+            rows, x32, M = None, local32, local32.shape[0]
+            cu, max_len = torch.arange(0, M + T, T, device=dev, dtype=torch.int32), T
         else:
-            pm = padding_mask.to(dev).reshape(B, 1, T).contiguous()
-            mi = ops.mask_indices(pm.view(B, T), torch.zeros_like(pm), pm)
-            ctx_rows, cu_c, Nc, max_nc = mi.ctx_rows, mi.cu_c, mi.Nc, mi.max_nc
-        xc32 = torch.empty(Nc, D, device=dev)
-        ops.gather_rows(local32, ctx_rows, Nc, xc32, None)
-        xs32 = self._enc_stack.forward_tf32(w["layers"], xc32, ops.tf32_round(xc32), cu_c, B, max_nc)
-        packed = torch.empty(Nc, D, device=dev)
-        ops.layernorm_fwd(xs32, p32("encoder.norm.weight"), p32("encoder.norm.bias"), self.encoder.norm.eps, packed,
-                          None, None, None)
-        out = torch.zeros(B * T, D, device=dev)
-        ops.scatter_rows(packed, ctx_rows, Nc, out)
-        return out.view(B, T, D)
+            rows, cu, M, max_len = index
+            x32 = torch.empty(M, D, device=dev)
+        x16 = torch.empty(M, D, device=dev, dtype=torch.bfloat16) if bf16 else None
+        if index is not None or bf16:
+            ops.gather_rows(local32, rows, M, None if index is None else x32, x16)
+        return x32, x16, cu, max_len
+
+    def _final_norm(self, xs32: torch.Tensor, index, B: int, st: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """The encoder's final LayerNorm of its output rows into the features [B, T, D] fp32, scattered to the visible
+        rows when packed (padded rows are zeros); st: LayerNorm statistics for the backward."""
+        T, D = self.total_patches, self.encoder_embedding_dim
+        dev = xs32.device
+        M = xs32.shape[0]
+        out = torch.empty(B, T, D, device=dev) if index is None else torch.zeros(B, T, D, device=dev)
+        packed = out.view(B * T, D) if index is None else torch.empty(M, D, device=dev)
+        ops.layernorm_fwd(xs32, self._view(self._flat_p, "encoder.norm.weight"),
+                          self._view(self._flat_p, "encoder.norm.bias"), self.encoder.norm.eps, packed, None, st, None)
+        if index is not None:
+            ops.scatter_rows(packed, index[0], M, out.view(B * T, D))
+        return out
+
+    def _audio_representation_tf32(self, audio: torch.Tensor, index) -> torch.Tensor:
+        """get_audio_representation with inference_precision == "tf32" (same masking semantics)."""
+        w = self._tf32_weights()
+        x32 = audio.to(device=self.device, dtype=torch.float32).contiguous()
+        B = x32.shape[0]
+        xv32, _, cu, max_len = self._visible_rows(self._local_features_tf32(x32, w), index, bf16=False)
+        xs32 = self._enc_stack.forward_tf32(w["layers"], xv32, ops.tf32_round(xv32), cu, B, max_len)
+        return self._final_norm(xs32, index, B)
 
     # ------------------------------------------------------------------------------------------- fine-tuning
-    def _feature_grad_plan(self, audio_grad: bool = False) -> Optional[_FeaturePlan]:
-        """None unless grad mode is on and the waveform (audio_grad) or a feature-path parameter requires grad (the
-        rule of `forward`)."""
-        if not torch.is_grad_enabled():
-            return None
-        params = dict(self.named_parameters())
+    def _feature_plan(self, trainable, audio_grad: bool = False) -> Optional[_FeaturePlan]:
+        """What a backward through the features computes: the weight gradients of the feature-path parameters named in
+        `trainable` (other names are ignored) and, with audio_grad, the waveform gradient.  None when it computes
+        neither."""
+        trainable = set(trainable)
         names = [n for n in self._train_names if n.startswith(_FEATURE_PATH)]
-        trainable = [n for n in names if params[n].requires_grad]
+        trainable = [n for n in names if n in trainable]
         if not (trainable or audio_grad):
             return None
         plan = _FeaturePlan()
@@ -1069,62 +1077,36 @@ class JEPA(_ModuleBase):
         plan.first_layer = 0 if plan.local else min(layers, default=n_layers)
         return plan
 
-    def _audio_representation_grad(self, audio, padding_mask, host_mask, plan: _FeaturePlan) -> torch.Tensor:
-        """Differentiable get_audio_representation (same masking semantics and checks as the inference path).  audio:
-        the waveform already on the model's device (moved outside the Function, so that autograd's copy backward
-        returns its gradient to the caller's device)."""
-        B, T = audio.shape[0], self.total_patches
-        index = None
-        if host_mask is not None:
-            index = self._periodic_index(host_mask, B, T)
-        elif padding_mask is not None:
-            pm = padding_mask.to(self.device).reshape(B, 1, T).contiguous()
-            mi = ops.mask_indices(pm.view(B, T), torch.zeros_like(pm), pm)
-            index = (mi.ctx_rows, mi.cu_c, mi.Nc, mi.max_nc)
-        params = dict(self.named_parameters())
-        return _FeatureBridge.apply(self, audio, index, plan, *[params[n] for n in plan.names])
-
-    def _features_saving(self, x16: torch.Tensor, index, plan: _FeaturePlan) -> _Ctx:
-        """Forward of `_FeatureBridge`: the inference kernels plus the activations the backward needs, kept from the
-        lowest trainable point upward.  index: None (dense) or (ctx_rows, cu, Nc, max_len) of the visible rows."""
-        dev = x16.device
+    def _features_forward(self, x16: torch.Tensor, index, plan: Optional[_FeaturePlan] = None):
+        """The bf16 feature forward (bf16 [B, Cin, L] waveform -> features [B, T, D] fp32) of get_audio_representation,
+        of `_FeatureBridge` and of the denoiser's student.  index: None (dense) or (ctx_rows, cu, Nc, max_len) of the
+        visible rows.  Without a plan nothing is saved and the context is None; with one, the activations the backward
+        needs are kept from the lowest trainable point upward.  Returns (features, context)."""
         B = x16.shape[0]
-        T, D = self.total_patches, self.encoder_embedding_dim
-        p32 = lambda n: self._view(self._flat_p, n)
-        c = _Ctx()
-        c.B, c.index, c.plan = B, index, plan
+        save = plan is not None
         # (the waveform gradient runs the whole conv stack backward: its GELU' copies are kept even when it is frozen)
-        local32, local_saved = self._local_features(x16, save=plan.local, save_conv=plan.conv or plan.dx)
-        c.x_shape = x16.shape
-        c.local_saved = local_saved if plan.local else None
-        if index is None:
-            M = B * T
-            c.cu, c.max_len = torch.arange(0, (B + 1) * T, T, device=dev, dtype=torch.int32), T
-            x16r = torch.empty(M, D, device=dev, dtype=torch.bfloat16)
-            ops.gather_rows(local32, None, M, None, x16r)
-            xs32, _, c.enc_saved = self._enc_stack.forward(self._W_enc, local32, x16r, c.cu, B, T, True,
-                                                           save_from=plan.first_layer)
-        else:
-            ctx_rows, c.cu, M, c.max_len = index
-            xc32 = torch.empty(M, D, device=dev)
-            xc16 = torch.empty(M, D, device=dev, dtype=torch.bfloat16)
-            ops.gather_rows(local32, ctx_rows, M, xc32, xc16)
-            xs32, _, c.enc_saved = self._enc_stack.forward(self._W_enc, xc32, xc16, c.cu, B, c.max_len, True,
-                                                           save_from=plan.first_layer)
+        local32, local_saved = self._local_features(x16, save=save and plan.local,
+                                                    save_conv=save and (plan.conv or plan.dx))
+        x32, xv16, cu, max_len = self._visible_rows(local32, index, bf16=True)
         del local32
-        c.out = torch.empty(B, T, D, device=dev) if index is None else torch.zeros(B, T, D, device=dev)
-        packed = c.out.view(B * T, D) if index is None else torch.empty(M, D, device=dev)
-        c.norm_st = torch.empty(M, 2, device=dev)
-        ops.layernorm_fwd(xs32, p32("encoder.norm.weight"), p32("encoder.norm.bias"), self.encoder.norm.eps, packed,
-                          None, c.norm_st, None)
-        if index is not None:
-            ops.scatter_rows(packed, index[0], M, c.out.view(B * T, D))
-        c.xs32, c.M = xs32, M
-        return c
+        xs32, _, enc_saved = self._enc_stack.forward(self._W_enc, x32, xv16, cu, B, max_len, save,
+                                                     save_from=plan.first_layer if save else 0)
+        M = xs32.shape[0]
+        norm_st = torch.empty(M, 2, device=x16.device) if save else None
+        out = self._final_norm(xs32, index, B, norm_st)
+        if not save:
+            return out, None
+        c = _Ctx()
+        c.B, c.index, c.plan, c.x_shape, c.cu, c.max_len, c.M = B, index, plan, x16.shape, cu, max_len, M
+        c.local_saved = local_saved if plan.local else None
+        c.enc_saved, c.xs32, c.norm_st = enc_saved, xs32, norm_st
+        return out, c
 
-    def _features_backward(self, c: _Ctx, grad_out: torch.Tensor):
-        """Backward of `_FeatureBridge` from the fp32 gradient of the features [B, T, D].  Returns (a gradient buffer
-        over the extractor..encoder span of the flat layout, owned by this call: several graphs may be alive; the fp32
+    def _features_backward(self, c: _Ctx, grad_out: torch.Tensor, gflat: Optional[torch.Tensor] = None,
+                           on_ready: Optional[Callable] = None):
+        """Backward of `_features_forward` from the fp32 gradient of the features [B, T, D].  gflat: the gradient buffer
+        (zeroed, flat layout), by default one owned by this call over the extractor..encoder span (several graphs may be
+        alive); on_ready(offset) announces that gflat[offset:] is final (bucketed all-reduce).  Returns (gflat, the fp32
         gradient of the bf16 waveform [B, Cin, L] when plan.dx, else None).  Only the parts with a trainable tensor
         compute weight gradients."""
         dev = c.xs32.device
@@ -1132,8 +1114,10 @@ class JEPA(_ModuleBase):
         T, D = self.total_patches, self.encoder_embedding_dim
         n_layers = self._enc_stack.n_layers
         p32 = lambda n: self._view(self._flat_p, n)
-        gflat = torch.zeros(self._enc_range[1], device=dev)
+        if gflat is None:
+            gflat = torch.zeros(self._enc_range[1], device=dev)
         g = lambda n: self._view(gflat, n)
+        ready = (lambda name: on_ready(self._offsets[name][0])) if on_ready is not None else (lambda name: None)
         dy = grad_out.to(device=dev, dtype=torch.float32).contiguous().view(B * T, D)
         if c.index is not None:   # padded rows are constants: only the visible rows' gradient enters
             dyp = torch.empty(M, D, device=dev)
@@ -1143,12 +1127,16 @@ class JEPA(_ModuleBase):
         ops.layernorm_bwd(dy, c.xs32, c.norm_st, p32("encoder.norm.weight"), dxs, None,
                           *((g("encoder.norm.weight"), g("encoder.norm.bias")) if plan.final_norm else (None, None)),
                           None)
+        ready("encoder.norm.weight")
         c.xs32 = None
         daudio = torch.empty(c.x_shape, device=dev) if plan.dx else None
         if plan.first_layer < n_layers:
-            dx = self._enc_stack.backward(self._W_enc, self._stack_grads("encoder.", n_layers, g), c.enc_saved, dxs,
-                                          c.cu, B, c.max_len, stop_at=plan.first_layer, need_dx=plan.local,
-                                          need_wgrad=plan.layer_w)
+            # (the cached views of _grad_views slice the whole layout: a call-owned buffer gets its own encoder views)
+            G_enc = self._grad_views(gflat)[0] if gflat is self._flat_g else \
+                self._stack_views("encoder.", n_layers, g, g)
+            dx = self._enc_stack.backward(self._W_enc, G_enc, c.enc_saved, dxs, c.cu, B, c.max_len,
+                                          lambda i: ready(f"encoder.layers.{i}.self_attn.in_proj_weight"),
+                                          stop_at=plan.first_layer, need_dx=plan.local, need_wgrad=plan.layer_w)
             if plan.local:
                 # the mapper output is bf16 (autocast), so is its gradient on the dense token grid
                 if c.index is None:
@@ -1158,7 +1146,7 @@ class JEPA(_ModuleBase):
                     dlocal16 = torch.zeros(B * T, D, device=dev, dtype=torch.bfloat16)
                     ops.scatter_dgelu(dx, c.index[0], None, M, dlocal16)
                 del dx
-                self._local_backward(c.local_saved, dlocal16, B, g, lambda name: None,
+                self._local_backward(c.local_saved, dlocal16, B, g, ready,
                                      norm=plan.norm or plan.conv or plan.dx, conv=plan.conv or plan.dx, dx=daudio,
                                      wg_mapper=plan.mapper, wg_norm=plan.norm, wg_conv=plan.conv)
         c.enc_saved = c.local_saved = None
@@ -1194,42 +1182,15 @@ class JEPA(_ModuleBase):
         self.eval()
         self._ensure_ready()
         self._sync_weights()
+        index = self._visible_index(audio.shape[0], padding_mask, host_mask)
         if self.inference_precision == "tf32":
-            return self._audio_representation_tf32(audio, padding_mask, host_mask)
+            return self._audio_representation_tf32(audio, index)
         dev = self.device
-        plan = self._feature_grad_plan(audio.requires_grad)
-        if plan is not None:
-            if plan.dx:   # moved outside the Function: autograd's copy backward takes the gradient back to audio.device
-                return self._audio_representation_grad(audio.to(device=dev), padding_mask, host_mask, plan)
-            return self._audio_representation_grad(audio.to(device=dev, dtype=torch.bfloat16).contiguous(),
-                                                   padding_mask, host_mask, plan)
-        x16 = audio.to(device=dev, dtype=torch.bfloat16).contiguous()
-        B = x16.shape[0]
-        T, D = self.total_patches, self.encoder_embedding_dim
-        local32, _ = self._local_features(x16, save=False)
-        p32 = lambda n: self._view(self._flat_p, n)
-        if padding_mask is None and host_mask is None:
-            cu = torch.arange(0, (B + 1) * T, T, device=dev, dtype=torch.int32)
-            x16r = torch.empty(B * T, D, device=dev, dtype=torch.bfloat16)
-            ops.gather_rows(local32, None, B * T, None, x16r)
-            xs32, _, _ = self._enc_stack.forward(self._W_enc, local32, x16r, cu, B, T, False)
-            out = torch.empty(B * T, D, device=dev)
-            ops.layernorm_fwd(xs32, p32("encoder.norm.weight"), p32("encoder.norm.bias"), self.encoder.norm.eps, out,
-                              None, None, None)
-            return out.view(B, T, D)
-        if host_mask is not None:
-            ctx_rows, cu_c, Nc, max_nc = self._periodic_index(host_mask, B, T)
-        else:
-            pm = padding_mask.to(dev).reshape(B, 1, T).contiguous()
-            mi = ops.mask_indices(pm.view(B, T), torch.zeros_like(pm), pm)
-            ctx_rows, cu_c, Nc, max_nc = mi.ctx_rows, mi.cu_c, mi.Nc, mi.max_nc
-        xc32 = torch.empty(Nc, D, device=dev)
-        xc16 = torch.empty(Nc, D, device=dev, dtype=torch.bfloat16)
-        ops.gather_rows(local32, ctx_rows, Nc, xc32, xc16)
-        xs32, _, _ = self._enc_stack.forward(self._W_enc, xc32, xc16, cu_c, B, max_nc, False)
-        packed = torch.empty(Nc, D, device=dev)
-        ops.layernorm_fwd(xs32, p32("encoder.norm.weight"), p32("encoder.norm.bias"), self.encoder.norm.eps, packed,
-                          None, None, None)
-        out = torch.zeros(B * T, D, device=dev)
-        ops.scatter_rows(packed, ctx_rows, Nc, out)
-        return out.view(B, T, D)
+        plan = None
+        if torch.is_grad_enabled():   # the rule of `forward`
+            plan = self._feature_plan([n for n, p in self.named_parameters() if p.requires_grad], audio.requires_grad)
+        if plan is None:
+            return self._features_forward(audio.to(device=dev, dtype=torch.bfloat16).contiguous(), index)[0]
+        params = dict(self.named_parameters())
+        # audio moves to the device outside the Function: autograd's copy backward takes the gradient back to audio.device
+        return _FeatureBridge.apply(self, audio.to(device=dev), index, plan, *[params[n] for n in plan.names])
