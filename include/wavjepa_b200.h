@@ -273,6 +273,10 @@ int wj_gather_rows(const void* src, int src_is_bf16, const int* idx, int N, int 
 /* out[idx[i], :] = src[i, :] (fp32): packed encoder rows back to their dense [B*T, D] positions
  * (JEPA.get_audio_representation, wavjepa/jepa.py:456-467). */
 int wj_scatter_rows(const float* src, const int* idx, int N, int D, float* out, void* stream);
+/* a[r, :] += b[idx[r], :] for r < N (fp32; idx NULL = identity): the gradient of a returned hidden state added into the
+ * encoder backward at its layer boundary, read from the dense [B*T, D] gradient through the packed-row index
+ * (JEPA.get_hidden_states).  One writer per element: bit-identical from run to run. */
+int wj_add_rows_f32(float* a, const float* b, const int* idx, int N, int D, void* stream);
 /* out_bf16[idx[i], :] = src[i, :] * h[idx[i], :] (h = the GELU' factors saved by an act == 1 GEMM epilogue; may be
  * NULL; idx NULL = identity); rows not listed are left untouched. */
 int wj_scatter_dgelu(const float* src, const int* idx, const void* h_bf16, int N, int D, void* out_bf16, void* stream);

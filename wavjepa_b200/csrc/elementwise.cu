@@ -72,6 +72,25 @@ __global__ void __launch_bounds__(256) scatter_rows_kernel(const float* __restri
   }
 }
 
+// a[r, :] += b[idx ? idx[r] : r, :]: one warp per row, float4 loads and stores.  Every element has one writer, so the
+// sum is the same bits from run to run without a deterministic-mode variant.
+__global__ void __launch_bounds__(256) add_rows_f32_kernel(float* __restrict__ a, const float* __restrict__ b,
+                                                           const int* __restrict__ idx, int N, int D4) {
+  const int lane = threadIdx.x & 31;
+  const long long warps = (static_cast<long long>(gridDim.x) * blockDim.x) >> 5;
+  for (long long r = (blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x) >> 5; r < N; r += warps) {
+    const long long sr = idx ? idx[r] : r;
+    float4* ar = reinterpret_cast<float4*>(a) + r * D4;
+    const float4* br = reinterpret_cast<const float4*>(b) + sr * D4;
+    for (int c = lane; c < D4; c += 32) {
+      float4 x = ar[c];
+      const float4 y = br[c];
+      x.x += y.x; x.y += y.y; x.z += y.z; x.w += y.w;
+      ar[c] = x;
+    }
+  }
+}
+
 // gain[clip] = 10^((target_dbfs - 20 log10(rms)) / 20), rms over all channels and samples of the clip; 1 if rms == 0
 __global__ void __launch_bounds__(512) clip_gain_kernel(const float* __restrict__ audio, long long per_clip,
                                                         float target_dbfs, float* __restrict__ gain) {
@@ -489,6 +508,13 @@ extern "C" int wj_scatter_rows(const float* src, const int* idx, int N, int D, f
   const long long n4 = static_cast<long long>(N) * (D / 4);
   scatter_rows_kernel<<<grid_for(n4), 256, 0, WJ_STREAM(stream)>>>(src, idx, n4, D / 4, out);
   return check_launch("scatter_rows");
+}
+
+extern "C" int wj_add_rows_f32(float* a, const float* b, const int* idx, int N, int D, void* stream) {
+  if (N <= 0) return WJ_OK;
+  if (D % 4) { set_error("wj_add_rows_f32: D %% 4 != 0"); return WJ_ERR_ARG; }
+  add_rows_f32_kernel<<<grid_for(static_cast<long long>(N) * 32), 256, 0, WJ_STREAM(stream)>>>(a, b, idx, N, D / 4);
+  return check_launch("add_rows_f32");
 }
 
 extern "C" int wj_clip_gain(const float* audio, int n_clips, int channels, int64_t clip_len, float target_dbfs,

@@ -96,10 +96,11 @@ class TransformerStack:
         return x32, x16, saved
 
     def forward_tf32(self, layers: List[LayerViews], x32: torch.Tensor, xop: torch.Tensor, cu: torch.Tensor, n_seqs: int,
-                     max_len: int) -> torch.Tensor:
+                     max_len: int, layer_hook: Optional[Callable] = None) -> torch.Tensor:
         """Inference forward at reference precision (the reference's fp32 feature extraction): the same packed layout,
         `layers` hold fp32 weight matrices rounded to nearest tf32.  x32: [M, d] fp32 residual stream, xop: its copy
-        rounded to nearest tf32.  Returns the fp32 output of the last layer.
+        rounded to nearest tf32.  Returns the fp32 output of the last layer; layer_hook(i, x32) is called with the
+        output of layer i (a buffer the stack does not write again).
 
         Every GEMM runs on the tf32 tensor cores with operands rounded to nearest as they are written (the tensor core
         would truncate raw fp32); attention keeps bf16 Q/K/V and P but writes O in fp32; the Linear outputs stay fp32
@@ -108,7 +109,7 @@ class TransformerStack:
         M = x32.shape[0]
         dev = x32.device
         bf, f32 = torch.bfloat16, torch.float32
-        for w in layers:
+        for i, w in enumerate(layers):
             qkv = _empty((M, 3 * d), bf, dev)
             ops.gemm_tf32(ops.plain_operand(xop), w.w_in, M, 1, qkv, bias=w.b_in)
             att = _empty((M, d), f32, dev)
@@ -129,14 +130,21 @@ class TransformerStack:
             x32 = _empty((M, d), f32, dev)
             xop = _empty((M, d), f32, dev)
             ops.add_layernorm_fwd_f32(x1_32, o2, w.g2, w.be2, self.eps, x32, xop)
+            if layer_hook is not None:
+                layer_hook(i, x32)
         return x32
 
     # ------------------------------------------------------------------------------------------------ backward
     def backward(self, layers: List[LayerViews], grads: List[LayerViews], saved: List[LayerSaved], dx: torch.Tensor,
                  cu: torch.Tensor, n_seqs: int, max_len: int, on_layer_done: Optional[Callable] = None,
-                 stop_at: int = 0, need_dx: bool = True, need_wgrad: Optional[Sequence[bool]] = None):
-        """dx: fp32 [M, d] gradient w.r.t. the stack output (before any final norm).  Accumulates parameter
+                 stop_at: int = 0, need_dx: bool = True, need_wgrad: Optional[Sequence[bool]] = None,
+                 inject: Optional[Callable] = None):
+        """dx: fp32 [M, d] gradient w.r.t. the stack output (before any final norm), only read.  Accumulates parameter
         gradients into `grads` (pre-zeroed) and returns the gradient w.r.t. the stack input (fp32).
+
+        inject(i, dx): called at the top of the iteration of every layer i below the last one, before its LayerNorm
+        backward, with the fp32 half of the gradient w.r.t. layer i's output (a buffer of the stack); it may add a
+        gradient of that output which reaches it from outside the stack (a returned hidden state).
 
         Between layers the gradient travels as a pair (fp32 residual branch, bf16 Linear data gradient -- bf16 is
         what autocast's Linear backward returns); the pair is summed inside the next LayerNorm backward.
@@ -153,6 +161,8 @@ class TransformerStack:
         for i in range(len(layers) - 1, stop_at - 1, -1):
             w, gw, s = layers[i], grads[i], saved[i]
             wg = need_wgrad is None or need_wgrad[i]
+            if inject is not None and dx_b is not None:
+                inject(i, dx)
             # ---- LN2 and the MLP
             dy2 = _empty((M, d), f32, dev)
             dy2_16 = _empty((M, d), bf, dev)

@@ -18,7 +18,9 @@ B200-first differences (results identical at every returned frame):
                         features agree with the fp32 reference to <= 1e-2 relative L2 (tests/test_gpu_model.py);
       "tf32"            the reference's fp32 feature extraction with every GEMM operand rounded to nearest tf32, fp32
                         accumulation, residual stream and chunk audio, exact erf GELU: <= 2e-3 relative L2
-                        (tests/test_gpu_tf32.py), at a lower throughput (DESIGN.md 2.1).
+                        (tests/test_gpu_tf32.py), at a lower throughput (DESIGN.md 2.1);
+  * `layer=k` on the loaders embeds encoder hidden state k (JEPA.get_hidden_states) instead of the final features, so a
+    layer sweep is one more runner option; only the first k encoder layers run (DESIGN.md 2.4).
 """
 from __future__ import annotations
 
@@ -66,11 +68,12 @@ def get_timestamps(sample_rate: int, B: int, input_audio_len: int, n_frames: int
 
 @torch.no_grad()
 def embed_chunks(model: JEPA, a: torch.Tensor, gain: Optional[torch.Tensor], unit: int, steps: int, sr: int,
-                 channel_tokens: int = 1):
+                 channel_tokens: int = 1, layer: Optional[int] = None):
     """The chunk loop of hear_api/runtime.py:107-142 (and ARCH/configs/wavjepa_wrapper.py:67-110) as ONE batched pass:
     a [B, C, L] fp32 on the device, gain [B] or None.  Chunk i of clip b = gain * a[b, :, i*unit:(i+1)*unit] (zeros past
     L), normalised per chunk (mean / unbiased std including the zero padding, runtime.py:12-16); the frames that fall
-    into the padding are key-masked and cut off.  Returns (emb [B, cut_off, D] fp32, cut_off)."""
+    into the padding are key-masked and cut off.  layer: embed hidden state `layer` of `JEPA.get_hidden_states`
+    instead of the final features (None).  Returns (emb [B, cut_off, D] fp32, cut_off)."""
     B, C, L = a.shape
     pad, n_chunks, cut_off, total_steps = hear_geometry(L, unit, sr, steps)
     dev = a.device
@@ -87,13 +90,18 @@ def embed_chunks(model: JEPA, a: torch.Tensor, gain: Optional[torch.Tensor], uni
     mask = torch.zeros(max(total_steps, n_chunks * steps), dtype=torch.bool)
     mask[cut_off:total_steps] = True
     mask = mask[:n_chunks * steps].reshape(n_chunks, steps)
+
+    def features(host_mask):
+        if layer is None:
+            return model.get_audio_representation(x16, None, host_mask=host_mask)
+        return model.get_hidden_states(x16, None, host_mask=host_mask, layers=[layer])[0]
     if channel_tokens > 1:
         # WavJEPA-Nat (hear_api/runtime_natjepa.py:142-147): the model emits channel-major tokens [c0 t0.., c1 t0..]; the
         # time mask is repeated "B E -> B (C E)" and the per-channel embeddings are averaged
-        emb = model.get_audio_representation(x16, None, host_mask=mask.repeat(1, channel_tokens).numpy())   # [B*n_chunks, C*steps, D]
+        emb = features(mask.repeat(1, channel_tokens).numpy())   # [B*n_chunks, C*steps, D]
         emb = emb.view(B * n_chunks, channel_tokens, steps, -1).mean(dim=1)
     else:
-        emb = model.get_audio_representation(x16, None, host_mask=mask.numpy())   # [B*n_chunks, steps, D] fp32
+        emb = features(mask.numpy())   # [B*n_chunks, steps, D] fp32
     return emb.reshape(B, n_chunks * steps, -1)[:, :cut_off], cut_off
 
 
@@ -101,7 +109,8 @@ class RuntimeJEPA(nn.Module):
     """reference hear_api/runtime.py:39-155."""
 
     def __init__(self, in_channels: int, weights, is_spectrogram: bool, process_seconds: float, extractor,
-                 model_size: str, sr: int, device: Optional[str] = None, precision: str = "bf16", **kwargs) -> None:
+                 model_size: str, sr: int, device: Optional[str] = None, precision: str = "bf16",
+                 layer: Optional[int] = None, **kwargs) -> None:
         super().__init__()
         if is_spectrogram:
             raise WavJepaLibError("spectrogram front-ends are not part of WavJEPA")
@@ -115,6 +124,9 @@ class RuntimeJEPA(nn.Module):
                           transformer_decoder_layers_cfg=TransformerLayerCFG.create(d_model=384), resample_sr=sr,
                           size=model_size, process_audio_seconds=process_seconds)
         self.model.inference_precision = precision   # "bf16" or "tf32" (ValueError otherwise), see the module docstring
+        if layer is not None:
+            self.model._hidden_layers([layer])        # ValueError unless an int in [0, N]
+        self.layer = layer
         if weights is None:
             raise TypeError("load_model needs a checkpoint: weights['state_dict'] (the reference fails here too, "
                             "hear_api/runtime.py:64)")
@@ -152,7 +164,8 @@ class RuntimeJEPA(nn.Module):
     def get_timestamp_embeddings(self, audio: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
         a, gain = self.to_feature(audio)
         B, _, L = a.shape
-        emb, _ = embed_chunks(self.model, a, gain, self.unit_frames, self.output_steps, self.sample_rate)
+        emb, _ = embed_chunks(self.model, a, gain, self.unit_frames, self.output_steps, self.sample_rate,
+                              layer=self.layer)
         ts = get_timestamps(self.sample_rate, B, L, emb.shape[1])
         return emb, ts
 
@@ -204,7 +217,8 @@ class RuntimeNatJEPA(RuntimeJEPA):
     def get_timestamp_embeddings(self, audio: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
         a, gain = self.to_feature(audio)
         B, C, L = a.shape
-        emb, _ = embed_chunks(self.model, a, gain, self.unit_frames, self.output_steps, self.sample_rate, channel_tokens=C)
+        emb, _ = embed_chunks(self.model, a, gain, self.unit_frames, self.output_steps, self.sample_rate, channel_tokens=C,
+                              layer=self.layer)
         ts = get_timestamps(self.sample_rate, B, L, emb.shape[1])
         return emb, ts
 
@@ -221,29 +235,34 @@ def _load_weights(args):
     return torch.load(w, weights_only=False, map_location="cpu")
 
 
-def load_model(*args, precision: str = "bf16", **kwargs) -> RuntimeJEPA:
+def load_model(*args, precision: str = "bf16", layer: Optional[int] = None, **kwargs) -> RuntimeJEPA:
     """hear_configs/WavJEPA.py:11-35.  args[0]: checkpoint path (or an already loaded dict with 'state_dict').
-    precision: "bf16" (default) or "tf32" (reference-precision features, see the module docstring)."""
+    precision: "bf16" (default) or "tf32" (reference-precision features, see the module docstring).
+    layer: None (default) embeds the final features; an int k in [0, N] embeds encoder hidden state k
+    (`JEPA.get_hidden_states`: 0 the encoder input, k the output of layer k - 1), for layer-wise probing."""
     extractor = ConvFeatureExtractor(conv_layers_spec=BASE_SPEC, in_channels=1)
     return RuntimeJEPA(in_channels=1, process_seconds=2.01, weights=_load_weights(args), sr=SR, model_size="base",
-                       is_spectrogram=False, extractor=extractor, precision=precision, **kwargs)
+                       is_spectrogram=False, extractor=extractor, precision=precision, layer=layer, **kwargs)
 
 
-def load_model_w2v2(*args, precision: str = "bf16", **kwargs) -> RuntimeJEPA:
-    """hear_configs/WavJEPA_w2v2.py:11-35: 7-layer wav2vec2 extractor (stride 320), 4.02 s windows -> 200 tokens."""
+def load_model_w2v2(*args, precision: str = "bf16", layer: Optional[int] = None, **kwargs) -> RuntimeJEPA:
+    """hear_configs/WavJEPA_w2v2.py:11-35: 7-layer wav2vec2 extractor (stride 320), 4.02 s windows -> 200 tokens.
+    precision, layer: as in load_model."""
     extractor = ConvFeatureExtractor(conv_layers_spec=W2V2_SPEC, in_channels=1)
     return RuntimeJEPA(in_channels=1, process_seconds=4.02, weights=_load_weights(args), sr=SR, model_size="base",
-                       is_spectrogram=False, extractor=extractor, precision=precision, **kwargs)
+                       is_spectrogram=False, extractor=extractor, precision=precision, layer=layer, **kwargs)
 
 
-def load_model_nat(*args, share_weights_over_channels: bool = False, precision: str = "bf16", **kwargs) -> RuntimeNatJEPA:
+def load_model_nat(*args, share_weights_over_channels: bool = False, precision: str = "bf16",
+                   layer: Optional[int] = None, **kwargs) -> RuntimeNatJEPA:
     """WavJEPA-Nat counterpart of load_model (README.md:93-108 `labhamlet/wavjepa-nat-base`): per-channel extractors
-    (wavjepa/extractors/audio_channel_feature_extractor.py), 2 x 200 tokens per 2.01 s window."""
+    (wavjepa/extractors/audio_channel_feature_extractor.py), 2 x 200 tokens per 2.01 s window.  precision, layer: as
+    in load_model (the hidden state is averaged over the two channels like the final features)."""
     from .extractors import ConvChannelFeatureExtractor
     extractor = ConvChannelFeatureExtractor(conv_layers_spec=BASE_SPEC, in_channels=2,
                                             share_weights_over_channels=share_weights_over_channels)
     return RuntimeNatJEPA(in_channels=2, process_seconds=2.01, weights=_load_weights(args), sr=SR, model_size="base",
-                          is_spectrogram=False, extractor=extractor, precision=precision, **kwargs)
+                          is_spectrogram=False, extractor=extractor, precision=precision, layer=layer, **kwargs)
 
 
 def get_scene_embeddings(audio, model):

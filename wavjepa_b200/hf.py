@@ -80,7 +80,9 @@ class WavJEPAModel(nn.Module):
                         **kwargs) -> "WavJEPAModel":
         """checkpoint: path to (or dict of) a Lightning checkpoint with 'state_dict' (hub names cannot be resolved here:
         there is no network).  nat: build the binaural WavJEPA-Nat runtime (default: inferred from the state-dict keys).
-        precision: "bf16" (default) or "tf32" (reference-precision features, wavjepa_b200.hear)."""
+        precision: "bf16" (default) or "tf32" (reference-precision features, wavjepa_b200.hear).  Other keyword
+        arguments go to the HEAR loader, e.g. layer=k: embed encoder hidden state k instead of the final features
+        (hear.load_model, JEPA.get_hidden_states)."""
         for k in ("trust_remote_code", "force_download"):
             kwargs.pop(k, None)
         ck = hear._load_weights((checkpoint,))
@@ -99,7 +101,7 @@ extractor = WavJEPAFeatureExtractor()
 
 def load_model(*args, precision: str = "bf16", **kwargs) -> WavJEPAModel:
     """hear_configs/WavJEPA_huggingface.py:19-24 (there: the hub model; here: args[0] = local checkpoint path / dict).
-    precision: "bf16" (default) or "tf32"."""
+    precision: "bf16" (default) or "tf32"; other keyword arguments (e.g. layer=k) as in WavJEPAModel.from_pretrained."""
     model = WavJEPAModel.from_pretrained(args[0], precision=precision, **kwargs)
     model.sample_rate = SAMPLING_RATE
     return model

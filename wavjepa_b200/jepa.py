@@ -141,32 +141,37 @@ class _FeaturePlan:
 
 
 class _FeatureBridge(torch.autograd.Function):
-    """Makes the features of `get_audio_representation` differentiable: the forward runs the saving kernels, the
-    backward runs the hand-written chain (final LayerNorm -> encoder layers -> mapper / feature norm / conv stack, down
+    """Makes the features of `get_audio_representation` (collect None) or the hidden states `collect` of
+    `get_hidden_states` (a tuple) differentiable: the forward runs the saving kernels, the backward runs the hand-written
+    chain (final LayerNorm or the hidden states' gradients -> encoder layers -> mapper / feature norm / conv stack, down
     to conv block 0's data gradient when the waveform requires grad) into a gradient buffer owned by this call and hands
     autograd the gradients of the inputs it asks for.  `audio` is the waveform on the model's device in the caller's
     dtype; its gradient is returned in that dtype."""
 
     @staticmethod
-    def forward(ctx, model, audio, index, plan, *params):
+    def forward(ctx, model, audio, index, plan, collect, *params):
         ctx.model = model
         ctx.audio_dtype = audio.dtype
-        out, ctx.fctx = model._features_forward(audio.to(torch.bfloat16).contiguous(), index, plan)
-        return out
+        out, ctx.fctx = model._features_forward(audio.to(torch.bfloat16).contiguous(), index, plan, collect)
+        if collect is None:
+            return out
+        ctx.set_materialize_grads(False)   # hidden states the loss does not read arrive as None and cost nothing
+        return tuple(out)
 
     @staticmethod
-    def backward(ctx, grad_out):
+    def backward(ctx, *grad_out):
         c = ctx.fctx
         if c is None:
-            raise RuntimeError("get_audio_representation: this graph was already backpropagated and its saved "
-                               "activations are freed; run the forward again (retain_graph is not supported)")
+            raise RuntimeError("get_audio_representation / get_hidden_states: this graph was already backpropagated "
+                               "and its saved activations are freed; run the forward again (retain_graph is not "
+                               "supported)")
         ctx.fctx = None
         model = ctx.model
-        gflat, dx = model._features_backward(c, grad_out)
-        needs = ctx.needs_input_grad[4:]
+        gflat, dx = model._features_backward(c, grad_out[0] if c.collect is None else list(grad_out))
+        needs = ctx.needs_input_grad[5:]
         grads = [model._view(gflat, n) if needs[i] else None for i, n in enumerate(c.plan.names)]
         daudio = dx.to(ctx.audio_dtype) if dx is not None and ctx.needs_input_grad[1] else None
-        return (None, daudio, None, None, *grads)
+        return (None, daudio, None, None, None, *grads)
 
 
 # =================================================================================================== model
@@ -1054,12 +1059,16 @@ class JEPA(_ModuleBase):
         return self._final_norm(xs32, index, B)
 
     # ------------------------------------------------------------------------------------------- fine-tuning
-    def _feature_plan(self, trainable, audio_grad: bool = False) -> Optional[_FeaturePlan]:
+    def _feature_plan(self, trainable, audio_grad: bool = False, top: Optional[int] = None) -> Optional[_FeaturePlan]:
         """What a backward through the features computes: the weight gradients of the feature-path parameters named in
         `trainable` (other names are ignored) and, with audio_grad, the waveform gradient.  None when it computes
-        neither."""
+        neither.  top (hidden states up to `top`): the path ends at the output of encoder layer top - 1, so the layers
+        from `top` on and the final norm are not part of it."""
         trainable = set(trainable)
         names = [n for n in self._train_names if n.startswith(_FEATURE_PATH)]
+        if top is not None:
+            names = [n for n in names if not n.startswith("encoder.") or
+                     (n.startswith("encoder.layers.") and int(n.split(".")[2]) < top)]
         trainable = [n for n in names if n in trainable]
         if not (trainable or audio_grad):
             return None
@@ -1077,39 +1086,73 @@ class JEPA(_ModuleBase):
         plan.first_layer = 0 if plan.local else min(layers, default=n_layers)
         return plan
 
-    def _features_forward(self, x16: torch.Tensor, index, plan: Optional[_FeaturePlan] = None):
+    def _dense_rows(self, x32: torch.Tensor, index, B: int, copy: bool = False) -> torch.Tensor:
+        """Encoder rows [M, D] fp32 on the token grid [B, T, D]: scattered into zeros when packed (a fresh buffer);
+        dense: x32 itself, or with `copy` a copy of it (a buffer the backward reads must not be handed out)."""
+        T, D = self.total_patches, self.encoder_embedding_dim
+        if index is None:
+            if copy:
+                out = torch.empty_like(x32)
+                ops.gather_rows(x32, None, x32.shape[0], out, None)
+                x32 = out
+            return x32.view(B, T, D)
+        out = torch.zeros(B, T, D, device=x32.device)
+        ops.scatter_rows(x32, index[0], x32.shape[0], out.view(B * T, D))
+        return out
+
+    def _features_forward(self, x16: torch.Tensor, index, plan: Optional[_FeaturePlan] = None,
+                          collect: Optional[List[int]] = None):
         """The bf16 feature forward (bf16 [B, Cin, L] waveform -> features [B, T, D] fp32) of get_audio_representation,
         of `_FeatureBridge` and of the denoiser's student.  index: None (dense) or (ctx_rows, cu, Nc, max_len) of the
-        visible rows.  Without a plan nothing is saved and the context is None; with one, the activations the backward
-        needs are kept from the lowest trainable point upward.  Returns (features, context)."""
+        visible rows.  collect (get_hidden_states): instead of the features, the list of hidden states `collect` [B, T, D]
+        fp32 (0: the encoder input, k: the output of layer k - 1); only the layers below max(collect) run and the final
+        norm does not.  Without a plan nothing is saved and the context is None; with one, the activations the backward
+        needs are kept from the lowest trainable point upward.  Returns (features or hidden states, context)."""
         B = x16.shape[0]
         save = plan is not None
+        top = self._enc_stack.n_layers if collect is None else max(collect)
         # (the waveform gradient runs the whole conv stack backward: its GELU' copies are kept even when it is frozen)
         local32, local_saved = self._local_features(x16, save=save and plan.local,
                                                     save_conv=save and (plan.conv or plan.dx))
-        x32, xv16, cu, max_len = self._visible_rows(local32, index, bf16=True)
+        x32, xv16, cu, max_len = self._visible_rows(local32, index, bf16=top > 0)
         del local32
-        xs32, _, enc_saved = self._enc_stack.forward(self._W_enc, x32, xv16, cu, B, max_len, save,
+        M = x32.shape[0]
+        hook, hidden = None, {}
+        if collect is not None:
+            # every hidden state below the top is an input the backward reads (the top one nothing else holds)
+            if 0 in collect:
+                hidden[0] = self._dense_rows(x32, index, B, copy=save and top > 0)
+
+            def hook(i, y, _):
+                if i + 1 in collect:
+                    hidden[i + 1] = self._dense_rows(y, index, B, copy=save and i + 1 < top)
+        xs32, _, enc_saved = self._enc_stack.forward(self._W_enc[:top], x32, xv16, cu, B, max_len, save, hook,
                                                      save_from=plan.first_layer if save else 0)
-        M = xs32.shape[0]
-        norm_st = torch.empty(M, 2, device=x16.device) if save else None
-        out = self._final_norm(xs32, index, B, norm_st)
+        norm_st = None
+        if collect is None:
+            norm_st = torch.empty(M, 2, device=x16.device) if save else None
+            out = self._final_norm(xs32, index, B, norm_st)
+        else:
+            out = [hidden[k] for k in collect]
         if not save:
             return out, None
         c = _Ctx()
         c.B, c.index, c.plan, c.x_shape, c.cu, c.max_len, c.M = B, index, plan, x16.shape, cu, max_len, M
+        c.collect = collect
         c.local_saved = local_saved if plan.local else None
-        c.enc_saved, c.xs32, c.norm_st = enc_saved, xs32, norm_st
+        c.enc_saved, c.xs32, c.norm_st = enc_saved, (xs32 if collect is None else None), norm_st
         return out, c
 
-    def _features_backward(self, c: _Ctx, grad_out: torch.Tensor, gflat: Optional[torch.Tensor] = None,
+    def _features_backward(self, c: _Ctx, grad_out, gflat: Optional[torch.Tensor] = None,
                            on_ready: Optional[Callable] = None):
-        """Backward of `_features_forward` from the fp32 gradient of the features [B, T, D].  gflat: the gradient buffer
-        (zeroed, flat layout), by default one owned by this call over the extractor..encoder span (several graphs may be
-        alive); on_ready(offset) announces that gflat[offset:] is final (bucketed all-reduce).  Returns (gflat, the fp32
-        gradient of the bf16 waveform [B, Cin, L] when plan.dx, else None).  Only the parts with a trainable tensor
-        compute weight gradients."""
-        dev = c.xs32.device
+        """Backward of `_features_forward` from the fp32 gradient of the features [B, T, D], or (a context with
+        `collect`) from the list of the gradients of the hidden states, None for those the loss does not read: the
+        highest one that is read starts the encoder backward, every other one is added to the gradient at its layer
+        boundary (ops.add_rows).  gflat: the gradient buffer (zeroed, flat layout), by default one owned by this call over
+        the extractor..encoder span (several graphs may be alive); on_ready(offset) announces that gflat[offset:] is
+        final (bucketed all-reduce).  Returns (gflat, the fp32 gradient of the bf16 waveform [B, Cin, L] when plan.dx,
+        else None).  Only the parts with a trainable tensor compute weight gradients."""
+        dev = self._flat_p.device
         B, M, plan = c.B, c.M, c.plan
         T, D = self.total_patches, self.encoder_embedding_dim
         n_layers = self._enc_stack.n_layers
@@ -1118,37 +1161,65 @@ class JEPA(_ModuleBase):
             gflat = torch.zeros(self._enc_range[1], device=dev)
         g = lambda n: self._view(gflat, n)
         ready = (lambda name: on_ready(self._offsets[name][0])) if on_ready is not None else (lambda name: None)
-        dy = grad_out.to(device=dev, dtype=torch.float32).contiguous().view(B * T, D)
-        if c.index is not None:   # padded rows are constants: only the visible rows' gradient enters
+        rows = None if c.index is None else c.index[0]
+
+        def dense(gr):
+            return gr.to(device=dev, dtype=torch.float32).contiguous().view(B * T, D)
+
+        def packed(dy):   # padded rows are constants: only the visible rows' gradient enters
+            if rows is None:
+                return dy
             dyp = torch.empty(M, D, device=dev)
-            ops.gather_rows(dy, c.index[0], M, dyp, None)
-            dy = dyp
-        dxs = torch.empty(M, D, device=dev)
-        ops.layernorm_bwd(dy, c.xs32, c.norm_st, p32("encoder.norm.weight"), dxs, None,
-                          *((g("encoder.norm.weight"), g("encoder.norm.bias")) if plan.final_norm else (None, None)),
-                          None)
-        ready("encoder.norm.weight")
-        c.xs32 = None
+            ops.gather_rows(dy, rows, M, dyp, None)
+            return dyp
+
         daudio = torch.empty(c.x_shape, device=dev) if plan.dx else None
-        if plan.first_layer < n_layers:
+        inject, dh0 = None, None
+        if c.collect is None:
+            top = n_layers
+            dx = torch.empty(M, D, device=dev)
+            ops.layernorm_bwd(packed(dense(grad_out)), c.xs32, c.norm_st, p32("encoder.norm.weight"), dx, None,
+                              *((g("encoder.norm.weight"), g("encoder.norm.bias")) if plan.final_norm else (None, None)),
+                              None)
+            ready("encoder.norm.weight")
+            c.xs32 = None
+        else:
+            # a hidden state at or below the lowest layer the backward visits reaches nothing trainable, unless the
+            # local features or the waveform want their gradient
+            low = 0 if plan.local else plan.first_layer + 1
+            dh = {k: dense(gr) for k, gr in zip(c.collect, grad_out) if gr is not None and k >= low}
+            if not dh:
+                c.enc_saved = c.local_saved = None
+                return gflat, (daudio.zero_() if plan.dx else None)
+            top = max(dh)
+            dx = packed(dh.pop(top))
+            dh0 = dh.pop(0, None) if top > 0 else None
+
+            def inject(i, x):
+                if i + 1 in dh:
+                    ops.add_rows(x, dh[i + 1], rows, M)
+        if plan.first_layer < top:
             # (the cached views of _grad_views slice the whole layout: a call-owned buffer gets its own encoder views)
             G_enc = self._grad_views(gflat)[0] if gflat is self._flat_g else \
                 self._stack_views("encoder.", n_layers, g, g)
-            dx = self._enc_stack.backward(self._W_enc, G_enc, c.enc_saved, dxs, c.cu, B, c.max_len,
+            dx = self._enc_stack.backward(self._W_enc[:top], G_enc, c.enc_saved, dx, c.cu, B, c.max_len,
                                           lambda i: ready(f"encoder.layers.{i}.self_attn.in_proj_weight"),
-                                          stop_at=plan.first_layer, need_dx=plan.local, need_wgrad=plan.layer_w)
-            if plan.local:
-                # the mapper output is bf16 (autocast), so is its gradient on the dense token grid
-                if c.index is None:
-                    dlocal16 = torch.empty(B * T, D, device=dev, dtype=torch.bfloat16)
-                    ops.gather_rows(dx, None, M, None, dlocal16)
-                else:
-                    dlocal16 = torch.zeros(B * T, D, device=dev, dtype=torch.bfloat16)
-                    ops.scatter_dgelu(dx, c.index[0], None, M, dlocal16)
-                del dx
-                self._local_backward(c.local_saved, dlocal16, B, g, ready,
-                                     norm=plan.norm or plan.conv or plan.dx, conv=plan.conv or plan.dx, dx=daudio,
-                                     wg_mapper=plan.mapper, wg_norm=plan.norm, wg_conv=plan.conv)
+                                          stop_at=plan.first_layer, need_dx=plan.local, need_wgrad=plan.layer_w,
+                                          inject=inject)
+        if plan.local:
+            if dh0 is not None:
+                ops.add_rows(dx, dh0, rows, M)
+            # the mapper output is bf16 (autocast), so is its gradient on the dense token grid
+            if c.index is None:
+                dlocal16 = torch.empty(B * T, D, device=dev, dtype=torch.bfloat16)
+                ops.gather_rows(dx, None, M, None, dlocal16)
+            else:
+                dlocal16 = torch.zeros(B * T, D, device=dev, dtype=torch.bfloat16)
+                ops.scatter_dgelu(dx, rows, None, M, dlocal16)
+            del dx
+            self._local_backward(c.local_saved, dlocal16, B, g, ready,
+                                 norm=plan.norm or plan.conv or plan.dx, conv=plan.conv or plan.dx, dx=daudio,
+                                 wg_mapper=plan.mapper, wg_norm=plan.norm, wg_conv=plan.conv)
         c.enc_saved = c.local_saved = None
         return gflat, daudio
 
@@ -1193,4 +1264,82 @@ class JEPA(_ModuleBase):
             return self._features_forward(audio.to(device=dev, dtype=torch.bfloat16).contiguous(), index)[0]
         params = dict(self.named_parameters())
         # audio moves to the device outside the Function: autograd's copy backward takes the gradient back to audio.device
-        return _FeatureBridge.apply(self, audio.to(device=dev), index, plan, *[params[n] for n in plan.names])
+        return _FeatureBridge.apply(self, audio.to(device=dev), index, plan, None, *[params[n] for n in plan.names])
+
+    def _hidden_layers(self, layers) -> List[int]:
+        """The hidden-state indices of `get_hidden_states(layers=...)`: None -> all N + 1, else a non-empty sequence of
+        distinct ints in [0, N] (ValueError otherwise).  Host-side only."""
+        n = self._enc_stack.n_layers
+        if layers is None:
+            return list(range(n + 1))
+        if isinstance(layers, (str, bytes)) or not hasattr(layers, "__iter__"):
+            raise ValueError(f"layers must be a sequence of ints in [0, {n}], got {layers!r}")
+        out = []
+        for k in layers:
+            if isinstance(k, bool) or not isinstance(k, (int, np.integer)):
+                raise ValueError(f"layers must hold ints in [0, {n}], got {k!r}")
+            if not 0 <= int(k) <= n:
+                raise ValueError(f"hidden state {int(k)} is out of range: this encoder has {n} layers, [0, {n}]")
+            if int(k) in out:
+                raise ValueError(f"hidden state {int(k)} is requested twice")
+            out.append(int(k))
+        if not out:
+            raise ValueError("layers is empty: request at least one hidden state (None requests all)")
+        return out
+
+    def _hidden_states_tf32(self, audio: torch.Tensor, index, collect: List[int]) -> List[torch.Tensor]:
+        """get_hidden_states with inference_precision == "tf32" (the path of _audio_representation_tf32, stopped after
+        layer max(collect) - 1)."""
+        w = self._tf32_weights()
+        x32 = audio.to(device=self.device, dtype=torch.float32).contiguous()
+        B = x32.shape[0]
+        top = max(collect)
+        xv32, _, cu, max_len = self._visible_rows(self._local_features_tf32(x32, w), index, bf16=False)
+        hidden = {}
+        if 0 in collect:
+            hidden[0] = self._dense_rows(xv32, index, B)
+
+        def hook(i, y):
+            if i + 1 in collect:
+                hidden[i + 1] = self._dense_rows(y, index, B)
+        if top > 0:
+            self._enc_stack.forward_tf32(w["layers"][:top], xv32, ops.tf32_round(xv32), cu, B, max_len, hook)
+        return [hidden[k] for k in collect]
+
+    def get_hidden_states(self, audio: torch.Tensor, padding_mask: Optional[torch.Tensor] = None, host_mask=None,
+                          layers=None) -> List[torch.Tensor]:
+        """The student encoder's per-layer hidden states (the `hidden_states` convention of HF transformers), fp32
+        [B, T, D] each on the model's device, in the order of `layers`:
+          hidden state 0        the encoder input: post_extraction_mapper output + pos_encoding_encoder;
+          hidden state k        the output of encoder.layers[k-1] (after its norm2), 1 <= k <= N (12 base, 24 large);
+        so `get_audio_representation == encoder.norm(hidden state N)`.  layers: distinct ints in [0, N] (None: all
+        N + 1); anything else raises ValueError before any device work.  Only the layers below max(layers) run, and
+        the final norm never does: layers=[6] runs 6 encoder layers, layers=[0] none.
+
+        Token layout, padding_mask / host_mask and the zero rows of hidden tokens are those of
+        `get_audio_representation`; so is inference_precision ("tf32": the reference-precision forward, no grad_fn).
+
+        Gradients ("bf16"): under the rule of `get_audio_representation` (some feature-path parameter requires grad,
+        or audio does) the hidden states carry a grad_fn, and any subset of them may feed the loss.  The graph holds the
+        path up to layer max(layers) - 1: the parameters of the layers above and of encoder.norm keep grad None.  A
+        hidden state the loss does not read costs nothing in the backward; the others' gradients are added at their
+        layer boundaries of the one encoder backward.  Frozen parts save nothing, the waveform gradient arrives in
+        audio's dtype on audio's device, one graph supports one backward (DESIGN.md 2.4)."""
+        collect = self._hidden_layers(layers)
+        self.eval()
+        self._ensure_ready()
+        self._sync_weights()
+        index = self._visible_index(audio.shape[0], padding_mask, host_mask)
+        if self.inference_precision == "tf32":
+            return self._hidden_states_tf32(audio, index, collect)
+        dev = self.device
+        plan = None
+        if torch.is_grad_enabled():
+            plan = self._feature_plan([n for n, p in self.named_parameters() if p.requires_grad], audio.requires_grad,
+                                      top=max(collect))
+        if plan is None:
+            return self._features_forward(audio.to(device=dev, dtype=torch.bfloat16).contiguous(), index, None,
+                                          collect)[0]
+        params = dict(self.named_parameters())
+        return list(_FeatureBridge.apply(self, audio.to(device=dev), index, plan, collect,
+                                         *[params[n] for n in plan.names]))

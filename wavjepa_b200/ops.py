@@ -561,6 +561,17 @@ def scatter_rows(src: torch.Tensor, idx: torch.Tensor, N: int, out: torch.Tensor
     check(lib.wj_scatter_rows(p(src), p(idx), N, src.shape[-1], p(out), _stream()))
 
 
+def add_rows(a: torch.Tensor, b: torch.Tensor, idx: Optional[torch.Tensor], N: int):
+    """a[r, :] += b[idx[r] if idx is not None else r, :] for r < N, fp32 (wj_add_rows_f32)."""
+    assert a.dtype == torch.float32 and b.dtype == torch.float32 and a.is_contiguous() and b.is_contiguous()
+    assert idx is None or idx.dtype == torch.int32
+    lib = _lib.load()
+    p = lambda t: C.c_void_p(_ptr(t))
+    if _lib._profile is not None:   # read a and b, write a
+        _lib._profile.nbytes = N * a.shape[-1] * 12
+    check(lib.wj_add_rows_f32(p(a), p(b), p(idx), N, a.shape[-1], _stream()))
+
+
 def target_accum(x: torch.Tensor, rowsum, B: int, T: int, D: int, scale: float, first: bool, inst_stats, targets,
                  eps: float = 1e-5):
     lib = _lib.load()
