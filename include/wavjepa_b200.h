@@ -305,6 +305,11 @@ int wj_masked_mse(const void* pred_bf16, const float* targets, const int* tgt_ro
  * i.e. loss_clean = sums[0] / M, loss_denoise_dereverb = sums[1] / M; dpred (optional, fp32 [2, M]) = gradient of
  * alpha * loss_clean + (1 - alpha) * loss_denoise_dereverb. */
 int wj_mse_pair(const float* pred, const float* target, int64_t M, float alpha, double* sums, float* dpred, void* stream);
+/* Backward of the two losses of wj_mse_pair with upstream weights on the device: w fp32 [2] = (d L / d loss_clean,
+ * d L / d loss_denoise_dereverb); dpred fp32 [2, M], dpred[h] = fp32(2 * w[h] / M, formed in fp64) * (pred[h] - target).
+ * w = (alpha, 1 - alpha) gives wj_mse_pair's dpred bit for bit.  No host read of w, no reduction: bit-identical from
+ * run to run in both modes. */
+int wj_mse_pair_bwd(const float* pred, const float* target, int64_t M, const float* w, float* dpred, void* stream);
 
 /* Segmental-SNR mixing (data_modules/scene_module/generate_scenes_batch.py:107-146 add_noise): rows b of source / noise
  * [B, T] fp32; energies over the window [start_b, start_b + length_b); out = source + a_b * noise with

@@ -42,6 +42,23 @@ __global__ void __launch_bounds__(256) mse_pair_kernel(const float4* __restrict_
   }
 }
 
+// dpred[h] = (2 / M) * w[h] * (pred[h] - target), w [2] on the device: the backward of the two losses of mse_pair_kernel
+// under autograd.  The scale is formed in fp64 and rounded once, as wj_mse_pair does on the host, so w = (alpha,
+// 1 - alpha) gives mse_pair_kernel's dpred bit for bit.  One writer per element: no reduction, no atomics.
+__global__ void __launch_bounds__(256) mse_pair_bwd_kernel(const float4* __restrict__ pred,
+                                                           const float4* __restrict__ target, long long m4,
+                                                           const float* __restrict__ w, float4* __restrict__ dpred) {
+  const double m = static_cast<double>(4 * m4);
+  const float w0 = static_cast<float>(2.0 * static_cast<double>(w[0]) / m);
+  const float w1 = static_cast<float>(2.0 * static_cast<double>(w[1]) / m);
+  for (long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; i < m4;
+       i += static_cast<long long>(gridDim.x) * blockDim.x) {
+    const float4 t = target[i], a = pred[i], b = pred[m4 + i];
+    dpred[i] = make_float4(w0 * (a.x - t.x), w0 * (a.y - t.y), w0 * (a.z - t.z), w0 * (a.w - t.w));
+    dpred[m4 + i] = make_float4(w1 * (b.x - t.x), w1 * (b.y - t.y), w1 * (b.z - t.z), w1 * (b.w - t.w));
+  }
+}
+
 // energy[b] = (sum source^2, sum noise^2) over the active window [start_b, start_b + len_b) of row b
 __global__ void __launch_bounds__(256) snr_energy_kernel(const float* __restrict__ source, const float* __restrict__ noise,
                                                          const int* __restrict__ start, const int* __restrict__ len,
@@ -109,6 +126,20 @@ extern "C" int wj_mse_pair(const float* pred, const float* target, int64_t M, fl
       reinterpret_cast<const float4*>(pred), reinterpret_cast<const float4*>(target), m4, w0, w1, sums,
       reinterpret_cast<float4*>(dpred));
   return check_launch("mse_pair");
+}
+
+extern "C" int wj_mse_pair_bwd(const float* pred, const float* target, int64_t M, const float* w, float* dpred,
+                               void* stream) {
+  if (M <= 0) return WJ_OK;
+  if (M % 4) { set_error("wj_mse_pair_bwd: M %% 4 != 0"); return WJ_ERR_ARG; }
+  const long long m4 = M / 4;
+  long long blocks = (m4 + 255) / 256;
+  const long long cap = static_cast<long long>(sm_count()) * 8;
+  if (blocks > cap) blocks = cap;
+  mse_pair_bwd_kernel<<<static_cast<unsigned>(blocks), 256, 0, WJ_STREAM(stream)>>>(
+      reinterpret_cast<const float4*>(pred), reinterpret_cast<const float4*>(target), m4, w,
+      reinterpret_cast<float4*>(dpred));
+  return check_launch("mse_pair_bwd");
 }
 
 extern "C" int wj_snr_mix(const float* source, const float* noise, const int* start, const int* length, const float* snr,

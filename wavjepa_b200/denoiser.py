@@ -11,8 +11,11 @@ B200-first differences (results identical up to the documented tolerances):
   * the reference runs the student twice (clean, generated) and the teacher once; here the two student passes are ONE
     packed batch of 2N sequences through the same kernels (no cross-sequence interaction anywhere in the stack), the
     teacher is `JEPA.get_audio_representation` on the same kernels;
-  * forward, hand-written backward, AdamW (+ cosine schedule with 5000 warm-up steps, denoiser.py:208-209) and the bf16
-    weight refresh are one fused `train_step`; there is no autograd graph;
+  * two training paths: `forward` in grad mode is differentiable (the student through `_FeatureBridge`, the two MSE
+    losses through `_MsePair`), so `loss.backward()` with a stock optimizer, gradient clipping and a pl.Trainer work as
+    in the reference (`training_step` returns the forward); or forward, hand-written backward, AdamW (+ cosine schedule
+    with 5000 warm-up steps, denoiser.py:208-209) and the bf16 weight refresh are one fused `train_step` with no
+    autograd graph;
   * scene generation: the RIR convolutions are FFT convolutions of full length (`torch.fft`, i.e. cuFFT as a plain
     library, exactly torchaudio.functional.fftconvolve's rfft -> product -> irfft with n = L1 + L2 - 1); the segmental
     SNR mix, the resampler, the crop + normalise pass are kernels of libwavjepa_b200.so.
@@ -32,7 +35,8 @@ from ._lib import WavJepaLibError
 from .extractors import ConvFeatureExtractor
 from .hear import fix_state_dict_keys
 from ._lightning import Base as _ModuleBase
-from .jepa import JEPA
+from ._lightning import attached_trainer
+from .jepa import JEPA, _FeatureBridge
 from .preprocess import sinc_resample_table
 from .types import ForwardReturn, TransformerEncoderCFG, TransformerLayerCFG
 
@@ -119,6 +123,29 @@ def resample(audio: torch.Tensor, resample_sr: int, original_sr: int = ORIGINAL_
 
 
 # ------------------------------------------------------------------------------------------------- the module
+class _MsePair(torch.autograd.Function):
+    """loss_clean, loss_denoise_dereverb (fp32 scalars) of the packed student features [2N, T, D] (clean half,
+    generated half) against the teacher's [N * T, D]: the sums of wj_mse_pair forward, wj_mse_pair_bwd backward with
+    the two upstream gradients as its device weights (an unused loss arrives as None and weighs 0)."""
+
+    @staticmethod
+    def forward(ctx, feats, targets):
+        ctx.set_materialize_grads(False)
+        M = targets.numel()
+        sums = torch.zeros(2, device=feats.device, dtype=torch.float64)
+        ops.mse_pair(feats, targets, 0.0, sums)
+        ctx.save_for_backward(feats, targets)
+        return (sums[0] / M).float(), (sums[1] / M).float()
+
+    @staticmethod
+    def backward(ctx, g_clean, g_dd):
+        feats, targets = ctx.saved_tensors
+        w = torch.stack([feats.new_zeros(()) if g is None else g.reshape(()).float() for g in (g_clean, g_dd)])
+        dfeats = torch.empty_like(feats)
+        ops.mse_pair_bwd(feats, targets, w, dfeats)
+        return dfeats, None
+
+
 class Denoiser(_ModuleBase):
     """reference wavjepa/denoiser.py:43-376."""
     TARGET_SECONDS: int = 10
@@ -213,6 +240,14 @@ class Denoiser(_ModuleBase):
         opt = torch.optim.AdamW(trainables, lr=self.hparams.lr, betas=self.hparams.adam_betas,
                                 eps=self.hparams.adam_eps, weight_decay=self.hparams.adam_weight_decay)
         sched = torch.optim.lr_scheduler.LambdaLR(opt, lambda s: self.lr_at(s) / self.hparams.lr)
+
+        # as JEPA.configure_optimizers: without a trainer, each optimizer step advances global_step, so this path and
+        # train_step agree on the schedule position and the checkpointed step
+        def _count(optimizer, args, kwargs):
+            if attached_trainer(self) is None:
+                self._core._step += 1
+
+        opt.register_step_post_hook(_count)
         return {"optimizer": opt, "lr_scheduler": {"scheduler": sched, "interval": "step"}}
 
     # ------------------------------------------------------------------------------------------- batch preparation
@@ -255,10 +290,13 @@ class Denoiser(_ModuleBase):
         return outs[0][idx], outs[1][idx]
 
     # ------------------------------------------------------------------------------------------- forward / backward
-    def _run(self, generated_scene: torch.Tensor, clean_scene: torch.Tensor, backward: bool):
+    def _check_teacher(self) -> None:
         if self.teacher is None:
             raise WavJepaLibError("Denoiser needs its frozen teacher: call _set_teacher(checkpoint) first "
                                   "(the reference has no attribute `teacher` before that either)")
+
+    def _run(self, generated_scene: torch.Tensor, clean_scene: torch.Tensor, backward: bool):
+        self._check_teacher()
         core = self._core
         core._ensure_ready()
         core._sync_weights()
@@ -300,11 +338,39 @@ class Denoiser(_ModuleBase):
             world = ddp.world_size
         return out, world
 
-    @torch.no_grad()
     def forward(self, generated_scene: torch.Tensor, clean_scene: torch.Tensor) -> ForwardReturn:
         """reference Denoiser.forward (wavjepa/denoiser.py:308-364): dict with loss, loss_clean,
-        loss_denoise_dereverb (device scalars)."""
-        return self._run(generated_scene, clean_scene, backward=False)[0]
+        loss_denoise_dereverb (device scalars).
+
+        Training through autograd: in grad mode, when a student parameter (extract_audio, feature_norms,
+        post_extraction_mapper, encoder) requires grad or a scene does, the three losses carry a grad_fn and
+        `loss.backward()` (or any mix of loss_clean / loss_denoise_dereverb) fills `.grad` of the trainable student
+        parameters and of the scenes that require grad, on their device and in their dtype.  The values are bit-identical
+        to the no-grad call; the teacher is never differentiated, frozen student parts save nothing and are not
+        backpropagated, and one graph supports one backward (DESIGN.md 5b).  `train_step` is the fused alternative."""
+        self._check_teacher()
+        core = self._core
+        core._ensure_ready()
+        plan = None
+        if torch.is_grad_enabled():   # the rule of JEPA.get_audio_representation
+            plan = core._feature_plan([n for n, p in self.named_parameters() if p.requires_grad],
+                                      generated_scene.requires_grad or clean_scene.requires_grad)
+        if plan is None:
+            with torch.no_grad():
+                return self._run(generated_scene, clean_scene, backward=False)[0]
+        core._sync_weights()
+        dev = self.device
+        # a scene that requires grad keeps its dtype up to the bridge, which reads it as bf16 and returns its gradient in
+        # that dtype; torch.cat and .to() route each half's gradient back to its scene
+        dt = torch.promote_types(generated_scene.dtype, clean_scene.dtype) if plan.dx else torch.bfloat16
+        clean = clean_scene.to(dev, dt)
+        x = torch.cat([clean, generated_scene.to(dev, dt)], dim=0)     # halves: [clean | generated]
+        params = dict(self.named_parameters())
+        feats = _FeatureBridge.apply(core, x, None, plan, None, *[params[n] for n in plan.names])
+        with torch.no_grad():
+            targets = self.teacher.get_audio_representation(clean.to(torch.bfloat16), padding_mask=None)
+        lc, ld = _MsePair.apply(feats, targets.reshape(-1, targets.shape[-1]).contiguous())
+        return ForwardReturn(loss=self.alpha * lc + (1 - self.alpha) * ld, loss_clean=lc, loss_denoise_dereverb=ld)
 
     @torch.no_grad()
     def forward_backward(self, generated_scene: torch.Tensor, clean_scene: torch.Tensor):
@@ -337,5 +403,8 @@ class Denoiser(_ModuleBase):
         return out
 
     def training_step(self, batch, batch_idx: int = 0) -> ForwardReturn:
+        """reference Denoiser.training_step: the forward, whose differentiable `loss` the caller (a pl.Trainer in
+        automatic optimization, or a plain loop) backpropagates and steps with the optimizer of `configure_optimizers`,
+        exactly like JEPA.training_step.  `train_step` is the fused step (forward, backward and AdamW in one call)."""
         generated_scene, clean_scene = batch
-        return self.train_step(generated_scene, clean_scene)
+        return self(generated_scene, clean_scene)

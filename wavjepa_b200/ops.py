@@ -776,6 +776,19 @@ def mse_pair(pred: torch.Tensor, target: torch.Tensor, alpha: float, sums_f64: t
     check(lib.wj_mse_pair(p(pred), p(target), C.c_int64(M), C.c_float(alpha), p(sums_f64), p(dpred), _stream()))
 
 
+def mse_pair_bwd(pred: torch.Tensor, target: torch.Tensor, w: torch.Tensor, dpred: torch.Tensor):
+    """dpred fp32 [2, M] = gradient of w[0] * loss_clean + w[1] * loss_denoise_dereverb (the losses of mse_pair); w fp32
+    [2] stays on the device (no host read)."""
+    assert pred.dtype == torch.float32 and target.dtype == torch.float32 and w.dtype == torch.float32
+    assert dpred.dtype == torch.float32 and w.numel() == 2 and w.is_contiguous()
+    M = target.numel()
+    assert pred.numel() == 2 * M and dpred.numel() == 2 * M
+    assert pred.is_contiguous() and target.is_contiguous() and dpred.is_contiguous()
+    lib = _lib.load()
+    p = lambda t: C.c_void_p(_ptr(t))
+    check(lib.wj_mse_pair_bwd(p(pred), p(target), C.c_int64(M), p(w), p(dpred), _stream()))
+
+
 def snr_mix(source: torch.Tensor, noise: torch.Tensor, start: torch.Tensor, length: torch.Tensor, snr: torch.Tensor,
             out: torch.Tensor):
     """source, noise, out fp32 [B, T]; start, length int32 [B]; snr fp32 [B]."""
