@@ -2,13 +2,15 @@
 (UTCHMMA = tcgen05.mma, LDTM / STTM = tcgen05.ld / st, UTMALDG / UTMASTG = TMA load / store, UTCBAR = tcgen05.commit,
 SYNCS = mbarrier) next to the legacy tensor-core (HMMA) and special-function (MUFU) counts, from
     cuobjdump -sass wavjepa_b200/libwavjepa_b200.so
-    python scripts/sass_summary.py > profiles/r02_sass_summary.txt"""
+    python scripts/sass_summary.py [library] > profiles/r02_sass_summary.txt     (default: the in-tree library)"""
 import collections
 import os
 import re
 import subprocess
+import sys
 
-LIB = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "wavjepa_b200", "libwavjepa_b200.so")
+LIB = sys.argv[1] if len(sys.argv) > 1 else \
+    os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "wavjepa_b200", "libwavjepa_b200.so")
 KEYS = ["UTCHMMA", "UTCHMMA.2CTA", "LDTM", "STTM", "UTMALDG", "UTMASTG", "UTCBAR", "SYNCS", "HMMA", "MUFU", "HFMA2", "total"]
 out = subprocess.run(["cuobjdump", "-sass", LIB], capture_output=True, text=True).stdout
 kern, counts = None, collections.OrderedDict()

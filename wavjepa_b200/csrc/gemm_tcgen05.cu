@@ -1,6 +1,6 @@
 // tcgen05 / TMEM / TMA GEMM core for the WavJEPA hot path (sm_100a only).
 //
-// One persistent, warp-specialised kernel serves every GEMM-shaped op of the path:
+// One persistent, warp-specialised kernel body (gemm_body) serves every GEMM-shaped op of the path:
 //   * Linear layers fwd / dgrad            (reference: torch.nn.Linear inside nn.TransformerEncoderLayer,
 //                                            wavjepa/jepa.py:126-132; MHA in/out-proj, MLP, the three mappers)
 //   * Conv1d 512->512 (k3 s2, k2 s2) fwd / dgrad as implicit GEMM over channels-last activations
@@ -13,6 +13,10 @@
 //   warp 2      : TMEM allocator / deallocator
 //   warp 3      : idle
 //   warps 4..19 : epilogue: tcgen05.ld -> registers -> fused bias / GELU / GELU' / residual -> global
+//
+// The body has two entry points: gemm_kernel runs it on single CTAs (128-row tiles), gemm_pair_kernel on CTA pairs
+// (__cluster_dims__(2, 1, 1), 256-row tiles, tcgen05.mma.cta_group::2, grid = 2 * min(#tiles, #SMs / 2)); every
+// pair-specific step is an `if constexpr (CTAS == 2)` inside the one body.
 //
 // Operand addressing is "virtual column" based so that the same kernel covers implicit-GEMM convolutions: the
 // reduction (normal mode) or output-column (WGRAD mode) index vc is split into segments of `seg.width` columns;
@@ -95,13 +99,15 @@ struct RegSplit {   // WIDE: the two-output GELU epilogue holds 64 accumulator +
 
 // AUX: the GELU-backward dgrad (MODE 2, HEAVY): every epilogue warp owns TWO 2 KB tiles (one per 32-column chunk of its
 // tile) that first receive the saved GELU' factors by TMA -- a whole tile ahead of their use -- and then stage the
-// output; the extra 32 KB come out of the operand ring (3 stages: that kernel is epilogue-bound, not operand-bound).
-template <int BN, bool AUX = false>
+// output; the extra 32 KB come out of the operand ring (3 stages on single CTAs, 5 on pairs: that kernel is
+// epilogue-bound, not operand-bound).  CTAS = 2: each CTA of a pair stages its 128 rows of A and HALF of the B tile.
+template <int BN, bool AUX, int CTAS>
 struct Cfg {
   static constexpr int A_BYTES = BM * BK * 2;
-  static constexpr int B_BYTES = BN * BK * 2;
+  static constexpr int B_BYTES = (BN / CTAS) * BK * 2;
   static constexpr int STAGE_BYTES = A_BYTES + B_BYTES;
-  static constexpr int STAGES = AUX ? ((BN == 256) ? 3 : 4) : ((BN == 256) ? 4 : ((BN == 192) ? 4 : ((BN == 128) ? 6 : 8)));
+  static constexpr int STAGES = CTAS == 2 ? (AUX ? 5 : ((BN == 256) ? 6 : 8))
+                                          : AUX ? ((BN == 256) ? 3 : 4) : ((BN == 256) ? 4 : ((BN == 192) ? 4 : ((BN == 128) ? 6 : 8)));
   static constexpr int STAGING_OFF = STAGES * STAGE_BYTES + 1024;   // barriers live in the 1 KB before it
   static constexpr int WARP_STAGING = AUX ? 4096 : 2048;
   static constexpr int SMEM_BYTES = STAGING_OFF + 1024 /*align slack*/ + kEpiWarps * WARP_STAGING /*TMA-store staging*/;
@@ -119,6 +125,68 @@ __device__ __forceinline__ void seg_coords(const SegInfo& s, int vc, int& c0, in
     q = 0;
     p = 0;
   }
+}
+
+// Tile decode.  normal: tile -> (m_blk, n_blk), n fastest (CTAs running together share the A rows through L2), then
+// m_blk -> (batch entry b, row0 = this CTA's first row inside it).  wgrad: tile -> (split, m_blk, n_blk), row0 = this
+// CTA's first output row.  tile_rows: rows of an m-block (BM, or 2 * BM for a CTA pair); row_off: this CTA's offset in it.
+struct TileCoords {
+  int split, m_blk, n_blk, b, row0;
+};
+
+template <bool WGRAD>
+__device__ __forceinline__ TileCoords tile_coords(const GemmParams& p, int tile, int tile_rows, int row_off) {
+  TileCoords t;
+  t.split = 0;
+  t.b = 0;
+  if constexpr (WGRAD) {
+    const int mn = p.m_blocks * p.n_blocks;
+    t.split = tile / mn;
+    tile -= t.split * mn;
+  }
+  t.m_blk = tile / p.n_blocks;
+  t.n_blk = tile - t.m_blk * p.n_blocks;
+  if constexpr (!WGRAD) {
+    t.b = t.m_blk / p.mb_per_batch;
+    t.row0 = (t.m_blk - t.b * p.mb_per_batch) * tile_rows + row_off;
+  } else {
+    t.row0 = t.m_blk * tile_rows + row_off;
+  }
+  return t;
+}
+
+// wgrad: the k-blocks [lo, hi) of the (batch, 64-token block) reduction that token split `split` covers (may be empty)
+__device__ __forceinline__ void wgrad_kb_range(const GemmParams& p, int split, int& lo, int& hi) {
+  const int kb_total = p.batch * p.kb_per_batch;
+  const int per = (kb_total + p.splits - 1) / p.splits;
+  lo = split * per;
+  hi = min(lo + per, kb_total);
+}
+
+// One TMA load into a stage of the operand ring.  Its bytes are counted on the stage's full barrier: this CTA's own
+// (`bar`), or on CTA pairs the leader's (`fb`, a shared::cluster address).
+template <int CTAS>
+__device__ __forceinline__ void stage_load(void* dst, const CUtensorMap* tm, uint64_t* bar, uint32_t fb, int c0, int c1) {
+  if constexpr (CTAS == 1) tma_load_2d(dst, tm, bar, c0, c1);
+  else tma_load_2d_pair(dst, tm, fb, c0, c1);
+}
+template <int CTAS>
+__device__ __forceinline__ void stage_load(void* dst, const CUtensorMap* tm, uint64_t* bar, uint32_t fb, int c0, int c1,
+                                           int c2) {
+  if constexpr (CTAS == 1) tma_load_3d(dst, tm, bar, c0, c1, c2);
+  else tma_load_3d_pair(dst, tm, fb, c0, c1, c2);
+}
+template <int CTAS>
+__device__ __forceinline__ void stage_load(void* dst, const CUtensorMap* tm, uint64_t* bar, uint32_t fb, int c0, int c1,
+                                           int c2, int c3) {
+  if constexpr (CTAS == 1) tma_load_4d(dst, tm, bar, c0, c1, c2, c3);
+  else tma_load_4d_pair(dst, tm, fb, c0, c1, c2, c3);
+}
+template <int CTAS>
+__device__ __forceinline__ void stage_load(void* dst, const CUtensorMap* tm, uint64_t* bar, uint32_t fb, int c0, int c1,
+                                           int c2, int c3, int c4) {
+  if constexpr (CTAS == 1) tma_load_5d(dst, tm, bar, c0, c1, c2, c3, c4);
+  else tma_load_5d_pair(dst, tm, fb, c0, c1, c2, c3, c4);
 }
 
 // One accumulator tile (this warp's 32 TMEM lanes x BN/4 columns) -> fused epilogue -> global memory.
@@ -452,27 +520,26 @@ struct AuxPipe {
 
 template <int BN>
 __device__ __forceinline__ bool aux_issue(const GemmParams& p, const OutMaps& om, AuxPipe& ap, int lane, int lane_grp,
-                                          int col_q, int tile, int ch, int tile_rows = BM, int row_off = 0) {
-  // tile_rows / row_off: rows of an m-block and this CTA's offset inside it (CTA pairs: 256 and rank * 128)
+                                          int col_q, int tile, int ch, int tile_rows, int row_off) {
+  // tile_rows / row_off: rows of an m-block and this CTA's offset inside it (see tile_coords)
   constexpr int CHUNKS = BN / 32 / 4;
   if (tile >= p.total_tiles) return false;
-  const int m_blk = tile / p.n_blocks, n_blk = tile - m_blk * p.n_blocks;
-  const int b = m_blk / p.mb_per_batch;
-  const int row0 = (m_blk - b * p.mb_per_batch) * tile_rows + row_off + lane_grp * 32;
-  const int n0 = n_blk * BN + (col_q * CHUNKS + ch) * 32;
+  const TileCoords tc = tile_coords<false>(p, tile, tile_rows, row_off);
+  const int row0 = tc.row0 + lane_grp * 32;
+  const int n0 = tc.n_blk * BN + (col_q * CHUNKS + ch) * 32;
   const bool live = n0 < p.N && row0 < p.L;   // warp-uniform; the same predicate gates the consumer
   if (live && lane == 0) {
     mbar_arrive_expect_tx(&ap.bar[ch], 2048);   // (TMA always delivers the whole box: out-of-range parts are zero-filled)
-    tma_load_3d(ap.buf + ch * 2048, &om.o2, &ap.bar[ch], n0, row0, b);
+    tma_load_3d(ap.buf + ch * 2048, &om.o2, &ap.bar[ch], n0, row0, tc.b);
   }
   return live;
 }
 
 template <int BN, typename Arrive>
 __device__ __forceinline__ void epilogue_tile_tma_aux(const GemmParams& p, const OutMaps& om, uint32_t t_base, AuxPipe& ap,
-                                                      int lane, int lane_grp, int col_q, int tile, int n_blk, int b,
-                                                      int row_in_batch0, int next_tile, Arrive arrive, int tile_rows = BM,
-                                                      int row_off = 0) {
+                                                      int lane, int lane_grp, int col_q, int n_blk, int b,
+                                                      int row_in_batch0, int next_tile, Arrive arrive, int tile_rows,
+                                                      int row_off) {
   constexpr int CHUNKS = BN / 32 / 4;
   const int row0 = row_in_batch0 + lane_grp * 32;
   const int sw = (lane >> 1) & 3;
@@ -551,17 +618,29 @@ __device__ __forceinline__ void epilogue_tile_tma_aux(const GemmParams& p, const
 // TF32 (MODE 0 only): fp32 operands, tcgen05.mma.kind::tf32.  A 128-byte swizzle row holds 64 bf16 or 32 fp32, and one
 // UMMA consumes 32 bytes of K either way, so the shared-memory ring, descriptors and barriers are byte-identical; only
 // the element count of a k-block (KB), the instruction kind and the descriptor's operand formats change.
-template <int BN, int MODE, bool HEAVY, bool TF32 = false>
-__global__ void __launch_bounds__(kThreads, 1)
-gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
-            const __grid_constant__ CUtensorMap tmB1, const __grid_constant__ OutMaps om, const GemmParams p) {
-  static_assert(!TF32 || (MODE == 0 && !HEAVY), "the tf32 kernel is the plain forward");
+//
+// CTAS = 2: two CTAs of a cluster (one TPC) work on one 256 x BN tile with tcgen05.mma.cta_group::2: each CTA stages
+// its own 128 rows of A and its own HALF of B (BN/2 columns), the leader's single MMA thread drives both tensor cores,
+// and each CTA's TMEM receives its 128 accumulator rows.  Per SM that is 32 KB of operands per 128 x 256 x 64 of MMA
+// work instead of 48 KB (less L2 -> SM traffic, 6 pipeline stages instead of 4 in the same shared memory, and only 2/3
+// of the shared-memory read bandwidth), which is what a single CTA runs out of.  Barrier protocol: both producers
+// signal the LEADER's full barriers (TMA .cta_group::2), the leader's commits are multicast to the empty /
+// accumulator-full barriers of both CTAs, the epilogue warps of both CTAs arrive on the leader's accumulator-empty
+// barrier.
+// `tid` is threadIdx.x as read by the __global__ entry point, where __launch_bounds__ tells the compiler it is below
+// kThreads (a read in this inlined body would not carry that range, which costs registers in the control warps).
+template <int BN, int MODE, bool HEAVY, bool TF32, int CTAS>
+__device__ __forceinline__ void gemm_body(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMap& tmB1,
+                                          const OutMaps& om, const GemmParams& p, uint32_t tid) {
+  static_assert(!TF32 || (MODE == 0 && !HEAVY && CTAS == 1), "the tf32 kernel is the plain single-CTA forward");
   constexpr bool AUXQ = (MODE == 2 && HEAVY);   // GELU-backward dgrad: TMA-fed factor tiles (see epilogue_tile_tma_aux)
-  using C = Cfg<BN, AUXQ>;
+  using C = Cfg<BN, AUXQ, CTAS>;
   constexpr bool WGRAD = (MODE == 1);
   constexpr bool B_MN = (MODE != 0);
+  constexpr bool DBG = (CTAS == 1);   // wj_gemm_debug cycle counters: single-CTA launches
   constexpr int STAGES = C::STAGES;
   constexpr int KB = TF32 ? BK / 2 : BK;   // elements of K per k-block (128 bytes of each operand row)
+  constexpr int TILE_ROWS = CTAS * BM;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   uint64_t* full_bar = reinterpret_cast<uint64_t*>(smem + STAGES * C::STAGE_BYTES);
@@ -571,8 +650,18 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tempty_bar + 2);
   uint64_t* aux_bar = full_bar + 64;            // [kEpiWarps][2], 512 bytes into the barrier KB
 
-  const int warp = threadIdx.x >> 5;
-  const int lane = threadIdx.x & 31;
+  const int warp = tid >> 5;
+  const int lane = tid & 31;
+  const int rank = CTAS == 2 ? static_cast<int>(cluster_ctarank()) : 0;   // this CTA's rows of a pair tile: rank * BM
+  const bool leader = rank == 0;
+  // static round-robin tile schedule over CTAs (CTA pairs); read where used rather than kept live through all roles
+  auto first_tile = [] { return static_cast<int>(blockIdx.x / CTAS); };
+  auto tile_step = [] { return static_cast<int>(gridDim.x / CTAS); };
+  // single CTAs sleep between probes of the empty / accumulator-empty barriers (see mbar_wait_relaxed)
+  auto wait_free = [](uint64_t* bar, uint32_t parity) {
+    if constexpr (CTAS == 1) mbar_wait_relaxed(bar, parity);
+    else mbar_wait(bar, parity);
+  };
 
   if (warp == 0 && lane == 0) {
     tma_prefetch_desc(&tmA);
@@ -585,32 +674,29 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
     }
     for (int i = 0; i < 2; ++i) {
       mbar_init(&tfull_bar[i], 1);
-      mbar_init(&tempty_bar[i], kEpiWarps);
+      mbar_init(&tempty_bar[i], CTAS * kEpiWarps);
     }
     if constexpr (AUXQ) {
       for (int i = 0; i < 2 * kEpiWarps; ++i) mbar_init(&aux_bar[i], 1);
     }
     fence_mbar_init();
   }
-  if (warp == 2) tmem_alloc(tmem_slot, 512);
+  if (warp == 2) {
+    if constexpr (CTAS == 1) tmem_alloc(tmem_slot, 512);
+    else tmem_alloc_pair(tmem_slot, 512);
+  }
   tc_fence_before();
-  __syncthreads();
+  if constexpr (CTAS == 1) __syncthreads();
+  else cluster_sync_all();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
 
-  // ------------------------------------------------------------------------------------------ tile decode helpers
-  // normal: tile -> (m_blk, n_blk), n fastest (CTAs running together share the A rows through L2)
-  // wgrad : tile -> (split, m_blk, n_blk)
   auto num_kb = [&](int tile) -> int {
     if constexpr (!WGRAD) {
       return p.K / KB;
     } else {
-      const int split = tile / (p.m_blocks * p.n_blocks);
-      const int kb_total = p.batch * p.kb_per_batch;
-      const int per = (kb_total + p.splits - 1) / p.splits;
-      const int lo = split * per;
-      int hi = lo + per;
-      if (hi > kb_total) hi = kb_total;
+      int lo, hi;
+      wgrad_kb_range(p, tile_coords<true>(p, tile, TILE_ROWS, rank * BM).split, lo, hi);
       return hi > lo ? hi - lo : 0;
     }
   };
@@ -623,96 +709,91 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
       int stage = 0;
       uint32_t phase = 0;
       long long dbg_prod = 0;
-      for (int tile = blockIdx.x; tile < p.total_tiles; tile += gridDim.x) {
+      for (int tile = first_tile(); tile < p.total_tiles; tile += tile_step()) {
+        const TileCoords tc = tile_coords<WGRAD>(p, tile, TILE_ROWS, rank * BM);
+        // this CTA's B columns: the whole tile, or its half of a pair tile
+        const int nb0 = tc.n_blk * BN + rank * (BN / CTAS);
         if constexpr (!WGRAD) {
-          const int m_blk = tile / p.n_blocks;
-          const int n_blk = tile - m_blk * p.n_blocks;
-          const int b = m_blk / p.mb_per_batch;
-          const int row0 = (m_blk - b * p.mb_per_batch) * BM;
           const int nkb = p.K / KB;
           for (int kb = 0; kb < nkb; ++kb) {
-            const long long tw = p.dbg ? clock64() : 0;
-            mbar_wait_relaxed(&empty_bar[stage], phase ^ 1);
-            if (p.dbg) dbg_prod += clock64() - tw;
+            const long long tw = (DBG && p.dbg) ? clock64() : 0;
+            wait_free(&empty_bar[stage], phase ^ 1);
+            if (DBG && p.dbg) dbg_prod += clock64() - tw;
             uint8_t* sa = smem + stage * C::STAGE_BYTES;
             uint8_t* sb = sa + C::A_BYTES;
+            const uint32_t fb = CTAS == 2 ? mapa_shared(smem_u32(&full_bar[stage]), 0) : 0u;
             int c0, q, po;
             seg_coords(p.seg, kb * KB, c0, q, po);
-            mbar_arrive_expect_tx(&full_bar[stage], C::STAGE_BYTES);
-            tma_load_4d(sa, &tmA, &full_bar[stage], c0, q, row0 + po, b);
+            if (leader) mbar_arrive_expect_tx(&full_bar[stage], CTAS * C::STAGE_BYTES);
+            stage_load<CTAS>(sa, &tmA, &full_bar[stage], fb, c0, q, tc.row0 + po, tc.b);
             if constexpr (!B_MN) {
-              tma_load_2d(sb, &tmB, &full_bar[stage], kb * KB, n_blk * BN);
+              stage_load<CTAS>(sb, &tmB, &full_bar[stage], fb, kb * KB, nb0);
             } else {
-              // dgrad: W is [reduction rows, output cols] row-major -> BN/64 MN-major atoms of 64 reduction rows, all
-              // fetched by ONE TMA instruction through a 3-D view {64 cols, rows, column atoms} (the TMA unit is
+              // dgrad: W is [reduction rows, output cols] row-major -> BN/CTAS/64 MN-major atoms of 64 reduction rows,
+              // all fetched by ONE TMA instruction through a 3-D view {64 cols, rows, column atoms} (the TMA unit is
               // instruction-rate limited: 5-6 small boxes per k-block held these modes at ~600-900 TFLOP/s)
               const int si = p.seg.width > 0 ? (kb * BK) / p.seg.width : 0;
               const int r0 = kb * BK - si * (p.seg.width > 0 ? p.seg.width : 0);
-              tma_load_3d(sb, &tmB, &full_bar[stage], 0, r0, (p.segB_col[si] + n_blk * BN) >> 6);
+              stage_load<CTAS>(sb, &tmB, &full_bar[stage], fb, 0, r0, (p.segB_col[si] + nb0) >> 6);
             }
             if (++stage == STAGES) { stage = 0; phase ^= 1; }
           }
         } else {
-          const int mn = p.m_blocks * p.n_blocks;
-          const int split = tile / mn;
-          const int rem = tile - split * mn;
-          const int m_blk = rem / p.n_blocks;
-          const int n_blk = rem - m_blk * p.n_blocks;
-          const int kb_total = p.batch * p.kb_per_batch;
-          const int per = (kb_total + p.splits - 1) / p.splits;
-          const int lo = split * per;
-          const int hi = min(lo + per, kb_total);
+          int lo, hi;
+          wgrad_kb_range(p, tc.split, lo, hi);
           for (int kb = lo; kb < hi; ++kb) {
             const int b = kb / p.kb_per_batch;
             const int row0 = (kb - b * p.kb_per_batch) * BK;
-            mbar_wait_relaxed(&empty_bar[stage], phase ^ 1);
+            wait_free(&empty_bar[stage], phase ^ 1);
             uint8_t* sa = smem + stage * C::STAGE_BYTES;
             uint8_t* sb = sa + C::A_BYTES;
-            mbar_arrive_expect_tx(&full_bar[stage], C::STAGE_BYTES);
-            // A operand: dY[b, row, m] (m contiguous): BM/64 MN atoms of 64 reduction rows, one 5-D TMA
+            const uint32_t fb = CTAS == 2 ? mapa_shared(smem_u32(&full_bar[stage]), 0) : 0u;
+            if (leader) mbar_arrive_expect_tx(&full_bar[stage], CTAS * C::STAGE_BYTES);
+            // A operand: dY[b, row, m] (m contiguous): this CTA's BM/64 MN atoms of 64 reduction rows, one 5-D TMA
             // {64 cols, rows, column atoms, q, batch}
-            tma_load_5d(sa, &tmA, &full_bar[stage], 0, row0, (m_blk * BM) >> 6, 0, b);
-            // B operand: X[b, row + p, (q), n]: BN/64 atoms; one TMA when the tile lies inside one segment
-            if (p.b_single) {
+            stage_load<CTAS>(sa, &tmA, &full_bar[stage], fb, 0, row0, tc.row0 >> 6, 0, b);
+            // B operand: X[b, row + p, (q), n]: BN/CTAS/64 atoms; one TMA when they lie inside one segment (the host
+            // routes pairs here only then), else one per atom
+            if (CTAS == 2 || p.b_single) {
               int c0, q, po;
-              seg_coords(p.seg, n_blk * BN, c0, q, po);
-              tma_load_5d(sb, &tmB, &full_bar[stage], 0, row0 + po, c0 >> 6, q, b);
+              seg_coords(p.seg, nb0, c0, q, po);
+              stage_load<CTAS>(sb, &tmB, &full_bar[stage], fb, 0, row0 + po, c0 >> 6, q, b);
             } else {
 #pragma unroll
               for (int a = 0; a < BN / 64; ++a) {
                 int c0, q, po;
-                seg_coords(p.seg, n_blk * BN + a * 64, c0, q, po);
-                tma_load_5d(sb + a * (BK * 128), &tmB1, &full_bar[stage], 0, row0 + po, c0 >> 6, q, b);
+                seg_coords(p.seg, nb0 + a * 64, c0, q, po);
+                stage_load<CTAS>(sb + a * (BK * 128), &tmB1, &full_bar[stage], fb, 0, row0 + po, c0 >> 6, q, b);
               }
             }
             if (++stage == STAGES) { stage = 0; phase ^= 1; }
           }
         }
       }
-      if (p.dbg) p.dbg[blockIdx.x * 8 + 3] = dbg_prod;
+      if (DBG && p.dbg) p.dbg[blockIdx.x * 8 + 3] = dbg_prod;
     }
   } else if (warp == 1) {
-    // ======================================================================================= MMA issuer
-    if (lane == 0) {
-      constexpr uint32_t idesc = TF32 ? umma_idesc_tf32(BM, BN) : umma_idesc_bf16(BM, BN, WGRAD, B_MN);
+    // ======================================================================================= MMA issuer (leader CTA)
+    if (leader && lane == 0) {
+      constexpr uint32_t idesc = TF32 ? umma_idesc_tf32(TILE_ROWS, BN) : umma_idesc_bf16(TILE_ROWS, BN, WGRAD, B_MN);
       int stage = 0;
       uint32_t phase = 0;
       int it = 0;
       long long dbg_full = 0, dbg_empty = 0;
-      const long long dbg_t0 = p.dbg ? clock64() : 0;
-      for (int tile = blockIdx.x; tile < p.total_tiles; tile += gridDim.x, ++it) {
+      const long long dbg_t0 = (DBG && p.dbg) ? clock64() : 0;
+      for (int tile = first_tile(); tile < p.total_tiles; tile += tile_step(), ++it) {
         const int acc = it & 1;
         const uint32_t acc_phase = (it >> 1) & 1;
         const int nkb = num_kb(tile);
-        long long tw = p.dbg ? clock64() : 0;
-        mbar_wait_relaxed(&tempty_bar[acc], acc_phase ^ 1);
-        if (p.dbg) dbg_empty += clock64() - tw;
+        long long tw = (DBG && p.dbg) ? clock64() : 0;
+        wait_free(&tempty_bar[acc], acc_phase ^ 1);
+        if (DBG && p.dbg) dbg_empty += clock64() - tw;
         tc_fence_after();
         const uint32_t d_tmem = tmem_base + acc * BN;
         for (int kb = 0; kb < nkb; ++kb) {
-          tw = p.dbg ? clock64() : 0;
+          tw = (DBG && p.dbg) ? clock64() : 0;
           mbar_wait(&full_bar[stage], phase);
-          if (p.dbg) dbg_full += clock64() - tw;
+          if (DBG && p.dbg) dbg_full += clock64() - tw;
           tc_fence_after();
           const uint32_t sa = smem_u32(smem + stage * C::STAGE_BYTES);
           const uint32_t sb = sa + C::A_BYTES;
@@ -726,15 +807,21 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
             else da = umma_smem_desc_sw128(sa + k * 2048, BK * 128, 1024);
             if constexpr (!B_MN) db = umma_smem_desc_sw128(sb + k * 32, 0, 1024);
             else db = umma_smem_desc_sw128(sb + k * 2048, BK * 128, 1024);
-            if constexpr (TF32) umma_tf32(d_tmem, da, db, idesc, (kb > 0 || k > 0) ? 1u : 0u);
-            else umma_bf16(d_tmem, da, db, idesc, (kb > 0 || k > 0) ? 1u : 0u);
+            const uint32_t accum = (kb > 0 || k > 0) ? 1u : 0u;
+            if constexpr (CTAS == 2) umma_bf16_pair(d_tmem, da, db, idesc, accum);
+            else if constexpr (TF32) umma_tf32(d_tmem, da, db, idesc, accum);
+            else umma_bf16(d_tmem, da, db, idesc, accum);
           }
-          umma_commit(&empty_bar[stage]);  // frees the smem slot when these MMAs retire
+          // frees the smem slot (of both CTAs) when these MMAs retire
+          if constexpr (CTAS == 1) umma_commit(&empty_bar[stage]);
+          else umma_commit_pair(&empty_bar[stage]);
           if (++stage == STAGES) { stage = 0; phase ^= 1; }
         }
-        umma_commit(&tfull_bar[acc]);  // accumulator complete -> epilogue
+        // accumulator complete -> epilogue (of both CTAs)
+        if constexpr (CTAS == 1) umma_commit(&tfull_bar[acc]);
+        else umma_commit_pair(&tfull_bar[acc]);
       }
-      if (p.dbg) {
+      if (DBG && p.dbg) {
         p.dbg[blockIdx.x * 8 + 0] = dbg_full;
         p.dbg[blockIdx.x * 8 + 1] = dbg_empty;
         p.dbg[blockIdx.x * 8 + 2] = clock64() - dbg_t0;
@@ -757,7 +844,7 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
     constexpr int CHUNKS = (BN / 32 + 3) / 4; // 32-column chunks per warp (TMA-store paths)
     int it = 0;
     long long dbg_epi = 0;
-    const long long dbg_e0 = p.dbg ? clock64() : 0;
+    const long long dbg_e0 = (DBG && p.dbg) ? clock64() : 0;
     AuxPipe ap;
     ap.buf = smem + C::STAGING_OFF + ew * C::WARP_STAGING;
     ap.bar = aux_bar + ew * 2;
@@ -765,317 +852,71 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
     if constexpr (AUXQ) {
       if (p.tma_store) {   // factors of this CTA's first tile
 #pragma unroll
-        for (int ch = 0; ch < BN / 128; ++ch) aux_issue<BN>(p, om, ap, lane, lane_grp, col_q, blockIdx.x, ch);
+        for (int ch = 0; ch < BN / 128; ++ch) aux_issue<BN>(p, om, ap, lane, lane_grp, col_q, first_tile(), ch, TILE_ROWS, rank * BM);
       }
     }
-    for (int tile = blockIdx.x; tile < p.total_tiles; tile += gridDim.x, ++it) {
+    for (int tile = first_tile(); tile < p.total_tiles; tile += tile_step(), ++it) {
       const int acc = it & 1;
       const uint32_t acc_phase = (it >> 1) & 1;
-      int m_blk, n_blk, b = 0, row_in_batch0 = 0;
-      bool have_k = true;
-      if constexpr (!WGRAD) {
-        m_blk = tile / p.n_blocks;
-        n_blk = tile - m_blk * p.n_blocks;
-        b = m_blk / p.mb_per_batch;
-        row_in_batch0 = (m_blk - b * p.mb_per_batch) * BM;
-      } else {
-        const int mn = p.m_blocks * p.n_blocks;
-        const int rem = tile % mn;
-        m_blk = rem / p.n_blocks;
-        n_blk = rem - m_blk * p.n_blocks;
-        have_k = num_kb(tile) > 0;
-      }
-      const long long tw = (p.dbg && warp == kEpiWarp0) ? clock64() : 0;
+      const TileCoords tc = tile_coords<WGRAD>(p, tile, TILE_ROWS, rank * BM);
+      const bool have_k = !WGRAD || num_kb(tile) > 0;
+      const long long tw = (DBG && p.dbg && warp == kEpiWarp0) ? clock64() : 0;
       mbar_wait(&tfull_bar[acc], acc_phase);
-      if (p.dbg && warp == kEpiWarp0) dbg_epi += clock64() - tw;
+      if (DBG && p.dbg && warp == kEpiWarp0) dbg_epi += clock64() - tw;
       tc_fence_after();
       const uint32_t t_acc = tmem_base + (static_cast<uint32_t>(lane_grp * 32) << 16) + acc * BN;
       const uint32_t t_base = t_acc + col_q * (CHUNKS * 32);   // (TMA-store paths: CHUNKS consecutive chunks per warp)
+      // the accumulator goes back to the MMA warp through the (leader's) accumulator-empty barrier
+      const uint32_t te = CTAS == 2 ? mapa_shared(smem_u32(&tempty_bar[acc]), 0) : 0u;
+      auto arrive = [&]() {
+        if constexpr (CTAS == 1) mbar_arrive(&tempty_bar[acc]);
+        else mbar_arrive_cluster(te);
+      };
       if constexpr (!WGRAD && !TF32) {
         if (p.tma_store) {
           if constexpr (AUXQ) {   // (for dgrad the second instantiation is the GELU-backward path)
-            epilogue_tile_tma_aux<BN>(p, om, t_base, ap, lane, lane_grp, col_q, tile, n_blk, b, row_in_batch0,
-                                      tile + static_cast<int>(gridDim.x), [&]() { mbar_arrive(&tempty_bar[acc]); });
+            epilogue_tile_tma_aux<BN>(p, om, t_base, ap, lane, lane_grp, col_q, tc.n_blk, tc.b, tc.row0,
+                                      tile + tile_step(), arrive, TILE_ROWS, rank * BM);
           } else {
-            epilogue_tile_tma<BN, HEAVY>(p, om, t_base, ap.buf, lane, lane_grp, col_q, n_blk, b, row_in_batch0,
-                                         [&]() { mbar_arrive(&tempty_bar[acc]); });
+            epilogue_tile_tma<BN, HEAVY>(p, om, t_base, ap.buf, lane, lane_grp, col_q, tc.n_blk, tc.b, tc.row0, arrive);
           }
           continue;
         }
       }
       long long out_off = 0;
-      if constexpr (WGRAD) out_off = static_cast<long long>(tile / (p.m_blocks * p.n_blocks)) * p.split_stride;
-      epilogue_tile<BN, WGRAD, TF32>(p, t_acc, lane, lane_grp, col_q, n_blk, b, row_in_batch0,
-                                     static_cast<long long>(m_blk) * BM, have_k, [&]() { mbar_arrive(&tempty_bar[acc]); },
+      if constexpr (WGRAD) out_off = static_cast<long long>(tc.split) * p.split_stride;
+      epilogue_tile<BN, WGRAD, TF32>(p, t_acc, lane, lane_grp, col_q, tc.n_blk, tc.b, tc.row0, tc.row0, have_k, arrive,
                                      out_off);
     }
     if (p.tma_store && lane == 0) bulk_wait0();   // all TMA stores of this warp are complete before smem goes away
-    if (p.dbg && warp == kEpiWarp0 && lane == 0) {
+    if (DBG && p.dbg && warp == kEpiWarp0 && lane == 0) {
       p.dbg[blockIdx.x * 8 + 4] = dbg_epi;
       p.dbg[blockIdx.x * 8 + 5] = clock64() - dbg_e0;
     }
   }
 
   tc_fence_before();
-  __syncthreads();
+  if constexpr (CTAS == 1) __syncthreads();
+  else cluster_sync_all();
   if (warp == 2) {
     tc_fence_after();
-    tmem_dealloc(tmem_base, 512);
+    if constexpr (CTAS == 1) tmem_dealloc(tmem_base, 512);
+    else tmem_dealloc_pair(tmem_base, 512);
   }
 }
 
-// =================================================================================================== CTA-pair kernel
-// Same roles as gemm_kernel, but two CTAs of a cluster (one TPC) work on one 256 x BN tile with
-// tcgen05.mma.cta_group::2: each CTA stages its own 128 rows of A and its own HALF of B (BN/2 columns), the leader's
-// single MMA thread drives both tensor cores, and each CTA's TMEM receives its 128 accumulator rows.  Per SM that is
-// 32 KB of operands per 128 x 256 x 64 of MMA work instead of 48 KB (less L2 -> SM traffic, 6 pipeline stages instead
-// of 4 in the same shared memory, and only 2/3 of the shared-memory read bandwidth), which is what the single-CTA
-// kernel runs out of.  Barrier protocol: both producers signal the LEADER's full barriers (TMA .cta_group::2), the
-// leader's commits are multicast to the empty / accumulator-full barriers of both CTAs, the epilogue warps of both
-// CTAs arrive on the leader's accumulator-empty barrier.
-template <int BN, bool AUX = false>
-struct CfgPair {
-  static constexpr int A_BYTES = BM * BK * 2;
-  static constexpr int B_BYTES = (BN / 2) * BK * 2;
-  static constexpr int STAGE_BYTES = A_BYTES + B_BYTES;
-  static constexpr int STAGES = AUX ? 5 : ((BN == 256) ? 6 : 8);   // AUX (GELU-backward dgrad): see Cfg
-  static constexpr int STAGING_OFF = STAGES * STAGE_BYTES + 1024;   // barriers live in the 1 KB before it
-  static constexpr int WARP_STAGING = AUX ? 4096 : 2048;
-  static constexpr int SMEM_BYTES = STAGING_OFF + 1024 /*align slack*/ + kEpiWarps * WARP_STAGING /*TMA-store staging*/;
-  static_assert(SMEM_BYTES <= 232448, "shared memory budget");
-};
+template <int BN, int MODE, bool HEAVY, bool TF32 = false>
+__global__ void __launch_bounds__(kThreads, 1)
+gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
+            const __grid_constant__ CUtensorMap tmB1, const __grid_constant__ OutMaps om, const GemmParams p) {
+  gemm_body<BN, MODE, HEAVY, TF32, 1>(tmA, tmB, tmB1, om, p, threadIdx.x);
+}
 
 template <int BN, int MODE, bool HEAVY>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
 gemm_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
                  const __grid_constant__ OutMaps om, const GemmParams p) {
-  constexpr bool AUXQ = (MODE == 2 && HEAVY);   // GELU-backward dgrad: TMA-fed factor tiles (see epilogue_tile_tma_aux)
-  using C = CfgPair<BN, AUXQ>;
-  constexpr bool WGRAD = (MODE == 1);
-  constexpr bool B_MN = (MODE != 0);
-  constexpr int STAGES = C::STAGES;
-  constexpr int BMP = 2 * BM;   // rows of a pair tile
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  uint64_t* full_bar = reinterpret_cast<uint64_t*>(smem + STAGES * C::STAGE_BYTES);
-  uint64_t* empty_bar = full_bar + STAGES;
-  uint64_t* tfull_bar = empty_bar + STAGES;
-  uint64_t* tempty_bar = tfull_bar + 2;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tempty_bar + 2);
-  uint64_t* aux_bar = full_bar + 64;            // [kEpiWarps][2], 512 bytes into the barrier KB
-
-  const int warp = threadIdx.x >> 5;
-  const int lane = threadIdx.x & 31;
-  const uint32_t rank = cluster_ctarank();
-  const bool leader = rank == 0;
-  const int pair_id = blockIdx.x >> 1;
-  const int n_pairs = gridDim.x >> 1;
-
-  if (warp == 0 && lane == 0) {
-    tma_prefetch_desc(&tmA);
-    tma_prefetch_desc(&tmB);
-  }
-  if (warp == 1 && lane == 0) {
-    for (int i = 0; i < STAGES; ++i) {
-      mbar_init(&full_bar[i], 1);
-      mbar_init(&empty_bar[i], 1);
-    }
-    for (int i = 0; i < 2; ++i) {
-      mbar_init(&tfull_bar[i], 1);
-      mbar_init(&tempty_bar[i], 2 * kEpiWarps);
-    }
-    if constexpr (AUXQ) {
-      for (int i = 0; i < 2 * kEpiWarps; ++i) mbar_init(&aux_bar[i], 1);
-    }
-    fence_mbar_init();
-  }
-  if (warp == 2) tmem_alloc_pair(tmem_slot, 512);
-  tc_fence_before();
-  cluster_sync_all();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-
-  auto num_kb = [&](int tile) -> int {
-    if constexpr (!WGRAD) {
-      return p.K / BK;
-    } else {
-      const int split = tile / (p.m_blocks * p.n_blocks);
-      const int kb_total = p.batch * p.kb_per_batch;
-      const int per = (kb_total + p.splits - 1) / p.splits;
-      const int lo = split * per;
-      int hi = lo + per;
-      if (hi > kb_total) hi = kb_total;
-      return hi > lo ? hi - lo : 0;
-    }
-  };
-
-  using RS = RegSplit<(MODE == 0 && HEAVY)>;
-  if (warp < kEpiWarp0) reg_dealloc<RS::CTRL>();
-  if (warp == 0) {
-    // ======================================================================================= TMA producer (both CTAs)
-    if (lane == 0) {
-      int stage = 0;
-      uint32_t phase = 0;
-      for (int tile = pair_id; tile < p.total_tiles; tile += n_pairs) {
-        if constexpr (!WGRAD) {
-          const int m_blk = tile / p.n_blocks;
-          const int n_blk = tile - m_blk * p.n_blocks;
-          const int b = m_blk / p.mb_per_batch;
-          const int row0 = (m_blk - b * p.mb_per_batch) * BMP + static_cast<int>(rank) * BM;
-          const int nkb = p.K / BK;
-          for (int kb = 0; kb < nkb; ++kb) {
-            mbar_wait(&empty_bar[stage], phase ^ 1);
-            uint8_t* sa = smem + stage * C::STAGE_BYTES;
-            uint8_t* sb = sa + C::A_BYTES;
-            const uint32_t fb = mapa_shared(smem_u32(&full_bar[stage]), 0);
-            int c0, q, po;
-            seg_coords(p.seg, kb * BK, c0, q, po);
-            if (leader) mbar_arrive_expect_tx(&full_bar[stage], 2 * C::STAGE_BYTES);
-            tma_load_4d_pair(sa, &tmA, fb, c0, q, row0 + po, b);
-            if constexpr (!B_MN) {
-              tma_load_2d_pair(sb, &tmB, fb, kb * BK, n_blk * BN + static_cast<int>(rank) * (BN / 2));
-            } else {
-              // dgrad: this CTA's BN/2 output columns = BN/128 MN-major atoms, one 3-D TMA (see gemm_kernel)
-              const int si = p.seg.width > 0 ? (kb * BK) / p.seg.width : 0;
-              const int r0 = kb * BK - si * (p.seg.width > 0 ? p.seg.width : 0);
-              tma_load_3d_pair(sb, &tmB, fb, 0, r0, (p.segB_col[si] + n_blk * BN + static_cast<int>(rank) * (BN / 2)) >> 6);
-            }
-            if (++stage == STAGES) { stage = 0; phase ^= 1; }
-          }
-        } else {
-          const int mn = p.m_blocks * p.n_blocks;
-          const int split = tile / mn;
-          const int rem = tile - split * mn;
-          const int m_blk = rem / p.n_blocks;
-          const int n_blk = rem - m_blk * p.n_blocks;
-          const int kb_total = p.batch * p.kb_per_batch;
-          const int per = (kb_total + p.splits - 1) / p.splits;
-          const int lo = split * per;
-          const int hi = min(lo + per, kb_total);
-          for (int kb = lo; kb < hi; ++kb) {
-            const int b = kb / p.kb_per_batch;
-            const int row0 = (kb - b * p.kb_per_batch) * BK;
-            mbar_wait(&empty_bar[stage], phase ^ 1);
-            uint8_t* sa = smem + stage * C::STAGE_BYTES;
-            uint8_t* sb = sa + C::A_BYTES;
-            const uint32_t fb = mapa_shared(smem_u32(&full_bar[stage]), 0);
-            if (leader) mbar_arrive_expect_tx(&full_bar[stage], 2 * C::STAGE_BYTES);
-            // A: this CTA's 128 of the pair tile's 256 dY columns (BM/64 MN-major atoms, one 5-D TMA);
-            // B: its BN/2 of the X columns (BN/128 atoms, one 5-D TMA: the host only routes here when a CTA's half tile
-            // lies inside one segment)
-            tma_load_5d_pair(sa, &tmA, fb, 0, row0, (m_blk * BMP + static_cast<int>(rank) * BM) >> 6, 0, b);
-            {
-              int c0, q, po;
-              seg_coords(p.seg, n_blk * BN + static_cast<int>(rank) * (BN / 2), c0, q, po);
-              tma_load_5d_pair(sb, &tmB, fb, 0, row0 + po, c0 >> 6, q, b);
-            }
-            if (++stage == STAGES) { stage = 0; phase ^= 1; }
-          }
-        }
-      }
-    }
-  } else if (warp == 1) {
-    // ======================================================================================= MMA issuer (leader CTA)
-    if (leader && lane == 0) {
-      constexpr uint32_t idesc = umma_idesc_bf16(BMP, BN, WGRAD, B_MN);
-      int stage = 0;
-      uint32_t phase = 0;
-      int it = 0;
-      for (int tile = pair_id; tile < p.total_tiles; tile += n_pairs, ++it) {
-        const int acc = it & 1;
-        const uint32_t acc_phase = (it >> 1) & 1;
-        const int nkb = num_kb(tile);
-        mbar_wait(&tempty_bar[acc], acc_phase ^ 1);
-        tc_fence_after();
-        const uint32_t d_tmem = tmem_base + acc * BN;
-        for (int kb = 0; kb < nkb; ++kb) {
-          mbar_wait(&full_bar[stage], phase);
-          tc_fence_after();
-          const uint32_t sa = smem_u32(smem + stage * C::STAGE_BYTES);
-          const uint32_t sb = sa + C::A_BYTES;
-#pragma unroll
-          for (int k = 0; k < BK / 16; ++k) {
-            uint64_t da, db;
-            if constexpr (!WGRAD) da = umma_smem_desc_sw128(sa + k * 32, 0, 1024);
-            else da = umma_smem_desc_sw128(sa + k * 2048, BK * 128, 1024);
-            if constexpr (!B_MN) db = umma_smem_desc_sw128(sb + k * 32, 0, 1024);
-            else db = umma_smem_desc_sw128(sb + k * 2048, BK * 128, 1024);
-            umma_bf16_pair(d_tmem, da, db, idesc, (kb > 0 || k > 0) ? 1u : 0u);
-          }
-          umma_commit_pair(&empty_bar[stage]);   // frees this smem slot in both CTAs
-          if (++stage == STAGES) { stage = 0; phase ^= 1; }
-        }
-        umma_commit_pair(&tfull_bar[acc]);       // accumulator complete -> epilogue warps of both CTAs
-      }
-    }
-  } else if (warp >= kEpiWarp0) {
-    // ======================================================================================= epilogue (both CTAs)
-    reg_alloc<RS::EPI>();
-    const int ew = warp - kEpiWarp0;
-    const int lane_grp = warp & 3;
-    const int col_q = ew >> 2;
-    constexpr int CHUNKS = BN / 32 / 4;
-    int it = 0;
-    AuxPipe ap;
-    ap.buf = smem + C::STAGING_OFF + ew * C::WARP_STAGING;
-    ap.bar = aux_bar + ew * 2;
-    ap.phase[0] = ap.phase[1] = 0;
-    if constexpr (AUXQ) {
-      if (p.tma_store) {   // factors of this pair's first tile (this CTA's 128 rows)
-#pragma unroll
-        for (int ch = 0; ch < BN / 128; ++ch)
-          aux_issue<BN>(p, om, ap, lane, lane_grp, col_q, pair_id, ch, BMP, static_cast<int>(rank) * BM);
-      }
-    }
-    for (int tile = pair_id; tile < p.total_tiles; tile += n_pairs, ++it) {
-      const int acc = it & 1;
-      const uint32_t acc_phase = (it >> 1) & 1;
-      int m_blk, n_blk, b = 0, row_in_batch0 = 0;
-      bool have_k = true;
-      if constexpr (!WGRAD) {
-        m_blk = tile / p.n_blocks;
-        n_blk = tile - m_blk * p.n_blocks;
-        b = m_blk / p.mb_per_batch;
-        row_in_batch0 = (m_blk - b * p.mb_per_batch) * BMP + static_cast<int>(rank) * BM;
-      } else {
-        const int mn = p.m_blocks * p.n_blocks;
-        const int rem = tile % mn;
-        m_blk = rem / p.n_blocks;
-        n_blk = rem - m_blk * p.n_blocks;
-        have_k = num_kb(tile) > 0;
-      }
-      mbar_wait(&tfull_bar[acc], acc_phase);
-      tc_fence_after();
-      const uint32_t t_base = tmem_base + (static_cast<uint32_t>(lane_grp * 32) << 16) + acc * BN;
-      const uint32_t te = mapa_shared(smem_u32(&tempty_bar[acc]), 0);
-      if constexpr (!WGRAD) {
-        if (p.tma_store) {   // bf16 outputs: the same staged TMA-store epilogues as the single-CTA kernel
-          if constexpr (AUXQ) {
-            epilogue_tile_tma_aux<BN>(p, om, t_base + col_q * (CHUNKS * 32), ap, lane, lane_grp, col_q, tile, n_blk, b,
-                                      row_in_batch0, tile + n_pairs, [&]() { mbar_arrive_cluster(te); }, BMP,
-                                      static_cast<int>(rank) * BM);
-          } else {
-            epilogue_tile_tma<BN, HEAVY>(p, om, t_base + col_q * (CHUNKS * 32), ap.buf, lane, lane_grp, col_q, n_blk, b,
-                                         row_in_batch0, [&]() { mbar_arrive_cluster(te); });
-          }
-          continue;
-        }
-      }
-      long long out_off = 0;
-      if constexpr (WGRAD) out_off = static_cast<long long>(tile / (p.m_blocks * p.n_blocks)) * p.split_stride;
-      epilogue_tile<BN, WGRAD>(p, t_base, lane, lane_grp, col_q, n_blk, b, row_in_batch0,
-                               static_cast<long long>(m_blk) * BMP + static_cast<long long>(rank) * BM, have_k,
-                               [&]() { mbar_arrive_cluster(te); }, out_off);
-    }
-    if (p.tma_store && lane == 0) bulk_wait0();   // all TMA stores of this warp are complete before smem goes away
-  }
-
-  tc_fence_before();
-  cluster_sync_all();
-  if (warp == 2) {
-    tc_fence_after();
-    tmem_dealloc_pair(tmem_base, 512);
-  }
+  gemm_body<BN, MODE, HEAVY, false, 2>(tmA, tmB, tmB, om, p, threadIdx.x);
 }
 
 // =================================================================================================== host side
@@ -1192,25 +1033,31 @@ static int encode_out_map(CUtensorMap* tm, const void* ptr, int N, int L, int ba
   return WJ_OK;
 }
 
-// Decides whether the epilogue can take the TMA-store path and builds its maps.
-static int setup_out_maps(GemmParams& p, OutMaps& om, int N, int L, int batch, bool dgrad = false) {
+// Whether the epilogue can take the TMA-store path: bf16 outputs with bias / GELU (optionally saving GELU'), and in
+// dgrads also the GELU-backward form out = acc * aux (+ fused column sums), no bias.  Everything else (fp32 outputs,
+// reduce-add, residual, row scatter) takes the generic epilogue.
+static bool tma_store_ok(const wj_epilogue_t* e, int N, bool dgrad) {
+  if (e == nullptr) return false;
+  const bool gelu_bwd = dgrad && e->act == 2 && e->aux != nullptr && e->bias == nullptr && e->out2 == nullptr &&
+                        e->ld_aux % 8 == 0 && reinterpret_cast<uintptr_t>(e->aux) % 16 == 0 && N % 8 == 0;
+  return !e->out_f32 && !e->accumulate && e->resid == nullptr && e->out_rows == nullptr &&
+         (gelu_bwd || (e->colsum == nullptr && (e->act == 0 || e->act == 1))) && e->ld_out % 8 == 0 &&
+         reinterpret_cast<uintptr_t>(e->out) % 16 == 0 &&
+         (e->out2 == nullptr || (e->ld_out2 % 8 == 0 && reinterpret_cast<uintptr_t>(e->out2) % 16 == 0));
+}
+
+// Decides whether the epilogue takes the TMA-store path and builds its maps.
+static int setup_out_maps(GemmParams& p, OutMaps& om, const wj_epilogue_t* e, int N, int L, int batch, bool dgrad) {
   memset(&om, 0, sizeof(om));
   p.tma_store = 0;
-  // dgrad also takes the GELU-backward form: out = acc * aux (+ fused column sums), no bias
-  const bool gelu_bwd = dgrad && p.act == 2 && p.aux != nullptr && p.bias == nullptr && p.out2 == nullptr &&
-                        p.ld_aux % 8 == 0 && reinterpret_cast<uintptr_t>(p.aux) % 16 == 0 && N % 8 == 0;
-  const bool ok = !p.out_f32 && !p.accumulate && p.resid == nullptr && p.out_rows == nullptr &&
-                  (gelu_bwd || (p.colsum == nullptr && (p.act == 0 || p.act == 1))) && (p.ld_out % 8 == 0) &&
-                  (reinterpret_cast<uintptr_t>(p.out) % 16 == 0) &&
-                  (p.out2 == nullptr || (p.ld_out2 % 8 == 0 && reinterpret_cast<uintptr_t>(p.out2) % 16 == 0));
-  if (!ok) return WJ_OK;
+  if (!tma_store_ok(e, N, dgrad)) return WJ_OK;
   int rc = encode_out_map(&om.o, p.out, N, L, batch, p.ld_out);
   if (rc) return rc;
   if (p.out2 != nullptr) {
     rc = encode_out_map(&om.o2, p.out2, N, L, batch, p.ld_out2);
     if (rc) return rc;
   }
-  if (gelu_bwd) {   // the saved factors have the output's shape: same box geometry, read by TMA loads (OutMaps::o2)
+  if (p.act == 2) {   // GELU backward: the saved factors have the output's shape, read by TMA loads (OutMaps::o2)
     rc = encode_out_map(&om.o2, p.aux, N, L, batch, p.ld_aux);
     if (rc) return rc;
   }
@@ -1222,73 +1069,41 @@ static int num_sms() { return sm_count(); }
 
 // 192-column tiles exist for the generic (fp32-output) epilogue and for the plain bf16 TMA-store epilogue
 static bool tile192_ok(const wj_epilogue_t* e, int N) {
-  if (e == nullptr || N % 192 != 0) return false;
-  if (e->out_f32) return true;
-  return !e->accumulate && e->resid == nullptr && e->out_rows == nullptr && e->colsum == nullptr && e->out2 == nullptr &&
-         (e->act == 0 || e->act == 1) && e->ld_out % 8 == 0 && reinterpret_cast<uintptr_t>(e->out) % 16 == 0;
+  return e != nullptr && N % 192 == 0 && (e->out_f32 || (tma_store_ok(e, N, false) && e->out2 == nullptr));
 }
 
-template <int BN, int MODE, bool HEAVY, bool TF32 = false>
+// Grid: one CTA (CTA pair) per tile, at most one per SM (pair of SMs); the kernels loop over the remaining tiles.
+template <int BN, int MODE, bool HEAVY, bool TF32, int CTAS>
 static int launch_variant(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMap& tmB1, const OutMaps& om,
-                          const GemmParams& p, int grid, cudaStream_t st) {
+                          const GemmParams& p, cudaStream_t st) {
   static bool attr_set = false;
-  auto kern = gemm_kernel<BN, MODE, HEAVY, TF32>;
-  constexpr int kSmem = Cfg<BN, (MODE == 2 && HEAVY)>::SMEM_BYTES;
+  constexpr int kSmem = Cfg<BN, (MODE == 2 && HEAVY), CTAS>::SMEM_BYTES;
   if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem);
+    cudaError_t e;
+    if constexpr (CTAS == 1) e = cudaFuncSetAttribute(gemm_kernel<BN, MODE, HEAVY, TF32>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem);
+    else e = cudaFuncSetAttribute(gemm_pair_kernel<BN, MODE, HEAVY>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem);
     if (e != cudaSuccess) { set_error("cudaFuncSetAttribute: %s", cudaGetErrorString(e)); return WJ_ERR_RUNTIME; }
     attr_set = true;
   }
-  kern<<<grid, kThreads, kSmem, st>>>(tmA, tmB, tmB1, om, p);
-  return check_launch("gemm_tcgen05 launch");
+  const int units = p.total_tiles < num_sms() / CTAS ? p.total_tiles : num_sms() / CTAS;
+  if constexpr (CTAS == 1) gemm_kernel<BN, MODE, HEAVY, TF32><<<units, kThreads, kSmem, st>>>(tmA, tmB, tmB1, om, p);
+  else gemm_pair_kernel<BN, MODE, HEAVY><<<CTAS * units, kThreads, kSmem, st>>>(tmA, tmB, om, p);
+  return check_launch(CTAS == 1 ? "gemm_tcgen05 launch" : "gemm_tcgen05 pair launch");
 }
 
-template <int BN, int MODE, bool HEAVY>
-static int launch_pair_variant(const CUtensorMap& tmA, const CUtensorMap& tmB, const OutMaps& om, const GemmParams& p,
-                               cudaStream_t st) {
-  static bool attr_set = false;
-  auto kern = gemm_pair_kernel<BN, MODE, HEAVY>;
-  constexpr int kSmem = CfgPair<BN, (MODE == 2 && HEAVY)>::SMEM_BYTES;
-  if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem);
-    if (e != cudaSuccess) { set_error("cudaFuncSetAttribute(pair): %s", cudaGetErrorString(e)); return WJ_ERR_RUNTIME; }
-    attr_set = true;
-  }
-  int pairs = num_sms() / 2;
-  if (p.total_tiles < pairs) pairs = p.total_tiles;
-  kern<<<2 * pairs, kThreads, kSmem, st>>>(tmA, tmB, om, p);
-  return check_launch("gemm_tcgen05 pair launch");
-}
-
-template <int BN, int MODE>
-static int launch_pair(const CUtensorMap& tmA, const CUtensorMap& tmB, const OutMaps& om, const GemmParams& p,
-                       cudaStream_t st) {
-  if constexpr (MODE == 0) {
-    if (p.tma_store && p.out2 != nullptr) return launch_pair_variant<BN, MODE, true>(tmA, tmB, om, p, st);
-  }
-  if constexpr (MODE == 2) {   // GELU-backward data gradient: the TMA-fed factor pipeline
-    if (p.tma_store && p.act == 2) return launch_pair_variant<BN, MODE, true>(tmA, tmB, om, p, st);
-  }
-  return launch_pair_variant<BN, MODE, false>(tmA, tmB, om, p, st);
-}
-
-template <int BN, int MODE>
+// The two-output epilogue (GELU + saved GELU') and the GELU-backward dgrad (TMA-fed factor tiles) are their own
+// instantiations of the TMA-store path (HEAVY: register budget, shared-memory layout).  192-column tiles (N = 384-like
+// shapes) have the generic epilogue and the plain bf16 TMA-store epilogue (bias / GELU) only.
+template <int BN, int MODE, int CTAS>
 static int launch(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMap& tmB1, const OutMaps& om,
-                  const GemmParams& p, int grid, cudaStream_t st) {
+                  const GemmParams& p, cudaStream_t st) {
+  const bool heavy = p.tma_store && (p.out2 != nullptr || p.act == 2);
   if constexpr (BN == 192) {
-    // 192-column tiles (N = 384-like shapes): generic epilogue, or the plain bf16 TMA-store epilogue (bias / GELU)
-    if (p.tma_store && (p.out2 != nullptr || p.act == 2)) { set_error("gemm: BN = 192 has only the plain TMA-store epilogue"); return WJ_ERR_ARG; }
-    return launch_variant<BN, MODE, false>(tmA, tmB, tmB1, om, p, grid, st);
-  } else {
-    if constexpr (MODE != 1) {
-      // the two-output epilogue (GELU + saved GELU') has its own instantiation of the TMA-store path (register budget)
-      if (p.tma_store && p.out2 != nullptr) return launch_variant<BN, MODE, true>(tmA, tmB, tmB1, om, p, grid, st);
-    }
-    if constexpr (MODE == 2) {
-      if (p.tma_store && p.act == 2) return launch_variant<BN, MODE, true>(tmA, tmB, tmB1, om, p, grid, st);
-    }
+    if (heavy) { set_error("gemm: BN = 192 has only the plain TMA-store epilogue"); return WJ_ERR_ARG; }
+  } else if constexpr (MODE != 1) {
+    if (heavy) return launch_variant<BN, MODE, true, false, CTAS>(tmA, tmB, tmB1, om, p, st);
   }
-  return launch_variant<BN, MODE, false>(tmA, tmB, tmB1, om, p, grid, st);
+  return launch_variant<BN, MODE, false, false, CTAS>(tmA, tmB, tmB1, om, p, st);
 }
 
 static void fill_seg(SegInfo& s, const wj_operand_t* op) {
@@ -1305,6 +1120,20 @@ static void fill_epilogue(GemmParams& p, const wj_epilogue_t* e) {
   p.bias = e->bias; p.resid = e->resid; p.resid_f32 = e->resid_f32; p.ld_resid = e->ld_resid;
   p.resid_mod = e->resid_mod; p.aux = reinterpret_cast<const bf16*>(e->aux); p.ld_aux = e->ld_aux;
   p.act = e->act; p.out_rows = e->out_rows; p.colsum = e->colsum;
+}
+
+// Parameters of the row-tiled modes (forward, dgrad, tf32): m-blocks of tile_rows rows (BM, or 2 * BM for CTA pairs)
+// per batch entry, BN-column n-blocks.
+static void row_tiled_params(GemmParams& p, const wj_operand_t* A, const wj_epilogue_t* epi, int L, int batch, int N,
+                             int K, int block_n, int tile_rows) {
+  memset(&p, 0, sizeof(p));
+  p.L = L; p.batch = batch; p.N = N; p.K = K;
+  p.mb_per_batch = (L + tile_rows - 1) / tile_rows;
+  p.m_blocks = batch * p.mb_per_batch;
+  p.n_blocks = (N + block_n - 1) / block_n;
+  p.total_tiles = p.m_blocks * p.n_blocks;
+  fill_seg(p.seg, A);
+  fill_epilogue(p, epi);
 }
 
 }  // namespace wj
@@ -1349,10 +1178,7 @@ extern "C" int wj_gemm_bf16(const wj_operand_t* A, const void* W, int64_t ldw, i
   // on the TMA-store epilogue with K >= 768 -- measured +5..11 % on the teacher / student / conv forward shapes
   // (1257 vs 1170, 1275 vs 1190, 1360 vs 1271, 1377 vs 1235 TFLOP/s); the K = 384 shapes and the generic fp32 epilogue
   // are faster on single CTAs (607 vs 696 TFLOP/s on the predictor's fc1)
-  if (block_n == 0 && K >= 768 && N % 256 == 0 && static_cast<long long>(L) * batch >= 4096 && epi != nullptr &&
-      !epi->out_f32 && !epi->accumulate && epi->resid == nullptr && epi->out_rows == nullptr && epi->colsum == nullptr &&
-      (epi->act == 0 || epi->act == 1) && epi->ld_out % 8 == 0 && reinterpret_cast<uintptr_t>(epi->out) % 16 == 0 &&
-      (epi->out2 == nullptr || (epi->ld_out2 % 8 == 0 && reinterpret_cast<uintptr_t>(epi->out2) % 16 == 0))) {
+  if (block_n == 0 && K >= 768 && N % 256 == 0 && static_cast<long long>(L) * batch >= 4096 && tma_store_ok(epi, N, false)) {
     pair = true;
     block_n = 256;
   }
@@ -1367,36 +1193,15 @@ extern "C" int wj_gemm_bf16(const wj_operand_t* A, const void* W, int64_t ldw, i
   rc = encode_map_2d(&tmB, W, (uint64_t)K, (uint64_t)N, (uint64_t)ldw * 2, BK, (uint32_t)(pair ? block_n / 2 : block_n));
   if (rc) return rc;
   GemmParams p;
-  memset(&p, 0, sizeof(p));
-  p.L = L; p.batch = batch; p.N = N; p.K = K;
-  if (pair) {
-    p.mb_per_batch = (L + 2 * BM - 1) / (2 * BM);
-    p.m_blocks = batch * p.mb_per_batch;
-    p.n_blocks = (N + block_n - 1) / block_n;
-    p.total_tiles = p.m_blocks * p.n_blocks;
-    fill_seg(p.seg, A);
-    fill_epilogue(p, epi);
-    cudaStream_t stp = reinterpret_cast<cudaStream_t>(stream);
-    OutMaps omp;
-    rc = setup_out_maps(p, omp, N, L, batch);
-    if (rc) return rc;
-    if (block_n == 256) return launch_pair<256, 0>(tmA, tmB, omp, p, stp);
-    return launch_pair<128, 0>(tmA, tmB, omp, p, stp);
-  }
-  p.mb_per_batch = (L + BM - 1) / BM;
-  p.m_blocks = batch * p.mb_per_batch;
-  p.n_blocks = (N + block_n - 1) / block_n;
-  p.total_tiles = p.m_blocks * p.n_blocks;
-  fill_seg(p.seg, A);
-  fill_epilogue(p, epi);
-  const int grid = p.total_tiles < num_sms() ? p.total_tiles : num_sms();
+  row_tiled_params(p, A, epi, L, batch, N, K, block_n, pair ? 2 * BM : BM);
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   OutMaps om;
-  rc = setup_out_maps(p, om, N, L, batch);
+  rc = setup_out_maps(p, om, epi, N, L, batch, /*dgrad=*/false);
   if (rc) return rc;
-  if (block_n == 256) return launch<256, 0>(tmA, tmB, tmB, om, p, grid, st);
-  if (block_n == 192) return launch<192, 0>(tmA, tmB, tmB, om, p, grid, st);
-  return launch<128, 0>(tmA, tmB, tmB, om, p, grid, st);
+  if (pair) return block_n == 256 ? launch<256, 0, 2>(tmA, tmB, tmB, om, p, st) : launch<128, 0, 2>(tmA, tmB, tmB, om, p, st);
+  if (block_n == 256) return launch<256, 0, 1>(tmA, tmB, tmB, om, p, st);
+  if (block_n == 192) return launch<192, 0, 1>(tmA, tmB, tmB, om, p, st);
+  return launch<128, 0, 1>(tmA, tmB, tmB, om, p, st);
 }
 
 // dW[m, vc] (+)= sum_{b, t} dY(b, t; m) * X(vc; t, b)      fp32 output, reduce-add when splits > 1 or accumulate.
@@ -1483,13 +1288,12 @@ extern "C" int wj_gemm_wgrad_bf16(const wj_operand_t* dY, const wj_operand_t* X,
                                       (size_t)(transposed ? N : M), reinterpret_cast<cudaStream_t>(stream));
     if (e != cudaSuccess) { set_error("memset2d: %s", cudaGetErrorString(e)); return WJ_ERR_RUNTIME; }
   }
-  const int grid = p.total_tiles < num_sms() ? p.total_tiles : num_sms();
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   OutMaps om;
   memset(&om, 0, sizeof(om));
-  if (pair) rc = launch_pair<256, 1>(tmA, tmB, om, p, st);
-  else if (block_n == 256) rc = launch<256, 1>(tmA, tmB, tmB1, om, p, grid, st);
-  else rc = launch<128, 1>(tmA, tmB, tmB1, om, p, grid, st);
+  if (pair) rc = launch<256, 1, 2>(tmA, tmB, tmB, om, p, st);
+  else if (block_n == 256) rc = launch<256, 1, 1>(tmA, tmB, tmB1, om, p, st);
+  else rc = launch<128, 1, 1>(tmA, tmB, tmB1, om, p, st);
   if (rc == WJ_OK && det_slabs != nullptr) rc = det_reduce_f32(det_slabs, splits, M, N, out, ld_out, st);
   return rc;
 }
@@ -1519,14 +1323,10 @@ extern "C" int wj_gemm_dgrad_bf16(const wj_operand_t* A, const void* W, int64_t 
   // CTA pairs for the plain bf16-output data gradients (TMA-store epilogue) with K >= 768 and whole 256-column tiles: the
   // same rule as the forward GEMMs (wj_gemm_bf16)
   // (plain bf16 outputs, or the GELU-backward form out = acc * saved factor with optional fused column sums)
-  const bool pair_gelu = epi != nullptr && epi->act == 2 && epi->aux != nullptr && epi->bias == nullptr &&
-                         epi->ld_aux % 8 == 0 && reinterpret_cast<uintptr_t>(epi->aux) % 16 == 0;
-  const bool pair_ok = epi != nullptr && !epi->out_f32 && !epi->accumulate && epi->resid == nullptr && epi->out_rows == nullptr &&
-                       epi->out2 == nullptr && ((epi->act == 0 && epi->colsum == nullptr) || pair_gelu) && epi->ld_out % 8 == 0 &&
-                       reinterpret_cast<uintptr_t>(epi->out) % 16 == 0 && N % 256 == 0;
+  const bool pair_ok = tma_store_ok(epi, N, /*dgrad=*/true) && epi->out2 == nullptr && epi->act != 1 && N % 256 == 0;
   if (pair && !(pair_ok && block_n == 256)) { set_error("wj_gemm_dgrad_bf16: the CTA-pair kernel takes plain bf16 outputs with N %% 256 == 0"); return WJ_ERR_ARG; }
   // (K >= 512 for plain outputs: +4 % on the K = 512 conv data gradient; the GELU-backward form loses there, 645 vs 738)
-  if (auto_bn && g_pair_dgrad && pair_ok && K >= (pair_gelu ? 768 : 512) && static_cast<long long>(L) * batch >= 4096) {
+  if (auto_bn && g_pair_dgrad && pair_ok && K >= (epi->act == 2 ? 768 : 512) && static_cast<long long>(L) * batch >= 4096) {
     pair = true;
     block_n = 256;
   }
@@ -1537,37 +1337,19 @@ extern "C" int wj_gemm_dgrad_bf16(const wj_operand_t* A, const void* W, int64_t 
   rc = encode_map_mn3(&tmB, W, (uint64_t)w_rows, (uint64_t)w_cols, (uint64_t)ldw * 2, (uint32_t)((pair ? block_n / 2 : block_n) / 64));
   if (rc) return rc;
   GemmParams p;
-  memset(&p, 0, sizeof(p));
-  p.L = L; p.batch = batch; p.N = N; p.K = K;
-  if (pair) {
-    p.mb_per_batch = (L + 2 * BM - 1) / (2 * BM);
-    p.m_blocks = batch * p.mb_per_batch;
-    p.n_blocks = N / block_n;
-    p.total_tiles = p.m_blocks * p.n_blocks;
-    fill_seg(p.seg, A);
-    for (int i = 0; i < 4; ++i) p.segB_col[i] = seg_col_off ? seg_col_off[i] : 0;
-    fill_epilogue(p, epi);
-    OutMaps omp;
-    rc = setup_out_maps(p, omp, N, L, batch, /*dgrad=*/true);
-    if (rc) return rc;
-    if (!p.tma_store) { set_error("wj_gemm_dgrad_bf16: pair kernel without a TMA-store epilogue"); return WJ_ERR_ARG; }
-    return launch_pair<256, 2>(tmA, tmB, omp, p, reinterpret_cast<cudaStream_t>(stream));
-  }
-  p.mb_per_batch = (L + BM - 1) / BM;
-  p.m_blocks = batch * p.mb_per_batch;
-  p.n_blocks = (N + block_n - 1) / block_n;
-  p.total_tiles = p.m_blocks * p.n_blocks;
-  fill_seg(p.seg, A);
+  row_tiled_params(p, A, epi, L, batch, N, K, block_n, pair ? 2 * BM : BM);
   for (int i = 0; i < 4; ++i) p.segB_col[i] = seg_col_off ? seg_col_off[i] : 0;
-  fill_epilogue(p, epi);
-  const int grid = p.total_tiles < num_sms() ? p.total_tiles : num_sms();
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   OutMaps om;
-  rc = setup_out_maps(p, om, N, L, batch, /*dgrad=*/true);
+  rc = setup_out_maps(p, om, epi, N, L, batch, /*dgrad=*/true);
   if (rc) return rc;
-  if (block_n == 192) return launch<192, 2>(tmA, tmB, tmB, om, p, grid, st);
-  if (block_n == 256) return launch<256, 2>(tmA, tmB, tmB, om, p, grid, st);
-  return launch<128, 2>(tmA, tmB, tmB, om, p, grid, st);
+  if (pair) {
+    if (!p.tma_store) { set_error("wj_gemm_dgrad_bf16: pair kernel without a TMA-store epilogue"); return WJ_ERR_ARG; }
+    return launch<256, 2, 2>(tmA, tmB, tmB, om, p, st);
+  }
+  if (block_n == 192) return launch<192, 2, 1>(tmA, tmB, tmB, om, p, st);
+  if (block_n == 256) return launch<256, 2, 1>(tmA, tmB, tmB, om, p, st);
+  return launch<128, 2, 1>(tmA, tmB, tmB, om, p, st);
 }
 
 // Reference-precision (TF32) inference GEMM: out[b*L + t, n] = epilogue( sum_vc A(vc; t, b) * W[n, vc] ) with A and W fp32
@@ -1600,19 +1382,11 @@ extern "C" int wj_gemm_tf32(const wj_operand_t* A, const float* W, int64_t ldw, 
   rc = encode_map_2d(&tmB, W, (uint64_t)K, (uint64_t)N, (uint64_t)ldw * 4, KB, (uint32_t)block_n, CU_TENSOR_MAP_DATA_TYPE_FLOAT32);
   if (rc) return rc;
   GemmParams p;
-  memset(&p, 0, sizeof(p));
-  p.L = L; p.batch = batch; p.N = N; p.K = K;
-  p.mb_per_batch = (L + BM - 1) / BM;
-  p.m_blocks = batch * p.mb_per_batch;
-  p.n_blocks = N / block_n;
-  p.total_tiles = p.m_blocks * p.n_blocks;
-  fill_seg(p.seg, A);
-  fill_epilogue(p, epi);
+  row_tiled_params(p, A, epi, L, batch, N, K, block_n, BM);
   p.round_tf32 = round_out ? 1 : 0;
-  const int grid = p.total_tiles < num_sms() ? p.total_tiles : num_sms();
   OutMaps om;
   memset(&om, 0, sizeof(om));   // (generic epilogue: no TMA stores)
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  if (block_n == 256) return launch_variant<256, 0, false, true>(tmA, tmB, tmB, om, p, grid, st);
-  return launch_variant<128, 0, false, true>(tmA, tmB, tmB, om, p, grid, st);
+  if (block_n == 256) return launch_variant<256, 0, false, true, 1>(tmA, tmB, tmB, om, p, st);
+  return launch_variant<128, 0, false, true, 1>(tmA, tmB, tmB, om, p, st);
 }
