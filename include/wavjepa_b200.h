@@ -211,6 +211,19 @@ int wj_crop_norm(const float* audio, const int* starts, const float* gain, int n
  * normalize_audio (hear_api/feature_helper.py:5-13). */
 int wj_clip_gain(const float* audio, int n_clips, int channels, int64_t clip_len, float target_dbfs, float* gain,
                  void* stream);
+/* Backward of wj_crop_norm for the HEAR chunking only: crop j of a clip starts at j*crop_len and crops_per_clip ==
+ * clip_len / crop_len + 1 (the zero-padded chunks of hear_api/runtime.py:107-124); any other geometry is refused with
+ * WJ_ERR_ARG.  dy: fp32 gradient of the fp32 output [n_clips*crops_per_clip, channels, crop_len].  Writes daudio
+ * [n_clips, channels, clip_len] (every sample: each belongs to exactly one crop) = g * dz, and dgain_part
+ * [n_clips*crops_per_clip] (may be NULL) = sum over the crop of dz * audio, the crop's share of the gradient of gain[clip]
+ * (gain NULL = 1).  z, mean and std are recomputed as the forward forms them; fp64 block reductions, no atomics. */
+int wj_crop_norm_bwd(const float* audio, const float* gain, const float* dy, int n_clips, int channels,
+                     int64_t clip_len, int crops_per_clip, int crop_len, float* daudio, float* dgain_part, void* stream);
+/* Backward of wj_clip_gain (target_dbfs does not enter it): dgain = sum_{j < parts} dgain_part[clip*parts + j] in index
+ * order, dx[clip] = -dgain * gain[clip] * audio[clip] / sum(audio[clip]^2) (0 for a silent clip, whose gain is the
+ * constant 1).  One block per clip, no atomics. */
+int wj_clip_gain_bwd(const float* audio, const float* gain, const float* dgain_part, int n_clips, int channels,
+                     int64_t clip_len, int parts, float* dx, void* stream);
 
 /* ------------------------------------------------------------------------------------------------------------------
  * On-GPU input pipeline (data_modules/WebAudioDataModule.py:43-61, dataset_functions.py:92-114).

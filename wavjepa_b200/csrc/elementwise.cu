@@ -115,6 +115,36 @@ __global__ void __launch_bounds__(512) clip_gain_kernel(const float* __restrict_
   }
 }
 
+// Backward of clip_gain_kernel: g = 10^(target / 20) / rms with rms^2 = sum x^2 / N, so dg/dx_j = -g x_j / sum x^2.
+// dgain = sum of the clip's `parts` partial gain gradients in index order; dx = dgain * dg/dx (0 when rms == 0: g = 1 is
+// then a constant).  The sum of squares is reduced in the forward's order.
+__global__ void __launch_bounds__(512) clip_gain_bwd_kernel(const float* __restrict__ audio, long long per_clip,
+                                                            const float* __restrict__ gain,
+                                                            const float* __restrict__ dgain_part, int parts,
+                                                            float* __restrict__ dx) {
+  __shared__ double s_red[16];
+  __shared__ float s_coef;
+  const float* src = audio + static_cast<size_t>(blockIdx.x) * per_clip;
+  float* dst = dx + static_cast<size_t>(blockIdx.x) * per_clip;
+  double acc = 0.0;
+  for (long long i = threadIdx.x; i < per_clip; i += blockDim.x) { const double v = src[i]; acc += v * v; }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+  if ((threadIdx.x & 31) == 0) s_red[threadIdx.x >> 5] = acc;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    double t = 0.0;
+    for (int w = 0; w < 16; ++w) t += s_red[w];
+    const float rms = sqrtf(static_cast<float>(t / static_cast<double>(per_clip)));
+    double dg = 0.0;
+    for (int j = 0; j < parts; ++j) dg += dgain_part[static_cast<size_t>(blockIdx.x) * parts + j];
+    s_coef = rms != 0.f ? static_cast<float>(-dg * gain[blockIdx.x] / t) : 0.f;
+  }
+  __syncthreads();
+  const float coef = s_coef;
+  for (long long i = threadIdx.x; i < per_clip; i += blockDim.x) dst[i] = coef * src[i];
+}
+
 // x0[r, :] = (src[r] >= 0 ? ctx[src[r], :] : bf16(mask_token)) + pos[pos_idx[r], :]
 __global__ void __launch_bounds__(256) predictor_assemble_kernel(const bf16* __restrict__ ctx,
                                                                  const float* __restrict__ mask_token,
@@ -523,6 +553,15 @@ extern "C" int wj_clip_gain(const float* audio, int n_clips, int channels, int64
   clip_gain_kernel<<<n_clips, 512, 0, WJ_STREAM(stream)>>>(audio, static_cast<long long>(channels) * clip_len,
                                                           target_dbfs, gain);
   return check_launch("clip_gain");
+}
+
+extern "C" int wj_clip_gain_bwd(const float* audio, const float* gain, const float* dgain_part, int n_clips,
+                                int channels, int64_t clip_len, int parts, float* dx, void* stream) {
+  if (n_clips <= 0) return WJ_OK;
+  if (parts <= 0) { set_error("wj_clip_gain_bwd: parts = %d, need >= 1", parts); return WJ_ERR_ARG; }
+  clip_gain_bwd_kernel<<<n_clips, 512, 0, WJ_STREAM(stream)>>>(audio, static_cast<long long>(channels) * clip_len, gain,
+                                                              dgain_part, parts, dx);
+  return check_launch("clip_gain_bwd");
 }
 
 extern "C" int wj_predictor_assemble(const void* ctx_bf16, const float* mask_token, const float* pos,

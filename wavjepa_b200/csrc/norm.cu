@@ -285,6 +285,89 @@ __global__ void __launch_bounds__(512) crop_norm_kernel(const float* __restrict_
   }
 }
 
+__device__ __forceinline__ double warp_sum_f64(double v) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+  return v;
+}
+
+// Backward of crop_norm_kernel for the HEAR chunking (start = chunk * Lc, S = Lfull / Lc + 1 chunks): one block / chunk,
+// so every sample < Lfull has exactly one writer.  z, mean and std are recomputed as the forward forms them; with
+// S1 = sum dy, S2 = sum dy (z - mean) and inv = 1 / (std + 1e-5):
+//   dz = inv (dy - S1 / n) - inv^2 (z - mean) S2 / ((n - 1) std)      (the S2 term is 0 when std == 0)
+// da = g dz for the samples inside the clip.  dgain_part[chunk] = sum dz a, this chunk's share of the gain gradient, is
+// taken in closed form: with z = g a (zero in the padding), sum dz z = inv S2 - inv^2 S2 std = 1e-5 inv^2 S2, so
+// sum dz a = 1e-5 inv^2 S2 / g.  (The normalisation is scale-invariant up to the 1e-5, so the direct sum would cancel
+// down to fp32 rounding noise.)
+__global__ void __launch_bounds__(512, 1) crop_norm_bwd_kernel(const float* __restrict__ audio,
+                                                               const float* __restrict__ gain,
+                                                               const float* __restrict__ dy, int C, long long Lfull,
+                                                               int S, int Lc, float* __restrict__ da,
+                                                               float* __restrict__ dgain_part) {
+  __shared__ double2 s_red[32];
+  __shared__ double2 s_val;
+  const int inst = blockIdx.x;
+  const int clip = inst / S;
+  const long long start = static_cast<long long>(inst - clip * S) * Lc;
+  const float* src = audio + static_cast<size_t>(clip) * C * Lfull;
+  float* dst = da + static_cast<size_t>(clip) * C * Lfull;
+  const float* g_out = dy + static_cast<size_t>(inst) * C * Lc;
+  const int n = C * Lc;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
+  const float gn = gain ? gain[clip] : 1.0f;
+  auto raw = [=](int i) -> float {   // a, zero past the clip end
+    const int c = i / Lc, t = i - c * Lc;
+    const long long p = start + t;
+    return p < Lfull ? src[static_cast<size_t>(c) * Lfull + p] : 0.f;
+  };
+  auto block_sum = [&](double2 v) -> double2 {
+    v.x = warp_sum_f64(v.x);
+    v.y = warp_sum_f64(v.y);
+    __syncthreads();
+    if (lane == 0) s_red[warp] = v;
+    __syncthreads();
+    if (warp == 0) {
+      const double2 t = lane < nw ? s_red[lane] : make_double2(0.0, 0.0);
+      const double tx = warp_sum_f64(t.x), ty = warp_sum_f64(t.y);
+      if (lane == 0) s_val = make_double2(tx, ty);
+    }
+    __syncthreads();
+    return s_val;
+  };
+  // pass 1: sum z (the forward's mean) and S1
+  double2 acc = make_double2(0.0, 0.0);
+  for (int i = threadIdx.x; i < n; i += blockDim.x) {
+    acc.x += __fmul_rn(raw(i), gn);
+    acc.y += g_out[i];
+  }
+  double2 r = block_sum(acc);
+  const double mean = r.x / n, s1 = r.y;
+  // pass 2: the forward's sum of squares and S2
+  acc = make_double2(0.0, 0.0);
+  for (int i = threadIdx.x; i < n; i += blockDim.x) {
+    const double d = __fmul_rn(raw(i), gn) - mean;
+    acc.x += d * d;
+    acc.y += g_out[i] * d;
+  }
+  r = block_sum(acc);
+  const float sd = static_cast<float>(sqrt(r.x / (n - 1)));
+  const float inv = 1.0f / (sd + 1e-5f);
+  const float fm = static_cast<float>(mean);
+  const float c1 = static_cast<float>(s1 / n);
+  const float c2 = sd > 0.f ? static_cast<float>(static_cast<double>(inv) * inv * r.y / ((n - 1) * static_cast<double>(sd)))
+                            : 0.f;
+  if (threadIdx.x == 0 && dgain_part != nullptr)
+    dgain_part[inst] = static_cast<float>(1e-5 * static_cast<double>(inv) * inv * r.y / gn);
+  // pass 3: dz and the data gradient of the samples inside the clip
+  for (int i = threadIdx.x; i < n; i += blockDim.x) {
+    const int c = i / Lc, t = i - c * Lc;
+    const long long p = start + t;
+    if (p >= Lfull) continue;
+    const float dz = inv * (g_out[i] - c1) - c2 * (__fmul_rn(src[static_cast<size_t>(c) * Lfull + p], gn) - fm);
+    dst[static_cast<size_t>(c) * Lfull + p] = gn * dz;
+  }
+}
+
 // ------------------------------------------------------------------------------------------------ teacher targets
 // inst_stats[b] = {mean, rstd} over the T*D values of instance b, from per-row (sum, sumsq) pairs.
 __global__ void __launch_bounds__(256) instance_stats_kernel(const float* __restrict__ rowsum, int B, int T, int D,
@@ -491,6 +574,22 @@ extern "C" int wj_crop_norm(const float* audio, const int* starts, const float* 
   crop_norm_kernel<<<n, 512, 0, WJ_STREAM(stream)>>>(audio, starts, channels, clip_len, crops_per_clip, crop_len, gain,
                                                     reinterpret_cast<bf16*>(out_bf16), out_f32);
   return check_launch("crop_norm");
+}
+
+extern "C" int wj_crop_norm_bwd(const float* audio, const float* gain, const float* dy, int n_clips, int channels,
+                                int64_t clip_len, int crops_per_clip, int crop_len, float* daudio, float* dgain_part,
+                                void* stream) {
+  if (n_clips <= 0) return WJ_OK;
+  if (crop_len <= 1 || clip_len < 0 || crops_per_clip != clip_len / crop_len + 1) {
+    set_error("wj_crop_norm_bwd: only the HEAR chunking has a backward (crop i at i * crop_len, clip_len / crop_len + 1 "
+              "crops per clip); got %d crops of %d samples over clips of %lld", crops_per_clip, crop_len,
+              static_cast<long long>(clip_len));
+    return WJ_ERR_ARG;
+  }
+  crop_norm_bwd_kernel<<<n_clips * crops_per_clip, 512, 0, WJ_STREAM(stream)>>>(audio, gain, dy, channels, clip_len,
+                                                                               crops_per_clip, crop_len, daudio,
+                                                                               dgain_part);
+  return check_launch("crop_norm_bwd");
 }
 
 extern "C" int wj_target_combine(const float* const* xs, const float* const* rowsums, int n_layers, int B, int T, int D,

@@ -20,7 +20,12 @@ B200-first differences (results identical at every returned frame):
                         accumulation, residual stream and chunk audio, exact erf GELU: <= 2e-3 relative L2
                         (tests/test_gpu_tf32.py), at a lower throughput (DESIGN.md 2.1);
   * `layer=k` on the loaders embeds encoder hidden state k (JEPA.get_hidden_states) instead of the final features, so a
-    layer sweep is one more runner option; only the first k encoder layers run (DESIGN.md 2.4).
+    layer sweep is one more runner option; only the first k encoder layers run (DESIGN.md 2.4);
+  * whole clips are differentiable in training mode (DESIGN.md 2.5): the loaders return the runtime in eval mode, and
+    after `.train()` a call in grad mode with precision "bf16" builds a graph when a feature-path parameter or the audio
+    requires grad -- loudness gain, down-mix / channel fix-up, chunking and per-chunk normalisation, encoder, cut-off,
+    channel and scene means all backpropagate, to the parameters and to the audio.  The embeddings are bit-identical to
+    the eval-mode call; every other case runs under no_grad.
 """
 from __future__ import annotations
 
@@ -32,7 +37,7 @@ from torch import nn
 from . import ops
 from ._lib import WavJepaLibError
 from .extractors import ConvFeatureExtractor
-from .jepa import JEPA
+from .jepa import _FEATURE_PATH, JEPA
 from .types import TransformerEncoderCFG, TransformerLayerCFG
 
 SR = 16000
@@ -66,47 +71,103 @@ def get_timestamps(sample_rate: int, B: int, input_audio_len: int, n_frames: int
     return torch.tensor([step * i for i in range(n_frames)]).unsqueeze(0).repeat(B, 1)
 
 
-@torch.no_grad()
+class _ClipGain(torch.autograd.Function):
+    """The -14 dBFS loudness gain of `to_feature` (ops.clip_gain over the whole [B, C, L] clip) under autograd.  The
+    gain comes out once per chunk, [B, n_chunks] (a broadcast view of [B]), so that `_ChunkNorm` hands back each chunk's
+    share of the gain gradient and the backward (ops.clip_gain_bwd) sums them in a fixed order."""
+
+    @staticmethod
+    def forward(ctx, a, n_chunks):
+        gain = ops.clip_gain(a, -14.0)
+        ctx.save_for_backward(a, gain)
+        return gain[:, None].expand(-1, n_chunks)
+
+    @staticmethod
+    def backward(ctx, dgain):
+        a, gain = ctx.saved_tensors
+        return ops.clip_gain_bwd(a, gain, dgain.contiguous()), None
+
+
+class _ChunkNorm(torch.autograd.Function):
+    """The chunking + per-chunk normalisation of `embed_chunks` (ops.crop_norm at starts i * unit) under autograd: a
+    [B, C, L] fp32, gain [B, n_chunks] from `_ClipGain` -> the fp32 chunks [B * n_chunks, C, unit].  The backward
+    (ops.crop_norm_bwd) returns (da, dgain), dgain per chunk."""
+
+    @staticmethod
+    def forward(ctx, a, gain, unit):
+        B, C, _ = a.shape
+        n_chunks = gain.shape[1]
+        g = gain[:, 0]   # the clip's gain: [B], contiguous (gain is a broadcast view)
+        starts = (torch.arange(n_chunks, device=a.device, dtype=torch.int32) * unit).repeat(B)
+        out = torch.empty(B * n_chunks, C, unit, device=a.device, dtype=torch.float32)
+        ops.crop_norm(a, starts, n_chunks, unit, None, out, gain=g)
+        ctx.save_for_backward(a, g)
+        ctx.unit = unit
+        return out
+
+    @staticmethod
+    def backward(ctx, dy):
+        a, g = ctx.saved_tensors
+        da, dgain = ops.crop_norm_bwd(a, g, dy.contiguous(), ctx.unit)
+        return da, dgain, None
+
+
 def embed_chunks(model: JEPA, a: torch.Tensor, gain: Optional[torch.Tensor], unit: int, steps: int, sr: int,
-                 channel_tokens: int = 1, layer: Optional[int] = None):
+                 channel_tokens: int = 1, layer: Optional[int] = None, graph: bool = False):
     """The chunk loop of hear_api/runtime.py:107-142 (and ARCH/configs/wavjepa_wrapper.py:67-110) as ONE batched pass:
     a [B, C, L] fp32 on the device, gain [B] or None.  Chunk i of clip b = gain * a[b, :, i*unit:(i+1)*unit] (zeros past
     L), normalised per chunk (mean / unbiased std including the zero padding, runtime.py:12-16); the frames that fall
     into the padding are key-masked and cut off.  layer: embed hidden state `layer` of `JEPA.get_hidden_states`
-    instead of the final features (None).  Returns (emb [B, cut_off, D] fp32, cut_off)."""
+    instead of the final features (None).  Returns (emb [B, cut_off, D] fp32, cut_off).
+    graph: build the autograd graph (DESIGN.md 2.5; "bf16" only): gain is then `_ClipGain`'s [B, n_chunks], the chunks
+    are `_ChunkNorm`'s fp32 output, which the model rounds to the bf16 the kernel would write; otherwise the pass runs
+    under no_grad."""
     B, C, L = a.shape
     pad, n_chunks, cut_off, total_steps = hear_geometry(L, unit, sr, steps)
-    dev = a.device
-    starts = (torch.arange(n_chunks, device=dev, dtype=torch.int32) * unit).repeat(B)
-    if model.inference_precision == "tf32":   # conv block 0 reads the fp32 chunks
-        x16 = torch.empty(B * n_chunks, C, unit, device=dev, dtype=torch.float32)
-        ops.crop_norm(a, starts, n_chunks, unit, None, x16, gain=gain)
-    else:
-        x16 = torch.empty(B * n_chunks, C, unit, device=dev, dtype=torch.bfloat16)
-        ops.crop_norm(a, starts, n_chunks, unit, x16, None, gain=gain)
     # The padding mask depends on the geometry only (the same for every clip), so it is built on the HOST and handed over as
     # a pattern that repeats every n_chunks sequences: the packed-token index then needs no device read-back, and calls
     # can be issued back to back without a host synchronisation.
     mask = torch.zeros(max(total_steps, n_chunks * steps), dtype=torch.bool)
     mask[cut_off:total_steps] = True
     mask = mask[:n_chunks * steps].reshape(n_chunks, steps)
+    with torch.set_grad_enabled(graph):
+        dev = a.device
+        if graph:
+            x = _ChunkNorm.apply(a, gain, unit)
+        else:
+            starts = (torch.arange(n_chunks, device=dev, dtype=torch.int32) * unit).repeat(B)
+            if model.inference_precision == "tf32":   # conv block 0 reads the fp32 chunks
+                x = torch.empty(B * n_chunks, C, unit, device=dev, dtype=torch.float32)
+                ops.crop_norm(a, starts, n_chunks, unit, None, x, gain=gain)
+            else:
+                x = torch.empty(B * n_chunks, C, unit, device=dev, dtype=torch.bfloat16)
+                ops.crop_norm(a, starts, n_chunks, unit, x, None, gain=gain)
 
-    def features(host_mask):
-        if layer is None:
-            return model.get_audio_representation(x16, None, host_mask=host_mask)
-        return model.get_hidden_states(x16, None, host_mask=host_mask, layers=[layer])[0]
-    if channel_tokens > 1:
-        # WavJEPA-Nat (hear_api/runtime_natjepa.py:142-147): the model emits channel-major tokens [c0 t0.., c1 t0..]; the
-        # time mask is repeated "B E -> B (C E)" and the per-channel embeddings are averaged
-        emb = features(mask.repeat(1, channel_tokens).numpy())   # [B*n_chunks, C*steps, D]
-        emb = emb.view(B * n_chunks, channel_tokens, steps, -1).mean(dim=1)
-    else:
-        emb = features(mask.numpy())   # [B*n_chunks, steps, D] fp32
-    return emb.reshape(B, n_chunks * steps, -1)[:, :cut_off], cut_off
+        def features(host_mask):
+            if layer is None:
+                return model.get_audio_representation(x, None, host_mask=host_mask)
+            return model.get_hidden_states(x, None, host_mask=host_mask, layers=[layer])[0]
+        if channel_tokens > 1:
+            # WavJEPA-Nat (hear_api/runtime_natjepa.py:142-147): the model emits channel-major tokens [c0 t0.., c1 t0..];
+            # the time mask is repeated "B E -> B (C E)" and the per-channel embeddings are averaged
+            emb = features(mask.repeat(1, channel_tokens).numpy())   # [B*n_chunks, C*steps, D]
+            emb = emb.view(B * n_chunks, channel_tokens, steps, -1).mean(dim=1)
+        else:
+            emb = features(mask.numpy())   # [B*n_chunks, steps, D] fp32
+        return emb.reshape(B, n_chunks * steps, -1)[:, :cut_off], cut_off
 
 
 class RuntimeJEPA(nn.Module):
-    """reference hear_api/runtime.py:39-155."""
+    """reference hear_api/runtime.py:39-155.
+
+    Built in eval mode: `get_timestamp_embeddings` / `get_scene_embeddings` / `forward` run under no_grad and their
+    outputs carry no graph, whatever requires grad.  After `.train()` (the flag of this module: the inner `model` is
+    always run in eval mode), a call in grad mode with precision "bf16" is differentiable when a feature-path parameter
+    of `model` (extract_audio, feature_norms, post_extraction_mapper, encoder) or the audio requires grad: `backward()`
+    fills `.grad` of the trainable path parameters and, when the audio requires grad, `audio.grad` (fp32, on the
+    audio's device) through the loudness gain, the channel fix-up, the chunking and the per-chunk normalisation.  The
+    embeddings are bit-identical to the eval-mode call.  Frozen parts, layer=, one backward per graph: as in
+    `JEPA.get_audio_representation` / `JEPA.get_hidden_states`; precision "tf32" stays forward-only (DESIGN.md 2.5)."""
 
     def __init__(self, in_channels: int, weights, is_spectrogram: bool, process_seconds: float, extractor,
                  model_size: str, sr: int, device: Optional[str] = None, precision: str = "bf16",
@@ -137,11 +198,26 @@ class RuntimeJEPA(nn.Module):
         self.unit_frames = int(process_seconds * self.sample_rate)
         self.output_steps = self.model.extract_audio.total_patches(self.unit_frames)
         self.model.to(device or "cuda")   # no CPU path: a machine without a B200 fails on the first call
-        self.model.eval()
+        self.eval()
+
+    def _graph(self, audio) -> bool:
+        """Whether a call builds an autograd graph: grad mode, training mode, precision "bf16", and the audio or a
+        feature-path parameter requires grad."""
+        if not (torch.is_grad_enabled() and self.training and self.model.inference_precision == "bf16"):
+            return False
+        return (torch.is_tensor(audio) and audio.requires_grad) or \
+            any(p.requires_grad for n, p in self.model.named_parameters() if n.startswith(_FEATURE_PATH))
+
+    def _gain(self, a: torch.Tensor, graph: bool) -> torch.Tensor:
+        """The loudness gain of the [B, C, L] clips before the channel fix-up: [B], or `_ClipGain`'s [B, n_chunks]."""
+        if not graph:
+            return ops.clip_gain(a, -14.0)
+        return _ClipGain.apply(a, hear_geometry(a.shape[2], self.unit_frames, self.sample_rate, self.output_steps)[1])
 
     # ---- hear_api/feature_helper.py:35-88 for tensors that are already batched [B, L] / [B, C, L]
-    def to_feature(self, audio: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
-        """-> (audio [B, 1, L] fp32 on the device, gain [B]); the gain is applied inside the chunk kernel."""
+    def to_feature(self, audio: torch.Tensor, graph: bool = False) -> Tuple[torch.Tensor, torch.Tensor]:
+        """-> (audio [B, 1, L] fp32 on the device, gain [B]); the gain is applied inside the chunk kernel.  graph: the
+        differentiable form of a graph-building call (gain [B, n_chunks], see `embed_chunks`)."""
         dev = self.model.device
         a = torch.as_tensor(audio).to(dev, torch.float32)
         if a.dim() == 2:
@@ -151,7 +227,7 @@ class RuntimeJEPA(nn.Module):
         if a.shape[1] > 100 and a.shape[2] <= 100:      # [B, T, C] -> [B, C, T]   (feature_helper.py:49-50)
             a = a.transpose(1, 2)
         a = a.contiguous()
-        gain = ops.clip_gain(a, -14.0)                   # RMS over the whole (C, L) clip BEFORE the down-mix (:53)
+        gain = self._gain(a, graph)                      # RMS over the whole (C, L) clip BEFORE the down-mix (:53)
         if a.shape[1] == 2:
             a = a.mean(dim=1, keepdim=True).contiguous()   # :66-67
         elif a.shape[1] == 4:
@@ -160,16 +236,16 @@ class RuntimeJEPA(nn.Module):
             raise WavJepaLibError("Unknown channel count")
         return a, gain
 
-    @torch.no_grad()
     def get_timestamp_embeddings(self, audio: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
-        a, gain = self.to_feature(audio)
+        graph = self._graph(audio)
+        with torch.set_grad_enabled(graph):
+            a, gain = self.to_feature(audio, graph)
         B, _, L = a.shape
         emb, _ = embed_chunks(self.model, a, gain, self.unit_frames, self.output_steps, self.sample_rate,
-                              layer=self.layer)
+                              layer=self.layer, graph=graph)
         ts = get_timestamps(self.sample_rate, B, L, emb.shape[1])
         return emb, ts
 
-    @torch.no_grad()
     def get_scene_embeddings(self, audio: torch.Tensor) -> torch.Tensor:
         emb, _ = self.get_timestamp_embeddings(audio)
         return emb.mean(dim=1)
@@ -194,7 +270,7 @@ class RuntimeNatJEPA(RuntimeJEPA):
                          precision, **kwargs)
         self.output_steps = self.model.extract_audio.total_patches(self.unit_frames) // in_channels
 
-    def to_feature(self, audio: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
+    def to_feature(self, audio: torch.Tensor, graph: bool = False) -> Tuple[torch.Tensor, torch.Tensor]:
         dev = self.model.device
         a = torch.as_tensor(audio).to(dev, torch.float32)
         if a.dim() == 2:
@@ -204,7 +280,7 @@ class RuntimeNatJEPA(RuntimeJEPA):
         if a.shape[1] > 100 and a.shape[2] <= 100:
             a = a.transpose(1, 2)
         a = a.contiguous()
-        gain = ops.clip_gain(a, -14.0)                   # RMS over the whole (C, L) clip BEFORE the channel fix-up
+        gain = self._gain(a, graph)                      # RMS over the whole (C, L) clip BEFORE the channel fix-up
         if a.shape[1] == 1:
             a = a.expand(-1, 2, -1).contiguous()           # feature_helper.py:57-58
         elif a.shape[1] == 4:
@@ -213,12 +289,13 @@ class RuntimeNatJEPA(RuntimeJEPA):
             raise WavJepaLibError("Unknown channel count")
         return a, gain
 
-    @torch.no_grad()
     def get_timestamp_embeddings(self, audio: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
-        a, gain = self.to_feature(audio)
+        graph = self._graph(audio)
+        with torch.set_grad_enabled(graph):
+            a, gain = self.to_feature(audio, graph)
         B, C, L = a.shape
         emb, _ = embed_chunks(self.model, a, gain, self.unit_frames, self.output_steps, self.sample_rate, channel_tokens=C,
-                              layer=self.layer)
+                              layer=self.layer, graph=graph)
         ts = get_timestamps(self.sample_rate, B, L, emb.shape[1])
         return emb, ts
 

@@ -67,11 +67,18 @@ class WavJEPAFeatureExtractor:
 
 
 class WavJEPAModel(nn.Module):
-    """`AutoModel` stand-in over the HEAR runtime: forward(input_values) -> (embeddings, timestamps)."""
+    """`AutoModel` stand-in over the HEAR runtime: forward(input_values) -> (embeddings, timestamps).
+
+    Like HF's `from_pretrained`, `from_pretrained` returns the model in eval mode, where forward runs under no_grad.
+    Fine-tuning is opt-in: after `model.train()`, forward in grad mode (precision "bf16") is differentiable --
+    `emb, _ = model(input_values); loss.backward()` fills `.grad` of the trainable feature-path parameters (model
+    parameters under `runtime.model.`) and, when input_values requires grad, `input_values.grad` (hear.RuntimeJEPA,
+    DESIGN.md 2.5)."""
 
     def __init__(self, runtime: hear.RuntimeJEPA):
         super().__init__()
         self.runtime = runtime
+        self.train(runtime.training)   # the runtime's mode (eval when it comes from a loader)
         self.sample_rate = runtime.sample_rate
         self.embedding_size = runtime.embedding_size
 

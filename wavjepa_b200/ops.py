@@ -554,6 +554,46 @@ def clip_gain(audio: torch.Tensor, target_dbfs: float = -14.0) -> torch.Tensor:
     return gain
 
 
+def crop_norm_bwd(audio: torch.Tensor, gain: Optional[torch.Tensor], dy: torch.Tensor, crop_len: int):
+    """Backward of `crop_norm` over the HEAR chunking (crop j of each clip at j * crop_len, clip_len // crop_len + 1
+    crops; the library refuses any other geometry).  audio [n, C, L] and gain [n] (or None) as given to the forward,
+    dy [n * crops, C, crop_len] fp32.  -> (daudio [n, C, L], dgain_part [n, crops]: each crop's share of the gain
+    gradient, summed by `clip_gain_bwd`)."""
+    n_clips, ch, clip_len = audio.shape
+    assert audio.dtype == torch.float32 and audio.is_contiguous()
+    assert dy.dtype == torch.float32 and dy.is_contiguous() and dy.dim() == 3 and dy.shape[1:] == (ch, crop_len)
+    assert dy.shape[0] % max(n_clips, 1) == 0
+    assert gain is None or (gain.dtype == torch.float32 and gain.is_contiguous() and gain.shape == (n_clips,))
+    crops = dy.shape[0] // max(n_clips, 1)
+    daudio = torch.empty_like(audio)
+    part = torch.empty(n_clips, crops, device=audio.device, dtype=torch.float32)
+    lib = _lib.load()
+    p = lambda t: C.c_void_p(_ptr(t))
+    if _lib._profile is not None:   # audio and dy read once each (the recomputations hit L2), daudio written once
+        _lib._profile.nbytes = 4 * (2 * audio.numel() + dy.numel())
+    check(lib.wj_crop_norm_bwd(p(audio), p(gain), p(dy), n_clips, ch, C.c_int64(clip_len), crops, crop_len, p(daudio),
+                               p(part), _stream()))
+    return daudio, part
+
+
+def clip_gain_bwd(audio: torch.Tensor, gain: torch.Tensor, dgain_part: torch.Tensor) -> torch.Tensor:
+    """Backward of `clip_gain`: audio [n, C, L] and gain [n] as in the forward, dgain_part [n, P] the gain gradient in
+    P parts (summed in index order).  -> dx [n, C, L]."""
+    n_clips, ch, clip_len = audio.shape
+    assert audio.dtype == torch.float32 and audio.is_contiguous()
+    assert gain.dtype == torch.float32 and gain.is_contiguous() and gain.shape == (n_clips,)
+    assert dgain_part.dtype == torch.float32 and dgain_part.is_contiguous() and dgain_part.dim() == 2
+    assert dgain_part.shape[0] == n_clips
+    dx = torch.empty_like(audio)
+    lib = _lib.load()
+    p = lambda t: C.c_void_p(_ptr(t))
+    if _lib._profile is not None:   # audio read once (the second read hits L2), dx written once
+        _lib._profile.nbytes = 8 * audio.numel()
+    check(lib.wj_clip_gain_bwd(p(audio), p(gain), p(dgain_part), n_clips, ch, C.c_int64(clip_len), dgain_part.shape[1],
+                               p(dx), _stream()))
+    return dx
+
+
 def scatter_rows(src: torch.Tensor, idx: torch.Tensor, N: int, out: torch.Tensor):
     assert src.dtype == torch.float32 and out.dtype == torch.float32 and idx.dtype == torch.int32
     lib = _lib.load()
