@@ -14,7 +14,7 @@ import torch
 import torch.nn.functional as F
 
 import wavjepa_b200 as w
-from wavjepa_b200 import _lib, hear, jepa, ops
+from wavjepa_b200 import _lib, extractors, hear, jepa, ops
 from oracle import inputs as oi
 from oracle import jepa_oracle as jo
 
@@ -272,9 +272,9 @@ def test_contract_bits_early_exit_and_inference_saves_nothing(monkeypatch):
     calls, saves = [], []
     real_bridge = jepa._FeatureBridge.apply
     monkeypatch.setattr(jepa._FeatureBridge, "apply", lambda *a_, **k_: calls.append(1) or real_bridge(*a_, **k_))
-    real_stack, real_conv, real_ln = model._enc_stack.forward, jepa.conv_stack_forward, ops.layernorm_fwd
+    real_stack, real_conv, real_ln = model._enc_stack.forward, extractors.conv_stack_forward, ops.layernorm_fwd
     monkeypatch.setattr(model._enc_stack, "forward", lambda *a_, **k_: saves.append(a_[6]) or real_stack(*a_, **k_))
-    monkeypatch.setattr(jepa, "conv_stack_forward", lambda *a_, **k_: saves.append(a_[6]) or real_conv(*a_, **k_))
+    monkeypatch.setattr(extractors, "conv_stack_forward", lambda *a_, **k_: saves.append(a_[6]) or real_conv(*a_, **k_))
     monkeypatch.setattr(ops, "layernorm_fwd", lambda *a_, **k_: saves.append(a_[6] is not None) or real_ln(*a_, **k_))
     hs = model.get_hidden_states(audio, pm, layers=[6])
     assert hs[0].grad_fn is None and not calls

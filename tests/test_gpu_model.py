@@ -726,6 +726,43 @@ def test_shared_conv_weights_are_announced_once_final():
             assert flat[off:].double().sum().item() == s1 and flat[off:].abs().double().sum().item() == s2, off
 
 
+@pytest.mark.parametrize("kind", ["mono", "w2v2", "nat", "nat_shared"])
+def test_standalone_extractor_forward_equals_the_models_conv_output(kind):
+    """`extract_audio(x)` is, bit for bit, the conv output the model computes from its flat buffers for the same audio
+    (w2v2 at 4.02 s: a 401-row input to its last block), and after a fused train_step, which updates the parameters in
+    place without bumping their versions, it reads the updated weights."""
+    spec, seconds = (hear.W2V2_SPEC, 4.02) if kind == "w2v2" else (hear.BASE_SPEC, 2.01)
+    if kind.startswith("nat"):
+        ex = w.ConvChannelFeatureExtractor(conv_layers_spec=spec, in_channels=2,
+                                           share_weights_over_channels=kind == "nat_shared")
+    else:
+        ex = w.ConvFeatureExtractor(conv_layers_spec=spec, in_channels=1)
+    model = w.JEPA(feature_extractor=ex, transformer_encoder_cfg=w.TransformerEncoderCFG.create(),
+                   transformer_encoder_layers_cfg=w.TransformerLayerCFG.create(),
+                   transformer_decoder_cfg=w.TransformerEncoderCFG.create(),
+                   transformer_decoder_layers_cfg=w.TransformerLayerCFG.create(d_model=384),
+                   process_audio_seconds=seconds, nr_samples_per_audio=2, average_top_k_layers=8).to(DEV)
+    model.global_step = 50000   # an lr at which one step moves the bf16 working weights
+    Cin, T = ex.in_channels, model.total_patches
+    g = torch.Generator().manual_seed(5)
+    x = torch.randn(2, Cin, model.target_length, generator=g).bfloat16().to(DEV)
+    mk = w.TimeInverseBlockMasker(4, 0.65, 10, 0.25, 10, 0.1, channel_based_masking=Cin == 2, seed=6, row0=0)
+    masks = mk(batch_size=2, n_times=T, in_channels=Cin)
+
+    def model_conv_output():
+        _, (_, f2, _, _) = model._local_features(x, save=False)
+        return f2.view(2, T, -1)
+
+    model.train_step(x, *masks)   # builds the flat buffers: the parameters keep their storage from here on
+    before = model.extract_audio(x)
+    assert before.shape == (2, T, ex.embedding_dim) and before.dtype == torch.bfloat16
+    assert torch.equal(before, model_conv_output())
+    model.train_step(x, *masks)
+    after = model.extract_audio(x)
+    assert not torch.equal(after, before)
+    assert torch.equal(after, model_conv_output())
+
+
 def test_hear_nat_runtime_matches_reference_goldens():
     """VERDICT r1 missing 5: the binaural HEAR runtime (hear_api/runtime_natjepa.py: channel fix-up, joint normalisation,
     channel-major mask, channel mean) against fixtures made by EXECUTING the reference's get_timestamp_embeddings

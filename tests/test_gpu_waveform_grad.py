@@ -17,7 +17,7 @@ import torch.nn.functional as F
 pytestmark = pytest.mark.gpu
 
 import wavjepa_b200 as w  # noqa: E402
-from wavjepa_b200 import _lib, hear, jepa, ops  # noqa: E402
+from wavjepa_b200 import _lib, extractors, hear, jepa, ops  # noqa: E402
 from oracle import inputs as oi  # noqa: E402
 from oracle import jepa_oracle as jo  # noqa: E402
 
@@ -274,9 +274,9 @@ def test_contract_device_dtype_and_inference_path_saves_nothing(monkeypatch):
     calls, saves = [], []
     real_bridge = jepa._FeatureBridge.apply
     monkeypatch.setattr(jepa._FeatureBridge, "apply", lambda *a_, **k_: calls.append(1) or real_bridge(*a_, **k_))
-    real_stack, real_conv, real_ln = model._enc_stack.forward, jepa.conv_stack_forward, ops.layernorm_fwd
+    real_stack, real_conv, real_ln = model._enc_stack.forward, extractors.conv_stack_forward, ops.layernorm_fwd
     monkeypatch.setattr(model._enc_stack, "forward", lambda *a_, **k_: saves.append(a_[6]) or real_stack(*a_, **k_))
-    monkeypatch.setattr(jepa, "conv_stack_forward", lambda *a_, **k_: saves.append(a_[6]) or real_conv(*a_, **k_))
+    monkeypatch.setattr(extractors, "conv_stack_forward", lambda *a_, **k_: saves.append(a_[6]) or real_conv(*a_, **k_))
     monkeypatch.setattr(ops, "layernorm_fwd", lambda *a_, **k_: saves.append(a_[6] is not None) or real_ln(*a_, **k_))
     f = model.get_audio_representation(base.to(DEV))
     assert f.grad_fn is None and not f.requires_grad and not calls

@@ -215,6 +215,110 @@ def conv_stack_backward(spec, sv: ConvSaved, dh_last: torch.Tensor, w0, gn_w, gn
         on_layer_done(0)
 
 
+def _stream_prefixes(ex) -> List[str]:
+    """Name prefix of the CNN that serves each conv stream, in channel order: the mono extractor runs one stream over
+    every input channel, the per-channel (Nat) extractor one mono stream per input channel, all through `cnns.0` when it
+    shares weights over channels."""
+    if isinstance(ex, ConvChannelFeatureExtractor):
+        return [f"cnns.{0 if ex.share_weights_over_channels else c}" for c in range(ex.in_channels)]
+    return ["cnn"]
+
+
+def gemm_weight_names(ex) -> List[str]:
+    """Names of the conv weights of blocks 1.. (the implicit GEMMs, which read tap-major copies), each CNN once."""
+    return [f"{p}.{i}.0.weight" for p in dict.fromkeys(_stream_prefixes(ex)) for i in range(1, len(ex.conv_layers_spec))]
+
+
+def _weights(prefix: str, n_blocks: int, p, wk):
+    """(block 0 weight, GroupNorm weight, GroupNorm bias, [blocks 1.. weights]) of the CNN at `prefix`: the first three
+    through the lookup p, the GEMM weights through wk."""
+    return (p(f"{prefix}.0.0.weight"), p(f"{prefix}.0.2.weight"), p(f"{prefix}.0.2.bias"),
+            [wk(f"{prefix}.{i}.0.weight") for i in range(1, n_blocks)])
+
+
+def _per_stream(ex, x: torch.Tensor, stack) -> torch.Tensor:
+    """Features [B, T, C] of the waveform x [B, Cin, L] from stack(prefix, stream input) -> [B, T_s, C] over the
+    extractor's streams: the mono extractor's one stream reads x itself; the per-channel streams read one channel each
+    and their tokens are laid out channel-major (audio_channel_feature_extractor.py:177-178)."""
+    prefixes = _stream_prefixes(ex)
+    if not isinstance(ex, ConvChannelFeatureExtractor):
+        return stack(prefixes[0], x)
+    B, Cin, L = x.shape
+    feats = None
+    xs = x.transpose(0, 1).contiguous()  # [Cin, B, L]: one mono stream per CNN
+    for c, prefix in enumerate(prefixes):
+        f = stack(prefix, xs[c].unsqueeze(1))
+        if feats is None:
+            Tc = f.shape[1]
+            feats = torch.empty(B, Cin * Tc, f.shape[2], device=x.device, dtype=f.dtype)
+        feats[:, c * Tc:(c + 1) * Tc].copy_(f)
+    return feats
+
+
+# The extractor's forward and backward take lookups from a parameter name relative to the extractor (`cnn.1.0.weight`,
+# `cnns.0.0.2.bias`) to a tensor: p the fp32 master, wk the tap-major working copy (kmajor_weight) of a block-1.. conv
+# weight, g the fp32 gradient view.
+def extractor_forward(ex, x16: torch.Tensor, p, wk, save: bool):
+    """x16 [B, Cin, L] bf16 -> (features [B, T, C] bf16, one ConvSaved per stream, None without save)."""
+    spec = ex.conv_layers_spec
+    saved = []
+
+    def stack(prefix, x):
+        f, sv = conv_stack_forward(spec, x, *_weights(prefix, len(spec), p, wk), save)
+        saved.append(sv)
+        return f
+    return _per_stream(ex, x16, stack), saved
+
+
+def extractor_forward_tf32(ex, x32: torch.Tensor, p, wk) -> torch.Tensor:
+    """Inference at reference precision (conv_stack_forward_tf32): x32 [B, Cin, L] fp32 -> features [B, T, C] fp32; wk
+    looks up the fp32 tap-major weights rounded to nearest tf32."""
+    spec = ex.conv_layers_spec
+    return _per_stream(ex, x32, lambda prefix, x: conv_stack_forward_tf32(spec, x, *_weights(prefix, len(spec), p, wk)))
+
+
+def extractor_backward(ex, saved: List[ConvSaved], dfeat: torch.Tensor, p, wk, g, ready,
+                       dx: Optional[torch.Tensor] = None, weights: bool = True) -> None:
+    """Backward of extractor_forward(save=True) from the fp32 gradient of the features [B*T, C]: accumulates into the
+    gradient views g(name), announces ready(name) for each conv weight once its gradient is final, and with dx (fp32
+    [B, Cin, L], overwritten) runs down to the waveform.  weights=False (frozen extractor, needs dx): data gradients
+    only, g is not read.  The streams run in reverse channel order; a CNN shared over channels adds every pass into the
+    same gradients, so they are final (and may be all-reduced) only after its last pass."""
+    spec = ex.conv_layers_spec
+    n, C = len(spec), ex.embedding_dim
+    prefixes = _stream_prefixes(ex)
+    per_channel = isinstance(ex, ConvChannelFeatureExtractor)
+    B = saved[0].x16.shape[0]
+    Ts = dfeat.shape[0] // (B * len(prefixes))
+    dev = dfeat.device
+    dfeat3 = dfeat.view(B, -1, C)
+    gw = g if weights else (lambda name: None)
+    for s in range(len(prefixes) - 1, -1, -1):
+        prefix, sv = prefixes[s], saved[s]
+        dfs = dfeat3[:, s * Ts:(s + 1) * Ts].contiguous().view(B * Ts, C)   # (one stream: dfeat itself)
+        # each per-channel stream's waveform gradient lands in its channel
+        dxs = torch.empty(B, 1, dx.shape[2], device=dev) if per_channel and dx is not None else dx
+        dh = torch.empty(B, Ts, C, device=dev, dtype=torch.bfloat16)
+        ops.scatter_dgelu(dfs, None, sv.pre[n - 1].view(B * Ts, C), B * Ts, dh.view(B * Ts, C))
+        final = prefix not in prefixes[:s]
+        conv_stack_backward(spec, sv, dh, *_weights(prefix, n, p, wk), *_weights(prefix, n, gw, gw),
+                            on_layer_done=(lambda i: ready(f"{prefix}.{i}.0.weight")) if final else None,
+                            dx=dxs, weights=weights)
+        if dxs is not dx:
+            dx[:, s:s + 1].copy_(dxs)
+
+
+def _forward(ex, x: torch.Tensor) -> torch.Tensor:
+    """The extractor modules' standalone forward: x [B, Cin, L] -> local features [B, T, C] (bf16) from the extractor's
+    own parameters, tap-major copies built on every call."""
+    if x.dim() != 3 or x.shape[1] != ex.in_channels:
+        raise ValueError(f"expected [B, {ex.in_channels}, L], got {tuple(x.shape)}")
+    params = {n: w.detach() for n, w in ex.named_parameters()}
+    wk = {n: kmajor_weight(params[n]) for n in gemm_weight_names(ex)}
+    feats, _ = extractor_forward(ex, x.to(torch.bfloat16).contiguous(), params.__getitem__, wk.__getitem__, False)
+    return feats
+
+
 # =============================================================================================== modules
 class ConvFeatureExtractor(Extractor, nn.Module):
     """reference wavjepa/extractors/audio_feature_extractor.py:13-154 (mode="default", no bias, not depthwise)."""
@@ -242,33 +346,12 @@ class ConvFeatureExtractor(Extractor, nn.Module):
             in_d = dim
         self.cnn = nn.Sequential(*blocks)
         self.embedding_dim = spec[-1][0]
-        self._wk_cache = None
-
-    # ---- weight access used by the JEPA engine
-    def conv_params(self):
-        return [blk[0].weight for blk in self.cnn]
-
-    def gn_params(self):
-        return self.cnn[0][2].weight, self.cnn[0][2].bias
-
-    def _working_weights(self):
-        ws = self.conv_params()
-        sig = tuple((w.data_ptr(), w._version) for w in ws)
-        if self._wk_cache is None or self._wk_cache[0] != sig:
-            self._wk_cache = (sig, [kmajor_weight(w) for w in ws[1:]])
-        return self._wk_cache[1]
 
     @torch.no_grad()
     def forward(self, x: torch.Tensor) -> torch.Tensor:
         """x [B, Cin, L] -> local features [B, T, C] (bf16).  Inference only; training goes through JEPA, whose
         backward owns the saved activations."""
-        if x.dim() != 3 or x.shape[1] != self.in_channels:
-            raise ValueError(f"expected [B, {self.in_channels}, L], got {tuple(x.shape)}")
-        x16 = x.to(torch.bfloat16).contiguous()
-        gw, gb = self.gn_params()
-        feats, _ = conv_stack_forward(self.conv_layers_spec, x16, self.conv_params()[0].detach(), gw.detach(),
-                                      gb.detach(), self._working_weights(), save=False)
-        return feats
+        return _forward(self, x)
 
     def total_patches(self, time: int, device: str = "cuda") -> int:
         return out_length(self.conv_layers_spec, time)
@@ -310,23 +393,17 @@ class ConvChannelFeatureExtractor(Extractor, nn.Module):
         self.share_weights_over_channels = share_weights_over_channels
         spec = [tuple(int(v) for v in cl) for cl in conv_layers_spec]
         n_cnn = 1 if share_weights_over_channels else in_channels
-        subs = [ConvFeatureExtractor(conv_layers_spec=spec, in_channels=1, dropout=dropout, mode=mode,
-                                     conv_bias=conv_bias, depthwise=depthwise) for _ in range(n_cnn)]
-        self._spec = spec
+        self.cnns = nn.ModuleList([ConvFeatureExtractor(conv_layers_spec=spec, in_channels=1, dropout=dropout, mode=mode,
+                                                        conv_bias=conv_bias, depthwise=depthwise).cnn
+                                   for _ in range(n_cnn)])
         self.conv_layers_spec = spec
-        self.cnns = nn.ModuleList([s.cnn for s in subs])
-        self._subs = subs  # plain list: the parameters are registered through self.cnns only
         self.embedding_dim = spec[-1][0]
-
-    def sub(self, c: int) -> ConvFeatureExtractor:
-        return self._subs[0 if self.share_weights_over_channels else c]
 
     @torch.no_grad()
     def forward(self, x: torch.Tensor) -> torch.Tensor:
-        if x.dim() != 3 or x.shape[1] != self.in_channels:
-            raise ValueError(f"expected [B, {self.in_channels}, L], got {tuple(x.shape)}")
-        outs = [self.sub(c)(x[:, c:c + 1].contiguous()) for c in range(self.in_channels)]
-        return torch.cat(outs, dim=1)
+        """x [B, Cin, L] -> local features [B, Cin * T, C] (bf16), channel-major.  Inference only, like
+        ConvFeatureExtractor.forward."""
+        return _forward(self, x)
 
     def total_patches(self, time: int, device: str = "cuda") -> int:
-        return out_length(self._spec, time) * self.in_channels
+        return out_length(self.conv_layers_spec, time) * self.in_channels

@@ -227,22 +227,26 @@ class RuntimeJEPA(nn.Module):
         if a.shape[1] > 100 and a.shape[2] <= 100:      # [B, T, C] -> [B, C, T]   (feature_helper.py:49-50)
             a = a.transpose(1, 2)
         a = a.contiguous()
-        gain = self._gain(a, graph)                      # RMS over the whole (C, L) clip BEFORE the down-mix (:53)
+        gain = self._gain(a, graph)                      # RMS over the whole (C, L) clip BEFORE the channel fix-up (:53)
+        return self._fix_channels(a), gain
+
+    def _fix_channels(self, a: torch.Tensor) -> torch.Tensor:
+        """The channel fix-up of FeatureExtractor(in_channels=1): [B, C, L] -> the mono [B, 1, L]."""
         if a.shape[1] == 2:
-            a = a.mean(dim=1, keepdim=True).contiguous()   # :66-67
-        elif a.shape[1] == 4:
-            a = a[:, :1].contiguous()                      # :73-74
-        elif a.shape[1] != 1:
+            return a.mean(dim=1, keepdim=True).contiguous()   # :66-67
+        if a.shape[1] == 4:
+            return a[:, :1].contiguous()                      # :73-74
+        if a.shape[1] != 1:
             raise WavJepaLibError("Unknown channel count")
-        return a, gain
+        return a
 
     def get_timestamp_embeddings(self, audio: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
         graph = self._graph(audio)
         with torch.set_grad_enabled(graph):
             a, gain = self.to_feature(audio, graph)
-        B, _, L = a.shape
+        B, C, L = a.shape
         emb, _ = embed_chunks(self.model, a, gain, self.unit_frames, self.output_steps, self.sample_rate,
-                              layer=self.layer, graph=graph)
+                              channel_tokens=C, layer=self.layer, graph=graph)
         ts = get_timestamps(self.sample_rate, B, L, emb.shape[1])
         return emb, ts
 
@@ -270,34 +274,15 @@ class RuntimeNatJEPA(RuntimeJEPA):
                          precision, **kwargs)
         self.output_steps = self.model.extract_audio.total_patches(self.unit_frames) // in_channels
 
-    def to_feature(self, audio: torch.Tensor, graph: bool = False) -> Tuple[torch.Tensor, torch.Tensor]:
-        dev = self.model.device
-        a = torch.as_tensor(audio).to(dev, torch.float32)
-        if a.dim() == 2:
-            a = a.unsqueeze(1)
-        if a.dim() != 3:
-            raise ValueError("audio input tensor must be (n_sounds, num_samples) or (n_sounds, n_channels, num_samples)")
-        if a.shape[1] > 100 and a.shape[2] <= 100:
-            a = a.transpose(1, 2)
-        a = a.contiguous()
-        gain = self._gain(a, graph)                      # RMS over the whole (C, L) clip BEFORE the channel fix-up
+    def _fix_channels(self, a: torch.Tensor) -> torch.Tensor:
+        """The channel fix-up of FeatureExtractor(in_channels=2): [B, C, L] -> [B, 2, L]."""
         if a.shape[1] == 1:
-            a = a.expand(-1, 2, -1).contiguous()           # feature_helper.py:57-58
-        elif a.shape[1] == 4:
-            a = a[:, :1].expand(-1, 2, -1).contiguous()    # :75-77
-        elif a.shape[1] != 2:
+            return a.expand(-1, 2, -1).contiguous()           # feature_helper.py:57-58
+        if a.shape[1] == 4:
+            return a[:, :1].expand(-1, 2, -1).contiguous()    # :75-77
+        if a.shape[1] != 2:
             raise WavJepaLibError("Unknown channel count")
-        return a, gain
-
-    def get_timestamp_embeddings(self, audio: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
-        graph = self._graph(audio)
-        with torch.set_grad_enabled(graph):
-            a, gain = self.to_feature(audio, graph)
-        B, C, L = a.shape
-        emb, _ = embed_chunks(self.model, a, gain, self.unit_frames, self.output_steps, self.sample_rate, channel_tokens=C,
-                              layer=self.layer, graph=graph)
-        ts = get_timestamps(self.sample_rate, B, L, emb.shape[1])
-        return emb, ts
+        return a
 
 
 def _load_weights(args):

@@ -30,8 +30,8 @@ from ._lib import WavJepaLibError, require_device
 from ._lightning import Base as _ModuleBase
 from ._lightning import attached_trainer
 from .engine import LayerViews, TransformerStack
-from .extractors import (ConvChannelFeatureExtractor, ConvFeatureExtractor, conv_stack_backward, conv_stack_forward,
-                         conv_stack_forward_tf32, kmajor_weight)
+from .extractors import (ConvChannelFeatureExtractor, ConvFeatureExtractor, extractor_backward, extractor_forward,
+                         extractor_forward_tf32, gemm_weight_names, kmajor_weight)
 from .pos_embed import get_1d_sincos_pos_embed_from_grid
 from .types import ForwardReturn, TransformerEncoderCFG, TransformerLayerCFG
 
@@ -395,8 +395,6 @@ class JEPA(_ModuleBase):
             tparams[tn].data = tflat[o - e0:o - e0 + cnt].view(shp)
         self._flat_t = tflat
         self._flat_t16 = torch.empty(e1 - e0, device=dev, dtype=torch.bfloat16)
-        # conv working weights (tap-major bf16) live outside the flat copy
-        self._conv_names = [n for n in order if n.startswith("extract_audio.") and n.endswith(".0.weight")]
         self._w_sig = None
         self._gviews_cache = None
         self._pos_enc = self.pos_encoding_encoder.detach().reshape(self.total_patches, -1).contiguous()
@@ -425,28 +423,15 @@ class JEPA(_ModuleBase):
         self._build_weight_views()
         self._w_sig = sig
 
-    def _conv_streams(self, wk: Optional[dict] = None) -> list:
-        """(prefix, weights) of the CNN that serves each conv stream, in channel order: the mono extractor runs one
-        stream over every input channel, the per-channel (Nat) extractor one mono stream per input channel, all through
-        `extract_audio.cnns.0` when it shares weights over channels.  weights: the tap-major working copies of blocks
-        1.. taken from `wk` (`_conv_wk`, or the tf32 copy), or their parameter names when wk is None."""
-        ex = self.extract_audio
-        if isinstance(ex, ConvChannelFeatureExtractor):
-            prefixes = [f"extract_audio.cnns.{0 if ex.share_weights_over_channels else c}" for c in range(ex.in_channels)]
-        else:
-            prefixes = ["extract_audio.cnn"]
-        names = lambda p: [f"{p}.{i}.0.weight" for i in range(1, len(ex.conv_layers_spec))]
-        return [(p, names(p) if wk is None else [wk[n] for n in names(p)]) for p in prefixes]
+    def _extractor_lookup(self, flat: torch.Tensor) -> Callable:
+        """Name relative to extract_audio -> its view of `flat` (the lookups of extractors.extractor_forward / _backward)."""
+        return lambda n: self._view(flat, "extract_audio." + n)
 
     def _tap_major(self, flat: torch.Tensor, dtype: torch.dtype, old: Optional[dict] = None) -> dict:
-        """Tap-major working copies (kmajor_weight) of the conv weights of blocks 1.. in `flat`, by name, written into
-        the buffers of `old` where it has them."""
-        out = {}
-        for _, names in self._conv_streams():
-            for name in names:
-                if name not in out:   # a CNN shared over channels serves several streams
-                    out[name] = kmajor_weight(self._view(flat, name), (old or {}).get(name), dtype=dtype)
-        return out
+        """Tap-major working copies (kmajor_weight) of the conv weights of blocks 1.. in `flat`, by name relative to
+        extract_audio, written into the buffers of `old` where it has them."""
+        view = self._extractor_lookup(flat)
+        return {n: kmajor_weight(view(n), (old or {}).get(n), dtype=dtype) for n in gemm_weight_names(self.extract_audio)}
 
     def _refresh_conv_weights(self) -> None:
         self._conv_wk = self._tap_major(self._flat_p, torch.bfloat16, getattr(self, "_conv_wk", None))
@@ -492,27 +477,12 @@ class JEPA(_ModuleBase):
         reference wavjepa/jepa.py:391-396.  Returns (local32 [B*T, D], ctx pieces for the backward).
         save_conv=False (with save): a frozen extractor keeps no activations; only the feature norm saves its stats."""
         save_conv = save if save_conv is None else (save and save_conv)
-        ex = self.extract_audio
         B = x16.shape[0]
         T, D = self.total_patches, self.encoder_embedding_dim
-        C = ex.embedding_dim
+        C = self.extract_audio.embedding_dim
         p32 = lambda n: self._view(self._flat_p, n)
-        streams = self._conv_streams(self._conv_wk)
-        conv_saved = []
-        if isinstance(ex, ConvChannelFeatureExtractor):
-            Tc = T // ex.in_channels
-            feats = torch.empty(B, T, C, device=x16.device, dtype=torch.bfloat16)
-            xs = x16.transpose(0, 1).contiguous()  # [Cin, B, L]: one mono stream per CNN
-            for c, (prefix, wks) in enumerate(streams):
-                f, sv = conv_stack_forward(ex.conv_layers_spec, xs[c].unsqueeze(1), p32(f"{prefix}.0.0.weight"),
-                                           p32(f"{prefix}.0.2.weight"), p32(f"{prefix}.0.2.bias"), wks, save_conv)
-                feats[:, c * Tc:(c + 1) * Tc].copy_(f)  # channel-major token order (audio_channel_feature_extractor.py:177-178)
-                conv_saved.append(sv)
-        else:
-            (prefix, wks), = streams
-            feats, sv = conv_stack_forward(ex.conv_layers_spec, x16, p32(f"{prefix}.0.0.weight"),
-                                           p32(f"{prefix}.0.2.weight"), p32(f"{prefix}.0.2.bias"), wks, save_conv)
-            conv_saved.append(sv)
+        feats, conv_saved = extractor_forward(self.extract_audio, x16, self._extractor_lookup(self._flat_p),
+                                              self._conv_wk.__getitem__, save_conv)
         f2 = feats.view(B * T, C)
         ln16 = torch.empty(B * T, C, device=x16.device, dtype=torch.bfloat16)
         st = torch.empty(B * T, 2, device=x16.device) if save else None
@@ -700,40 +670,9 @@ class JEPA(_ModuleBase):
         ready("feature_norms.weight")
         if not conv:
             return
-        # ---- conv stack(s)
-        ex = self.extract_audio
-        streams = self._conv_streams(self._conv_wk)
-        if isinstance(ex, ConvChannelFeatureExtractor):
-            Tc = T // ex.in_channels
-            dfeat3 = dfeat.view(B, T, C)
-            for ch in range(ex.in_channels - 1, -1, -1):
-                prefix, wks = streams[ch]
-                sv = conv_saved[ch]
-                dfc = dfeat3[:, ch * Tc:(ch + 1) * Tc].contiguous().view(B * Tc, C)
-                # with shared weights every channel pass adds into the SAME gradient region: it is final (and may be
-                # all-reduced) only after the last pass
-                last = (not ex.share_weights_over_channels) or ch == 0
-                # each mono stream's waveform gradient lands in its channel
-                dxc = None if dx is None else torch.empty(B, 1, dx.shape[2], device=dev)
-                self._conv_backward(prefix, wks, ex.conv_layers_spec, sv, dfc, B, Tc, C, g,
-                                    ready if last else (lambda name: None), dxc, wg_conv)
-                if dx is not None:
-                    dx[:, ch:ch + 1].copy_(dxc)
-        else:
-            (prefix, wks), = streams
-            self._conv_backward(prefix, wks, ex.conv_layers_spec, conv_saved[0], dfeat, B, T, C, g, ready, dx, wg_conv)
-
-    def _conv_backward(self, prefix, wks, spec, sv, dfeat, B, T, C, g, ready, dx=None, weights: bool = True):
-        n = len(spec)
-        dev = dfeat.device
-        p32 = lambda nm: self._view(self._flat_p, nm)
-        dh = torch.empty(B, T, C, device=dev, dtype=torch.bfloat16)
-        ops.scatter_dgelu(dfeat, None, sv.pre[n - 1].view(B * T, C), B * T, dh.view(B * T, C))
-        gw = g if weights else (lambda nm: None)
-        conv_stack_backward(spec, sv, dh, p32(f"{prefix}.0.0.weight"), p32(f"{prefix}.0.2.weight"),
-                            p32(f"{prefix}.0.2.bias"), wks, gw(f"{prefix}.0.0.weight"), gw(f"{prefix}.0.2.weight"),
-                            gw(f"{prefix}.0.2.bias"), [gw(f"{prefix}.{i}.0.weight") for i in range(1, n)],
-                            on_layer_done=lambda i: ready(f"{prefix}.{i}.0.weight"), dx=dx, weights=weights)
+        extractor_backward(self.extract_audio, conv_saved, dfeat, self._extractor_lookup(self._flat_p),
+                           self._conv_wk.__getitem__, lambda n: g("extract_audio." + n),
+                           lambda n: ready("extract_audio." + n), dx, wg_conv)
 
     # ------------------------------------------------------------------------------------------- public API
     def forward(self, audio: torch.Tensor, ctx_masks: torch.Tensor, target_indices: torch.Tensor,
@@ -992,25 +931,12 @@ class JEPA(_ModuleBase):
     def _local_features_tf32(self, x32: torch.Tensor, w: dict) -> torch.Tensor:
         """_local_features at reference precision (inference only): fp32 waveform -> conv stack (tf32) -> LayerNorm(512)
         -> tf32 Linear 512->D (+bias) + positional table, all fp32.  Returns local32 [B*T, D]."""
-        ex = self.extract_audio
         B = x32.shape[0]
         T, D = self.total_patches, self.encoder_embedding_dim
-        C = ex.embedding_dim
+        C = self.extract_audio.embedding_dim
         p32 = lambda n: self._view(self._flat_p, n)
-
-        def stack(prefix, wks, x):
-            return conv_stack_forward_tf32(ex.conv_layers_spec, x, p32(f"{prefix}.0.0.weight"), p32(f"{prefix}.0.2.weight"),
-                                           p32(f"{prefix}.0.2.bias"), wks)
-
-        streams = self._conv_streams(w["conv"])
-        if isinstance(ex, ConvChannelFeatureExtractor):
-            Tc = T // ex.in_channels
-            feats = torch.empty(B, T, C, device=x32.device)
-            xs = x32.transpose(0, 1).contiguous()  # [Cin, B, L]: one mono stream per CNN
-            for c, (prefix, wks) in enumerate(streams):
-                feats[:, c * Tc:(c + 1) * Tc].copy_(stack(prefix, wks, xs[c].unsqueeze(1)))
-        else:
-            feats = stack(*streams[0], x32)
+        feats = extractor_forward_tf32(self.extract_audio, x32, self._extractor_lookup(self._flat_p),
+                                       w["conv"].__getitem__)
         ln = torch.empty(B * T, C, device=x32.device)
         ops.add_layernorm_fwd_f32(feats.view(B * T, C), None, p32("feature_norms.weight"), p32("feature_norms.bias"),
                                   self.feature_norms.eps, None, ln)
@@ -1049,14 +975,28 @@ class JEPA(_ModuleBase):
             ops.scatter_rows(packed, index[0], M, out.view(B * T, D))
         return out
 
-    def _audio_representation_tf32(self, audio: torch.Tensor, index) -> torch.Tensor:
-        """get_audio_representation with inference_precision == "tf32" (same masking semantics)."""
+    def _features_tf32(self, audio: torch.Tensor, index, collect: Optional[List[int]] = None):
+        """The forward of `_features_forward` with inference_precision == "tf32" (same masking semantics, inference
+        only): the final-normed features [B, T, D] when collect is None, else the hidden states `collect`, running only
+        the layers below max(collect)."""
         w = self._tf32_weights()
         x32 = audio.to(device=self.device, dtype=torch.float32).contiguous()
         B = x32.shape[0]
-        xv32, _, cu, max_len = self._visible_rows(self._local_features_tf32(x32, w), index, bf16=False)
-        xs32 = self._enc_stack.forward_tf32(w["layers"], xv32, ops.tf32_round(xv32), cu, B, max_len)
-        return self._final_norm(xs32, index, B)
+        top = self._enc_stack.n_layers if collect is None else max(collect)
+        xs32, _, cu, max_len = self._visible_rows(self._local_features_tf32(x32, w), index, bf16=False)
+        hook, hidden = None, {}
+        if collect is not None:
+            if 0 in collect:
+                hidden[0] = self._dense_rows(xs32, index, B)
+
+            def hook(i, y):
+                if i + 1 in collect:
+                    hidden[i + 1] = self._dense_rows(y, index, B)
+        if top > 0:
+            xs32 = self._enc_stack.forward_tf32(w["layers"][:top], xs32, ops.tf32_round(xs32), cu, B, max_len, hook)
+        if collect is None:
+            return self._final_norm(xs32, index, B)
+        return [hidden[k] for k in collect]
 
     # ------------------------------------------------------------------------------------------- fine-tuning
     def _feature_plan(self, trainable, audio_grad: bool = False, top: Optional[int] = None) -> Optional[_FeaturePlan]:
@@ -1250,21 +1190,28 @@ class JEPA(_ModuleBase):
         One graph supports one backward.  inference_precision "tf32" stays forward-only (no grad_fn, whatever
         requires grad): fine-tuning and the waveform gradient run in the "bf16" training numerics (DESIGN.md 2.2,
         2.3)."""
+        return self._representation(audio, padding_mask, host_mask, None)
+
+    def _representation(self, audio: torch.Tensor, padding_mask, host_mask, collect: Optional[List[int]]):
+        """The body of `get_audio_representation` (collect None) and `get_hidden_states` (the hidden states collect)."""
         self.eval()
         self._ensure_ready()
         self._sync_weights()
         index = self._visible_index(audio.shape[0], padding_mask, host_mask)
         if self.inference_precision == "tf32":
-            return self._audio_representation_tf32(audio, index)
+            return self._features_tf32(audio, index, collect)
         dev = self.device
         plan = None
         if torch.is_grad_enabled():   # the rule of `forward`
-            plan = self._feature_plan([n for n, p in self.named_parameters() if p.requires_grad], audio.requires_grad)
+            plan = self._feature_plan([n for n, p in self.named_parameters() if p.requires_grad], audio.requires_grad,
+                                      top=None if collect is None else max(collect))
         if plan is None:
-            return self._features_forward(audio.to(device=dev, dtype=torch.bfloat16).contiguous(), index)[0]
+            return self._features_forward(audio.to(device=dev, dtype=torch.bfloat16).contiguous(), index, None,
+                                          collect)[0]
         params = dict(self.named_parameters())
         # audio moves to the device outside the Function: autograd's copy backward takes the gradient back to audio.device
-        return _FeatureBridge.apply(self, audio.to(device=dev), index, plan, None, *[params[n] for n in plan.names])
+        out = _FeatureBridge.apply(self, audio.to(device=dev), index, plan, collect, *[params[n] for n in plan.names])
+        return out if collect is None else list(out)
 
     def _hidden_layers(self, layers) -> List[int]:
         """The hidden-state indices of `get_hidden_states(layers=...)`: None -> all N + 1, else a non-empty sequence of
@@ -1287,25 +1234,6 @@ class JEPA(_ModuleBase):
             raise ValueError("layers is empty: request at least one hidden state (None requests all)")
         return out
 
-    def _hidden_states_tf32(self, audio: torch.Tensor, index, collect: List[int]) -> List[torch.Tensor]:
-        """get_hidden_states with inference_precision == "tf32" (the path of _audio_representation_tf32, stopped after
-        layer max(collect) - 1)."""
-        w = self._tf32_weights()
-        x32 = audio.to(device=self.device, dtype=torch.float32).contiguous()
-        B = x32.shape[0]
-        top = max(collect)
-        xv32, _, cu, max_len = self._visible_rows(self._local_features_tf32(x32, w), index, bf16=False)
-        hidden = {}
-        if 0 in collect:
-            hidden[0] = self._dense_rows(xv32, index, B)
-
-        def hook(i, y):
-            if i + 1 in collect:
-                hidden[i + 1] = self._dense_rows(y, index, B)
-        if top > 0:
-            self._enc_stack.forward_tf32(w["layers"][:top], xv32, ops.tf32_round(xv32), cu, B, max_len, hook)
-        return [hidden[k] for k in collect]
-
     def get_hidden_states(self, audio: torch.Tensor, padding_mask: Optional[torch.Tensor] = None, host_mask=None,
                           layers=None) -> List[torch.Tensor]:
         """The student encoder's per-layer hidden states (the `hidden_states` convention of HF transformers), fp32
@@ -1325,21 +1253,4 @@ class JEPA(_ModuleBase):
         hidden state the loss does not read costs nothing in the backward; the others' gradients are added at their
         layer boundaries of the one encoder backward.  Frozen parts save nothing, the waveform gradient arrives in
         audio's dtype on audio's device, one graph supports one backward (DESIGN.md 2.4)."""
-        collect = self._hidden_layers(layers)
-        self.eval()
-        self._ensure_ready()
-        self._sync_weights()
-        index = self._visible_index(audio.shape[0], padding_mask, host_mask)
-        if self.inference_precision == "tf32":
-            return self._hidden_states_tf32(audio, index, collect)
-        dev = self.device
-        plan = None
-        if torch.is_grad_enabled():
-            plan = self._feature_plan([n for n, p in self.named_parameters() if p.requires_grad], audio.requires_grad,
-                                      top=max(collect))
-        if plan is None:
-            return self._features_forward(audio.to(device=dev, dtype=torch.bfloat16).contiguous(), index, None,
-                                          collect)[0]
-        params = dict(self.named_parameters())
-        return list(_FeatureBridge.apply(self, audio.to(device=dev), index, plan, collect,
-                                         *[params[n] for n in plan.names]))
+        return self._representation(audio, padding_mask, host_mask, self._hidden_layers(layers))
